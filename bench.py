@@ -54,7 +54,14 @@ def parse():
     ap.add_argument('--no-long-history', action='store_true', help='skip the configs[4] leg (B=4096, H=256)')
     ap.add_argument('--no-dp-check', action='store_true', help='skip the N-rank vs single-process numerical pre-flight (world > 1)')
     ap.add_argument('--no-affinity', action='store_true', help='do not bind each rank to the CPU cores local to its GPU')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', help='after the timed steps write what the last of them computed (loss, logits, '
+                                                          'gradients, model state after the update) as DIR/<name>.npy; see dump_outputs')
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl != 'ours' or int(os.environ.get('WORLD_SIZE', '1')) > 1):
+        ap.error('--dump-outputs writes the outputs of --impl ours in one process')
+    return args
 
 
 def load_weights():
@@ -181,7 +188,7 @@ def run_reference(args):
     rank = int(os.environ.get('RANK', '0'))
     if rank != 0:
         return
-    steps, warmup = max(1, min(args.steps, 100)), max(1, min(args.warmup, 5))
+    steps, warmup = args.steps, max(1, min(args.warmup, 5))
     rate, ms, cores, kind = cpu_reference_rate(args, steps, warmup)
     line = {
         'impl': 'reference', 'metric': 'train_impressions_per_sec', 'value': rate, 'unit': 'impressions/s',
@@ -323,6 +330,29 @@ def scoring_cpu_baseline(host_batch, user_num):
                       '2-model ensemble'}
 
 
+DUMP_ELEMENTS = 1 << 20       # per array: logits or delta of a large --batch / --user-num are stored as a fixed seeded sample
+
+
+def dump_outputs(out_dir, tr, model, loss):
+    """What the last timed FusedTrainStep step of a single process computed, as out_dir/<name>.npy: loss, logits,
+    grad.<parameter> (the gradient the update used) and state.<key> (model.state_dict() after the update), float32 (float64 for integer buffers).  An array
+    of more than DUMP_ELEMENTS elements keeps the same seeded sample of its flattened values in every run, so two builds run
+    with the same arguments compare array for array."""
+    arrays = {'loss': torch.tensor([loss.item()]), 'logits': tr.logits}
+    arrays.update({'grad.' + name: tr.grads[off:off + n].view(shape) for name, off, n, shape in tr.flat.slots})
+    arrays.update({'state.' + k: v for k, v in model.state_dict().items()})
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        a = a.astype(np.float32 if a.dtype == np.float32 else np.float64)
+        if a.size > DUMP_ELEMENTS:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, DUMP_ELEMENTS, replace=False))]
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+        total += a.nbytes
+    assert total <= 64 << 20, f'{total} bytes of outputs'
+
+
 def make_records(n, H, C, seed, user_num):
     """Synthetic impressions in the reference's record-list layout (tool/process_data.py:252; what import_processed_data returns)."""
     from news_recommendation_model_b200.synthetic import make_batch
@@ -398,11 +428,13 @@ def run_ours(args):
     with ClockSampler(local) as clk:
         e0.record()
         for i in range(K):
-            tr.run(slots[i % N_POOL])
+            last = tr.run(slots[i % N_POOL])
         e1.record()
         barrier()
     ms_total = max_over_ranks(e0.elapsed_time(e1))
     value = world * B * K / (ms_total / 1e3)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, tr, model, last)     # before the legs below train the same model further
 
     # ---- B. end to end through the same API: every step copies its batch from pinned host memory
     #         into a device slot (copy stream, one batch ahead) and the host reads every step's loss.

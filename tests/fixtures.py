@@ -20,6 +20,18 @@ def load_case(name: str):
     return np.load(os.path.join(GOLDEN, name + '.npz'))
 
 
+def stored(case, key, a):
+    """`a`, a whole tensor, at the elements the case stores for `key`: all of them, or the fixed sample in sample/<key>
+    (tests/golden/make_golden.py:sample_large)."""
+    a = np.asarray(a)
+    return a.reshape(-1)[case['sample/' + key]] if 'sample/' + key in case.files else a
+
+
+def grad_scale(case, key):
+    """Largest |gradient| of the whole tensor (the stored gradient may be a sample)."""
+    return float(case['gradmax/' + key]) if 'gradmax/' + key in case.files else float(np.abs(case['grad/' + key]).max())
+
+
 def _sha(*arrays):
     h = hashlib.sha256()
     for a in arrays:

@@ -10,7 +10,10 @@ and stores what the reference computed:
   weights_*.npz          the 37 tensors of ckpt/ckpt_ebnerd_large_*_final.pth
   case_train_b16.npz     train-mode logits, loss, all 37 gradients (incl. dense
                          delta), post-Adam parameters and BN buffers for one
-                         train.py:69-75 step (B=16,H=50,C=5,user_num=1000)
+                         train.py:69-75 step (B=16,H=50,C=5,user_num=1000);
+                         tensors of more than SAMPLE elements are stored at a
+                         fixed seeded sample of them (sample_large), inputs
+                         regenerated from the seed
   case_cfg1_b64.npz      BASELINE config 1 (B=64,H=50,C=5): train-mode logits,
                          loss, gradient norms (inputs regenerated from the seed)
   case_eval_b8.npz       test.py:31-74 scoring of ragged-candidate impressions
@@ -45,6 +48,25 @@ def import_reference():
     import test as ref_test                    # /root/reference/test.py (model_test)
     from tool.evaluation import auc_score
     return UserModel, ref_test, auc_score
+
+
+SAMPLE = 8192          # keeps every fixture file under 1 MB
+
+
+def sample_large(d):
+    """For every gradient of more than SAMPLE elements: keep it and the updated tensor at a fixed seeded sample of SAMPLE
+    flat indices (sample/<key>), plus the largest magnitude and the norm of the whole gradient (gradmax/, gradnorm/)."""
+    for key in [k for k in d if k.startswith('grad/')]:
+        k, g = key[len('grad/'):], d[key]
+        if g.size <= SAMPLE:
+            continue
+        idx = np.sort(np.random.default_rng(0).choice(g.size, SAMPLE, replace=False)).astype(np.int64)
+        d['sample/' + k] = idx
+        d['gradmax/' + k] = np.array(np.abs(g).max(), dtype=np.float64)
+        d['gradnorm/' + k] = np.array(np.linalg.norm(g.astype(np.float64)))
+        d[key] = g.reshape(-1)[idx]
+        d['after/' + k] = d['after/' + k].reshape(-1)[idx]
+    return d
 
 
 def sha(*arrays):
@@ -93,6 +115,7 @@ def train_case(UserModel, sd, path, *, B, H, C, user_num, seed, store_inputs, fu
             d['grad/' + k] = g.numpy()
         for k, v in model.state_dict().items():
             d['after/' + k] = v.numpy()
+        sample_large(d)
     else:
         for k, g in grads.items():
             d['gradnorm/' + k] = np.array(g.double().norm().item())
@@ -139,7 +162,7 @@ def main():
     sd_t = dump_weights('train')
     sd_v = dump_weights('validation')
     train_case(UserModel, sd_t, f'{HERE}/case_train_b16.npz', B=16, H=50, C=5, user_num=1000, seed=1234,
-               store_inputs=True, full=True)
+               store_inputs=False, full=True)
     train_case(UserModel, sd_t, f'{HERE}/case_cfg1_b64.npz', B=64, H=50, C=5, user_num=1000, seed=4321,
                store_inputs=False, full=False)
     eval_case(UserModel, ref_test, auc_score, [sd_t, sd_v], f'{HERE}/case_eval_b8.npz', B=8, H=200, C=24, seed=99)

@@ -1,8 +1,9 @@
 #!/usr/bin/env python
-"""Drive the reference's OWN scripts (unmodified byte copies in baseline/_ref: test.py:model_test, verify.py:model_validation and
-the train.py:69-75 loop body) over the drop-in shim on the GPU, in a fresh interpreter:
+"""Drive the reference's OWN scripts (unmodified byte copies in baseline/_ref: test.py:model_test, verify.py:model_validation) and
+the train.py:69-75 loop body over the drop-in shim on the GPU, in a fresh interpreter:
 
-    PYTHONPATH=<repo>/shim:<repo>:<repo>/baseline/_ref  python tests/run_reference_scripts.py
+    PYTHONPATH=<repo>/shim:<repo>:<repo>/baseline/_ref  python tests/run_reference_scripts.py scripts train
+    PYTHONPATH=<repo>/shim:<repo>  python tests/run_reference_scripts.py train        (needs no reference files)
 
 sys.path order is the one INTEGRATION.md section 1 prescribes, so the scripts' own `from models.user_model import UserModel`
 (test.py:7, verify.py:5, train.py:9) binds to the B200 implementation while `configs.run_config`, `tool.*`, `test`, `verify`
@@ -21,20 +22,19 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, HERE)
 sys.modules.setdefault('zstandard', types.ModuleType('zstandard'))     # tool/process_data.py:16 imports it; never called here
 
-import test as ref_test                 # baseline/_ref/test.py      (not the stdlib package: the reference root precedes it)
-import verify as ref_verify             # baseline/_ref/verify.py
 from models.user_model import UserModel  # shim -> news_recommendation_model_b200
 import news_recommendation_model_b200 as nrm
-from fixtures import case_batch, load_case, load_weights
+from fixtures import case_batch, load_case, load_weights, stored
 
 
-def main():
+def scripts(out, dev):
+    import test as ref_test                 # baseline/_ref/test.py      (not the stdlib package: the reference root precedes it)
+    import verify as ref_verify             # baseline/_ref/verify.py
     ref_root = os.path.join(os.path.dirname(HERE), 'baseline', '_ref')
     assert os.path.abspath(ref_test.__file__).startswith(ref_root), ref_test.__file__
     assert os.path.abspath(ref_verify.__file__).startswith(ref_root), ref_verify.__file__
-    assert UserModel is nrm.UserModel and ref_test.UserModel is nrm.UserModel and ref_verify.UserModel is nrm.UserModel
-    dev = torch.device('cuda:0')
-    out = {'test_py': os.path.abspath(ref_test.__file__), 'verify_py': os.path.abspath(ref_verify.__file__)}
+    assert ref_test.UserModel is nrm.UserModel and ref_verify.UserModel is nrm.UserModel
+    out.update({'test_py': os.path.abspath(ref_test.__file__), 'verify_py': os.path.abspath(ref_verify.__file__)})
 
     # ---- test.py:31-74 and verify.py:19-43 on the ragged-candidate golden case, ensemble of the two shipped checkpoints
     case = load_case('case_eval_b8')
@@ -61,6 +61,8 @@ def main():
     auc, tpr = ref_verify.model_validation(models, records, dev, batch_size=4)
     out['auc'], out['tpr'] = float(auc), float(tpr)
 
+
+def train(out, dev):
     # ---- the train.py:46-48, 69-75 loop body on the golden training case (torch.optim.Adam, as the script has it)
     tc = load_case('case_train_b16')
     tb = case_batch(tc)
@@ -86,13 +88,21 @@ def main():
     for k in sd:
         if ('after/' + k) not in tc.files:
             continue
-        ref = torch.from_numpy(tc['after/' + k]).double()
-        err = float((sd[k].detach().cpu().double() - ref).abs().max())
-        moved = float((ref - before[k].double()).abs().max()) if k in before else 0.0
+        ref = tc['after/' + k].astype(np.float64)
+        err = float(np.abs(stored(tc, k, sd[k].detach().cpu().double().numpy()) - ref).max())
+        moved = float(np.abs(ref - stored(tc, k, before[k].double().numpy())).max()) if k in before else 0.0
         out['after_err'][k] = [err, moved]
     model_ckpt = model.state_dict()
     model_ckpt.pop('delta')                                                         # train.py:95-96
     out['ckpt_keys'] = list(model_ckpt.keys())
+
+
+def main():
+    assert UserModel is nrm.UserModel
+    dev = torch.device('cuda:0')
+    out = {}
+    for part in sys.argv[1:]:
+        {'scripts': scripts, 'train': train}[part](out, dev)
     print('RESULT ' + json.dumps(out))
 
 

@@ -17,20 +17,29 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REF = os.path.join(ROOT, 'baseline', '_ref')
 
 
-@pytest.fixture(scope='module')
-def result():
-    if not os.path.isfile(os.path.join(REF, 'test.py')):
-        pytest.skip('baseline/_ref is absent (python oracle/make_ref.py in the build container)')
-    from oracle.make_ref import verify_copy
-    assert verify_copy(), 'baseline/_ref differs from the checksums recorded when it was copied from /root/reference'
+def _run(part, path):
     env = dict(os.environ)
-    env['PYTHONPATH'] = os.pathsep.join([os.path.join(ROOT, 'shim'), ROOT, REF])
+    env['PYTHONPATH'] = os.pathsep.join([os.path.join(ROOT, 'shim'), ROOT] + path)
     env['PYTHONDONTWRITEBYTECODE'] = '1'
-    out = subprocess.run([sys.executable, os.path.join(ROOT, 'tests', 'run_reference_scripts.py')], capture_output=True, text=True,
+    out = subprocess.run([sys.executable, os.path.join(ROOT, 'tests', 'run_reference_scripts.py'), part], capture_output=True, text=True,
                          env=env, cwd=ROOT, timeout=600)
     assert out.returncode == 0, out.stderr[-4000:]
     line = [ln for ln in out.stdout.splitlines() if ln.startswith('RESULT ')][-1]
     return json.loads(line[len('RESULT '):])
+
+
+@pytest.fixture(scope='module')
+def result():
+    if not os.path.isfile(os.path.join(REF, 'test.py')):
+        pytest.skip("the original project's scripts are not in the tree (baseline/_ref, oracle/make_ref.py)")
+    from oracle.make_ref import verify_copy
+    assert verify_copy(), 'baseline/_ref differs from the checksums recorded when it was copied'
+    return _run('scripts', [REF])
+
+
+@pytest.fixture(scope='module')
+def train_result():
+    return _run('train', [])
 
 
 def test_reference_model_test_over_the_shim_reproduces_the_golden_scores_and_submission_lines(result):
@@ -56,8 +65,9 @@ def test_reference_model_validation_over_the_shim_reproduces_the_golden_auc(resu
     assert abs(result['tpr'] - sum(hits) / B) <= 1e-9
 
 
-def test_reference_training_loop_body_over_the_shim_reproduces_the_golden_step(result):
+def test_reference_training_loop_body_over_the_shim_reproduces_the_golden_step(train_result):
     """train.py:46-48, 69-75 with torch.optim.Adam (as the script has it), weights after the step against the reference's."""
+    result = train_result
     tc = load_case('case_train_b16')
     assert abs(result['train_loss'] - float(tc['loss'])) <= 1e-5
     assert np.abs(np.asarray(result['train_logits'], dtype=np.float32) - tc['logits']).max() <= 1e-4

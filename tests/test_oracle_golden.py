@@ -4,7 +4,7 @@ import numpy as np
 import pytest
 import torch
 
-from fixtures import case_batch, load_case, load_weights
+from fixtures import case_batch, grad_scale, load_case, load_weights, stored
 from oracle import reference_port as O
 
 # identical ATen kernels on the same host give bit-equal results; leave a little room for
@@ -31,21 +31,28 @@ def test_train_step_matches_reference_b16():
     assert abs(loss.item() - float(case['loss'])) <= TOL
     for k, leaf in leaves.items():
         ref = case['grad/' + k]
-        err = np.abs(leaf.grad.numpy() - ref).max()
-        assert err <= TOL * max(1.0, np.abs(ref).max()), (k, err)
+        err = np.abs(stored(case, k, leaf.grad.numpy()) - ref).max()
+        tol = TOL * max(1.0, grad_scale(case, k))
+        assert err <= tol, (k, err)
+        if 'gradnorm/' + k in case.files:     # a sampled tensor: its whole gradient through the norm
+            n_err = abs(leaf.grad.double().norm().item() - float(case['gradnorm/' + k]))
+            assert n_err <= tol * np.sqrt(leaf.numel()), (k, n_err)
     # BN buffers after the training forward (momentum 0.1, unbiased running_var)
     for k in ('bn.running_mean', 'bn.running_var'):
         ref = case['after/' + k]
         assert np.abs(p[k].detach().numpy() - ref).max() <= TOL * max(1.0, np.abs(ref).max()), k
     assert int(p['bn.num_batches_tracked']) == int(case['after/bn.num_batches_tracked'])
-    # one Adam step (train.py:48,74): first step => m = (1-b1) g, v = (1-b2) g^2
+    # one Adam step (train.py:48,74): first step => m = (1-b1) g, v = (1-b2) g^2.  It is fed the reference's gradient (checked
+    # above): an element whose gradient is near eps moves by up to lr when that gradient changes in its last bits.  Fed the
+    # oracle's own gradient, invariant_interest_model.text_img_attention.mlp.fc1.weight came out 8.5e-6 from the reference's
+    # on the Intel Xeon host of a B200 machine (ATen AVX512 kernels), while another Xeon host with the same kernels matched
     with torch.no_grad():
         for k, leaf in leaves.items():
-            m = torch.zeros_like(leaf)
-            v = torch.zeros_like(leaf)
-            O.adam_step(leaf, leaf.grad, m, v, 1)
+            param = torch.from_numpy(stored(case, k, leaf.detach().numpy()).copy())
+            grad = torch.from_numpy(case['grad/' + k].copy())
+            O.adam_step(param, grad, torch.zeros_like(param), torch.zeros_like(param), 1)
             ref = case['after/' + k]
-            assert np.abs(leaf.numpy() - ref).max() <= TOL * max(1.0, np.abs(ref).max()), k
+            assert np.abs(param.numpy() - ref).max() <= TOL * max(1.0, np.abs(ref).max()), k
 
 
 def test_config1_b64_matches_reference():
