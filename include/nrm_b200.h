@@ -18,6 +18,7 @@
  *                 models/attention_model.py:52-97             (inside nrm_forward)
  *     UserInstantInterestModel.forward
  *                 models/user_instant_interest_model.py:20-23 (inside nrm_forward)
+ *   s_label / s_ti            user_invariant_interest_model.py:83-87   nrm_forward_scores, nrm_history_topk
  *   UserModel.loss            models/user_model.py:37-43      nrm_loss_forward
  *   loss.backward()           train.py:73                     nrm_loss_backward, nrm_backward
  *   optimizer.step()          train.py:48,74                  nrm_adam_step
@@ -220,7 +221,29 @@ int nrm_backward_encoder_compact(const nrm_compact_batch* batch, int B, int H, i
                                  const double* bn_bwd_sums, long long bn_global_rows, float* grads, void* workspace,
                                  size_t workspace_bytes, void* stream);
 
-
+/* ---- attention scores: "which past clicks made the model rank this article high?" -------------------------------------------
+ * The pairwise attention scores s[c][h] of both branches (PointwiseAttentionExpanded.forward, attention_model.py:52-97, called at
+ * user_invariant_interest_model.py:83-87: label_attention, text_img_attention) for every (candidate, history row) pair, computed by
+ * the kernels that compute the logits.  scores: float32 [2,B,C,H], branch 0 = label_attention, 1 = text_img_attention.  Pad history
+ * rows get scores too (the reference does not mask them; they contribute to the pooled sum).
+ *   nrm_forward_scores[_compact]: nrm_forward[_compact] in mode NRM_MODE_EVAL (any other mode: NRM_EINVAL; BatchNorm reads its
+ *     running statistics and nothing is written to them) that also writes `scores`; the logits are bit-identical to nrm_forward's
+ *     for the same precision, the workspace is nrm_workspace_bytes(B, H, C, NRM_MODE_EVAL).  The compact variant has
+ *     nrm_forward_compact's precision limits.  With NRM_ATT_ITEM_TILES=1 in the environment: NRM_EUNSUPPORTED (those kernels do
+ *     not export scores).
+ *   nrm_history_topk: per (branch, b, c) row the k largest scores and their history positions, descending, ties to the lower
+ *     position (Python's stable sorted(..., reverse=True)); idx_out int32 / val_out float32 [2,B,C,k], 1 <= k <= min(H, 64).  Pad rows
+ *     are left out: all-zero rows of x_history [B,H,80] or hist_article [B,H] == 0 (at most one of the two; both null: none); slots
+ *     beyond the real rows get index -1 and score NaN. */
+int nrm_forward_scores(const double* x_history, const double* x_target, long long x_target_batch_stride,
+                       const double* x_global, long long x_global_batch_stride, int B, int H, int C,
+                       const float* params, float* bn_running_mean, float* bn_running_var, long long* bn_num_batches_tracked,
+                       int mode, int precision, float* logits, float* scores, void* workspace, size_t workspace_bytes, void* stream);
+int nrm_forward_scores_compact(const nrm_compact_batch* batch, int B, int H, int C, const float* params, float* bn_running_mean,
+                               float* bn_running_var, long long* bn_num_batches_tracked, int mode, int precision,
+                               float* logits, float* scores, void* workspace, size_t workspace_bytes, void* stream);
+int nrm_history_topk(const float* scores, int B, int C, int H, int k, const double* x_history, const int* hist_article,
+                     int* idx_out, float* val_out, void* stream);
 
 /* ---- UserModel.loss (user_model.py:37-43) ---------------------------------------- */
 /* loss = (1-alpha) BCE(softmax(out), y) + alpha BCE(softmax(out + delta[id]), y), mean

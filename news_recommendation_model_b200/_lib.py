@@ -68,6 +68,9 @@ SIGNATURES = {
     'nrm_rank_strings_capacity': (sz, [i32, i32]),
     'nrm_rank_strings': (i32, [vp, vp, vp, i32, i32, vp, vp, ll, vp]),
     'nrm_expand_compact': (i32, [vp, i32, vp, vp, vp, vp, vp, vp, i32, i32, i32, vp, vp, vp, vp, vp]),
+    'nrm_forward_scores': (i32, [vp, vp, ll, vp, ll, i32, i32, i32, vp, vp, vp, vp, i32, i32, vp, vp, vp, sz, vp]),
+    'nrm_forward_scores_compact': (i32, [vp, i32, i32, i32, vp, vp, vp, vp, i32, i32, vp, vp, vp, sz, vp]),
+    'nrm_history_topk': (i32, [vp, i32, i32, i32, i32, vp, vp, vp, vp, vp]),
 }
 
 

@@ -519,6 +519,49 @@ extern "C" int nrm_forward_compact(const nrm_compact_batch* batch, int B, int H,
                             logits, workspace, workspace_bytes, stream);
 }
 
+// ---- attention scores (explanations): eval-mode forward that also exports s_label / s_ti -----------------------------------------
+static int forward_scores_impl(const char* fn, const BatchPtrs& in, int B, int H, int C, const float* params, float* bn_running_mean,
+                               float* bn_running_var, long long* bn_num_batches_tracked, int mode, int precision, float* logits,
+                               float* scores, void* workspace, size_t workspace_bytes, void* stream) {
+  if (mode != NRM_MODE_EVAL) { set_error("%s: scores are exported by eval-mode forwards only (mode must be NRM_MODE_EVAL, got %d)", fn, mode); return NRM_EINVAL; }
+  if (!scores) { set_error("%s: null scores", fn); return NRM_EINVAL; }
+  if (!use_rowstacked()) {
+    set_error("%s: the item-tile attention kernels (NRM_ATT_ITEM_TILES) do not export scores", fn);
+    return NRM_EUNSUPPORTED;
+  }
+  Workspace w;
+  NRM_TRY(get_workspace(fn, w, workspace, workspace_bytes, B, H, C, mode));
+  w.scores = scores;
+  NRM_TRY(encoder_forward(in, params, w, mode, precision, (cudaStream_t)stream));
+  return nrm_forward_head(B, H, C, params, bn_running_mean, bn_running_var, bn_num_batches_tracked, mode, precision, nullptr, 0,
+                          logits, workspace, workspace_bytes, stream);
+}
+
+extern "C" int nrm_forward_scores(const double* x_history, const double* x_target, long long xt_bs, const double* x_global,
+                                  long long xg_bs, int B, int H, int C, const float* params, float* bn_running_mean,
+                                  float* bn_running_var, long long* bn_num_batches_tracked, int mode, int precision,
+                                  float* logits, float* scores, void* workspace, size_t workspace_bytes, void* stream) {
+  NRM_TRY(check_shape("nrm_forward_scores", B, H, C));
+  if (!x_history || !x_target || !x_global || !params) { set_error("nrm_forward_scores: null pointer"); return NRM_EINVAL; }
+  if (xt_bs < (long long)C * TC || xg_bs < (long long)C * GC) { set_error("nrm_forward_scores: batch stride smaller than one impression"); return NRM_EINVAL; }
+  const BatchPtrs in{x_history, x_target, xt_bs, x_global, xg_bs};
+  return forward_scores_impl("nrm_forward_scores", in, B, H, C, params, bn_running_mean, bn_running_var, bn_num_batches_tracked, mode,
+                             precision, logits, scores, workspace, workspace_bytes, stream);
+}
+
+extern "C" int nrm_forward_scores_compact(const nrm_compact_batch* batch, int B, int H, int C, const float* params, float* bn_running_mean,
+                                          float* bn_running_var, long long* bn_num_batches_tracked, int mode, int precision,
+                                          float* logits, float* scores, void* workspace, size_t workspace_bytes, void* stream) {
+  NRM_TRY(check_shape("nrm_forward_scores_compact", B, H, C));
+  if (!params) { set_error("nrm_forward_scores_compact: null pointer"); return NRM_EINVAL; }
+  CompactPtrs cp;
+  NRM_TRY(compact_batch("nrm_forward_scores_compact", batch, precision, cp));
+  BatchPtrs in{nullptr, nullptr, 0, nullptr, 0};
+  in.compact = &cp;
+  return forward_scores_impl("nrm_forward_scores_compact", in, B, H, C, params, bn_running_mean, bn_running_var, bn_num_batches_tracked,
+                             mode, precision, logits, scores, workspace, workspace_bytes, stream);
+}
+
 static int backward_head(const char* fn, bool defer_wgrad, int B, int H, int C, const float* params, int precision, const float* dlogits, float* grads,
                          double* bn_bwd_sums, void* workspace, size_t workspace_bytes, void* stream) {
   NRM_TRY(check_shape(fn, B, H, C));

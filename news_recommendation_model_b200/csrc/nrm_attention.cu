@@ -136,10 +136,12 @@ __device__ __forceinline__ float reduce16(float v) {   // sum over the 16 lanes 
 // ---------------------------------------------------------------------------------
 // forward: grid = B (one impression per CTA), 256 threads, ~108 KB shared
 // ---------------------------------------------------------------------------------
-template <int BRANCH>
+// kScores: also store every valid row's score s[c][h] to scores [2][B][C][H] (nrm_forward_scores); with kScores = false the kernel
+// is the one nrm_forward has always launched.
+template <int BRANCH, bool kScores>
 __global__ void __launch_bounds__(ATT_THREADS, 2)
 attention_forward_kernel(const double* __restrict__ xh, const float* __restrict__ xhp, int B, int H, int C,
-                         const float* __restrict__ P, float* __restrict__ e) {
+                         const float* __restrict__ P, float* __restrict__ e, float* __restrict__ scores) {
   pdl_wait();                                          // programmatic dependent launch: see nrm_common.cuh
   pdl_trigger();
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -184,6 +186,8 @@ attention_forward_kernel(const double* __restrict__ xh, const float* __restrict_
             for (int j = 0; j < 4; ++j) part = fmaf(gelu_f(acc[r][j] + tpv[j]), w2v[j], part);
             part = reduce16(part);
             if (tc == 0) sm.s[cl * HT + 4 * tr + r] = part + b2;
+            if (kScores && tc == 0 && r0 + 4 * tr + r < H)
+              scores[((BRANCH * (long long)B + b) * C + c0 + cl) * H + r0 + 4 * tr + r] = part + b2;
           }
         }
         __syncthreads();
@@ -499,13 +503,12 @@ int launch_attention_forward(const BatchPtrs& in, const float* P, Workspace& w, 
   if (precision == NRM_PRECISION_BF16 || precision == NRM_PRECISION_BF16X3) return launch_attention_forward_tc(in, w, branch, precision, s);
   if (precision != NRM_PRECISION_FP32) { set_error("attention: precision %d not built", precision); return NRM_EUNSUPPORTED; }
   const size_t smem = sizeof(AttSmemFwd);
-  if (branch == 0) {
-    NRM_CUDA(cudaFuncSetAttribute(attention_forward_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    launch_pdl(attention_forward_kernel<0>, dim3(w.B), dim3(ATT_THREADS), smem, s, in.xh, w.xh, w.B, w.H, w.C, P, w.e);
-  } else {
-    NRM_CUDA(cudaFuncSetAttribute(attention_forward_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    launch_pdl(attention_forward_kernel<1>, dim3(w.B), dim3(ATT_THREADS), smem, s, in.xh, w.xh, w.B, w.H, w.C, P, w.e);
-  }
+  // w.scores non-null: the score-exporting instantiations
+  void (*k)(const double*, const float*, int, int, int, const float*, float*, float*) =
+      w.scores != nullptr ? (branch == 0 ? attention_forward_kernel<0, true> : attention_forward_kernel<1, true>)
+                          : (branch == 0 ? attention_forward_kernel<0, false> : attention_forward_kernel<1, false>);
+  NRM_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  launch_pdl(k, dim3(w.B), dim3(ATT_THREADS), smem, s, in.xh, (const float*)w.xh, w.B, w.H, w.C, P, w.e, w.scores);
   NRM_LAUNCH_CHECK("attention_forward_kernel");
   return NRM_OK;
 }

@@ -31,7 +31,7 @@
 namespace nrm {
 namespace rs {
 
-
+#ifndef NRM_RS_SCORES_TU
 __global__ void __launch_bounds__(256)
 att_prep_rs_kernel(const float* __restrict__ P, unsigned char* __restrict__ img_all) {
   pdl_wait();
@@ -54,6 +54,7 @@ att_prep_rs_kernel(const float* __restrict__ P, unsigned char* __restrict__ img_
     if (threadIdx.x == 0) tail[64] = P[off.fc2_b];
   }
 }
+#endif
 
 
 struct Stage {
@@ -98,10 +99,16 @@ __device__ __forceinline__ void issue_stage(Stage& st, const float* __restrict__
   cp_async_commit();
 }
 
-template <int SPLIT>
-__global__ void __launch_bounds__(THREADS, 1)
-attention_forward_rs_kernel(const float* __restrict__ pca32, const float* __restrict__ xhp, int B, int H, int C,
-                            const unsigned char* __restrict__ img, const float* __restrict__ tp_all, float* __restrict__ e) {
+// kScores: also store every valid row's fp32 score s[c][h] to scores [2][B][C][H] (nrm_forward_scores).  The four column-quarter
+// partials of a row meet in shared memory behind sizeof(Smem<NP>) (SCORE_XCHG_BYTES more dynamic shared memory).  The kScores kernels
+// are compiled in a translation unit of their own (nrm_attention_rs_scores.cu includes this file with NRM_RS_SCORES_TU defined):
+// ptxas compiles a module as a whole, and any further kernel here changes the register assignment of the ones nrm_forward launches.
+constexpr int SCORE_XCHG_BYTES = 2 * 3 * 128 * 4;    // [tile parity][column quarter 1..3][row of the tile]
+
+template <int SPLIT, bool kScores>
+__device__ __forceinline__ void attention_forward_rs(const float* __restrict__ pca32, const float* __restrict__ xhp, int B, int H, int C,
+                                                     const unsigned char* __restrict__ img, const float* __restrict__ tp_all,
+                                                     float* __restrict__ e, float* __restrict__ scores) {
   pdl_wait();
   pdl_trigger();
   constexpr int NP = SPLIT == 3 ? 2 : 1;
@@ -406,6 +413,17 @@ attention_forward_rs_kernel(const float* __restrict__ pca32, const float* __rest
             *reinterpret_cast<__nv_bfloat16*>(st.s2[0] + off) = hi;
             if (NP == 2) *reinterpret_cast<__nv_bfloat16*>(st.s2[1] + off) = __float2bfloat16_rn(acc - __bfloat162float(hi));
           }
+          if constexpr (kScores) {
+            // s = (quarter 0 + quarter 1) + (quarter 2 + quarter 3), each quarter's partial as the epilogue computed it (fp32, before
+            // the bf16 split).  The four warps of sub-partition sp meet at named barrier 1 + sp; the exchange slots alternate with the
+            // tile parity, and a warp cannot overwrite a slot before quarter 0 has passed the NEXT barrier, i.e. read this one.
+            float* xchg = reinterpret_cast<float*>(smem_raw + sizeof(Smem<NP>)) + (tile_seq & 1) * (3 * 128) + 32 * sp + lane;
+            if (cq > 0) xchg[(cq - 1) * 128] = acc;
+            __syncwarp();                                  // bar.sync is the ALIGNED barrier: the warp must arrive converged
+            asm volatile("bar.sync %0, 128;\n" ::"r"(1 + sp) : "memory");
+            if (cq == 0 && valid)
+              scores[(((long long)branch * B + b) * C + c0 + cl) * H + h0 + hloc] = (acc + xchg[0]) + (xchg[128] + xchg[256]);
+          }
           if (ti == ntiles - 1) {
             umma::fence_async_smem();                      // scores are read by the tensor core (async proxy)
             arrive_warp(&sm.s_full[s]);
@@ -424,8 +442,26 @@ attention_forward_rs_kernel(const float* __restrict__ pca32, const float* __rest
   if (warp == 0) umma::tmem_dealloc(tmem, TMEM_COLS);
 }
 
+#ifndef NRM_RS_SCORES_TU
+template <int SPLIT>
+__global__ void __launch_bounds__(THREADS, 1)
+attention_forward_rs_kernel(const float* __restrict__ pca32, const float* __restrict__ xhp, int B, int H, int C,
+                            const unsigned char* __restrict__ img, const float* __restrict__ tp_all, float* __restrict__ e) {
+  attention_forward_rs<SPLIT, false>(pca32, xhp, B, H, C, img, tp_all, e, nullptr);
+}
+#else
+template <int SPLIT>
+__global__ void __launch_bounds__(THREADS, 1)
+attention_forward_rs_scores_kernel(const float* __restrict__ pca32, const float* __restrict__ xhp, int B, int H, int C,
+                                   const unsigned char* __restrict__ img, const float* __restrict__ tp_all, float* __restrict__ e,
+                                   float* __restrict__ scores) {
+  attention_forward_rs<SPLIT, true>(pca32, xhp, B, H, C, img, tp_all, e, scores);
+}
+#endif
+
 }  // namespace rs
 
+#ifndef NRM_RS_SCORES_TU
 int launch_attention_prep_rs(const float* P, Workspace& w, cudaStream_t s) {
   launch_pdl(rs::att_prep_rs_kernel, dim3(8, 2), dim3(256), 0, s, P, reinterpret_cast<unsigned char*>(w.att_rs_img));
   NRM_LAUNCH_CHECK("att_prep_rs_kernel");
@@ -445,8 +481,9 @@ static int launch_fwd_rs(const BatchPtrs& in, Workspace& w, cudaStream_t s) {
   return NRM_OK;
 }
 
-// both branches in one launch
+// both branches in one launch; w.scores non-null: the score-exporting kernels (nrm_attention_rs_scores.cu)
 int launch_attention_forward_rs(const BatchPtrs& in, Workspace& w, int precision, cudaStream_t s) {
+  if (w.scores != nullptr) return launch_attention_forward_rs_scores(w, precision, s);
   return precision == NRM_PRECISION_BF16 ? launch_fwd_rs<1>(in, w, s) : launch_fwd_rs<3>(in, w, s);
 }
 
@@ -465,5 +502,24 @@ int rsprof_read(long long* host_out64) {
   return NRM_EUNSUPPORTED;
 #endif
 }
+
+#else
+template <int SPLIT>
+static int launch_fwd_rs_scores(Workspace& w, cudaStream_t s) {
+  constexpr int NP = SPLIT == 3 ? 2 : 1;
+  const size_t smem = sizeof(rs::Smem<NP>) + rs::SCORE_XCHG_BYTES;
+  const long long G = (w.C + rs::CG - 1) / rs::CG, U = 2LL * w.B * G;
+  const int grid = (int)min(U, (long long)sm_count());
+  NRM_CUDA(cudaFuncSetAttribute(rs::attention_forward_rs_scores_kernel<SPLIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  launch_pdl(rs::attention_forward_rs_scores_kernel<SPLIT>, dim3(grid), dim3(rs::THREADS), smem, s, w.pca_h, w.xh, w.B, w.H, w.C,
+             reinterpret_cast<const unsigned char*>(w.att_rs_img), w.tp, w.e, w.scores);
+  NRM_LAUNCH_CHECK("attention_forward_rs_scores_kernel");
+  return NRM_OK;
+}
+
+int launch_attention_forward_rs_scores(Workspace& w, int precision, cudaStream_t s) {
+  return precision == NRM_PRECISION_BF16 ? launch_fwd_rs_scores<1>(w, s) : launch_fwd_rs_scores<3>(w, s);
+}
+#endif
 
 }  // namespace nrm

@@ -194,6 +194,7 @@ struct Workspace {
   unsigned int* head_arrive;   // arrival counter: the last CTA of the tensor-core head backward sums the BatchNorm partials
   float* head_img;     // operand images of the ten head products (nrm_head_tc.cu): bf16 parts, chunked in ring order
   float* att_rs_img;   // weight image of the row-stacked attention kernels (nrm_attention_rs.cu): bf16 operand tiles, hi | lo
+  float* scores;       // caller's [2][B][C][H] attention scores (nrm_forward_scores; not carved: null = the forward stores none)
   // backward (training only)
   float* da3; float* da2; float* da1;   // [R,66]
   float* dy;           // [R,264]

@@ -49,6 +49,7 @@ size_t attention_rs_image_bytes();
 int rsprof_read(long long* host_out64);                                         // -DNRM_RS_PROFILE builds only
 int launch_attention_prep_rs(const float* P, Workspace& w, cudaStream_t s);       // weight image -> w.att_rs_img (weights only)
 int launch_attention_forward_rs(const BatchPtrs& in, Workspace& w, int precision, cudaStream_t s);   // both branches, one launch
+int launch_attention_forward_rs_scores(Workspace& w, int precision, cudaStream_t s);   // the same + scores to w.scores (nrm_attention_rs_scores.cu)
 // nrm_attention_rs_bwd.cu: sums over rows (weight gradients, dtp) of one branch; export_dhid also writes the dhid tiles / scores
 int launch_attention_backward_rs(Workspace& w, int branch, int precision, bool export_dhid, cudaStream_t s);
 int launch_attention_input_grad_rs(Workspace& w, int precision, cudaStream_t s);   // label branch: dxh, dxt from the exported tiles
