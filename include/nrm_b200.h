@@ -19,6 +19,7 @@
  *     UserInstantInterestModel.forward
  *                 models/user_instant_interest_model.py:20-23 (inside nrm_forward)
  *   s_label / s_ti            user_invariant_interest_model.py:83-87   nrm_forward_scores, nrm_history_topk
+ *   ensemble softmax + order  test.py:58-63, 124-127 over a shared pool  nrm_forward_pool, nrm_pool_topk
  *   UserModel.loss            models/user_model.py:37-43      nrm_loss_forward
  *   loss.backward()           train.py:73                     nrm_loss_backward, nrm_backward
  *   optimizer.step()          train.py:48,74                  nrm_adam_step
@@ -244,6 +245,30 @@ int nrm_forward_scores_compact(const nrm_compact_batch* batch, int B, int H, int
                                float* logits, float* scores, void* workspace, size_t workspace_bytes, void* stream);
 int nrm_history_topk(const float* scores, int B, int C, int H, int k, const double* x_history, const int* hist_article,
                      int* idx_out, float* val_out, void* stream);
+
+/* ---- recommendation: every user against a shared pool of N articles -------------------------------------------------------------
+ * The other way round from the [B,C] impressions above: score all N articles of a pool (e.g. the articles live now) for each of B
+ * users and keep each user's k best unread ones.
+ *   nrm_forward_pool: logits [B,N] float32; logits[b][n] is, bit for bit, what nrm_forward in mode NRM_MODE_EVAL returns for
+ *     impression b with the user's history and the whole pool as its candidates (x_target[b] / x_global[b] = the pool's rows for
+ *     every b), in the same precision (all three; NRM_ATT_ITEM_TILES=1 too).  BatchNorm reads its running statistics only.
+ *     users->hist_* are the users' [B,H] / [B,H,2] compact histories; users->cand_article / cand_time are the pool's [N] ids and
+ *     packed time buckets (one time for all users); label32 / label64 must be null.  The pool is processed in chunks of `chunk`
+ *     articles (a positive multiple of 8, the attention's candidate group: any such chunk gives the same bits); the workspace
+ *     is nrm_pool_workspace_bytes(B, H, N, chunk) bytes, 256-byte aligned, and grows with B * chunk.
+ *   nrm_pool_topk: per user b the k pool positions with the largest score, descending, ties to the lower position (Python's
+ *     stable sorted(..., reverse=True), test.py:124-127); pos_out int32 / val_out float32 [B,k], 1 <= k <= min(N, 1024).
+ *     logits: n_models >= 1 (at most 16) stacked [B,N] slices, model m at logits + m * model_stride.  Position n is eligible
+ *     unless pool_article[n] is 0 or outside [1, n_articles), a logit of n is NaN in any model, or (hist_article [B,H] given;
+ *     null = no exclusion) pool_article[n] equals one of the user's non-pad history ids.  Score: the logit for one model; for
+ *     n_models >= 2 the mean over the models of the softmax over the user's eligible positions (test.py:58-63),
+ *     (1/M) sum_m exp(x_m - max_m) / sum_eligible exp(x_m - max_m), in float32.  Slots beyond the eligible count get position
+ *     -1 and score NaN.  H <= 16384 when hist_article is given. */
+size_t nrm_pool_workspace_bytes(int B, int H, int N, int chunk);
+int nrm_forward_pool(const nrm_compact_batch* users, int B, int H, int N, int chunk, const float* params, const float* bn_running_mean,
+                     const float* bn_running_var, int precision, float* logits, void* workspace, size_t workspace_bytes, void* stream);
+int nrm_pool_topk(const float* logits, int n_models, long long model_stride, int B, int N, int k, const int* pool_article, int n_articles,
+                  const int* hist_article, int H, int* pos_out, float* val_out, void* stream);
 
 /* ---- UserModel.loss (user_model.py:37-43) ---------------------------------------- */
 /* loss = (1-alpha) BCE(softmax(out), y) + alpha BCE(softmax(out + delta[id]), y), mean

@@ -5,7 +5,7 @@ from .models import (MLP, PointwiseAttention, PointwiseAttentionExpanded, UserIn
 from .optim import FusedAdam
 from .trainer import FusedTrainStep
 from ._lib import NrmError, build
-from . import dp, explain, metrics, scoring, wire
+from . import dp, explain, metrics, recommend, scoring, wire
 
 __all__ = ['MLP', 'PointwiseAttention', 'PointwiseAttentionExpanded', 'UserInstantInterestModel',
-           'UserInvariantInterestModel', 'UserModel', 'FusedAdam', 'FusedTrainStep', 'NrmError', 'build', 'dp', 'explain', 'metrics', 'scoring', 'wire']
+           'UserInvariantInterestModel', 'UserModel', 'FusedAdam', 'FusedTrainStep', 'NrmError', 'build', 'dp', 'explain', 'metrics', 'recommend', 'scoring', 'wire']

@@ -71,6 +71,9 @@ SIGNATURES = {
     'nrm_forward_scores': (i32, [vp, vp, ll, vp, ll, i32, i32, i32, vp, vp, vp, vp, i32, i32, vp, vp, vp, sz, vp]),
     'nrm_forward_scores_compact': (i32, [vp, i32, i32, i32, vp, vp, vp, vp, i32, i32, vp, vp, vp, sz, vp]),
     'nrm_history_topk': (i32, [vp, i32, i32, i32, i32, vp, vp, vp, vp, vp]),
+    'nrm_pool_workspace_bytes': (sz, [i32, i32, i32, i32]),
+    'nrm_forward_pool': (i32, [vp, i32, i32, i32, i32, vp, vp, vp, i32, vp, vp, sz, vp]),
+    'nrm_pool_topk': (i32, [vp, i32, ll, i32, i32, i32, vp, i32, vp, i32, vp, vp, vp]),
 }
 
 

@@ -562,6 +562,78 @@ extern "C" int nrm_forward_scores_compact(const nrm_compact_batch* batch, int B,
                              mode, precision, logits, scores, workspace, workspace_bytes, stream);
 }
 
+// ---- recommendation from a shared pool: every user against the same N articles, in chunks of the pool ------------------------------
+// Workspace: the users' history as packed float64 rows (expanded once), one pool chunk as packed x_target / x_global rows, the chunk's
+// [B,C] logits and the eval workspace of a (B, H, C) forward.  The encoder reads the chunk's candidate rows with batch stride 0, so
+// all B users see the same rows without a copy per user.  C is a multiple of 8, the row-stacked attention's candidate group (rs::CG),
+// so every chunk groups candidates exactly as one forward over all N columns would: the logits are that forward's, bit for bit.
+struct PoolCarve { double* xh; double* xt; double* xg; float* out; void* ws; size_t ws_bytes, bytes; };
+static void carve_pool(PoolCarve& pc, void* base, int B, int H, int N, int chunk) {
+  const int C = chunk < N ? chunk : N;
+  size_t off = 0;
+  auto take = [&](size_t bytes) -> void* {
+    void* p = base ? (char*)base + off : nullptr;
+    off += (bytes + 255) & ~(size_t)255;
+    return p;
+  };
+  pc.xh = (double*)take(sizeof(double) * B * H * HC);
+  pc.xt = (double*)take(sizeof(double) * C * TC);
+  pc.xg = (double*)take(sizeof(double) * C * GC);
+  pc.out = (float*)take(sizeof(float) * B * C);
+  Workspace w;
+  pc.ws_bytes = carve_workspace(w, nullptr, B, H, C, NRM_MODE_EVAL);
+  pc.ws = take(pc.ws_bytes);
+  pc.bytes = off;
+}
+
+extern "C" size_t nrm_pool_workspace_bytes(int B, int H, int N, int chunk) {
+  if (B <= 0 || H <= 0 || N <= 0 || chunk <= 0) return 0;
+  PoolCarve pc;
+  carve_pool(pc, nullptr, B, H, N, chunk);
+  return pc.bytes;
+}
+
+extern "C" int nrm_forward_pool(const nrm_compact_batch* users, int B, int H, int N, int chunk, const float* params,
+                                const float* bn_running_mean, const float* bn_running_var, int precision, float* logits,
+                                void* workspace, size_t workspace_bytes, void* stream) {
+  const char* fn = "nrm_forward_pool";
+  if (B <= 0 || H <= 0 || N <= 0) { set_error("%s: B, H, N must be positive (got %d, %d, %d)", fn, B, H, N); return NRM_EINVAL; }
+  if (chunk <= 0 || chunk % 8 != 0) { set_error("%s: chunk must be a positive multiple of 8 (got %d)", fn, chunk); return NRM_EINVAL; }
+  if (precision < NRM_PRECISION_FP32 || precision > NRM_PRECISION_BF16X3) { set_error("%s: unknown precision %d", fn, precision); return NRM_EINVAL; }
+  if (!users || !users->articles || users->n_articles <= 0 || !users->hist_article || !users->hist_time || !users->hist_click ||
+      !users->cand_article || !users->cand_time) {
+    set_error("%s: bad compact batch", fn); return NRM_EINVAL;
+  }
+  if (users->label32 || users->label64) { set_error("%s: the pool has no labels (label32 / label64 must be null)", fn); return NRM_EINVAL; }
+  if ((reinterpret_cast<uintptr_t>(users->articles) & 15) != 0) { set_error("%s: the article table must be 16-byte aligned", fn); return NRM_EINVAL; }
+  if (!params || !bn_running_mean || !bn_running_var || !logits) { set_error("%s: null pointer", fn); return NRM_EINVAL; }
+  const int C = chunk < N ? chunk : N;
+  NRM_TRY(check_shape(fn, B, H, C));
+  if (workspace == nullptr || ((uintptr_t)workspace & 255) != 0) { set_error("%s: workspace must be non-null and 256-byte aligned", fn); return NRM_EWORKSPACE; }
+  PoolCarve pc;
+  carve_pool(pc, workspace, B, H, N, chunk);
+  if (pc.bytes > workspace_bytes) { set_error("%s: workspace too small (%zu < %zu bytes)", fn, workspace_bytes, pc.bytes); return NRM_EWORKSPACE; }
+  cudaStream_t s = (cudaStream_t)stream;
+  const nrm_compact_batch& u = *users;
+  NRM_TRY(launch_expand_compact(u.articles, u.n_articles, u.hist_article, u.hist_time, u.hist_click, nullptr, nullptr, nullptr, (long long)B * H, 0,
+                                pc.xh, nullptr, nullptr, nullptr, s));
+  // the BatchNorm buffers are only read in eval mode: the head's training-only writes never happen
+  float* run_mean = const_cast<float*>(bn_running_mean);
+  float* run_var = const_cast<float*>(bn_running_var);
+  for (int c0 = 0; c0 < N; c0 += C) {
+    const int nc = N - c0 < C ? N - c0 : C;
+    NRM_TRY(launch_expand_compact(u.articles, u.n_articles, nullptr, nullptr, nullptr, u.cand_article + c0, u.cand_time + c0, nullptr, 0, nc,
+                                  nullptr, pc.xt, pc.xg, nullptr, s));
+    const BatchPtrs in{pc.xh, pc.xt, 0, pc.xg, 0};
+    NRM_TRY(forward_encoder_impl(fn, in, B, H, nc, params, NRM_MODE_EVAL, precision, nullptr, pc.ws, pc.ws_bytes, stream));
+    float* out = nc == N ? logits : pc.out;                 // a single chunk writes the [B,N] logits directly
+    NRM_TRY(nrm_forward_head(B, H, nc, params, run_mean, run_var, nullptr, NRM_MODE_EVAL, precision, nullptr, 0, out, pc.ws, pc.ws_bytes, stream));
+    if (out != logits)
+      NRM_CUDA(cudaMemcpy2DAsync(logits + c0, sizeof(float) * N, out, sizeof(float) * nc, sizeof(float) * nc, B, cudaMemcpyDeviceToDevice, s));
+  }
+  return NRM_OK;
+}
+
 static int backward_head(const char* fn, bool defer_wgrad, int B, int H, int C, const float* params, int precision, const float* dlogits, float* grads,
                          double* bn_bwd_sums, void* workspace, size_t workspace_bytes, void* stream) {
   NRM_TRY(check_shape(fn, B, H, C));

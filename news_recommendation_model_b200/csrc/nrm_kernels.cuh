@@ -76,6 +76,15 @@ int launch_head_backward_dgrad_tc(const float* P, Workspace& w, int precision, c
 int launch_head_forward_tc(const float* P, Workspace& w, int precision, float* run_mean, float* run_var, long long* nbt, int training, int keep,
                            const double* bn_sums, long long bn_rows, float* logits, cudaStream_t s);
 
+// nrm_wire.cu: NH history rows and R candidate rows of the compact format -> packed float64 rows (either count may be 0)
+int launch_expand_compact(const float* articles, int n_articles, const int* hist_article, const unsigned* hist_time, const float* hist_click,
+                          const int* cand_article, const unsigned* cand_time, const float* label32, long long NH, long long R,
+                          double* x_history, double* x_target, double* x_global, double* label64, cudaStream_t s);
+
+// nrm_recommend.cu: per user, the k best eligible positions of a shared article pool (nrm_pool_topk)
+int launch_pool_topk(const float* logits, int n_models, long long model_stride, int B, int N, int k, const int* pool_article, int n_articles,
+                     const int* hist_article, int H, int* pos_out, float* val_out, cudaStream_t s);
+
 // nrm_head.cu
 int launch_bn_partial_sums(Workspace& w, cudaStream_t s);                 // -> w.bn_sums
 int launch_head_forward(const float* P, Workspace& w, float* run_mean, float* run_var, long long* nbt,

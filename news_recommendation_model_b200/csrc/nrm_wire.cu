@@ -62,6 +62,16 @@ expand_compact_kernel(const float* __restrict__ articles, int n_articles,
   }
 }
 
+int launch_expand_compact(const float* articles, int n_articles, const int* hist_article, const unsigned* hist_time, const float* hist_click,
+                          const int* cand_article, const unsigned* cand_time, const float* label32, long long NH, long long R,
+                          double* x_history, double* x_target, double* x_global, double* label64, cudaStream_t s) {
+  const long long warps = NH + R + (R + 31) / 32;
+  expand_compact_kernel<<<(unsigned)((warps + 7) / 8), 256, 0, s>>>(articles, n_articles, hist_article, hist_time, hist_click, cand_article,
+                                                                    cand_time, label32, NH, R, x_history, x_target, x_global, label64);
+  NRM_LAUNCH_CHECK("expand_compact_kernel");
+  return NRM_OK;
+}
+
 }  // namespace nrm
 
 using namespace nrm;
@@ -77,11 +87,6 @@ extern "C" int nrm_expand_compact(const float* articles, int n_articles, const i
   if ((reinterpret_cast<uintptr_t>(articles) | reinterpret_cast<uintptr_t>(x_history) | reinterpret_cast<uintptr_t>(x_target)) & 15) {
     set_error("nrm_expand_compact: articles / x_history / x_target must be 16-byte aligned"); return NRM_EINVAL;
   }
-  const long long NH = (long long)B * H, R = (long long)B * C;
-  const long long warps = NH + R + (R + 31) / 32;
-  expand_compact_kernel<<<(unsigned)((warps + 7) / 8), 256, 0, (cudaStream_t)stream>>>(articles, n_articles, hist_article, hist_time, hist_click,
-                                                                                     cand_article, cand_time, label32, NH, R, x_history,
-                                                                                     x_target, x_global, label64);
-  NRM_LAUNCH_CHECK("expand_compact_kernel");
-  return NRM_OK;
+  return launch_expand_compact(articles, n_articles, hist_article, hist_time, hist_click, cand_article, cand_time, label32, (long long)B * H,
+                               (long long)B * C, x_history, x_target, x_global, label64, (cudaStream_t)stream);
 }
