@@ -101,8 +101,8 @@ def attention_forward(p, prefix, t: T, h: T):
 
 
 def attention_backward(p, prefix, t: T, h: T, saved, dP: T, grads, need_input_grads: bool):
-    """dP [B,C,64] -> (dt, dh) (None for the text/img branch whose inputs are data)
-    and fc1/fc2 gradients accumulated into `grads`."""
+    """dP [B,C,64] -> (dt, dh, Gt): dt, dh are None for the text/img branch whose inputs are data; Gt [B,C,64] = dL/dtp
+    (the sum of dhid over the history rows).  fc1/fc2 gradients are accumulated into `grads`."""
     A, Bm, Wd, b1, w2, b2 = derived_weights(p, prefix)
     Wc, hid, s = saved
     ds = torch.einsum('bck,bhk->bch', dP, h)
@@ -118,42 +118,55 @@ def attention_backward(p, prefix, t: T, h: T, saved, dP: T, grads, need_input_gr
     grads[prefix + 'mlp.fc1.bias'] += Gt.sum((0, 1))
     grads[prefix + 'mlp.fc1.weight'] += torch.cat([dA, dBm, dBm - dA, dWd], dim=1)
     if not need_input_grads:
-        return None, None
+        return None, None, Gt
     dt = Gt @ Bm + torch.einsum('bcjk,jk->bck', S, Wd)
     dh = torch.einsum('bch,bck->bhk', s, dP) + torch.einsum('bchj,bcjk->bhk', dhid, Wc)
-    return dt, dh
+    return dt, dh, Gt
 
 
 # ---------------------------------------------------------------------------
-# whole training step in kernel form
+# stages of the training step.  Each takes its inputs as arguments, so that a test can feed one stage the
+# upstream buffers of another implementation (tests/test_gpu_stagewise.py feeds the GPU's own).
 # ---------------------------------------------------------------------------
 
-def forward_backward(p, x_history, x_target, x_global, user_id, label, *, training=True, alpha=0.95,
-                     dtype=torch.float32):
-    """Returns (logits, loss, grads dict incl. 'delta', bn batch stats)."""
-    B, H, _ = x_history.shape
-    C = x_target.shape[1]
-    R = B * C
-    grads = {k: torch.zeros_like(v) for k, v in p.items() if v.dtype.is_floating_point and not k.startswith('bn.running')}
+def grad_buffers(p) -> Dict[str, T]:
+    return {k: torch.zeros_like(v) for k, v in p.items() if v.dtype.is_floating_point and not k.startswith('bn.running')}
 
-    # ---- encoder forward
-    dh_ = decode_rows(x_history.reshape(B * H, -1), dtype)
-    dt_ = decode_rows(x_target.reshape(R, -1), dtype)
-    xin_h = embed_rows(p, dh_)                                        # [BH,66]
-    xt = embed_rows(p, dt_)                                           # [R,64]
-    W1, b1w = p[II + 'w1.weight'], p[II + 'w1.bias']
-    xh = xin_h @ W1.t() + b1w                                         # [BH,64]
-    lab_P, lab_saved = attention_forward(p, II + 'label_attention.', xt.view(B, C, 64), xh.view(B, H, 64))
-    ti_P, ti_saved = attention_forward(p, II + 'text_img_attention.', dt_['pca'].view(B, C, 64), dh_['pca'].view(B, H, 64))
-    g = x_global.reshape(R, 3).to(dtype)
+
+def w1_forward(p, xin_h: T) -> T:
+    """xh = w1(xin_h)   (user_invariant_interest_model.py:78)"""
+    return xin_h @ p[II + 'w1.weight'].t() + p[II + 'w1.bias']
+
+
+def w1_backward(p, xin_h: T, dxh: T, grads) -> T:
+    """-> dxin_h; w1 gradients accumulated into `grads`."""
+    grads[II + 'w1.weight'] += dxh.t() @ xin_h
+    grads[II + 'w1.bias'] += dxh.sum(0)
+    return dxh @ p[II + 'w1.weight']
+
+
+def instant_forward(p, x_global: T, dtype) -> Tuple[T, T]:
+    """-> (g [R,3], eu_l [R,8] = relu(out_fc(g)))   (user_instant_interest_model.py)"""
+    g = x_global.reshape(-1, 3).to(dtype)
     Wi, bi = p['instant_interest_model.out_fc.0.weight'], p['instant_interest_model.out_fc.0.bias']
-    eu_l = torch.relu(g @ Wi.t() + bi)
-    e = torch.cat([lab_P.reshape(R, 64), ti_P.reshape(R, 64), eu_l, xt, dt_['pca']], dim=1)   # [R,264]
+    return g, torch.relu(g @ Wi.t() + bi)
 
-    # ---- head forward (user_model.py:31-35)
+
+def instant_backward(g: T, eu_l: T, de_l: T, grads) -> None:
+    """de_l = de[:, 128:136]"""
+    dpre = de_l * (eu_l > 0).to(de_l.dtype)
+    grads['instant_interest_model.out_fc.0.weight'] += dpre.t() @ g
+    grads['instant_interest_model.out_fc.0.bias'] += dpre.sum(0)
+
+
+def head_forward(p, e: T, training: bool = True, stats: Tuple[T, T] = None):
+    """e [R,264] -> (logits [R], saved).  training: BatchNorm over the batch's own (biased) statistics, computed from e; else
+    `stats` = (mean, var), the running statistics when None.  (user_model.py:31-35)"""
     if training:
         mean = e.mean(0)
         var = ((e - mean) ** 2).mean(0)                               # biased, used for normalisation
+    elif stats is not None:
+        mean, var = stats
     else:
         mean, var = p['bn.running_mean'], p['bn.running_var']
     rstd = 1.0 / torch.sqrt(var + 1e-5)
@@ -168,9 +181,44 @@ def forward_backward(p, x_history, x_target, x_global, user_id, label, *, traini
     a2 = x @ M1.t() + d1; u2 = gelu(a2)
     y = u2 @ M2.t() + d2
     a3 = y @ O1.t() + f1; u3 = gelu(a3)
-    r = (u3 @ O2.t() + f2).reshape(B, C)
+    r = (u3 @ O2.t() + f2).reshape(-1)
+    saved = dict(e=e, mean=mean, var=var, rstd=rstd, xhat=xhat, z=z, a1=a1, u1=u1, gate=gate, x=x, a2=a2, u2=u2, y=y, a3=a3, u3=u3,
+                 training=training)
+    return r, saved
 
-    # ---- loss forward + backward (user_model.py:37-43)
+
+def head_backward(p, saved, dlogits: T, grads) -> T:
+    """dlogits [R] -> de [R,264]; the head's weight gradients (bn, gate, mlp, out_mlp) accumulated into `grads`."""
+    s = saved
+    G1, G2, M1, M2, O1, O2 = (p[k] for k in ('gate.fc1.weight', 'gate.fc2.weight', 'mlp.fc1.weight', 'mlp.fc2.weight',
+                                             'out_mlp.fc1.weight', 'out_mlp.fc2.weight'))
+    dr = dlogits.reshape(-1, 1)
+    grads['out_mlp.fc2.weight'] += dr.t() @ s['u3']
+    grads['out_mlp.fc2.bias'] += dr.sum(0)
+    da3 = (dr @ O2) * gelu_grad(s['a3'])
+    grads['out_mlp.fc1.weight'] += da3.t() @ s['y']; grads['out_mlp.fc1.bias'] += da3.sum(0)
+    dy = da3 @ O1
+    grads['mlp.fc2.weight'] += dy.t() @ s['u2']; grads['mlp.fc2.bias'] += dy.sum(0)
+    da2 = (dy @ M2) * gelu_grad(s['a2'])
+    grads['mlp.fc1.weight'] += da2.t() @ s['x']; grads['mlp.fc1.bias'] += da2.sum(0)
+    dx = da2 @ M1
+    dgate = dx * s['e']
+    de = dx * s['gate']
+    grads['gate.fc2.weight'] += dgate.t() @ s['u1']; grads['gate.fc2.bias'] += dgate.sum(0)
+    da1 = (dgate @ G2) * gelu_grad(s['a1'])
+    grads['gate.fc1.weight'] += da1.t() @ s['z']; grads['gate.fc1.bias'] += da1.sum(0)
+    dz = da1 @ G1
+    xhat, rstd = s['xhat'], s['rstd']
+    grads['bn.weight'] += (dz * xhat).sum(0); grads['bn.bias'] += dz.sum(0)
+    dxhat = dz * p['bn.weight']
+    if s['training']:
+        return de + rstd * (dxhat - dxhat.mean(0) - xhat * (dxhat * xhat).mean(0))
+    return de + rstd * dxhat
+
+
+def loss_backward(p, r: T, user_id, label, grads, *, alpha=0.95, dtype=torch.float32) -> Tuple[T, T]:
+    """r [B,C] -> (loss, dlogits [B,C]); the delta gradient accumulated into `grads`.  (user_model.py:37-43)"""
+    B, C = r.shape
     yl = label.to(dtype)
     N = float(B * C)
 
@@ -182,46 +230,47 @@ def forward_backward(p, x_history, x_target, x_global, user_id, label, *, traini
         return lo, dlog
     l1, dl1 = bce_softmax(r)
     l2, dl2 = bce_softmax(r + p['delta'][user_id][:, None])
-    loss = (1 - alpha) * l1 + alpha * l2
-    dr = ((1 - alpha) * dl1 + alpha * dl2).reshape(R, 1)
     grads['delta'].index_add_(0, user_id, alpha * dl2.sum(1))
+    return (1 - alpha) * l1 + alpha * l2, (1 - alpha) * dl1 + alpha * dl2
 
-    # ---- head backward
-    grads['out_mlp.fc2.weight'] += dr.t() @ u3
-    grads['out_mlp.fc2.bias'] += dr.sum(0)
-    da3 = (dr @ O2) * gelu_grad(a3)
-    grads['out_mlp.fc1.weight'] += da3.t() @ y; grads['out_mlp.fc1.bias'] += da3.sum(0)
-    dy = da3 @ O1
-    grads['mlp.fc2.weight'] += dy.t() @ u2; grads['mlp.fc2.bias'] += dy.sum(0)
-    da2 = (dy @ M2) * gelu_grad(a2)
-    grads['mlp.fc1.weight'] += da2.t() @ x; grads['mlp.fc1.bias'] += da2.sum(0)
-    dx = da2 @ M1
-    dgate = dx * e
-    de = dx * gate
-    grads['gate.fc2.weight'] += dgate.t() @ u1; grads['gate.fc2.bias'] += dgate.sum(0)
-    da1 = (dgate @ G2) * gelu_grad(a1)
-    grads['gate.fc1.weight'] += da1.t() @ z; grads['gate.fc1.bias'] += da1.sum(0)
-    dz = da1 @ G1
-    grads['bn.weight'] += (dz * xhat).sum(0); grads['bn.bias'] += dz.sum(0)
-    dxhat = dz * p['bn.weight']
-    if training:
-        de = de + rstd * (dxhat - dxhat.mean(0) - xhat * (dxhat * xhat).mean(0))
-    else:
-        de = de + rstd * dxhat
+
+# ---------------------------------------------------------------------------
+# whole training step in kernel form
+# ---------------------------------------------------------------------------
+
+def forward_backward(p, x_history, x_target, x_global, user_id, label, *, training=True, alpha=0.95,
+                     dtype=torch.float32):
+    """Returns (logits, loss, grads dict incl. 'delta', bn batch stats)."""
+    B, H, _ = x_history.shape
+    C = x_target.shape[1]
+    R = B * C
+    grads = grad_buffers(p)
+
+    # ---- encoder forward
+    dh_ = decode_rows(x_history.reshape(B * H, -1), dtype)
+    dt_ = decode_rows(x_target.reshape(R, -1), dtype)
+    xin_h = embed_rows(p, dh_)                                        # [BH,66]
+    xt = embed_rows(p, dt_)                                           # [R,64]
+    xh = w1_forward(p, xin_h)                                         # [BH,64]
+    lab_P, lab_saved = attention_forward(p, II + 'label_attention.', xt.view(B, C, 64), xh.view(B, H, 64))
+    ti_P, ti_saved = attention_forward(p, II + 'text_img_attention.', dt_['pca'].view(B, C, 64), dh_['pca'].view(B, H, 64))
+    g, eu_l = instant_forward(p, x_global, dtype)
+    e = torch.cat([lab_P.reshape(R, 64), ti_P.reshape(R, 64), eu_l, xt, dt_['pca']], dim=1)   # [R,264]
+
+    # ---- head forward, loss forward + backward, head backward
+    r, head_saved = head_forward(p, e, training)
+    r = r.reshape(B, C)
+    loss, dr = loss_backward(p, r, user_id, label, grads, alpha=alpha, dtype=dtype)
+    de = head_backward(p, head_saved, dr.reshape(R), grads)
 
     # ---- encoder backward
-    dpre = de[:, 128:136] * (eu_l > 0).to(dtype)
-    grads['instant_interest_model.out_fc.0.weight'] += dpre.t() @ g
-    grads['instant_interest_model.out_fc.0.bias'] += dpre.sum(0)
-    dt_lab, dh_lab = attention_backward(p, II + 'label_attention.', xt.view(B, C, 64), xh.view(B, H, 64), lab_saved,
-                                        de[:, 0:64].reshape(B, C, 64), grads, True)
+    instant_backward(g, eu_l, de[:, 128:136], grads)
+    dt_lab, dh_lab, _ = attention_backward(p, II + 'label_attention.', xt.view(B, C, 64), xh.view(B, H, 64), lab_saved,
+                                           de[:, 0:64].reshape(B, C, 64), grads, True)
     attention_backward(p, II + 'text_img_attention.', dt_['pca'].view(B, C, 64), dh_['pca'].view(B, H, 64), ti_saved,
                        de[:, 64:128].reshape(B, C, 64), grads, False)
     dxt = dt_lab.reshape(R, 64) + de[:, 136:200]
-    dxh = dh_lab.reshape(B * H, 64)
-    grads[II + 'w1.weight'] += dxh.t() @ xin_h
-    grads[II + 'w1.bias'] += dxh.sum(0)
-    dxin_h = dxh @ W1
+    dxin_h = w1_backward(p, xin_h, dh_lab.reshape(B * H, 64), grads)
     embed_rows_backward(p, dh_, xin_h, dxin_h, grads)
     embed_rows_backward(p, dt_, xt, dxt, grads)
-    return r, loss, grads, (mean, var)
+    return r, loss, grads, (head_saved['mean'], head_saved['var'])
