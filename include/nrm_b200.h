@@ -97,8 +97,6 @@ int         nrm_debug_umma_selftest(const float* a0, const float* a1, const floa
  * 4: tcgen05.ld only.  `reps` products of `nk` K=16 steps each. */
 int         nrm_debug_mma_microbench(long long* out, int variant, int reps, int nk, void* stream);
 
-/* Phase cycle counters of the tensor-core attention forward (only in a -DNRM_TC_PROFILE build; otherwise returns
- * NRM_EUNSUPPORTED): 16 host int64 = clock64 cycles accumulated by CTA 0 per phase since the last call. */
 /* ---- data parallelism over peer memory (no counterpart in the single-process reference; north_star: gradient all-reduce) ----
  * The gradient average over the ranks is fused into the optimizer: every rank's flat gradient buffer sits in symmetric (peer-mapped)
  * memory and nrm_adam_step_allreduce reads all of them in rank order while it updates.  `peer_ctx` is a device struct
@@ -125,7 +123,6 @@ int         nrm_peer_allsum_stats(const double* local, int which, double* out, c
 int         nrm_debug_rsprof(long long* host_out64);   /* row-stacked attention kernels: per-role wait cycles (-DNRM_RS_PROFILE builds) */
 long long   nrm_debug_ws_field(int B, int H, int C, int mode, const char* name, long long* bytes);   /* byte offset of a workspace buffer (debugging) */
 int         nrm_debug_headprof(long long* host_out32); /* tensor-core head kernels: the same (-DNRM_RS_PROFILE builds) */
-int         nrm_debug_tcprof(long long* host_out32);
 
 /* ---- flat parameter layout (reference state_dict order; SURVEY.md section 8b) ---- */
 int         nrm_layout_entries(void);                 /* trainable tensors incl. delta     */
@@ -230,8 +227,7 @@ int nrm_backward_encoder_compact(const nrm_compact_batch* batch, int B, int H, i
  *   nrm_forward_scores[_compact]: nrm_forward[_compact] in mode NRM_MODE_EVAL (any other mode: NRM_EINVAL; BatchNorm reads its
  *     running statistics and nothing is written to them) that also writes `scores`; the logits are bit-identical to nrm_forward's
  *     for the same precision, the workspace is nrm_workspace_bytes(B, H, C, NRM_MODE_EVAL).  The compact variant has
- *     nrm_forward_compact's precision limits.  With NRM_ATT_ITEM_TILES=1 in the environment: NRM_EUNSUPPORTED (those kernels do
- *     not export scores).
+ *     nrm_forward_compact's precision limits.
  *   nrm_history_topk: per (branch, b, c) row the k largest scores and their history positions, descending, ties to the lower
  *     position (Python's stable sorted(..., reverse=True)); idx_out int32 / val_out float32 [2,B,C,k], 1 <= k <= min(H, 64).  Pad rows
  *     are left out: all-zero rows of x_history [B,H,80] or hist_article [B,H] == 0 (at most one of the two; both null: none); slots
@@ -251,7 +247,7 @@ int nrm_history_topk(const float* scores, int B, int C, int H, int k, const doub
  * users and keep each user's k best unread ones.
  *   nrm_forward_pool: logits [B,N] float32; logits[b][n] is, bit for bit, what nrm_forward in mode NRM_MODE_EVAL returns for
  *     impression b with the user's history and the whole pool as its candidates (x_target[b] / x_global[b] = the pool's rows for
- *     every b), in the same precision (all three; NRM_ATT_ITEM_TILES=1 too).  BatchNorm reads its running statistics only.
+ *     every b), in the same precision (all three).  BatchNorm reads its running statistics only.
  *     users->hist_* are the users' [B,H] / [B,H,2] compact histories; users->cand_article / cand_time are the pool's [N] ids and
  *     packed time buckets (one time for all users); label32 / label64 must be null.  The pool is processed in chunks of `chunk`
  *     articles (a positive multiple of 8, the attention's candidate group: any such chunk gives the same bits); the workspace

@@ -28,7 +28,6 @@ SIGNATURES = {
     'nrm_timing_report': (i32, [C.c_char_p, sz]),
     'nrm_debug_umma_selftest': (i32, [vp, vp, vp, vp, vp, i32, i32, vp]),
     'nrm_debug_mma_microbench': (i32, [vp, i32, i32, i32, vp]),
-    'nrm_debug_tcprof': (i32, [vp]),
     'nrm_debug_rsprof': (i32, [vp]),
     'nrm_debug_headprof': (i32, [vp]),
     'nrm_debug_ws_field': (ll, [i32, i32, i32, i32, C.c_char_p, vp]),

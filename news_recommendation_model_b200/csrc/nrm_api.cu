@@ -104,20 +104,6 @@ static SideStream* side_stream(cudaStream_t caller) {
   return ss;
 }
 
-// NRM_ATT_ITEM_TILES=1 selects the previous per-(pair, candidate) M = 64 tensor-core kernels (nrm_attention_tc.cu) instead of the
-// row-stacked ones (nrm_attention_rs.cu); kept as the second tensor-core implementation for A/B tests.
-bool use_rowstacked() {
-  static const bool on = getenv("NRM_ATT_ITEM_TILES") == nullptr;
-  return on;
-}
-
-// The FFMA forward of w1 streams at ~35 % of the HBM roofline once there are several tiles per SM; the tensor-core version only
-// pays when NRM_W1_FWD_TC=1 asks for it (kept for A/B runs): with <= 3 tiles per SM its per-CTA prologue is not amortised.
-bool w1_forward_on_tensor_cores(const Workspace&) {
-  static const bool on = getenv("NRM_W1_FWD_TC") != nullptr;
-  return on;
-}
-
 bool pdl_enabled() {
   static const bool on = getenv("NRM_NO_PDL") == nullptr;
   return on;
@@ -192,7 +178,6 @@ size_t carve_workspace(Workspace& w, void* base, int B, int H, int C, int mode) 
   w.y = (float*)take(f * R * E);
   w.a3 = (float*)take(f * R * HID);
   w.head_wt = (float*)take(f * (HEAD_WT_W1T + 64 * XIN));
-  w.att_derived = (float*)take(f * 2 * 12420);
   w.tp = (float*)take(f * 2 * R * 64);
   w.att_rs_img = (float*)take(attention_rs_image_bytes());
   w.head_img = (float*)take(head_tc_image_bytes());
@@ -238,12 +223,6 @@ size_t carve_workspace(Workspace& w, void* base, int B, int H, int C, int mode) 
   return off;
 }
 
-// NRM_HEAD_FFMA=1 keeps the scoring head on the FFMA kernels (nrm_head_fused.cu) in the tensor-core precisions too
-static bool head_on_tensor_cores(int precision) {
-  static const bool ffma = [] { const char* e = getenv("NRM_HEAD_FFMA"); return e != nullptr && e[0] == '1'; }();
-  return precision != NRM_PRECISION_FP32 && use_rowstacked() && !ffma;
-}
-
 static int check_shape(const char* fn, int B, int H, int C) {
   if (B <= 0 || H <= 0 || C <= 0) { set_error("%s: B, H, C must be positive (got %d, %d, %d)", fn, B, H, C); return NRM_EINVAL; }
   if (((long long)B * H + (long long)B * C) * 6 >= (1LL << 31)) { set_error("%s: batch too large for 32-bit entry ids", fn); return NRM_EINVAL; }
@@ -260,15 +239,15 @@ static int encoder_forward(const BatchPtrs& in, const float* P, Workspace& w, in
   SideStream* ss = side_stream(s);
   if (ss == nullptr) { set_error("encoder_forward: cannot create the side stream"); return NRM_ECUDA; }
   const bool tc = precision != NRM_PRECISION_FP32;
-  // fork 0: what depends on the weights only (derived attention matrices, transposed head matrices) runs on the side
-  // stream under the embedding kernel
+  // fork 0: what depends on the weights only (transposed head matrices, the operand images of the tensor-core attention and head)
+  // runs on the side stream under the embedding kernel
   NRM_CUDA(cudaEventRecord(ss->fork0, s));
   NRM_CUDA(cudaStreamWaitEvent(ss->stream, ss->fork0, 0));
   NRM_TRY(launch_head_transpose(P, w, ss->stream));          // includes w1^T for the history projection below
   NRM_CUDA(cudaEventRecord(ss->join0, ss->stream));
-  if (tc) {                                                  // derived weights of the path in use (weights only)
-    if (use_rowstacked()) NRM_TRY(launch_attention_prep_rs(P, w, ss->stream)); else NRM_TRY(launch_attention_prep(P, w, ss->stream));
-    if (head_on_tensor_cores(precision)) NRM_TRY(launch_head_images_tc(P, w, precision, (mode & NRM_MODE_KEEP_FOR_BWD) != 0, ss->stream));
+  if (tc) {
+    NRM_TRY(launch_attention_prep_rs(P, w, ss->stream));
+    NRM_TRY(launch_head_images_tc(P, w, precision, (mode & NRM_MODE_KEEP_FOR_BWD) != 0, ss->stream));
   }
   { KernelTimer t("embed_rows", s);
     NRM_TRY(launch_embed_rows(in, P, w, (mode & NRM_MODE_KEEP_FOR_BWD) != 0, s)); }
@@ -284,21 +263,15 @@ static int encoder_forward(const BatchPtrs& in, const float* P, Workspace& w, in
   }
   // xh = w1(xin_h)   (user_invariant_interest_model.py:78)
   NRM_CUDA(cudaStreamWaitEvent(s, ss->join0, 0));            // w1^T ready
-  { KernelTimer t("w1_forward", s);
-    if (tc && use_rowstacked() && w1_forward_on_tensor_cores(w)) NRM_TRY(launch_w1_forward_tc(P, w, precision, s)); else NRM_TRY(launch_w1_forward(P, w, s)); }
-  NRM_CUDA(cudaStreamWaitEvent(s, ss->join_tp, 0));          // join: derived weights, transposed head matrices, tp
+  { KernelTimer t("w1_forward", s); NRM_TRY(launch_w1_forward(P, w, s)); }
+  NRM_CUDA(cudaStreamWaitEvent(s, ss->join_tp, 0));          // join: operand images, transposed head matrices, tp
   if (!tc) {
     { KernelTimer t("attention_forward_label", s); NRM_TRY(launch_attention_forward(in, P, w, 0, precision, s)); }
     { KernelTimer t("attention_forward_textimg", s); NRM_TRY(launch_attention_forward(in, P, w, 1, precision, s)); }
   } else {
     // tensor-core path: one launch covers both branches
     KernelTimer t("attention_forward", s);
-    if (use_rowstacked()) {
-      NRM_TRY(launch_attention_forward_rs(in, w, precision, s));
-    } else {
-      NRM_TRY(launch_attention_forward(in, P, w, 0, precision, s));
-      NRM_TRY(launch_attention_forward(in, P, w, 1, precision, s));
-    }
+    NRM_TRY(launch_attention_forward_rs(in, w, precision, s));
   }
   // join: the id sort (long finished: it ran under the w1 / attention kernels) comes back to the caller's stream HERE, so a
   // training-mode forward that is never followed by a backward (validation with gradients enabled, a graph capture of the
@@ -310,9 +283,13 @@ static int encoder_forward(const BatchPtrs& in, const float* P, Workspace& w, in
 static int encoder_backward(const BatchPtrs& in, const float* P, Workspace& w, int precision, float* G, cudaStream_t s) {
   SideStream* ss = side_stream(s);
   if (ss == nullptr) { set_error("encoder_backward: cannot create the side stream"); return NRM_ECUDA; }
-  { KernelTimer t("attention_backward_label", s); NRM_TRY(launch_attention_backward(in, P, w, 0, precision, s)); }
-  if (precision != NRM_PRECISION_FP32 && use_rowstacked()) {
-    // row-stacked kernels: the label branch's input gradients (dxh, dxt) come from the dhid tiles the kernel above exported
+  const bool tc = precision != NRM_PRECISION_FP32;
+  // tensor-core precisions: the row-stacked backward sums over rows (weight gradients, dtp); its label branch exports dhid for the
+  // input-gradient kernel
+  { KernelTimer t("attention_backward_label", s);
+    if (tc) NRM_TRY(launch_attention_backward_rs(w, 0, precision, true, s)); else NRM_TRY(launch_attention_backward(in, P, w, 0, precision, s)); }
+  if (tc) {
+    // the label branch's input gradients (dxh, dxt) come from the dhid tiles the kernel above exported
     KernelTimer t("attention_input_grad_label", s);
     NRM_TRY(launch_attention_input_grad_rs(w, precision, s));
   }
@@ -321,11 +298,11 @@ static int encoder_backward(const BatchPtrs& in, const float* P, Workspace& w, i
   // attention kernel is on the critical path, the w1 backward then runs beside attention_finish in the latency-bound tail
   NRM_CUDA(cudaEventRecord(ss->fork2, s));
   NRM_CUDA(cudaStreamWaitEvent(ss->stream, ss->fork2, 0));
-  { KernelTimer t("attention_backward_textimg", s); NRM_TRY(launch_attention_backward(in, P, w, 1, precision, s)); }
+  { KernelTimer t("attention_backward_textimg", s);
+    if (tc) NRM_TRY(launch_attention_backward_rs(w, 1, precision, false, s)); else NRM_TRY(launch_attention_backward(in, P, w, 1, precision, s)); }
   // w1: dxin_h = dxh W1, dW1 = dxh^T xin_h, db1 = colsum(dxh)
   { KernelTimer t("w1_backward", ss->stream);
-    if (precision != NRM_PRECISION_FP32 && use_rowstacked()) NRM_TRY(launch_w1_backward_tc(P, w, G, precision, ss->stream));
-    else NRM_TRY(launch_w1_backward(P, w, G, ss->stream)); }
+    if (tc) NRM_TRY(launch_w1_backward_tc(P, w, G, precision, ss->stream)); else NRM_TRY(launch_w1_backward(P, w, G, ss->stream)); }
   NRM_CUDA(cudaEventRecord(ss->join2, ss->stream));
   if (ss->head_wgrad_pending) {                              // behind the w1 backward on the side stream; covered by join3 below
     ss->head_wgrad_pending = false;
@@ -333,8 +310,8 @@ static int encoder_backward(const BatchPtrs& in, const float* P, Workspace& w, i
     NRM_TRY(launch_head_backward_wgrad(ss->wg_params, w, ss->wg_grads, ss->stream, ss->wg_tiles, ss->wg_precision));
   }
   { KernelTimer t("attention_finish", s);
-    NRM_TRY(launch_attention_finish(P, w, 0, precision, G, s));
-    NRM_TRY(launch_attention_finish(P, w, 1, precision, G, s)); }
+    if (tc) NRM_TRY(launch_attention_finish_tc(P, w, G, s));   // one pass for both branches
+    else { NRM_TRY(launch_attention_finish(P, w, 0, precision, G, s)); NRM_TRY(launch_attention_finish(P, w, 1, precision, G, s)); } }
   NRM_CUDA(cudaStreamWaitEvent(s, ss->join2, 0));          // join: dxin_h ready
   // fork: the sentiment / instant Linear gradients (side stream) next to the table gradients (two latency-bound kernel
   // pairs that write disjoint gradient ranges)
@@ -450,7 +427,7 @@ static int compact_batch(const char* fn, const nrm_compact_batch* cb, int precis
     set_error("%s: bad compact batch", fn); return NRM_EINVAL;
   }
   if ((reinterpret_cast<uintptr_t>(cb->articles) & 15) != 0) { set_error("%s: the article table must be 16-byte aligned", fn); return NRM_EINVAL; }
-  if (precision == NRM_PRECISION_FP32 || !use_rowstacked()) {
+  if (precision == NRM_PRECISION_FP32) {
     set_error("%s: the compact wire format is read directly by the tensor-core precisions only (use nrm_expand_compact otherwise)", fn);
     return NRM_EUNSUPPORTED;
   }
@@ -493,7 +470,7 @@ extern "C" int nrm_forward_head(int B, int H, int C, const float* params, float*
   const double* sums = bn_sums ? bn_sums : w.bn_sums;
   const long long rows = bn_global_rows > 0 ? bn_global_rows : w.R;
   KernelTimer t("head_forward", (cudaStream_t)stream);
-  if (head_on_tensor_cores(precision))
+  if (precision != NRM_PRECISION_FP32)
     return launch_head_forward_tc(params, w, precision, bn_running_mean, bn_running_var, bn_num_batches_tracked, training,
                                   (mode & NRM_MODE_KEEP_FOR_BWD) != 0, sums, rows, logits, (cudaStream_t)stream);
   return launch_head_forward(params, w, bn_running_mean, bn_running_var, bn_num_batches_tracked, training,
@@ -525,10 +502,6 @@ static int forward_scores_impl(const char* fn, const BatchPtrs& in, int B, int H
                                float* scores, void* workspace, size_t workspace_bytes, void* stream) {
   if (mode != NRM_MODE_EVAL) { set_error("%s: scores are exported by eval-mode forwards only (mode must be NRM_MODE_EVAL, got %d)", fn, mode); return NRM_EINVAL; }
   if (!scores) { set_error("%s: null scores", fn); return NRM_EINVAL; }
-  if (!use_rowstacked()) {
-    set_error("%s: the item-tile attention kernels (NRM_ATT_ITEM_TILES) do not export scores", fn);
-    return NRM_EUNSUPPORTED;
-  }
   Workspace w;
   NRM_TRY(get_workspace(fn, w, workspace, workspace_bytes, B, H, C, mode));
   w.scores = scores;
@@ -641,7 +614,7 @@ static int backward_head(const char* fn, bool defer_wgrad, int B, int H, int C, 
   Workspace w;
   NRM_TRY(get_workspace(fn, w, workspace, workspace_bytes, B, H, C, NRM_MODE_KEEP_FOR_BWD));
   cudaStream_t s = (cudaStream_t)stream;
-  const bool tc = head_on_tensor_cores(precision);
+  const bool tc = precision != NRM_PRECISION_FP32;
   const int tiles = tc ? head_tc_tiles(w.R) : 0;
   if (!defer_wgrad) {
     KernelTimer t("head_backward", s);
@@ -680,7 +653,7 @@ static int backward_encoder_impl(const char* fn, const BatchPtrs& in, int B, int
   cudaStream_t s = (cudaStream_t)stream;
   const double* sums = bn_bwd_sums ? bn_bwd_sums : w.bn_bwd_sums;
   const long long rows = bn_global_rows > 0 ? bn_global_rows : w.R;
-  NRM_TRY(launch_bn_backward_combine(params, w, training, sums, rows, head_on_tensor_cores(precision), s));
+  NRM_TRY(launch_bn_backward_combine(params, w, training, sums, rows, precision != NRM_PRECISION_FP32, s));
   return encoder_backward(in, params, w, precision, grads, s);   // also enqueues and joins the weight gradients nrm_backward_head_deferred left
 }
 
@@ -718,7 +691,7 @@ static int backward_impl(const char* fn, const BatchPtrs& in, int B, int H, int 
   cudaStream_t s = (cudaStream_t)stream;
   SideStream* ss = side_stream(s);
   if (ss == nullptr) { set_error("%s: cannot create the side stream", fn); return NRM_ECUDA; }
-  const bool htc = head_on_tensor_cores(precision);
+  const bool htc = precision != NRM_PRECISION_FP32;
   const int tiles = htc ? head_tc_tiles(w.R) : 0;
   { KernelTimer t("head_backward", s);
     if (htc) NRM_TRY(launch_head_backward_dgrad_tc(params, w, precision, dlogits, grads, s)); else NRM_TRY(launch_head_backward_dgrad(params, w, dlogits, s));

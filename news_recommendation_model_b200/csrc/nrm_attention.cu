@@ -500,8 +500,7 @@ attention_compose_kernel(const float* __restrict__ part, int nparts, AttOffsets 
 static int att_bwd_grid(int B) { return min(B, min(sm_count(), ATT_BWD_CTAS_MAX)); }
 
 int launch_attention_forward(const BatchPtrs& in, const float* P, Workspace& w, int branch, int precision, cudaStream_t s) {
-  if (precision == NRM_PRECISION_BF16 || precision == NRM_PRECISION_BF16X3) return launch_attention_forward_tc(in, w, branch, precision, s);
-  if (precision != NRM_PRECISION_FP32) { set_error("attention: precision %d not built", precision); return NRM_EUNSUPPORTED; }
+  if (precision != NRM_PRECISION_FP32) { set_error("attention: the FFMA kernels run precision fp32 only (got %d)", precision); return NRM_EUNSUPPORTED; }
   const size_t smem = sizeof(AttSmemFwd);
   // w.scores non-null: the score-exporting instantiations
   void (*k)(const double*, const float*, int, int, int, const float*, float*, float*) =
@@ -514,14 +513,7 @@ int launch_attention_forward(const BatchPtrs& in, const float* P, Workspace& w, 
 }
 
 int launch_attention_backward(const BatchPtrs& in, const float* P, Workspace& w, int branch, int precision, cudaStream_t s) {
-  if (precision == NRM_PRECISION_BF16 || precision == NRM_PRECISION_BF16X3) {
-    if (use_rowstacked()) {
-      // row-stacked kernels: sums over rows (weight gradients, dtp); the label branch exports dhid for its input-gradient kernel
-      return launch_attention_backward_rs(w, branch, precision, branch == 0, s);
-    }
-    return launch_attention_backward_tc(in, P, w, branch, precision, s);
-  }
-  if (precision != NRM_PRECISION_FP32) { set_error("attention: precision %d not built", precision); return NRM_EUNSUPPORTED; }
+  if (precision != NRM_PRECISION_FP32) { set_error("attention: the FFMA kernels run precision fp32 only (got %d)", precision); return NRM_EUNSUPPORTED; }
   const size_t smem = sizeof(AttSmemBwd);
   const int grid = att_bwd_grid(w.B);
   float* part = w.att_part + (long long)branch * ATT_BWD_CTAS_MAX * ATT_PARTIAL;
@@ -537,7 +529,7 @@ int launch_attention_backward(const BatchPtrs& in, const float* P, Workspace& w,
 }
 
 int launch_attention_finish(const float* P, Workspace& w, int branch, int precision, float* grads, cudaStream_t s) {
-  if (precision != NRM_PRECISION_FP32) return branch == 1 ? launch_attention_finish_tc(P, w, grads, s) : NRM_OK;   // one pass for both branches
+  if (precision != NRM_PRECISION_FP32) { set_error("attention: the FFMA kernels run precision fp32 only (got %d)", precision); return NRM_EUNSUPPORTED; }
   const float* part = w.att_part + (long long)branch * ATT_BWD_CTAS_MAX * ATT_PARTIAL;
   launch_pdl(attention_compose_kernel, dim3(64), dim3(256), 0, s, part, att_bwd_grid(w.B), branch == 0 ? ATT_LABEL : ATT_TI, grads);
   NRM_LAUNCH_CHECK("attention_compose_kernel");

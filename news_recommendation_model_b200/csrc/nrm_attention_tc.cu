@@ -1,86 +1,18 @@
-// Pairwise MLP attention + sum pooling on the 5th-generation tensor cores, forward AND backward.
-// Reference: PointwiseAttentionExpanded.forward (models/attention_model.py:52-97) and the pooling at
-// models/user_invariant_interest_model.py:83-87.
-//
-// Reduced algebra (nrm_attention.cu, DESIGN.md section 3): per ITEM = (impression b, candidate c)
-//     hid[h][j] = sum_k H[h][k] W_c[j][k] + tp[j],   W_c = Wd diag(t_c) + A,   tp = Bm t_c + b1
-//     s[h] = w2 . gelu(hid[h][:]) + b2,               pooled[k] = sum_h s[h] H[h][k]
-// and, given dP = dL/dpooled,
-//     ds[h] = sum_k dP[k] H[h][k];     dhid[h][j] = ds[h] w2[j] gelu'(hid[h][j])
-//     S^T[k][j] = sum_h H[h][k] dhid[h][j]  (= dL/dW_c^T);   dA += S;  dWd[j][k] += S[j][k] t[k]
-//     dt[k] = sum_j S[j][k] Wd[j][k] (+ the tp path, nrm_attention_post);   Gt[j] = sum_h dhid[h][j] = dL/dtp[j]
-//     dH[h][k] += sum_j dhid[h][j] W_c[j][k] + s[h] dP[k]
-//
-// Every contraction above is a tcgen05.mma (M = 64, bf16 operands in shared memory, fp32 accumulators in
-// tensor memory); the CUDA cores only generate operands and run the per-row epilogues:
-//
-//   product            M   N   K    A operand                     B operand
-//   hid    = H W_c^T   h   j   k    H tile, K-major               W_c tile, K-major      (per item)
-//   pooled = H^T s     k   c   h    H tile read MN-major          score tile [c][h]      (per impression, forward)
-//   ds     = H dP^T    h   c   k    H tile, K-major               dP tile [c][k]         (per impression)
-//   S^T    = H^T dhid  k   j   h    H tile read MN-major          dhid tile read MN-major
-//   dH    += dhid W_c  h   k   j    dhid tile, K-major            W_c tile read MN-major
-//   Gt     = dhid^T 1  j   8   h    dhid tile read MN-major       constant ones tile
-//
-// "read MN-major" = the same K-major tile consumed through a descriptor with the major bit set
-// (nrm_umma.cuh), so no transposed copy is ever written.
-//
-// An M = 64 accumulator fills only lanes 0-15 of each 32-lane TMEM sub-partition, so the CTA (128
-// threads) always works on a PAIR of impressions: impression 0's accumulators live in the lower
-// half-lanes, impression 1's in the upper half-lanes of the same columns, and thread (warp w, lane l)
-// owns row 16 w + (l & 15) of impression l >> 4 in every epilogue: it reads its 64 accumulator columns
-// with tcgen05.ld and does +tp, GELU, the fc2 dot product, dhid, ... entirely in registers.
-//
-// SPLIT = 1: plain bf16 operands ("bf16").  SPLIT = 3: every operand is written as hi + lo bf16 parts and every
-// product is issued as A_hi B_hi + A_hi B_lo + A_lo B_hi ("bf16x3", relative operand error 2^-16; this is
-// torch's float32 matmul precision "high").  Accumulation is fp32 in both.
+// The tensor-core attention's work outside the row-stacked kernels (nrm_attention_rs.cu, nrm_attention_rs_bwd.cu), for precision
+// bf16 / bf16x3, plus the tcgen05 building-block test and micro-benchmark.  Reduced algebra: DESIGN.md section 3.
+//   candidate_tp_kernel          tp = Bm t + b1 per candidate row, before the forward
+//   attention_finish_kernel      sums the row-stacked backward's per-CTA partials into dA, dWd, dw2, db2, and runs the tp path of
+//                                the backward (dBm, db1 partials; dxt += dtp Bm) over the candidate rows
+//   attention_tp_finish_kernel   sums the tp-path partials into dBm, dBm - dA and db1
+//   umma_selftest_kernel         nrm_debug_umma_selftest (tests/test_gpu_tensorcore.py)
+//   mma_microbench_kernel        nrm_debug_mma_microbench (tools/mma_microbench.py)
 #include "nrm_kernels.cuh"
-#include <cstddef>
 
 #include "nrm_umma.cuh"
 
 namespace nrm {
 
-// Optional phase timing (make EXTRA=-DNRM_TC_PROFILE): in CTA 0, thread 0 (the warp that issues the MMAs) and thread 32
-// (a warp that does not) accumulate clock64 deltas per phase into g_tcprof[i] / g_tcprof[16 + i]; nrm_debug_tcprof()
-// returns and clears them.  Compiled out by default.
-#ifdef NRM_TC_PROFILE
-__device__ long long g_tcprof[32];
-#define TCPROF_DECL long long tcp_t = clock64();
-#define TCPROF(i) do { if (blockIdx.x == 0 && (threadIdx.x == 0 || threadIdx.x == 32)) { const long long n__ = clock64(); g_tcprof[(i) + (threadIdx.x ? 16 : 0)] += n__ - tcp_t; tcp_t = n__; } } while (0)
-#else
-#define TCPROF_DECL
-#define TCPROF(i) do { } while (0)
-#endif
-
 constexpr int TC_THREADS = 256;       // 8 warps: warp w reads TMEM sub-partition w & 3 and accumulator columns 32 (w >> 2) .. +32
-constexpr int TC_MAXC = 8;           // candidates per chunk (N of the ds / pooling products)
-
-// derived weights per branch in the workspace (att_prep_kernel): Wd | A | w2 | b2.
-// Wd and A = Wa - Wc are stored in operand-build order [k/8][(k/4)%2][j][k%4]: the thread that builds the 8 k-values
-// (j, k/8) of a W_c tile reads two 16-byte vectors per matrix and consecutive lanes (j) read consecutive vectors,
-// from global memory when a CTA stages the blocks and from shared memory (conflict-free) for every item after that.
-constexpr int DER_WD = 0, DER_A = 4096, DER_W2 = 8192, DER_B2 = 8256, DER_SIZE = 12420;
-__host__ __device__ constexpr int wda_index(int j, int k) { return (((k >> 3) * 2 + ((k >> 2) & 1)) * 64 + j) * 4 + (k & 3); }
-
-__global__ void __launch_bounds__(256)
-att_prep_kernel(const float* __restrict__ P, float* __restrict__ der) {
-  pdl_wait();                                          // programmatic dependent launch: see nrm_common.cuh
-  pdl_trigger();
-  const AttOffsets off = blockIdx.y == 0 ? ATT_LABEL : ATT_TI;
-  float* d = der + (long long)blockIdx.y * DER_SIZE;
-  const float* W = P + off.fc1_w;
-  for (int i = blockIdx.x * 256 + threadIdx.x; i < 4096; i += gridDim.x * 256) {
-    const int j = i >> 6, k = i & 63;
-    const float wa = W[j * 256 + k], wc = W[j * 256 + 128 + k], wd = W[j * 256 + 192 + k];
-    d[DER_WD + wda_index(j, k)] = wd;
-    d[DER_A + wda_index(j, k)] = wa - wc;
-  }
-  if (blockIdx.x == 0 && threadIdx.x < 64) {
-    d[DER_W2 + threadIdx.x] = P[off.fc2_w + threadIdx.x];
-    if (threadIdx.x == 0) d[DER_B2] = P[off.fc2_b];
-  }
-}
 
 // tp[branch][r][j] = b1[j] + sum_k (Wb + Wc)[j][k] t[r][k] for every candidate row r (t = the candidate's label
 // features / PCA vector inside e_concat).  32 rows per CTA, blockIdx.y = branch.
@@ -122,767 +54,8 @@ candidate_tp_kernel(const float* __restrict__ P, const float* __restrict__ e, lo
   }
 }
 
-// ---- small operand tiles -------------------------------------------------------------------------
-// [8 rows][64 k] K-major: byte offset of (r, 8*kb) = kb*128 + r*16   (LBO = 128, one 8-row group)
-constexpr uint32_t T8_LBO = 128, T8_SBO = 128, T8_BYTES = 1024;
-__device__ __forceinline__ umma::Operand op_tile8_k(uint32_t addr) { return umma::make_operand(addr, T8_LBO, T8_SBO, 2 * T8_LBO, T8_BYTES); }
-// [16 rows][64 k] K-major: byte offset of (r, 8*kb) = kb*256 + (r/8)*128 + (r%8)*16; hi and lo parts 2048 bytes apart
-constexpr uint32_t T16_LBO = 256;
-__device__ __forceinline__ umma::Operand op_tile16_k(uint32_t addr) { return umma::make_operand(addr, T16_LBO, 128, 2 * T16_LBO, 2 * T8_BYTES); }
-
-template <int NP> struct TileBytes { static constexpr uint32_t T64 = NP * umma::TILE64_BYTES, T8 = NP * T8_BYTES; };
-
-// history rows [r0, r0+64) of impression b -> canonical K-major tile(s); rows >= H are zero.
-// All global loads of the tile are issued before the first conversion (one memory round trip per tile).
-// Work item -> (row, 8-column block): a warp covers 16 consecutive rows x 2 blocks, so its loads are 64-byte
-// segments (every fetched sector fully used) and its 16-byte tile stores fall into two 256-byte runs (2-way bank
-// conflict at worst); row-fastest would make every load touch 32 different rows.
-__device__ __forceinline__ void stage_item(int it, int& row, int& kb) {
-  const int lane = it & 31, w = it >> 5;
-  row = (w & 3) * 16 + (lane & 15);
-  kb = (w >> 2) * 2 + (lane >> 4);
-}
-template <int BRANCH, int NP>
-__device__ __forceinline__ void stage_history(const double* __restrict__ xh, const float* __restrict__ xhp,
-                                              long long b, int H, int r0, unsigned char* tile) {
-  constexpr int ITERS = 64 * 8 / TC_THREADS;
-  if (BRANCH == 0) {
-    float4 raw[ITERS][2];
-#pragma unroll
-    for (int u = 0; u < ITERS; ++u) {
-      int row, kb; stage_item(threadIdx.x + u * TC_THREADS, row, kb);
-      raw[u][0] = raw[u][1] = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (r0 + row < H) {
-        const float4* src = reinterpret_cast<const float4*>(xhp + (b * H + r0 + row) * 64 + kb * 8);
-        raw[u][0] = __ldg(src); raw[u][1] = __ldg(src + 1);
-      }
-    }
-#pragma unroll
-    for (int u = 0; u < ITERS; ++u) {
-      int row, kb; stage_item(threadIdx.x + u * TC_THREADS, row, kb);
-      const float v[8] = {raw[u][0].x, raw[u][0].y, raw[u][0].z, raw[u][0].w, raw[u][1].x, raw[u][1].y, raw[u][1].z, raw[u][1].w};
-      umma::store_operand8<NP>(tile, umma::tile64_offset(row, kb), umma::TILE64_BYTES, v);
-    }
-  } else {
-    double2 raw[ITERS][4];
-#pragma unroll
-    for (int u = 0; u < ITERS; ++u) {
-      int row, kb; stage_item(threadIdx.x + u * TC_THREADS, row, kb);
-#pragma unroll
-      for (int i = 0; i < 4; ++i) raw[u][i] = make_double2(0.0, 0.0);
-      if (r0 + row < H) {
-        const double2* src = reinterpret_cast<const double2*>(xh + (b * H + r0 + row) * HC + 4 + kb * 8);
-#pragma unroll
-        for (int i = 0; i < 4; ++i) raw[u][i] = __ldg(src + i);
-      }
-    }
-#pragma unroll
-    for (int u = 0; u < ITERS; ++u) {
-      int row, kb; stage_item(threadIdx.x + u * TC_THREADS, row, kb);
-      float v[8];
-#pragma unroll
-      for (int i = 0; i < 4; ++i) { v[2 * i] = (float)raw[u][i].x; v[2 * i + 1] = (float)raw[u][i].y; }
-      umma::store_operand8<NP>(tile, umma::tile64_offset(row, kb), umma::TILE64_BYTES, v);
-    }
-  }
-}
-
-// W_c[j][k] = Wd[j][k] * t[k] + A[j][k] -> K-major tile(s) (rows = j).  wda = Wd | A in shared memory (operand-build
-// order, see wda_index); t = the candidate vector in shared memory.
-// Both items of a pair in one pass: the Wd / A vectors are read once and combined with the two candidate vectors
-// (tt = [t of item 0 | tp | t of item 1 | tp], 128 floats per item).
-template <int NP>
-__device__ __forceinline__ void build_Wc_pair(const float* wda, const float* tt, int nimp, unsigned char* tile0, unsigned char* tile1) {
-#pragma unroll 2
-  for (int it = threadIdx.x; it < 64 * 8; it += TC_THREADS) {
-    const int j = it & 63, kb = it >> 6;
-    const float4 d0 = *reinterpret_cast<const float4*>(wda + DER_WD + ((kb * 2 + 0) * 64 + j) * 4);
-    const float4 d1 = *reinterpret_cast<const float4*>(wda + DER_WD + ((kb * 2 + 1) * 64 + j) * 4);
-    const float4 a0 = *reinterpret_cast<const float4*>(wda + DER_A + ((kb * 2 + 0) * 64 + j) * 4);
-    const float4 a1 = *reinterpret_cast<const float4*>(wda + DER_A + ((kb * 2 + 1) * 64 + j) * 4);
-    const uint32_t off = umma::tile64_offset(j, kb);
-    {
-      const float4 t0 = *reinterpret_cast<const float4*>(tt + kb * 8), t1 = *reinterpret_cast<const float4*>(tt + kb * 8 + 4);
-      float v[8];
-      v[0] = fmaf(d0.x, t0.x, a0.x); v[1] = fmaf(d0.y, t0.y, a0.y); v[2] = fmaf(d0.z, t0.z, a0.z); v[3] = fmaf(d0.w, t0.w, a0.w);
-      v[4] = fmaf(d1.x, t1.x, a1.x); v[5] = fmaf(d1.y, t1.y, a1.y); v[6] = fmaf(d1.z, t1.z, a1.z); v[7] = fmaf(d1.w, t1.w, a1.w);
-      umma::store_operand8<NP>(tile0, off, umma::TILE64_BYTES, v);
-    }
-    if (nimp == 2) {
-      const float4 t0 = *reinterpret_cast<const float4*>(tt + 128 + kb * 8), t1 = *reinterpret_cast<const float4*>(tt + 128 + kb * 8 + 4);
-      float v[8];
-      v[0] = fmaf(d0.x, t0.x, a0.x); v[1] = fmaf(d0.y, t0.y, a0.y); v[2] = fmaf(d0.z, t0.z, a0.z); v[3] = fmaf(d0.w, t0.w, a0.w);
-      v[4] = fmaf(d1.x, t1.x, a1.x); v[5] = fmaf(d1.y, t1.y, a1.y); v[6] = fmaf(d1.z, t1.z, a1.z); v[7] = fmaf(d1.w, t1.w, a1.w);
-      umma::store_operand8<NP>(tile1, off, umma::TILE64_BYTES, v);
-    }
-  }
-}
-
-// Candidate vector t and tp = Bm t + b1 of the two items of a pair: thread (q = tid / 64, i = tid % 64) moves t_q[i] and
-// tp_q[i].  Loaded one pair ahead into registers, parked in shared memory as tt[q][0:64] = t, tt[q][64:128] = tp.
-struct PairVec { float t, tp; };
-__device__ __forceinline__ PairVec load_pair_vec(const float* __restrict__ e, const float* __restrict__ tp, long long b0, int C,
-                                                 int c, int toff, int nimp) {
-  const int q = threadIdx.x >> 6, i = threadIdx.x & 63;
-  PairVec v{0.f, 0.f};
-  if (q < nimp) {       // q >= 2 for threads >= 128
-    const long long rc = (b0 + q) * C + c;
-    v.t = __ldg(e + rc * E + toff + i);
-    v.tp = __ldg(tp + rc * 64 + i);
-  }
-  return v;
-}
-__device__ __forceinline__ void park_pair_vec(float* tt, const PairVec v) {
-  const int q = threadIdx.x >> 6, i = threadIdx.x & 63;
-  if (q >= 2) return;
-  tt[q * 128 + i] = v.t;
-  tt[q * 128 + 64 + i] = v.tp;
-}
-
-__device__ __forceinline__ void st_bf16(unsigned char* p, float v) {
-  *reinterpret_cast<__nv_bfloat16*>(p) = __float2bfloat16_rn(v);
-}
-// one element of an operand tile (hi, and lo when NP == 2)
-template <int NP>
-__device__ __forceinline__ void store_operand1(unsigned char* tile, uint32_t off, uint32_t part_bytes, float v) {
-  const __nv_bfloat16 h = __float2bfloat16_rn(v);
-  *reinterpret_cast<__nv_bfloat16*>(tile + off) = h;
-  if (NP == 2) *reinterpret_cast<__nv_bfloat16*>(tile + part_bytes + off) = __float2bfloat16_rn(v - __bfloat162float(h));
-}
-
-// Work units = (impression pair, candidate), dealt to the CTAs as contiguous, equally long ranges so that the
-// last wave is as full as the first; `whole_pairs` keeps a pair's candidates together (needed when its outputs
-// are accumulated over candidates or history tiles inside one CTA).
-__device__ __forceinline__ void unit_range(int npairs, int C, bool whole_pairs, int& u0, int& u1) {
-  if (whole_pairs) {
-    u0 = (int)((long long)npairs * blockIdx.x / gridDim.x) * C;
-    u1 = (int)((long long)npairs * (blockIdx.x + 1) / gridDim.x) * C;
-  } else {
-    const long long U = (long long)npairs * C;
-    u0 = (int)(U * blockIdx.x / gridDim.x);
-    u1 = (int)(U * (blockIdx.x + 1) / gridDim.x);
-  }
-}
-
-// =====================================================================================================
-// forward
-// =====================================================================================================
-template <int NP>
-struct TcSmemFwd {
-  __align__(128) unsigned char opA[2][TileBytes<NP>::T64];   // history tiles, one per impression of the pair
-  __align__(128) unsigned char opB[2][TileBytes<NP>::T64];   // W_c of the two items of a candidate pair
-  __align__(128) unsigned char opS[2][2 * TileBytes<NP>::T8];   // partial scores [c + 8 column-half][h] per impression (B operand of the pooling product)
-  __align__(16) float wda[8192];                             // Wd | A, operand-build order
-  __align__(16) float tt[2][2 * 128];                        // [buffer][item q][t 64 | tp 64]
-  float w2[64];
-  uint64_t mbar;
-  uint64_t wbar;                                             // bulk copy of the derived weights has landed
-  uint32_t tmem_base;
-};
-
-// TMEM columns: [0,64) hid of the current pair, [64,80) pooled^T partials (N = 16: candidate c of column half 0 | 1)
-constexpr uint32_t FWD_TMEM_COLS = 128, FWD_COL_HID = 0, FWD_COL_POOL = 64;
-
-template <int BRANCH, int SPLIT>
-__device__ __forceinline__ void attention_forward_tc_body(const double* __restrict__ xh, const float* __restrict__ xhp, int B, int H, int C,
-                                                          const float* __restrict__ der_all, const float* __restrict__ tp_all,
-                                                          float* __restrict__ e) {
-  constexpr int NP = SPLIT == 3 ? 2 : 1;
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  TcSmemFwd<NP>& sm = *reinterpret_cast<TcSmemFwd<NP>*>(smem_raw);
-  constexpr int TOFF = BRANCH == 0 ? E_XT : E_PCAT;
-  constexpr int POFF = BRANCH == 0 ? E_LAB : E_TI;
-  constexpr uint32_t IDESC_HID = umma::make_idesc_bf16(64, 64);
-  constexpr uint32_t IDESC_POOL = umma::make_idesc_bf16(64, 16, true, false);
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const float* der = der_all + (long long)BRANCH * DER_SIZE;
-
-  const float* tpg = tp_all + (long long)BRANCH * B * C * 64;
-  if (tid < 64) sm.w2[tid] = __ldg(der + DER_W2 + tid);
-  if (tid == 0) {                                      // Wd | A (32 KB): one bulk copy by the TMA engine, under the rest of the prologue
-    umma::mbar_init(&sm.mbar, 1);
-    umma::mbar_init(&sm.wbar, 1);
-    umma::bulk_load(sm.wda, der, 8192 * sizeof(float), &sm.wbar);
-  }
-  const float b2 = __ldg(der + DER_B2);
-  if (warp == 0) umma::tmem_alloc(&sm.tmem_base, FWD_TMEM_COLS);
-  umma::fence_before_sync();
-  __syncthreads();
-  umma::fence_after_sync();
-  umma::mbar_wait(&sm.wbar, 0);
-  const uint32_t tmem = sm.tmem_base;
-  uint32_t phase = 0;
-
-  // epilogue role: sub-partition = warp & 3, column half = warp >> 2, half-lanes = impression 0 / 1 of the pair
-  const int sp = warp & 3, ch = warp >> 2;
-  const int half = lane >> 4, row = sp * 16 + (lane & 15);
-  const uint32_t my_tmem = tmem + ((uint32_t)(sp * 32) << 16);
-
-  const int npairs_b = (B + 1) / 2;
-  int u0, u1;
-  TCPROF_DECL
-  // a (pair, candidate) unit accumulates its own pooled vector over the history tiles, so a pair's candidates may be
-  // dealt to several CTAs (each re-stages the pair's history tiles): long candidate lists fill the machine even with few pairs
-  unit_range(npairs_b, C, false, u0, u1);
-  for (int u = u0; u < u1;) {
-    const int pb = u / C, ca = u - pb * C, cend = min(C, ca + (u1 - u));   // candidates [ca, cend) of pair pb
-    u += cend - ca;
-    const long long b0 = 2LL * pb;
-    const int nimp = (b0 + 1 < B) ? 2 : 1;
-    for (int r0 = 0; r0 < H; r0 += 64) {
-      for (int c0 = ca; c0 < cend; c0 += TC_MAXC) {
-        const int nc = min(TC_MAXC, cend - c0);
-        if (c0 == ca) {
-          __syncthreads();                              // previous tile's products have completed (waited below)
-          TCPROF(0);
-          for (int imp = 0; imp < nimp; ++imp) stage_history<BRANCH, NP>(xh, xhp, b0 + imp, H, r0, sm.opA[imp]);
-          TCPROF(1);
-        }
-        park_pair_vec(sm.tt[0], load_pair_vec(e, tpg, b0, C, c0, TOFF, nimp));
-        __syncthreads();
-        TCPROF(2);
-        for (int c = 0; c < nc; ++c) {
-          const float* tt = sm.tt[c & 1];
-          PairVec nxt{0.f, 0.f};
-          if (c + 1 < nc) nxt = load_pair_vec(e, tpg, b0, C, c0 + c + 1, TOFF, nimp);     // one pair ahead
-          build_Wc_pair<NP>(sm.wda, tt, nimp, sm.opB[0], sm.opB[1]);
-          TCPROF(3);
-          umma::fence_async_smem();
-          umma::fence_before_sync();
-          __syncthreads();
-          TCPROF(4);
-          if (warp == 0 && umma::elect_one()) {
-            umma::fence_after_sync();
-            for (int q = 0; q < nimp; ++q)
-              umma::mma_product<SPLIT, 4>(tmem + FWD_COL_HID + ((uint32_t)(16 * q) << 16), umma::op_tile64_k(umma::smem_u32(sm.opA[q])),
-                                          umma::op_tile64_k(umma::smem_u32(sm.opB[q])), IDESC_HID, false);
-            umma::mma_commit(&sm.mbar);
-          }
-          TCPROF(5);
-          umma::mbar_wait(&sm.mbar, phase);
-          phase ^= 1;
-          umma::fence_after_sync();
-          TCPROF(6);
-          {
-            // this thread's 32 of the 64 hidden units; the two column halves become two rows (c, c + 8) of the score tile,
-            // and the pooling product, being linear in the scores, adds them
-            float acc = ch == 0 ? b2 : 0.f;
-            float v[32];
-            umma::tmem_ld32(my_tmem + FWD_COL_HID + ch * 32, v);       // all lanes take part (.sync.aligned)
-            if (half < nimp) {
-              const float* tp = tt + half * 128 + 64 + ch * 32;
-#pragma unroll
-              for (int j = 0; j < 32; ++j) acc = fmaf(gelu_f(v[j] + tp[j]), sm.w2[ch * 32 + j], acc);
-              store_operand1<NP>(sm.opS[half], (uint32_t)(row >> 3) * T16_LBO + (uint32_t)ch * 128 + (uint32_t)c * 16 + (uint32_t)(row & 7) * 2,
-                                 2 * T8_BYTES, acc);
-            }
-          }
-          TCPROF(7);
-          if (c + 1 < nc) park_pair_vec(sm.tt[(c + 1) & 1], nxt);
-          umma::fence_async_smem();
-          umma::fence_before_sync();
-          __syncthreads();                                    // TMEM hid, opB and tp free for the next pair; opS visible
-        }
-        TCPROF(8);
-        // pooled^T[k][c] = sum_h H[h][k] s[c][h]  for both impressions (columns c >= nc are never read)
-        if (warp == 0 && umma::elect_one()) {
-          umma::fence_after_sync();
-          for (int q = 0; q < nimp; ++q)
-            umma::mma_product<SPLIT, 4>(tmem + FWD_COL_POOL + ((uint32_t)(16 * q) << 16), umma::op_tile64_mn(umma::smem_u32(sm.opA[q])),
-                                        op_tile16_k(umma::smem_u32(sm.opS[q])), IDESC_POOL, false);
-          umma::mma_commit(&sm.mbar);
-        }
-        umma::mbar_wait(&sm.mbar, phase);
-        phase ^= 1;
-        umma::fence_after_sync();
-        if (ch == 0) {
-          float v[16];
-          umma::tmem_ld16(my_tmem + FWD_COL_POOL, v);
-          if (half < nimp) {
-            float* dst = e + ((b0 + half) * C + c0) * E + POFF + row;     // here `row` is the feature index k
-#pragma unroll
-            for (int c = 0; c < TC_MAXC; ++c)
-              if (c < nc) { const float p = v[c] + v[c + 8]; if (r0 == 0) dst[(long long)c * E] = p; else dst[(long long)c * E] += p; }
-          }
-        }
-        umma::fence_before_sync();
-        TCPROF(9);
-      }
-    }
-  }
-  __syncthreads();
-  if (warp == 0) umma::tmem_dealloc(tmem, FWD_TMEM_COLS);
-}
-
-// Both branches in ONE launch (blockIdx.y = branch: 0 label features, 1 text/img PCA): the CTAs of the second branch start
-// as soon as CTAs of the first retire, so the machine sees one ramp-up and one tail instead of two.
-template <int SPLIT>
-__global__ void __launch_bounds__(TC_THREADS, 2)
-attention_forward_tc_kernel(const double* __restrict__ xh, const float* __restrict__ xhp, int B, int H, int C,
-                            const float* __restrict__ der_all, const float* __restrict__ tp_all, float* __restrict__ e) {
-  pdl_wait();                                          // programmatic dependent launch: see nrm_common.cuh
-  pdl_trigger();
-  if (blockIdx.y == 0) attention_forward_tc_body<0, SPLIT>(xh, xhp, B, H, C, der_all, tp_all, e);
-  else attention_forward_tc_body<1, SPLIT>(xh, xhp, B, H, C, der_all, tp_all, e);
-}
-
-// =====================================================================================================
-// backward
-// =====================================================================================================
-// NBD = 2: separate W_c and dhid tiles (label branch: dH = dhid W_c needs both at once);
-// NBD = 1: dhid overwrites W_c once hid has been read (text/img branch: no input gradients)
-template <int NP, int NBD>
-struct TcSmemBwd {
-  __align__(128) unsigned char opA[2][TileBytes<NP>::T64];   // history tiles [h][k]
-  __align__(128) unsigned char opBD[NBD][2][TileBytes<NP>::T64];   // [0][q]: W_c [j][k] of item q;  [NBD-1][q]: dhid [h][j] of item q
-  __align__(128) unsigned char opW2[2][NBD == 2 ? TileBytes<NP>::T64 : 128];   // label branch: W_c of the odd candidates (software pipeline)
-  __align__(128) unsigned char opP[2][TileBytes<NP>::T8];    // dP [c][k] per impression (B operand of the ds product)
-  __align__(128) unsigned char ones[T8_BYTES];               // [8][64] ones (B operand of the Gt product)
-  float ds[2][TC_MAXC][64];                                  // [impression][candidate][history row]
-  float sc[NBD == 2 ? 2 * 2 * TC_MAXC * 64 : 64];            // partial attention scores [column half][impression][candidate][row] (label branch only)
-  float dtx[2 * 64];                                         // dt partial of column half 1, [impression][k]
-  __align__(16) float dpf[NBD == 2 ? 2 * TC_MAXC * 64 : 4];  // fp32 dP [impression][candidate][k] (pooling path of dH, label branch only)
-  __align__(16) float wda[8192];                             // Wd | A, operand-build order
-  __align__(16) float tt[2][2 * 128];                        // [buffer][item q][t 64 | tp 64]
-  float w2[64];
-  uint64_t mbar;
-  uint64_t mbar_h;                                           // hid products of the pipelined (label) kernel
-  uint64_t wbar;                                             // bulk copy of the derived weights has landed
-  uint32_t tmem_base;
-};
-
-// TMEM columns: [0,64) hid, then Gt in [0,8) (text/img);  [64,128) ds in [64,72), then S^T;  [128,192) dH (label);
-// [192,256) dA^T (text/img), Gt in [192,200) (label)
-constexpr uint32_t BWD_TMEM_COLS = 256, BWD_COL_HID = 0, BWD_COL_S = 64, BWD_COL_DH = 128, BWD_COL_DA = 192;
-// per-CTA partial sums (floats): dA^T [64 k][64 j] | dWd^T [64][64] | dw2 [64] | db2 [1] (+3 pad)
-constexpr int TCP_DA = 0, TCP_DWD = 4096, TCP_DW2 = 2 * 4096, TCP_DB2 = 2 * 4096 + 64, TC_PARTIAL = ATT_TC_PARTIAL;
-
-template <int BRANCH, int SPLIT>
-__global__ void __launch_bounds__(TC_THREADS, BRANCH == 0 ? 1 : 2)
-attention_backward_tc_kernel(const double* __restrict__ xh, const float* __restrict__ xhp, int B, int H, int C,
-                             const float* __restrict__ der_all, const float* __restrict__ tp_all, const float* __restrict__ P,
-                             const float* __restrict__ e, const float* __restrict__ de, float* __restrict__ dxh, float* __restrict__ dxt,
-                             float* __restrict__ dtp, float* __restrict__ part) {
-  pdl_wait();                                          // programmatic dependent launch: see nrm_common.cuh
-  pdl_trigger();
-  constexpr int NP = SPLIT == 3 ? 2 : 1;
-  constexpr bool INPUT_GRADS = (BRANCH == 0);
-  constexpr int NBD = INPUT_GRADS ? 2 : 1, DH = NBD - 1;
-  // dA^T = sum over items of S^T: the label kernel (one CTA per SM, registers to spare) adds the S^T it reads anyway in
-  // registers; the text/img kernel (128 registers per thread) lets the tensor core accumulate it in TMEM with a second product
-  constexpr bool DA_IN_REGS = INPUT_GRADS;
-  // Software pipeline (label kernel: one CTA per SM, nobody else hides its tensor-core latency): while the second group
-  // of products of candidate c (S^T, dH, Gt) runs, the CTA builds W_c of candidate c + 1 in a second buffer and queues its
-  // hid product behind them, so that product runs under epilogue 2 of candidate c.  hid is then only ever read by
-  // epilogue 1, and Gt moves out of its columns into the (unused, dA^T lives in registers) [192, 200).
-  constexpr bool PIPE = INPUT_GRADS;
-  constexpr uint32_t COL_GT = PIPE ? BWD_COL_DA : BWD_COL_HID;
-  static_assert(!PIPE || DA_IN_REGS, "the pipelined kernel parks Gt in the dA^T columns");
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  TcSmemBwd<NP, NBD>& sm = *reinterpret_cast<TcSmemBwd<NP, NBD>*>(smem_raw);
-  constexpr AttOffsets off = BRANCH == 0 ? ATT_LABEL : ATT_TI;
-  constexpr int TOFF = BRANCH == 0 ? E_XT : E_PCAT;
-  constexpr int POFF = BRANCH == 0 ? E_LAB : E_TI;
-  constexpr uint32_t IDESC_HID = umma::make_idesc_bf16(64, 64);               // H W_c^T
-  constexpr uint32_t IDESC_DS = umma::make_idesc_bf16(64, 8);                 // H dP^T
-  constexpr uint32_t IDESC_ST = umma::make_idesc_bf16(64, 64, true, true);    // H^T dhid
-  constexpr uint32_t IDESC_DH = umma::make_idesc_bf16(64, 64, false, true);   // dhid W_c
-  constexpr uint32_t IDESC_GT = umma::make_idesc_bf16(64, 8, true, false);    // dhid^T ones
-#ifdef NRM_TC_PROFILE_BWD
-#ifndef PROF_BRANCH
-#define PROF_BRANCH 0
-#endif
-  TCPROF_DECL
-#define BPROF(i) do { if (BRANCH == PROF_BRANCH) TCPROF(i); } while (0)
-#else
-#define BPROF(i) do { } while (0)
-#endif
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const float* der = der_all + (long long)BRANCH * DER_SIZE;
-  const float* Wd_rm = P + off.fc1_w + 192;            // Wd[j][k] = fc1.weight[j][192 + k]
-
-  const float* tpg = tp_all + (long long)BRANCH * B * C * 64;
-  if (tid < 64) sm.w2[tid] = __ldg(der + DER_W2 + tid);
-  if (tid == 0) {                                      // Wd | A (32 KB): one bulk copy by the TMA engine, under the rest of the prologue
-    umma::mbar_init(&sm.mbar, 1); umma::mbar_init(&sm.mbar_h, 1);
-    umma::mbar_init(&sm.wbar, 1);
-    umma::bulk_load(sm.wda, der, 8192 * sizeof(float), &sm.wbar);
-  }
-  for (int i = tid; i < (int)T8_BYTES / 2; i += TC_THREADS) reinterpret_cast<__nv_bfloat16*>(sm.ones)[i] = __float2bfloat16_rn(1.0f);
-  const float b2 = __ldg(der + DER_B2);
-  if (warp == 0) umma::tmem_alloc(&sm.tmem_base, BWD_TMEM_COLS);
-  umma::fence_async_smem();
-  umma::fence_before_sync();
-  __syncthreads();
-  umma::fence_after_sync();
-  umma::mbar_wait(&sm.wbar, 0);
-  const uint32_t tmem = sm.tmem_base;
-  uint32_t phase = 0, phase_h = 0;
-
-  // thread = (column half ch, TMEM sub-partition sp, impression half, row): every epilogue handles the 32 accumulator
-  // columns [32 ch, 32 ch + 32) of its row
-  const int sp = warp & 3, ch = warp >> 2;
-  const int half = lane >> 4, row = sp * 16 + (lane & 15);
-  const uint32_t my_tmem = tmem + ((uint32_t)(sp * 32) << 16);
-  const uint32_t half_off[2] = {0u, 16u << 16};
-  const int cb = ch;                                   // column block of this thread
-
-  // persistent per-thread accumulators
-  float dw2_acc[32];       // thread (ch, half, history row): sum over items of ds * gelu(hid[row][32 ch + j])
-  float dwd_acc[32];       // thread (ch, half, k):           sum over items of t[k] * S^T[k][32 ch + j]
-  float da_acc[DA_IN_REGS ? 32 : 1];   // thread (ch, half, k): sum over items of S^T[k][32 ch + j]
-#pragma unroll
-  for (int j = 0; j < 32; ++j) { dw2_acc[j] = 0.f; dwd_acc[j] = 0.f; if (DA_IN_REGS) da_acc[j] = 0.f; }
-  bool da_started[2] = {false, false};
-  float db2_acc = 0.f;
-
-  const int npairs_b = (B + 1) / 2;
-  int u0, u1;
-  // A pair's candidates may be split between two CTAs unless its outputs are accumulated in global memory over
-  // history tiles or candidate chunks.  With the label branch a split pair has exactly two contributors to dxh
-  // (ranges are at least C units long), each adding its finished partial sum once to a zeroed destination:
-  // 0 + a + b == 0 + b + a bit for bit, so the result does not depend on which CTA gets there first.
-  unit_range(npairs_b, C, H > 64 || (INPUT_GRADS && C > TC_MAXC), u0, u1);
-  BPROF(9);
-  for (int u = u0; u < u1;) {
-    const int pb = u / C, ca = u - pb * C, cend = min(C, ca + (u1 - u));   // candidates [ca, cend) of pair pb
-    u += cend - ca;
-    const bool split_pair = (ca > 0 || cend < C);
-    const bool single_chunk = (cend - ca <= TC_MAXC);
-    const long long b0 = 2LL * pb;
-    const int nimp = (b0 + 1 < B) ? 2 : 1;
-    const bool act = half < nimp;
-    const long long bmine = b0 + half;                 // this thread's impression (valid when act)
-    for (int r0 = 0; r0 < H; r0 += 64) {
-      __syncthreads();                                 // every product of the previous tile has completed
-      BPROF(0);
-      for (int imp = 0; imp < nimp; ++imp) stage_history<BRANCH, NP>(xh, xhp, b0 + imp, H, r0, sm.opA[imp]);
-      BPROF(1);
-      bool dh_started = false;
-      for (int c0 = ca; c0 < cend; c0 += TC_MAXC) {
-        const int nc = min(TC_MAXC, cend - c0);
-        // ---- ds[c][h] = sum_k dP_c[k] H[h][k] for the chunk's candidates of both impressions
-        for (int i = tid; i < nimp * TC_MAXC * 8; i += TC_THREADS) {
-          const int imp = i / (TC_MAXC * 8), c = (i / 8) % TC_MAXC, kb = i & 7;
-          float v[8];
-          if (c < nc) {
-            const float4* src = reinterpret_cast<const float4*>(de + ((b0 + imp) * C + c0 + c) * E + POFF + kb * 8);
-            const float4 a = __ldg(src), bq = __ldg(src + 1);
-            v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = bq.x; v[5] = bq.y; v[6] = bq.z; v[7] = bq.w;
-          } else {
-#pragma unroll
-            for (int q = 0; q < 8; ++q) v[q] = 0.f;
-          }
-          umma::store_operand8<NP>(sm.opP[imp], (uint32_t)kb * T8_LBO + (uint32_t)c * 16, T8_BYTES, v);
-          if (INPUT_GRADS) {
-            float4* dpd = reinterpret_cast<float4*>(sm.dpf + (imp * TC_MAXC + c) * 64 + kb * 8);
-            dpd[0] = make_float4(v[0], v[1], v[2], v[3]); dpd[1] = make_float4(v[4], v[5], v[6], v[7]);
-          }
-        }
-        umma::fence_async_smem();
-        umma::fence_before_sync();
-        __syncthreads();
-        if (warp == 0 && umma::elect_one()) {
-          umma::fence_after_sync();
-          for (int q = 0; q < nimp; ++q)
-            umma::mma_product<SPLIT, 4>(tmem + BWD_COL_S + half_off[q], umma::op_tile64_k(umma::smem_u32(sm.opA[q])),
-                                        op_tile8_k(umma::smem_u32(sm.opP[q])), IDESC_DS, false);
-          umma::mma_commit(&sm.mbar);
-        }
-        umma::mbar_wait(&sm.mbar, phase);
-        phase ^= 1;
-        umma::fence_after_sync();
-        if (ch == 0) {
-          float v[8];
-          umma::tmem_ld8(my_tmem + BWD_COL_S, v);
-          if (act) {
-#pragma unroll
-            for (int c = 0; c < TC_MAXC; ++c) sm.ds[half][c][row] = v[c];
-          }
-        }
-        umma::fence_before_sync();
-
-        park_pair_vec(sm.tt[0], load_pair_vec(e, tpg, b0, C, c0, TOFF, nimp));
-        __syncthreads();                                 // ds and the first pair's vectors visible
-        BPROF(2);
-        // W_c tiles of candidate c: the pipelined kernel alternates between two buffers
-        auto wc_tile = [&](int c, int q) -> unsigned char* { return (PIPE && (c & 1)) ? sm.opW2[q] : sm.opBD[0][q]; };
-        auto issue_hid = [&](int c, uint64_t* bar) {
-          if (warp == 0 && umma::elect_one()) {
-            umma::fence_after_sync();
-            for (int q = 0; q < nimp; ++q)
-              umma::mma_product<SPLIT, 4>(tmem + BWD_COL_HID + half_off[q], umma::op_tile64_k(umma::smem_u32(sm.opA[q])),
-                                          umma::op_tile64_k(umma::smem_u32(wc_tile(c, q))), IDESC_HID, false);
-            umma::mma_commit(bar);
-          }
-        };
-        if (PIPE) {                                        // prologue: hid product of the chunk's first candidate
-          build_Wc_pair<NP>(sm.wda, sm.tt[0], nimp, wc_tile(0, 0), wc_tile(0, 1));
-          umma::fence_async_smem();
-          umma::fence_before_sync();
-          __syncthreads();
-          issue_hid(0, &sm.mbar_h);
-        }
-        for (int c = 0; c < nc; ++c) {
-          const long long rcm = bmine * C + c0 + c;
-          const float* tt = sm.tt[c & 1];
-          PairVec nxt{0.f, 0.f};
-          if (c + 1 < nc) nxt = load_pair_vec(e, tpg, b0, C, c0 + c + 1, TOFF, nimp);     // one pair ahead
-          if (!PIPE) {
-            build_Wc_pair<NP>(sm.wda, tt, nimp, sm.opBD[0][0], sm.opBD[0][1]);
-            BPROF(3);
-            umma::fence_async_smem();
-            umma::fence_before_sync();
-            __syncthreads();                               // (1) operands visible; previous S^T / Gt reads done
-            issue_hid(c, &sm.mbar);
-            umma::mbar_wait(&sm.mbar, phase);
-            phase ^= 1;
-          } else {
-            umma::mbar_wait(&sm.mbar_h, phase_h);          // issued one candidate ago, ran under epilogue 2
-            phase_h ^= 1;
-          }
-          umma::fence_after_sync();
-          BPROF(4);
-          // ---- epilogue 1: thread = (column half, impression half, history row)
-          {
-            const float dsr = act ? sm.ds[half][c][row] : 0.f;
-            float sacc = (ch == 0) ? b2 : 0.f;
-            float v[32];
-            umma::tmem_ld32(my_tmem + BWD_COL_HID + cb * 32, v);
-            if (act) {
-              const float* tp = tt + half * 128 + 64 + cb * 32;
-              // packed pairs (fma.rn.f32x2): the epilogue is bound by issue slots
-              const f32x2 ds2 = pk(dsr, dsr);
-              f32x2 sacc2 = pk(0.f, 0.f);
-#pragma unroll
-              for (int j8 = 0; j8 < 4; ++j8) {
-                float dh[8];
-#pragma unroll
-                for (int jj = 0; jj < 8; jj += 2) {
-                  const int j = j8 * 8 + jj;
-                  const float2 tpp = *reinterpret_cast<const float2*>(tp + j);
-                  const float2 wp = *reinterpret_cast<const float2*>(&sm.w2[cb * 32 + j]);
-                  f32x2 g, gp;
-                  gelu_both2(add2(pk(v[j], v[j + 1]), pk(tpp.x, tpp.y)), g, gp);
-                  const f32x2 w = pk(wp.x, wp.y);
-                  if (INPUT_GRADS) sacc2 = fma2(g, w, sacc2);
-                  upk(fma2(ds2, g, pk(dw2_acc[j], dw2_acc[j + 1])), dw2_acc[j], dw2_acc[j + 1]);
-                  upk(mul2(mul2(ds2, w), gp), dh[jj], dh[jj + 1]);
-                }
-                umma::store_operand8<NP>(sm.opBD[DH][half], umma::tile64_offset(row, cb * 4 + j8), umma::TILE64_BYTES, dh);
-              }
-              if (INPUT_GRADS) { float s0, s1; upk(sacc2, s0, s1); sacc += s0 + s1; }
-              if (ch == 0) db2_acc += dsr;
-              if (INPUT_GRADS) sm.sc[((ch * 2 + half) * TC_MAXC + c) * 64 + row] = sacc;
-            }
-          }
-          BPROF(5);
-          if (c + 1 < nc) park_pair_vec(sm.tt[(c + 1) & 1], nxt);
-          umma::fence_async_smem();
-          umma::fence_before_sync();
-          __syncthreads();                               // (2) dhid tiles visible; hid columns free
-          if (warp == 0 && umma::elect_one()) {
-            umma::fence_after_sync();
-            for (int q = 0; q < nimp; ++q) {
-              const umma::Operand h_mn = umma::op_tile64_mn(umma::smem_u32(sm.opA[q]));
-              const umma::Operand d_mn = umma::op_tile64_mn(umma::smem_u32(sm.opBD[DH][q]));
-              const umma::Operand d_k = umma::op_tile64_k(umma::smem_u32(sm.opBD[DH][q]));
-              const umma::Operand w_mn = umma::op_tile64_mn(umma::smem_u32(wc_tile(c, q)));
-              umma::mma_product<SPLIT, 4>(tmem + BWD_COL_S + half_off[q], h_mn, d_mn, IDESC_ST, false);
-              if (!DA_IN_REGS) umma::mma_product<SPLIT, 4>(tmem + BWD_COL_DA + half_off[q], h_mn, d_mn, IDESC_ST, da_started[q]);
-              if (INPUT_GRADS) umma::mma_product<SPLIT, 4>(tmem + BWD_COL_DH + half_off[q], d_k, w_mn, IDESC_DH, dh_started);
-              // Gt: ones is exact in bf16, so only the (hi, hi) and (lo, hi) terms exist
-              {
-                const umma::Operand one = op_tile8_k(umma::smem_u32(sm.ones));
-#pragma unroll
-                for (int t = 0; t < NP; ++t)
-#pragma unroll
-                  for (int ks = 0; ks < 4; ++ks)
-                    umma::mma_bf16(tmem + COL_GT + half_off[q], d_mn.desc + (uint64_t)(t * d_mn.part16 + ks * d_mn.kstep16),
-                                   one.desc + (uint64_t)(ks * one.kstep16), IDESC_GT, (t > 0 || ks > 0) ? 1u : 0u);
-              }
-            }
-            umma::mma_commit(&sm.mbar);
-          }
-          dh_started = true;
-          for (int q = 0; q < nimp; ++q) da_started[q] = true;
-          if (PIPE && c + 1 < nc) {
-            // under the products just issued: W_c of the next candidate into the other buffer, its hid product queued
-            build_Wc_pair<NP>(sm.wda, sm.tt[(c + 1) & 1], nimp, wc_tile(c + 1, 0), wc_tile(c + 1, 1));
-            BPROF(3);
-            umma::fence_async_smem();
-            umma::fence_before_sync();
-            __syncthreads();
-            issue_hid(c + 1, &sm.mbar_h);
-          }
-          umma::mbar_wait(&sm.mbar, phase);
-          phase ^= 1;
-          umma::fence_after_sync();
-          BPROF(6);
-          // ---- epilogue 2: thread = (column half, impression half, feature k = row) for S^T, (half, j = row) for Gt
-          {
-            const float tk = act ? tt[half * 128 + row] : 0.f;
-            float dt = 0.f;
-            float v[32];
-            umma::tmem_ld32(my_tmem + BWD_COL_S + cb * 32, v);
-            if (act) {
-              const f32x2 tk2 = pk(tk, tk);
-#pragma unroll
-              for (int j = 0; j < 32; j += 2) {
-                const f32x2 v2 = pk(v[j], v[j + 1]);
-                upk(fma2(tk2, v2, pk(dwd_acc[j], dwd_acc[j + 1])), dwd_acc[j], dwd_acc[j + 1]);
-                if (DA_IN_REGS) upk(add2(pk(da_acc[j], da_acc[j + 1]), v2), da_acc[j], da_acc[j + 1]);
-                if (INPUT_GRADS) {
-                  dt = fmaf(v[j], __ldg(Wd_rm + (cb * 32 + j) * 256 + row), dt);
-                  dt = fmaf(v[j + 1], __ldg(Wd_rm + (cb * 32 + j + 1) * 256 + row), dt);
-                }
-              }
-            }
-            if (INPUT_GRADS) {
-              // dt[k] = sum over both column halves: half 1 parks its share, half 0 adds it and writes
-              if (ch == 1 && act) sm.dtx[half * 64 + row] = dt;
-              umma::fence_before_sync();
-              __syncthreads();
-              if (ch == 0 && act) {
-                dt += sm.dtx[half * 64 + row];
-                float* dst = dxt + rcm * 64 + row;
-                if (r0 == 0) *dst = dt + __ldg(de + rcm * E + E_XT + row);   // + the direct ec path (user_model.py:31)
-                else *dst += dt;
-              }
-            }
-            if (ch == 0) {
-              const float gt = umma::tmem_ld1(my_tmem + COL_GT);
-              if (act) {
-                float* gdst = dtp + rcm * 64 + row;
-                if (r0 == 0) *gdst = gt; else *gdst += gt;
-              }
-            }
-          }
-          umma::fence_before_sync();
-          BPROF(7);
-        }
-        __syncthreads();                                 // ds / opP of this chunk consumed before the next chunk rewrites them
-        if (INPUT_GRADS && !single_chunk) {
-          // several candidate chunks (whole pair in this CTA): the pooling path dxh[row][k] (+)= sum_c s_c[row] dP_c[k]
-          // of each chunk is accumulated in global memory (each thread owns 32 columns of its row)
-          if (act && r0 + row < H) {
-            float* dst = dxh + (bmine * H + r0 + row) * 64 + cb * 32;
-            for (int k4 = 0; k4 < 8; ++k4) {
-              float4 acc = (c0 == ca) ? make_float4(0.f, 0.f, 0.f, 0.f) : *reinterpret_cast<float4*>(dst + 4 * k4);
-              for (int c = 0; c < nc; ++c) {
-                const float s = sm.sc[((0 * 2 + half) * TC_MAXC + c) * 64 + row] + sm.sc[((1 * 2 + half) * TC_MAXC + c) * 64 + row];
-                const float4 dp = *reinterpret_cast<const float4*>(sm.dpf + (half * TC_MAXC + c) * 64 + cb * 32 + 4 * k4);
-                acc.x = fmaf(s, dp.x, acc.x); acc.y = fmaf(s, dp.y, acc.y); acc.z = fmaf(s, dp.z, acc.z); acc.w = fmaf(s, dp.w, acc.w);
-              }
-              *reinterpret_cast<float4*>(dst + 4 * k4) = acc;
-            }
-          }
-          __syncthreads();                               // sc consumed before the next chunk's epilogues overwrite it
-        }
-      }
-      if (INPUT_GRADS) {
-        // dH of this tile (W_c path, all candidates of the range) from tensor memory + the pooling path
-        const int ncs = cend - ca;                       // candidates of the single chunk
-        float v[32];
-        umma::tmem_ld32(my_tmem + BWD_COL_DH + cb * 32, v);
-        if (act && r0 + row < H) {
-          float* dstf = dxh + (bmine * H + r0 + row) * 64 + cb * 32;
-          // attention scores of this row (both column halves), once
-          float srow[TC_MAXC];
-#pragma unroll
-          for (int c = 0; c < TC_MAXC; ++c)
-            srow[c] = (single_chunk && c < ncs) ? sm.sc[((0 * 2 + half) * TC_MAXC + c) * 64 + row] + sm.sc[((1 * 2 + half) * TC_MAXC + c) * 64 + row] : 0.f;
-#pragma unroll
-          for (int k4 = 0; k4 < 8; ++k4) {
-            float4 a = make_float4(v[4 * k4], v[4 * k4 + 1], v[4 * k4 + 2], v[4 * k4 + 3]);
-            if (single_chunk) {
-#pragma unroll
-              for (int c = 0; c < TC_MAXC; ++c) {
-                if (c < ncs) {
-                  const float s = srow[c];
-                  const float4 dp = *reinterpret_cast<const float4*>(sm.dpf + (half * TC_MAXC + c) * 64 + cb * 32 + 4 * k4);
-                  a.x = fmaf(s, dp.x, a.x); a.y = fmaf(s, dp.y, a.y); a.z = fmaf(s, dp.z, a.z); a.w = fmaf(s, dp.w, a.w);
-                }
-              }
-            } else {
-              const float4 g = *reinterpret_cast<float4*>(dstf + 4 * k4);
-              a.x += g.x; a.y += g.y; a.z += g.z; a.w += g.w;
-            }
-            if (split_pair) {
-              atomicAdd(dstf + 4 * k4 + 0, a.x); atomicAdd(dstf + 4 * k4 + 1, a.y);
-              atomicAdd(dstf + 4 * k4 + 2, a.z); atomicAdd(dstf + 4 * k4 + 3, a.w);
-            } else {
-              *reinterpret_cast<float4*>(dstf + 4 * k4) = a;
-            }
-          }
-        }
-        umma::fence_before_sync();
-        BPROF(8);
-      }
-    }
-  }
-
-  // ---- per-CTA partial sums -> part[blockIdx.x]
-  __syncthreads();
-  float* out = part + (long long)blockIdx.x * TC_PARTIAL;
-  {
-    // dA^T and dWd^T from registers: thread (ch, half, k); the two impression halves (lanes l and l ^ 16) are
-    // summed in the warp and the lower half writes out[TCP_DA / TCP_DWD + k*64 + 32 ch + j]
-    float v[32];
-    if (!DA_IN_REGS) umma::tmem_ld32(my_tmem + BWD_COL_DA + cb * 32, v);
-#pragma unroll
-    for (int j = 0; j < 32; ++j) {
-      float a = DA_IN_REGS ? da_acc[j] : (da_started[half] ? v[j] : 0.f);
-      a += __shfl_xor_sync(0xffffffffu, a, 16);
-      v[j] = a;
-      float d = dwd_acc[j];
-      d += __shfl_xor_sync(0xffffffffu, d, 16);
-      dwd_acc[j] = d;
-    }
-    if (half == 0) {
-      float4* dst = reinterpret_cast<float4*>(out + TCP_DA + row * 64 + cb * 32);
-      float4* dst2 = reinterpret_cast<float4*>(out + TCP_DWD + row * 64 + cb * 32);
-#pragma unroll
-      for (int k4 = 0; k4 < 8; ++k4) {
-        dst[k4] = make_float4(v[4 * k4], v[4 * k4 + 1], v[4 * k4 + 2], v[4 * k4 + 3]);
-        dst2[k4] = make_float4(dwd_acc[4 * k4], dwd_acc[4 * k4 + 1], dwd_acc[4 * k4 + 2], dwd_acc[4 * k4 + 3]);
-      }
-    }
-  }
-  umma::fence_before_sync();
-  __syncthreads();
-  {
-    // dw2[32 ch + j] = sum over the 128 threads of column half ch: one pass per half through a [128][33] scratch
-    // (the operand buffers are free now; opA and opBD are contiguous)
-    float* red = reinterpret_cast<float*>(sm.opA);
-    using SmemT = TcSmemBwd<NP, NBD>;
-    static_assert(offsetof(SmemT, opBD) == sizeof(sm.opA), "opA / opBD must be contiguous");
-    static_assert(sizeof(sm.opA) + sizeof(sm.opBD) >= 128 * 33 * sizeof(float), "reduce scratch");
-    float* red2 = &sm.ds[0][0][0];                           // db2 partials (128 floats)
-    for (int pass = 0; pass < 2; ++pass) {
-      __syncthreads();
-      if (ch == pass) {
-#pragma unroll
-        for (int j = 0; j < 32; ++j) red[(tid & 127) * 33 + j] = dw2_acc[j];
-        if (pass == 0) red2[tid & 127] = db2_acc;
-      }
-      __syncthreads();
-      if (tid < 32) {
-        float sacc = 0.f;
-        for (int t = 0; t < 128; ++t) sacc += red[t * 33 + tid];
-        out[TCP_DW2 + pass * 32 + tid] = sacc;
-      }
-    }
-    if (tid == 0) {
-      float d = 0.f;
-      for (int t = 0; t < 128; ++t) d += red2[t];
-      out[TCP_DB2] = d;
-    }
-  }
-  __syncthreads();
-  BPROF(10);
-  if (warp == 0) umma::tmem_dealloc(tmem, BWD_TMEM_COLS);
-}
+// per-CTA partial sums of the row-stacked backward (floats, ATT_TC_PARTIAL per CTA): dA^T [64 k][64 j] | dWd^T [64][64] | dw2 [64] | db2 [1]
+constexpr int TCP_DA = 0, TCP_DWD = 4096, TCP_DW2 = 2 * 4096, TCP_DB2 = 2 * 4096 + 64;
 
 // Sum the per-CTA partials (fixed order) and write the attention-MLP gradients that do not depend on tp:
 //   fc1.weight grad blocks: [:, 0:64] = dA, [:, 192:256] = dWd   (the Bm-dependent blocks are completed by
@@ -893,7 +66,7 @@ attention_tc_compose_block(int block, const float* __restrict__ part_all, int np
                            float* __restrict__ dA_all) {
   const int branch = blockIdx.y;
   const AttOffsets off = branch == 0 ? ATT_LABEL : ATT_TI;
-  const float* part = part_all + (long long)branch * ATT_TC_PARTS_MAX * TC_PARTIAL;
+  const float* part = part_all + (long long)branch * ATT_TC_PARTS_MAX * ATT_TC_PARTIAL;
   const int nparts = branch == 0 ? nparts0 : nparts1;
   float* dA_out = dA_all + branch * 4096;
   // block = 64 consecutive (k,j) entries (two per lane) x 32 interleaved groups of partials, combined in group order;
@@ -905,7 +78,7 @@ attention_tc_compose_block(int block, const float* __restrict__ part_all, int np
     float dA0 = 0.f, dWd0 = 0.f, dA1 = 0.f, dWd1 = 0.f;
 #pragma unroll 4
     for (int p = grp; p < nparts; p += 32) {
-      const float* q = part + (long long)p * TC_PARTIAL;
+      const float* q = part + (long long)p * ATT_TC_PARTIAL;
       dA0 += q[TCP_DA + i]; dA1 += q[TCP_DA + i + 32];
       dWd0 += q[TCP_DWD + i]; dWd1 += q[TCP_DWD + i + 32];
     }
@@ -928,7 +101,7 @@ attention_tc_compose_block(int block, const float* __restrict__ part_all, int np
     float w = 0.f;
     if (ent <= 64) {
 #pragma unroll 4
-      for (int p = g8; p < nparts; p += 8) w += part[(long long)p * TC_PARTIAL + (ent < 64 ? TCP_DW2 + ent : TCP_DB2)];
+      for (int p = g8; p < nparts; p += 8) w += part[(long long)p * ATT_TC_PARTIAL + (ent < 64 ? TCP_DW2 + ent : TCP_DB2)];
     }
     r2[g8 * 128 + ent] = w;
     __syncthreads();
@@ -1092,6 +265,8 @@ attention_tp_finish_kernel(const float* __restrict__ part_all, int nparts, const
   }
 }
 
+template <int NP> struct TileBytes { static constexpr uint32_t T64 = NP * umma::TILE64_BYTES; };   // one [64][64] operand tile, all parts
+
 // ---------------------------------------------------------------------------------
 // Self test of the tensor-core building blocks (tests/test_gpu_tensorcore.py): four 64x64x64 products with the
 // interleaved half-lane accumulators:
@@ -1141,7 +316,7 @@ umma_selftest_kernel(const float* __restrict__ a0, const float* __restrict__ a1,
   }
   umma::mbar_wait(mbar, 0);
   umma::fence_after_sync();
-  // warp w reads sub-partition w & 3, column half w >> 2 (as the attention kernels do)
+  // warp w reads sub-partition w & 3, column half w >> 2
   const int half = lane >> 4, row = (warp & 3) * 16 + (lane & 15), cb = warp >> 2;
   {
     float v[32];
@@ -1157,71 +332,11 @@ umma_selftest_kernel(const float* __restrict__ a0, const float* __restrict__ a1,
 // ---------------------------------------------------------------------------------
 // launchers
 // ---------------------------------------------------------------------------------
-// weights only (no dependence on the batch)
-int launch_attention_prep(const float* P, Workspace& w, cudaStream_t s) {
-  launch_pdl(att_prep_kernel, dim3(dim3(4, 2)), dim3(256), 0, s, P, w.att_derived);
-  NRM_LAUNCH_CHECK("att_prep_kernel");
-  return NRM_OK;
-}
 // needs the candidate rows of e written by embed_rows_kernel
 int launch_candidate_tp(const float* P, Workspace& w, cudaStream_t s) {
   launch_pdl(candidate_tp_kernel, dim3(dim3((unsigned)((w.R + 31) / 32), 2)), dim3(256), 0, s, P, w.e, w.R, w.tp);
   NRM_LAUNCH_CHECK("candidate_tp_kernel");
   return NRM_OK;
-}
-
-// Shared memory is requested with some padding so that exactly `per_sm` CTAs fit: tensor memory serves at most
-// 512 columns per SM, and what the CTAs leave of the 228 KB stays L1, which has to hold the 48 KB of derived
-// weights every operand build reads.
-static size_t padded_smem(size_t need, int per_sm) {
-  const size_t floor_bytes = (227 * 1024) / (per_sm + 1) + 1024;     // one more CTA must not fit
-  return need > floor_bytes ? need : floor_bytes;
-}
-
-template <int SPLIT>
-static int launch_fwd_both(const BatchPtrs& in, Workspace& w, cudaStream_t s) {
-  constexpr int NP = SPLIT == 3 ? 2 : 1;
-  const int per_sm = 2;
-  const size_t smem = padded_smem(sizeof(TcSmemFwd<NP>), per_sm);
-  if (smem > 227 * 1024) { set_error("attention forward: shared memory"); return NRM_EUNSUPPORTED; }
-  // one CTA per pair or per candidate chunk of TC_MAXC units, whichever gives more CTAs; never more than fit at once
-  const long long npairs = (w.B + 1) / 2, units = npairs * w.C;
-  const int grid = (int)min(max(npairs, (units + TC_MAXC - 1) / TC_MAXC), (long long)per_sm * sm_count());
-  NRM_CUDA(cudaFuncSetAttribute(attention_forward_tc_kernel<SPLIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  launch_pdl(attention_forward_tc_kernel<SPLIT>, dim3(dim3(grid, 2)), dim3(TC_THREADS), smem, s, in.xh, w.xh, w.B, w.H, w.C, w.att_derived, w.tp, w.e);
-  NRM_LAUNCH_CHECK("attention_forward_tc_kernel");
-  return NRM_OK;
-}
-
-// branch 0 launches both branches; branch 1 is a no-op (kept so that the callers' per-branch sequence stays uniform)
-int launch_attention_forward_tc(const BatchPtrs& in, Workspace& w, int branch, int precision, cudaStream_t s) {
-  if (branch != 0) return NRM_OK;
-  return precision == NRM_PRECISION_BF16 ? launch_fwd_both<1>(in, w, s) : launch_fwd_both<3>(in, w, s);
-}
-
-static int ctas_per_sm(size_t smem, int cap) { return (int)max((size_t)1, min((size_t)cap, (size_t)(227 * 1024) / (smem + 1024))); }
-static int att_tc_bwd_grid(int B, int per_sm) { return min((B + 1) / 2, min(per_sm * sm_count(), ATT_TC_PARTS_MAX)); }
-
-template <int BRANCH, int SPLIT>
-static int launch_bwd(const BatchPtrs& in, const float* P, Workspace& w, cudaStream_t s) {
-  constexpr int NP = SPLIT == 3 ? 2 : 1;
-  constexpr int NBD = BRANCH == 0 ? 2 : 1;
-  const size_t smem = padded_smem(sizeof(TcSmemBwd<NP, NBD>), 2);    // at most two CTAs per SM (2 x 256 tensor-memory columns)
-  if (smem > 227 * 1024) { set_error("attention backward: shared memory"); return NRM_EUNSUPPORTED; }
-  const int grid = att_tc_bwd_grid(w.B, ctas_per_sm(smem, 2));
-  w.att_tc_parts[BRANCH] = grid;
-  if (BRANCH == 0) NRM_CUDA(cudaMemsetAsync(w.dxh, 0, sizeof(float) * (size_t)w.NH * 64, s));   // split pairs add into it
-  float* part = w.att_part + (long long)BRANCH * ATT_TC_PARTS_MAX * TC_PARTIAL;
-  float* dtp = w.dtp + (long long)BRANCH * w.R * 64;
-  NRM_CUDA(cudaFuncSetAttribute(attention_backward_tc_kernel<BRANCH, SPLIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  launch_pdl(attention_backward_tc_kernel<BRANCH, SPLIT>, dim3(grid), dim3(TC_THREADS), smem, s, in.xh, w.xh, w.B, w.H, w.C, w.att_derived, w.tp, P, w.e, w.de, w.dxh, w.dxt, dtp, part);
-  NRM_LAUNCH_CHECK("attention_backward_tc_kernel");
-  return NRM_OK;
-}
-
-int launch_attention_backward_tc(const BatchPtrs& in, const float* P, Workspace& w, int branch, int precision, cudaStream_t s) {
-  if (precision == NRM_PRECISION_BF16) return branch == 0 ? launch_bwd<0, 1>(in, P, w, s) : launch_bwd<1, 1>(in, P, w, s);
-  return branch == 0 ? launch_bwd<0, 3>(in, P, w, s) : launch_bwd<1, 3>(in, P, w, s);
 }
 
 // both branches at once (after both backward kernels)
@@ -1361,18 +476,4 @@ extern "C" int nrm_debug_mma_microbench(long long* out, int variant, int reps, i
   mma_microbench_kernel<<<1, TC_THREADS, smem, (cudaStream_t)stream>>>(out, variant, reps, nk);
   NRM_LAUNCH_CHECK("mma_microbench_kernel");
   return NRM_OK;
-}
-
-extern "C" int nrm_debug_tcprof(long long* host_out32) {
-#ifdef NRM_TC_PROFILE
-  long long zero[32] = {0};
-  NRM_CUDA(cudaDeviceSynchronize());
-  NRM_CUDA(cudaMemcpyFromSymbol(host_out32, nrm::g_tcprof, sizeof(zero)));
-  NRM_CUDA(cudaMemcpyToSymbol(nrm::g_tcprof, zero, sizeof(zero)));
-  return NRM_OK;
-#else
-  (void)host_out32;
-  set_error("nrm_debug_tcprof: library built without -DNRM_TC_PROFILE");
-  return NRM_EUNSUPPORTED;
-#endif
 }

@@ -158,7 +158,7 @@ constexpr int SORT_CHUNK = 2048;       // entries per counting-sort CTA
 constexpr int SEG_GROUP = 128;         // sorted entries per level-1 segment group
 constexpr int ATT_BWD_CTAS_MAX = 148;  // persistent grid of the attention backward
 constexpr int ATT_PARTIAL = 3 * D * D + 64 + 64 + 4;   // dA | dWd | dBm | dw2 | db1 | db2 (+pad) floats per CTA
-constexpr int ATT_TC_PARTS_MAX = 512; // CTAs of the tensor-core attention backward (2 per SM)
+constexpr int ATT_TC_PARTS_MAX = 512; // most CTAs (= partials) of the row-stacked attention backward (one CTA per SM)
 constexpr int ATT_TC_PARTIAL = 2 * 4096 + 68;   // dA^T | dWd^T | dw2 | db2 floats per CTA
 constexpr int HEAD_WG_CHUNKS_MAX = 64; // row chunks of the head weight-gradient kernel
 constexpr int STAT_BLOCKS = 256;       // row chunks of the column-statistics kernels
@@ -187,7 +187,6 @@ struct Workspace {
   float* head_part_f;  // [tiles][68]   out_mlp.fc2 partial gradients per row tile
   double* head_part_bn;// [tiles][2,264] BatchNorm backward partial sums per row tile
   float* head_part_w;  // [5][chunks][66*264+264] weight-gradient partials
-  float* att_derived;  // [2][12420] derived attention weights (tensor-core paths)
   float* tp;           // [2][R,64]  tp = (Wb + Wc) t + b1 per candidate row and branch (tensor-core paths)
   unsigned char* att_dhid;  // label branch, training: dhid tile images (hi | lo) exported by the row-stacked backward for the input-gradient kernel
   float* att_sc;       // label branch, training: partial scores [tiles][4][128]

@@ -1,6 +1,6 @@
-// Scoring head of UserModel (models/user_model.py:31-35), fused -- the FFMA implementation: precision = fp32, and the other
-// precisions with NRM_HEAD_FFMA=1 (their default is the tensor-core head, nrm_head_tc.cu; head_grad_finish_kernel and the
-// transposes below serve both):
+// Scoring head of UserModel (models/user_model.py:31-35), fused -- the FFMA implementation of precision = fp32 (the other
+// precisions run the tensor-core head, nrm_head_tc.cu; head_grad_finish_kernel and the transposes below serve both):
+//
 //     z = BatchNorm(e);  gate = fc2(gelu(fc1(z)));  x = gate * e;  y = fc2(gelu(fc1(x)));  r = fc2(gelu(fc1(y)))
 // Forward: ONE kernel takes a tile of candidate rows through all six layers with the activations in shared
 // memory (the five 264 <-> 66 matrices stream through L2, 350 KB per tile); only what the backward needs

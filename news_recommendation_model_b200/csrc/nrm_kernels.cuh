@@ -29,19 +29,15 @@ int launch_w1_forward(const float* P, Workspace& w, cudaStream_t s);            
 int launch_w1_backward(const float* P, Workspace& w, float* grads, cudaStream_t s);  // w.dxh -> w.dxin_h, w1 gradients
 
 // nrm_w1_tc.cu  (tensor-core tiles; precision = bf16 / bf16x3)
-int launch_w1_forward_tc(const float* P, Workspace& w, int precision, cudaStream_t s);
 int launch_w1_backward_tc(const float* P, Workspace& w, float* grads, int precision, cudaStream_t s);
 
-// nrm_attention.cu  (branch 0 = label attention on w1-projected features, 1 = text/img PCA)
+// nrm_attention.cu  (precision fp32: FFMA kernels; branch 0 = label attention on w1-projected features, 1 = text/img PCA)
 int launch_attention_forward(const BatchPtrs& in, const float* P, Workspace& w, int branch, int precision, cudaStream_t s);
 int launch_attention_backward(const BatchPtrs& in, const float* P, Workspace& w, int branch, int precision, cudaStream_t s);
 int launch_attention_finish(const float* P, Workspace& w, int branch, int precision, float* grads, cudaStream_t s);
 
 // nrm_attention_tc.cu  (precision = bf16 / bf16x3: tcgen05 tensor-core tiles)
-int launch_attention_prep(const float* P, Workspace& w, cudaStream_t s);          // derived weights -> w.att_derived (weights only)
 int launch_candidate_tp(const float* P, Workspace& w, cudaStream_t s);            // per-candidate tp -> w.tp (needs w.e target rows)
-int launch_attention_forward_tc(const BatchPtrs& in, Workspace& w, int branch, int precision, cudaStream_t s);
-int launch_attention_backward_tc(const BatchPtrs& in, const float* P, Workspace& w, int branch, int precision, cudaStream_t s);
 int launch_attention_finish_tc(const float* P, Workspace& w, float* grads, cudaStream_t s);   // both branches
 
 // nrm_attention_rs.cu  (row-stacked M = 128 formulation, operand rows in tensor memory; precision = bf16 / bf16x3)
@@ -54,7 +50,6 @@ int launch_attention_forward_rs_scores(Workspace& w, int precision, cudaStream_t
 int launch_attention_backward_rs(Workspace& w, int branch, int precision, bool export_dhid, cudaStream_t s);
 int launch_attention_input_grad_rs(Workspace& w, int precision, cudaStream_t s);   // label branch: dxh, dxt from the exported tiles
 long long attention_rs_tiles(int B, int H, int C);
-bool use_rowstacked();
 
 // nrm_head_fused.cu
 int launch_head_transpose(const float* P, Workspace& w, cudaStream_t s);          // transposed head matrices -> w.head_wt (weights only)

@@ -1,22 +1,20 @@
-// w1 = nn.Linear(66, 64) over the embedded history rows (models/user_invariant_interest_model.py:33,78) on the tensor cores.
-//   forward   xh[r][j]   = sum_k xin[r][k] W1[j][k] + b1[j]                                   M = rows, N = 64, K = 66 (padded to 80)
-//   backward  dxin[r][k] = sum_j dxh[r][j] W1[j][k]                                           M = rows, N = 80, K = 64
-//             dW1[j][k]  = sum_r dxh[r][j] xin[r][k],   db1[j] = sum_r dxh[r][j]              M = 64,  N = 80, K = rows
+// Backward of w1 = nn.Linear(66, 64) over the embedded history rows (models/user_invariant_interest_model.py:33,78) on the tensor cores.
+//   dxin[r][k] = sum_j dxh[r][j] W1[j][k]                                                     M = rows, N = 80, K = 64
+//   dW1[j][k]  = sum_r dxh[r][j] xin[r][k],   db1[j] = sum_r dxh[r][j]                        M = 64,  N = 80, K = rows
 // NH = B*H rows (51 200 at B = 1024, H = 50; 1 048 576 at B = 4096, H = 256): tall-skinny products whose FFMA versions
 // (nrm_w1.cu) spend 25 / 120 us on 0.4 / 0.9 GFLOP.  Here a CTA walks tiles of 128 rows: its threads turn the fp32 rows into
 // un-swizzled K-major bf16 operand tiles (hi | lo parts, 3 MMAs per product = fp32-grade, as in the attention kernels) and one
 // elected thread issues tcgen05.mma; the weight-gradient product reads the SAME two tiles MN-major (contraction over the rows) and
 // accumulates in tensor memory over all tiles of the CTA; db1 rides along as the product with a column of ones (K padding of xin).
-// Per-CTA partials are summed in CTA order by w1_finish_kernel (deterministic).  Used when precision != fp32.
+// Per-CTA partials are summed in CTA order by w1_finish_kernel (deterministic).  Used when precision != fp32; the forward is
+// nrm_w1.cu's FFMA kernel in every precision.
 #include "nrm_kernels.cuh"
-#include <cstddef>
 
 #include "nrm_umma.cuh"
 
 namespace nrm {
 namespace w1tc {
 
-constexpr int THREADS = 256;
 constexpr int ROWS = 128;
 constexpr int KX = 80;                        // xin columns padded to a multiple of 16 (66 real, column 66 = 1 in the backward, rest 0)
 constexpr uint32_t LBO = ROWS * 16;           // K-major tile of 128 rows: (r, 8 kb) at kb * 2048 + (r / 8) * 128 + (r % 8) * 16
@@ -29,50 +27,6 @@ __device__ __forceinline__ uint32_t tile_off(int r, int kb) { return (uint32_t)k
 __device__ __forceinline__ umma::Operand op_k(uint32_t addr, uint32_t part) { return umma::make_operand(addr, LBO, 128, 2 * LBO, part); }
 __device__ __forceinline__ umma::Operand op_mn(uint32_t addr, uint32_t part) { return umma::make_operand(addr, 128, LBO, 256, part); }
 
-// rows [r0, r0 + 128) of a row-major fp32 matrix with `cols` columns -> K-major bf16 tile(s) of KB 8-column blocks; rows >= nr and
-// columns >= cols are zero; `one_col` >= 0 sets that column to 1 in every real row.
-template <int NP, int KB>
-__device__ __forceinline__ void convert_rows(const float* __restrict__ src, int cols, long long r0, int nr, unsigned char* tile, uint32_t part, int one_col) {
-  // every load of the thread's items is issued before the first one is used: a load -> convert -> store loop pays one memory round
-  // trip per item (the kernel was latency-bound at 27 us for 26 MB with it)
-  constexpr int ITEMS = ROWS * KB, IT = (ITEMS + THREADS - 1) / THREADS;
-  float2 x[IT][4];
-#pragma unroll
-  for (int u = 0; u < IT; ++u) {
-    const int it = threadIdx.x + u * THREADS;
-    const int r = it & (ROWS - 1), kb = it >> 7;        // consecutive lanes -> consecutive rows: conflict-free 16-byte tile stores
-#pragma unroll
-    for (int i = 0; i < 4; ++i) x[u][i] = make_float2(0.f, 0.f);
-    if (it < ITEMS && r < nr) {
-      const float* p = src + (r0 + r) * cols + kb * 8;
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        if (kb * 8 + 2 * i + 2 <= cols) x[u][i] = __ldg(reinterpret_cast<const float2*>(p) + i);      // cols is even (66): pairs never straddle the end
-      }
-    }
-  }
-#pragma unroll
-  for (int u = 0; u < IT; ++u) {
-    const int it = threadIdx.x + u * THREADS;
-    if (it >= ITEMS) break;
-    const int r = it & (ROWS - 1), kb = it >> 7;
-    float v[8] = {x[u][0].x, x[u][0].y, x[u][1].x, x[u][1].y, x[u][2].x, x[u][2].y, x[u][3].x, x[u][3].y};
-    if (r < nr && one_col >= 0 && (one_col >> 3) == kb) v[one_col & 7] = 1.0f;
-    umma::store_operand8<NP>(tile, tile_off(r, kb), part, v);
-  }
-}
-
-// W1 [64][66] (row j, column k) -> K-major tile [64 rows j][KX k] (LBO = 64 rows * 16 B = 1024): B operand of the forward
-template <int NP>
-__device__ __forceinline__ void build_w_jk(const float* __restrict__ W, unsigned char* tile, uint32_t part) {
-  for (int it = threadIdx.x; it < 64 * (KX / 8); it += THREADS) {
-    const int j = it & 63, kb = it >> 6;
-    float v[8];
-#pragma unroll
-    for (int i = 0; i < 8; ++i) v[i] = (kb * 8 + i < XIN) ? __ldg(W + j * XIN + kb * 8 + i) : 0.f;
-    umma::store_operand8<NP>(tile, (uint32_t)kb * 1024u + (uint32_t)(j >> 3) * 128u + (uint32_t)(j & 7) * 16u, part, v);
-  }
-}
 // W1^T as a K-major tile [80 rows k][64 j] (LBO = 80 rows * 16 B = 1280): B operand of the dxin product
 template <int NP>
 __device__ __forceinline__ void build_w_kj(const float* __restrict__ W, unsigned char* tile, uint32_t part) {
@@ -83,69 +37,6 @@ __device__ __forceinline__ void build_w_kj(const float* __restrict__ W, unsigned
     for (int i = 0; i < 8; ++i) v[i] = (k < XIN) ? __ldg(W + (jb * 8 + i) * XIN + k) : 0.f;
     umma::store_operand8<NP>(tile, (uint32_t)jb * 1280u + (uint32_t)(k >> 3) * 128u + (uint32_t)(k & 7) * 16u, part, v);
   }
-}
-
-template <int NP>
-struct SmemFwd {
-  __align__(128) unsigned char xs[NP * X_TILE];
-  __align__(128) unsigned char ws[NP * 64 * KX * 2];
-  uint64_t mbar;
-  uint32_t tmem_base;
-};
-
-template <int SPLIT>
-__global__ void __launch_bounds__(THREADS)
-w1_forward_tc_kernel(const float* __restrict__ xin, const float* __restrict__ P, float* __restrict__ xh, long long NH) {
-  pdl_wait();
-  pdl_trigger();
-  constexpr int NP = SPLIT == 3 ? 2 : 1;
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  SmemFwd<NP>& sm = *reinterpret_cast<SmemFwd<NP>*>(smem_raw);
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  if (tid == 0) umma::mbar_init(&sm.mbar, 1);
-  if (warp == 0) umma::tmem_alloc(&sm.tmem_base, 64);
-  build_w_jk<NP>(P + P_W1_W, sm.ws, 64 * KX * 2);
-  umma::fence_async_smem();
-  umma::fence_before_sync();
-  __syncthreads();
-  umma::fence_after_sync();
-  const uint32_t tmem = sm.tmem_base;
-  constexpr uint32_t IDESC = umma::make_idesc_bf16(128, 64);
-  const int sp = warp & 3, half = warp >> 2;
-  const float4* bias = reinterpret_cast<const float4*>(P + P_W1_B + 32 * half);
-  uint32_t phase = 0;
-  const long long ntiles = (NH + ROWS - 1) / ROWS;
-  for (long long tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
-    const long long r0 = tile * ROWS;
-    const int nr = (int)min((long long)ROWS, NH - r0);
-    convert_rows<NP, KX / 8>(xin, XIN, r0, nr, sm.xs, X_TILE, -1);
-    umma::fence_async_smem();
-    umma::fence_before_sync();
-    __syncthreads();                                   // operands visible; the previous tile's accumulator has been read
-    if (warp == 0 && umma::elect_one()) {
-      umma::fence_after_sync();
-      umma::mma_product<SPLIT, KX / 16>(tmem, op_k(umma::smem_u32(sm.xs), X_TILE),
-                                        umma::make_operand(umma::smem_u32(sm.ws), 1024, 128, 2048, 64 * KX * 2), IDESC, false);
-      umma::mma_commit(&sm.mbar);
-    }
-    umma::mbar_wait(&sm.mbar, phase);
-    phase ^= 1;
-    umma::fence_after_sync();
-    float v[32];
-    umma::tmem_ld32(tmem + 32 * half + ((uint32_t)(32 * sp) << 16), v);
-    umma::fence_before_sync();
-    const int r = 32 * sp + lane;
-    if (r < nr) {
-      float4* dst = reinterpret_cast<float4*>(xh + (r0 + r) * 64 + 32 * half);
-#pragma unroll
-      for (int q = 0; q < 8; ++q) {
-        const float4 b = __ldg(bias + q);
-        dst[q] = make_float4(v[4 * q] + b.x, v[4 * q + 1] + b.y, v[4 * q + 2] + b.z, v[4 * q + 3] + b.w);
-      }
-    }
-  }
-  __syncthreads();
-  if (warp == 0) umma::tmem_dealloc(tmem, 64);
 }
 
 // fp32 rows already staged in shared memory (row-major, `cols` floats per row, cp.async) -> K-major bf16 tile(s)
@@ -292,21 +183,6 @@ w1_backward_tc_kernel(const float* __restrict__ xin, const float* __restrict__ d
 }  // namespace w1tc
 
 int launch_w1_finish(Workspace& w, int nparts, float* G, cudaStream_t s);   // nrm_w1.cu: sums the per-CTA partials in CTA order
-
-template <int SPLIT>
-static int launch_fwd(const float* P, Workspace& w, cudaStream_t s) {
-  constexpr int NP = SPLIT == 3 ? 2 : 1;
-  const size_t smem = sizeof(w1tc::SmemFwd<NP>);
-  const long long ntiles = (w.NH + w1tc::ROWS - 1) / w1tc::ROWS;
-  const int grid = (int)min(ntiles, (long long)3 * sm_count());
-  NRM_CUDA(cudaFuncSetAttribute(w1tc::w1_forward_tc_kernel<SPLIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  launch_pdl(w1tc::w1_forward_tc_kernel<SPLIT>, dim3(grid), dim3(w1tc::THREADS), smem, s, w.xin_h, P, w.xh, w.NH);
-  NRM_LAUNCH_CHECK("w1_forward_tc_kernel");
-  return NRM_OK;
-}
-int launch_w1_forward_tc(const float* P, Workspace& w, int precision, cudaStream_t s) {
-  return precision == NRM_PRECISION_BF16 ? launch_fwd<1>(P, w, s) : launch_fwd<3>(P, w, s);
-}
 
 template <int SPLIT>
 static int launch_bwd(const float* P, Workspace& w, float* G, cudaStream_t s) {

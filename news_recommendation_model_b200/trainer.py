@@ -18,7 +18,6 @@ Under data parallelism the graph is split around the gradient all-reduce.
 from __future__ import annotations
 
 import ctypes
-import os
 import struct
 from typing import List, Optional
 
@@ -77,9 +76,9 @@ class FusedTrainStep:
         world = self.dp.world if self.dp is not None else 1
         self.precision = model._precision_code()
         self.mode = engine.MODE_BN_BATCH_STATS | engine.MODE_KEEP_FOR_BWD
-        # compact batches go straight into the row kernels (no expansion to the packed float64 tensors) on the row-stacked tensor-core
-        # path; precision fp32 and the item-tile kernels read the packed rows, so they get nrm_expand_compact in front
-        self.compact_direct = self.precision != 0 and os.environ.get('NRM_ATT_ITEM_TILES') is None
+        # compact batches go straight into the row kernels (no expansion to the packed float64 tensors) in the tensor-core precisions;
+        # the FFMA attention of precision fp32 reads the packed rows, so it gets nrm_expand_compact in front
+        self.compact_direct = self.precision != 0
         n = self.flat.total
         # data parallel: the flat gradient buffer in symmetric (peer-mapped) memory, so that the Adam kernel of every rank can read
         # all of them (dp.PeerContext); None -> NCCL all-reduce between two graphs

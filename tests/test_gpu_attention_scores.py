@@ -1,9 +1,6 @@
 """Attention scores exported by the fused forward (nrm_forward_scores[_compact]) and the top-k "why this article" kernel
 (nrm_history_topk), through news_recommendation_model_b200.explain, in every precision."""
 import ctypes
-import os
-import subprocess
-import sys
 
 import pytest
 import torch
@@ -169,29 +166,3 @@ def test_k_larger_than_h_raises_value_error():
     s = torch.zeros(2, 1, 1, 3, device='cuda')
     with pytest.raises(ValueError):
         explain.top_history(s, 4)
-
-
-_ITEM_TILES_SCRIPT = r'''
-import sys, torch
-sys.path.insert(0, sys.argv[1]); sys.path.insert(0, sys.argv[1] + '/tests')
-import news_recommendation_model_b200 as nrm
-from news_recommendation_model_b200.synthetic import make_batch
-m = nrm.UserModel(40).to('cuda').set_precision(sys.argv[2])
-b = make_batch(2, 10, 3, seed=1, user_num=40).to('cuda')
-try:
-    nrm.explain.attention_scores(m, b.x_history, b.x_target, b.x_global)
-except nrm.NrmError as e:
-    print('NrmError:', e)
-    sys.exit(0)
-sys.exit(3)
-'''
-
-
-@pytest.mark.parametrize('precision', PRECISIONS)
-def test_item_tile_switch_raises_nrm_error(precision):
-    """NRM_ATT_ITEM_TILES=1 (read once per process) selects attention kernels that export no scores: an error, not another
-    kernel set whose logits would differ from nrm_forward's."""
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    env = dict(os.environ, NRM_ATT_ITEM_TILES='1')
-    out = subprocess.run([sys.executable, '-c', _ITEM_TILES_SCRIPT, root, precision], env=env, timeout=300, capture_output=True, text=True)
-    assert out.returncode == 0 and 'NRM_ATT_ITEM_TILES' in out.stdout, (out.returncode, out.stdout, out.stderr[-2000:])

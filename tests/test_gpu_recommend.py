@@ -2,9 +2,6 @@
 in every precision: the pool logits against the eval forward on the pool replicated per user, chunk invariance, BatchNorm left
 alone, and the selection against its host restatement (tests/recommend_ref.py)."""
 import ctypes
-import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
@@ -235,25 +232,3 @@ def test_bad_chunk_and_k_return_einval(precision):
     assert b'1024' in lib.nrm_last_error()
     assert lib.nrm_pool_topk(p(logits), 1, B * N, B, N, 1024, p(pa), table.n, p(ha), H, p(pos), p(val), None) == 0
     torch.cuda.synchronize()
-
-
-_ITEM_TILES_SCRIPT = r'''
-import sys, torch
-sys.path.insert(0, sys.argv[1]); sys.path.insert(0, sys.argv[1] + '/tests')
-import test_gpu_recommend as T
-from news_recommendation_model_b200 import recommend
-model = T._model(sys.argv[2])
-users, pool = T._users(3, 40, seed=23), T._pool(100, seed=24)
-got = recommend.pool_logits(model, T._table(), *users, pool[1], pool_article=pool[0], chunk=24)
-sys.exit(0 if torch.equal(got, T._expanded_logits(model, users, pool)) else 3)
-'''
-
-
-@pytest.mark.parametrize('precision', PRECISIONS)
-def test_item_tile_kernels_give_the_same_bits_as_their_forward(precision):
-    """NRM_ATT_ITEM_TILES=1 (read once per process) selects the item-tile attention kernels: the pool logits still equal that
-    process's eval forward on the replicated pool."""
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    env = dict(os.environ, NRM_ATT_ITEM_TILES='1')
-    out = subprocess.run([sys.executable, '-c', _ITEM_TILES_SCRIPT, root, precision], env=env, timeout=300, capture_output=True, text=True)
-    assert out.returncode == 0, (out.returncode, out.stdout, out.stderr[-2000:])

@@ -24,9 +24,9 @@ A row passes when |gpu - ref| <= rtol * max|ref over its impression| + atol * ma
 |gpu - ref| <= rtol * max|ref| of that tensor.  A failure names the buffer, the precision, the case's regime and the (b, c | h, column)
 of the worst element.
 
-Tolerances.  The floor of a buffer is the worst err / max|ref over the impression| over the cases of the matrix below (the
-item-tile runs included), with the case it came from; measured on one B200 at a 1000 W power limit, nvcc 12.9.  Cases with B >= 7
-(RTOL):
+Tolerances.  The floor of a buffer is the worst err / max|ref over the impression| over the cases of the matrix below (and over
+runs of the since-removed item-tile attention kernels), with the case it came from; measured on one B200 at a 1000 W power limit,
+nvcc 12.9.  Cases with B >= 7 (RTOL):
 
     buffer          fp32              bf16x3            bf16
     xh              4.4e-07 (b2000)   4.4e-07 (b2000)   4.4e-07 (b2000)
@@ -79,8 +79,6 @@ Set NRM_STAGEWISE_FLOORS=<path> to write the floors measured by a run as JSON.
 import ctypes
 import json
 import os
-import subprocess
-import sys
 import warnings
 
 import numpy as np
@@ -115,7 +113,6 @@ CASES = [
 ]
 CASE_IDS = [c[0] for c in CASES]
 CASE = {c[0]: c for c in CASES}
-ITEM_TILE_CASES = ('b7_h65_c8', 'b150_h50_c9', 'b160_h129_c17')
 
 # rtol per buffer and precision (see the module docstring for the floors they come from): RTOL for every case with B >= 7, RTOL_SMALL
 # for the two ill-conditioned smallest batches (SMALL_CASES)
@@ -298,34 +295,6 @@ def test_stagewise_against_float64(case_id, precision):
     failures = []
     check_step(case, precision, run_case(case_id, precision), failures)
     assert not failures, '\n'.join(failures)
-
-
-_ITEM_TILE_SCRIPT = r'''
-import sys, torch
-sys.path.insert(0, sys.argv[1]); sys.path.insert(0, sys.argv[1] + '/tests')
-import test_gpu_stagewise as S
-out = {}
-for prec in ('bf16x3', 'bf16'):
-    for cid in S.ITEM_TILE_CASES:
-        res = S.run_case(cid, prec)
-        out[(cid, prec)] = dict(logits=res['logits'].cpu(), bufs={k: v.cpu() for k, v in res['bufs'].items()},
-                                grads={k: v.cpu() for k, v in res['grads'].items()})
-torch.save(out, sys.argv[2])
-'''
-
-
-def test_item_tile_kernels_stagewise(tmp_path):
-    """The per-(pair, candidate) item-tile attention kernels (NRM_ATT_ITEM_TILES=1, read once per process, hence a child process)
-    at G = 1 with 64 + 1 history rows, G = 2 and G = 3, in both tensor-core precisions."""
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    path = str(tmp_path / 'item_tiles.pt')
-    env = dict(os.environ, NRM_ATT_ITEM_TILES='1')
-    subprocess.run([sys.executable, '-c', _ITEM_TILE_SCRIPT, root, path], check=True, env=env, timeout=600)
-    results = torch.load(path)
-    failures = []
-    for (cid, prec), res in results.items():
-        check_step(CASE[cid], prec, res, failures)
-    assert not failures, 'NRM_ATT_ITEM_TILES=1:\n' + '\n'.join(failures)
 
 
 @pytest.mark.parametrize('precision', PRECISIONS)

@@ -5,7 +5,6 @@ import numpy as np
 import pytest
 import torch
 
-import news_recommendation_model_b200 as nrm
 from news_recommendation_model_b200 import _lib
 from fixtures import load_weights
 from news_recommendation_model_b200.synthetic import make_batch
@@ -100,42 +99,3 @@ def test_bf16x3_eval_forward_meets_fp32_tolerance():
         out = model(d.x_history, d.x_target, d.x_global).cpu()
         ref = O.user_model_forward(p, b.x_history, b.x_target, b.x_global, training=False)
     assert (out - ref).abs().max().item() <= P.TOL_LOGITS
-
-
-_ALT_SCRIPT = r'''
-import sys, numpy as np, torch
-sys.path.insert(0, sys.argv[1]); sys.path.insert(0, sys.argv[1] + '/tests')
-import news_recommendation_model_b200 as nrm
-from fixtures import load_weights
-from news_recommendation_model_b200.synthetic import make_batch
-m = nrm.UserModel(300); m.load_state_dict(load_weights('train'), strict=False); m.to('cuda').train().set_precision('bf16x3')
-b = make_batch(96, 37, 7, seed=31, user_num=300).to('cuda')
-out = m(b.x_history, b.x_target, b.x_global); m.loss(b.user_id, out, b.label).backward()
-np.savez(sys.argv[2], logits=out.detach().cpu().numpy(), **{k: v.grad.detach().cpu().numpy() for k, v in m.named_parameters()})
-'''
-
-
-@pytest.mark.parametrize('env', [{'NRM_HEAD_FFMA': '1'}, {'NRM_ATT_ITEM_TILES': '1'}])
-def test_alternative_kernel_sets_agree_with_the_default_ones(env, tmp_path):
-    """The library keeps a second implementation of its two tensor-core blocks behind environment switches (read once per process):
-    the FFMA scoring head (NRM_HEAD_FFMA=1) against the tcgen05 head, the round-1 item-tile attention kernels (NRM_ATT_ITEM_TILES=1)
-    against the row-stacked ones.  One training step (B = 96: two head tiles, one ragged) in a child process per switch: logits and
-    every gradient agree with the default kernels within the fp32-grade tolerances."""
-    import os
-    import subprocess
-    import sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    res = {}
-    for name, extra in (('default', {}), ('alt', env)):
-        path = str(tmp_path / f'{name}.npz')
-        e = {k: v for k, v in os.environ.items() if k not in ('NRM_HEAD_FFMA', 'NRM_ATT_ITEM_TILES')}
-        e.update(extra)
-        subprocess.run([sys.executable, '-c', _ALT_SCRIPT, root, path], check=True, env=e, timeout=300)
-        res[name] = dict(np.load(path))
-    assert np.abs(res['default']['logits'] - res['alt']['logits']).max() <= P.TOL_LOGITS
-    for k, g in res['default'].items():
-        if k == 'logits':
-            continue
-        scale = np.abs(g).max()
-        tol = P.TOL_GRAD_ABS if k in P.NOISE_KEYS else 2 * P.TOL_GRAD_REL * scale + P.TOL_GRAD_ABS
-        assert np.abs(g - res['alt'][k]).max() <= tol, (env, k, float(np.abs(g - res['alt'][k]).max()), float(scale))
