@@ -19,7 +19,7 @@
  *     UserInstantInterestModel.forward
  *                 models/user_instant_interest_model.py:20-23 (inside nrm_forward)
  *   s_label / s_ti            user_invariant_interest_model.py:83-87   nrm_forward_scores, nrm_history_topk
- *   ensemble softmax + order  test.py:58-63, 124-127 over a shared pool  nrm_forward_pool, nrm_pool_topk
+ *   ensemble softmax + order  test.py:58-63, 124-127 over a shared pool  nrm_forward_pool, nrm_pool_topk, nrm_pool_rank
  *   UserModel.loss            models/user_model.py:37-43      nrm_loss_forward
  *   loss.backward()           train.py:73                     nrm_loss_backward, nrm_backward
  *   optimizer.step()          train.py:48,74                  nrm_adam_step
@@ -265,6 +265,21 @@ int nrm_forward_pool(const nrm_compact_batch* users, int B, int H, int N, int ch
                      const float* bn_running_var, int precision, float* logits, void* workspace, size_t workspace_bytes, void* stream);
 int nrm_pool_topk(const float* logits, int n_models, long long model_stride, int B, int N, int k, const int* pool_article, int n_articles,
                   const int* hist_article, int H, int* pos_out, float* val_out, void* stream);
+/*   nrm_pool_rank: where each of a user's held-out target articles lands in that user's ranking of the whole pool, the ranking
+ *     nrm_pool_topk returns the first k entries of (same logits, n_models, model_stride, pool_article, n_articles, hist_article, H,
+ *     eligibility and scores).  targets int32 [B,P], 1 <= P <= 1024: article ids, 0 = pad slot.  Target (b, p) is rankable if its
+ *     id is in [1, n_articles), no earlier slot of row b holds the same id, and an eligible pool position holds it (pool ids should
+ *     be distinct; a repeated one ranks by its occurrence that comes first).  Per target, int32 / float32 [B,P], counted over user
+ *     b's eligible positions:
+ *       pos_out      its pool position;
+ *       rank_out     the positions ahead of it in nrm_pool_topk's order: it is among nrm_pool_topk(k) iff rank < k;
+ *       greater_out  the positions with a strictly larger score;
+ *       equal_out    the other positions with an equal score (-0.0 == +0.0);
+ *       score_out    its score;
+ *     -1 / -1 / -1 / -1 / NaN for a target that is not rankable.  n_eligible_out int32 [B]: the user's eligible positions. */
+int nrm_pool_rank(const float* logits, int n_models, long long model_stride, int B, int N, const int* pool_article, int n_articles,
+                  const int* hist_article, int H, const int* targets, int P, int* pos_out, int* rank_out, int* greater_out,
+                  int* equal_out, float* score_out, int* n_eligible_out, void* stream);
 
 /* ---- UserModel.loss (user_model.py:37-43) ---------------------------------------- */
 /* loss = (1-alpha) BCE(softmax(out), y) + alpha BCE(softmax(out + delta[id]), y), mean

@@ -73,6 +73,7 @@ SIGNATURES = {
     'nrm_pool_workspace_bytes': (sz, [i32, i32, i32, i32]),
     'nrm_forward_pool': (i32, [vp, i32, i32, i32, i32, vp, vp, vp, i32, vp, vp, sz, vp]),
     'nrm_pool_topk': (i32, [vp, i32, ll, i32, i32, i32, vp, i32, vp, i32, vp, vp, vp]),
+    'nrm_pool_rank': (i32, [vp, i32, ll, i32, i32, vp, i32, vp, i32, vp, i32, vp, vp, vp, vp, vp, vp, vp]),
 }
 
 

@@ -79,6 +79,10 @@ int launch_expand_compact(const float* articles, int n_articles, const int* hist
 // nrm_recommend.cu: per user, the k best eligible positions of a shared article pool (nrm_pool_topk)
 int launch_pool_topk(const float* logits, int n_models, long long model_stride, int B, int N, int k, const int* pool_article, int n_articles,
                      const int* hist_article, int H, int* pos_out, float* val_out, cudaStream_t s);
+// nrm_recommend.cu: per user, where each held-out target lands in the ranking nrm_pool_topk takes the first k entries of (nrm_pool_rank)
+int launch_pool_rank(const float* logits, int n_models, long long model_stride, int B, int N, const int* pool_article, int n_articles,
+                     const int* hist_article, int H, const int* targets, int P, int* pos_out, int* rank_out, int* greater_out,
+                     int* equal_out, float* score_out, int* n_eligible_out, cudaStream_t s);
 
 // nrm_head.cu
 int launch_bn_partial_sums(Workspace& w, cudaStream_t s);                 // -> w.bn_sums

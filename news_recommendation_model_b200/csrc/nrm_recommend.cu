@@ -59,15 +59,19 @@ __device__ __forceinline__ bool pool_clicked(const int* tab, int lg, int id) {
 // any, so that a thread keeps POOL_BATCH independent loads in flight.
 constexpr int POOL_BATCH = 4;
 
+// The phases both kernels share take their argument struct (PoolTopkArgs or PoolRankArgs) as a template parameter: they read only
+// the pool and exclusion fields the two have in common, and each kernel keeps its own parameter layout.
+
 // a pool id that may be recommended: in range and not clicked by this user
-__device__ __forceinline__ bool pool_id_ok(const PoolTopkArgs& a, const int* tab, int id) {
+template <class Args>
+__device__ __forceinline__ bool pool_id_ok(const Args& a, const int* tab, int id) {
   return id >= 1 && id < a.n_articles && !pool_clicked(tab, a.hash_lg, id);
 }
 
 // keys of positions n0 + j * POOL_THREADS from the logits alone (0: past the pool or a NaN logit in some model) and their ids;
 // whether the id is eligible is left to the caller, which checks it only for the keys it wants
-template <bool ENSEMBLE>
-__device__ __forceinline__ void pool_raw_keys(const PoolTopkArgs& a, const float* row, const float* mx, const float* sum, int n0,
+template <bool ENSEMBLE, class Args>
+__device__ __forceinline__ void pool_raw_keys(const Args& a, const float* row, const float* mx, const float* sum, int n0,
                                               unsigned long long (&key)[POOL_BATCH], int (&id)[POOL_BATCH]) {
   float x[POOL_BATCH], acc[POOL_BATCH];
   bool ok[POOL_BATCH];
@@ -100,8 +104,8 @@ __device__ __forceinline__ void pool_raw_keys(const PoolTopkArgs& a, const float
 }
 
 // ensemble statistics: this thread's max (MAX) or sum of exp(x_m - vmax) over its eligible positions, for model m
-template <bool MAX>
-__device__ __forceinline__ float pool_model_partial(const PoolTopkArgs& a, const float* row, const int* tab, int m, float vmax) {
+template <bool MAX, class Args>
+__device__ __forceinline__ float pool_model_partial(const Args& a, const float* row, const int* tab, int m, float vmax) {
   float v = MAX ? -CUDART_INF_F : 0.f;
 #pragma unroll 1
   for (int n0 = threadIdx.x; n0 < a.N; n0 += POOL_BATCH * POOL_THREADS) {
@@ -154,6 +158,56 @@ __device__ __forceinline__ float pool_block_reduce(float v, float* red) {
   return red[POOL_THREADS / 32];
 }
 
+// user b's clicked ids into the hash table tab[1 << hash_lg] (pad rows and ids no pool position can carry are left out); ends with
+// a barrier
+template <class Args>
+__device__ __forceinline__ void pool_build_clicked(const Args& a, int b, int tid, int* tab) {
+  if (a.hash_lg > 0) {
+    const int cap = 1 << a.hash_lg;
+    for (int i = tid; i < cap; i += POOL_THREADS) tab[i] = 0;
+    __syncthreads();
+    for (int h = tid; h < a.H; h += POOL_THREADS) {
+      const int id = a.hist_article[(long long)b * a.H + h];
+      if (id < 1 || id >= a.n_articles) continue;
+      for (unsigned s = pool_hash(id, a.hash_lg);; s = (s + 1) & (unsigned)(cap - 1)) {
+        const int old = atomicCAS(&tab[s], 0, id);
+        if (old == 0 || old == id) break;
+      }
+    }
+  }
+  __syncthreads();
+}
+
+// ensemble: per model m, mx[m] / sum[m] = max and sum of exp(x - max) over the eligible positions; ends with a barrier
+template <class Args>
+__device__ __forceinline__ void pool_ensemble_stats(const Args& a, const float* row, const int* tab, float* mx, float* sum, float* red) {
+  for (int m = 0; m < a.n_models; ++m) {
+    const float vmax = pool_block_reduce<true>(pool_model_partial<true>(a, row, tab, m, 0.f), red);
+    const float vsum = pool_block_reduce<false>(pool_model_partial<false>(a, row, tab, m, vmax), red);
+    if (threadIdx.x == 0) { mx[m] = vmax; sum[m] = vsum; }
+  }
+  __syncthreads();
+}
+
+// sel[0, cnt) -> descending, bitonic over the next power of two (padded with 0 keys, which sort last); ends with a barrier
+__device__ __forceinline__ void pool_sort_desc(unsigned long long* sel, int cnt, int tid) {
+  int P = 1;
+  while (P < cnt) P <<= 1;
+  for (int i = cnt + tid; i < P; i += POOL_THREADS) sel[i] = 0ull;
+  __syncthreads();
+  for (int size = 2; size <= P; size <<= 1) {
+    for (int stride = size >> 1; stride > 0; stride >>= 1) {
+      for (int t = tid; t < P / 2; t += POOL_THREADS) {
+        const int lo = 2 * t - (t & (stride - 1)), hi = lo + stride;
+        const bool desc = (lo & size) == 0;
+        const unsigned long long x = sel[lo], y = sel[hi];
+        if ((x < y) == desc) { sel[lo] = y; sel[hi] = x; }
+      }
+      __syncthreads();
+    }
+  }
+}
+
 template <bool ENSEMBLE>
 __global__ void __launch_bounds__(POOL_THREADS, 3)
 pool_topk_kernel(const PoolTopkArgs a) {
@@ -167,31 +221,8 @@ pool_topk_kernel(const PoolTopkArgs a) {
   const int tid = threadIdx.x, b = blockIdx.x, N = a.N;
   const float* row = a.logits + (long long)b * N;
 
-  // the user's clicked ids (pad rows and ids no pool position can carry are left out)
-  if (a.hash_lg > 0) {
-    const int cap = 1 << a.hash_lg;
-    for (int i = tid; i < cap; i += POOL_THREADS) clicked_tab[i] = 0;
-    __syncthreads();
-    for (int h = tid; h < a.H; h += POOL_THREADS) {
-      const int id = a.hist_article[(long long)b * a.H + h];
-      if (id < 1 || id >= a.n_articles) continue;
-      for (unsigned s = pool_hash(id, a.hash_lg);; s = (s + 1) & (unsigned)(cap - 1)) {
-        const int old = atomicCAS(&clicked_tab[s], 0, id);
-        if (old == 0 || old == id) break;
-      }
-    }
-  }
-  __syncthreads();
-
-  // ensemble: per model, max and sum of exp(x - max) over the eligible positions
-  if (ENSEMBLE) {
-    for (int m = 0; m < a.n_models; ++m) {
-      const float vmax = pool_block_reduce<true>(pool_model_partial<true>(a, row, clicked_tab, m, 0.f), red);
-      const float vsum = pool_block_reduce<false>(pool_model_partial<false>(a, row, clicked_tab, m, vmax), red);
-      if (tid == 0) { mx[m] = vmax; sum[m] = vsum; }
-    }
-    __syncthreads();
-  }
+  pool_build_clicked(a, b, tid, clicked_tab);
+  if (ENSEMBLE) pool_ensemble_stats(a, row, clicked_tab, mx, sum, red);
 
   // radix select of the k-th largest key; threshold: the selected keys are exactly those >= it
   unsigned long long prefix = 0ull, mask = 0ull, threshold = 0ull;
@@ -267,21 +298,7 @@ pool_topk_kernel(const PoolTopkArgs a) {
   }
   __syncthreads();
   const int cnt = (int)s_count;
-  int P = 1;
-  while (P < cnt) P <<= 1;
-  for (int i = cnt + tid; i < P; i += POOL_THREADS) sel[i] = 0ull;
-  __syncthreads();
-  for (int size = 2; size <= P; size <<= 1) {
-    for (int stride = size >> 1; stride > 0; stride >>= 1) {
-      for (int t = tid; t < P / 2; t += POOL_THREADS) {
-        const int lo = 2 * t - (t & (stride - 1)), hi = lo + stride;
-        const bool desc = (lo & size) == 0;
-        const unsigned long long x = sel[lo], y = sel[hi];
-        if ((x < y) == desc) { sel[lo] = y; sel[hi] = x; }
-      }
-      __syncthreads();
-    }
-  }
+  pool_sort_desc(sel, cnt, tid);
   for (int j = tid; j < a.k; j += POOL_THREADS) {
     const long long o = (long long)b * a.k + j;
     if (j < cnt) {
@@ -295,18 +312,185 @@ pool_topk_kernel(const PoolTopkArgs a) {
   }
 }
 
+// ---- nrm_pool_rank: where each of a user's held-out targets lands in that user's ranking of the whole pool --------------------
+// The ranking is the one nrm_pool_topk returns a prefix of (same eligibility, scores and keys).  A target is rankable if its id is
+// in [1, n_articles), is held by an eligible pool position, and does not repeat an id of an earlier slot of the user's target row.
+// Two passes over the pool after the ensemble statistics: the first finds each target's key (ids -> first slot through a second
+// hash table); the T rankable keys are then sorted, and in the second pass every eligible position finds by binary search the gap
+// between consecutive target keys (and target scores) it falls into and counts itself there with a shared-memory integer atomic.
+// A prefix sum over the gaps gives every target's counts, exactly and independently of timing, in O(N log P) work per user.
+constexpr int POOL_TARGETS_MAX = 1024;
+constexpr int TARGET_HASH_LG = 11;            // 2048 slots for <= 1024 ids: load factor <= 1/2
+
+struct PoolRankArgs {
+  const float* logits; int n_models; long long model_stride;
+  int N;
+  const int* pool_article; int n_articles;
+  const int* hist_article; int H; int hash_lg;   // hash_lg 0: no exclusion
+  const int* targets; int P;
+  int* pos_out; int* rank_out; int* greater_out; int* equal_out; float* score_out; int* n_eligible_out;
+};
+
+// the first slot of the user's target row that holds `id`, -1 if none
+__device__ __forceinline__ int pool_target_slot(const int* tgt_id, const int* tgt_slot, int id) {
+  if (id < 1) return -1;                                   // 0 marks an empty table slot
+  constexpr unsigned m = (1u << TARGET_HASH_LG) - 1;
+  for (unsigned h = pool_hash(id, TARGET_HASH_LG);; h = (h + 1) & m) {
+    const int v = tgt_id[h];
+    if (v == id) return tgt_slot[h];
+    if (v == 0) return -1;
+  }
+}
+
+// lo + the number of entries of the descending run s[lo, hi) for which above(entry) holds (it holds on a prefix of the run)
+template <class Above>
+__device__ __forceinline__ int pool_count_above(const unsigned long long* s, int lo, int hi, Above above) {
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if (above(s[mid])) lo = mid + 1; else hi = mid;
+  }
+  return lo;
+}
+
+// inclusive prefix sum of v[0, n) by one warp
+__device__ __forceinline__ void pool_warp_scan(int* v, int n) {
+  const int lane = threadIdx.x & 31;
+  int carry = 0;
+  for (int i0 = 0; i0 < n; i0 += 32) {
+    int x = i0 + lane < n ? v[i0 + lane] : 0;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int y = __shfl_up_sync(0xffffffffu, x, o);
+      if (lane >= o) x += y;
+    }
+    if (i0 + lane < n) v[i0 + lane] = x + carry;
+    carry += __shfl_sync(0xffffffffu, x, 31);
+  }
+}
+
+template <bool ENSEMBLE>
+__global__ void __launch_bounds__(POOL_THREADS, 3)
+pool_rank_kernel(const PoolRankArgs a) {
+  extern __shared__ int clicked_tab[];                     // [1 << hash_lg] article ids, 0 = empty slot
+  __shared__ int tgt_id[1 << TARGET_HASH_LG], tgt_slot[1 << TARGET_HASH_LG];   // target id -> its first slot in the row
+  __shared__ unsigned long long slot_key[POOL_TARGETS_MAX];                    // per slot: the key of its position, 0 = not rankable
+  __shared__ unsigned long long tkey[POOL_TARGETS_MAX];                        // the T rankable keys, descending
+  // per gap j (between sorted targets j - 1 and j): eligible positions with a larger key than target j but not than j - 1, and the
+  // same for score > and score >=; after the prefix sums, entry j is target j's count
+  __shared__ int gap_rank[POOL_TARGETS_MAX], gap_greater[POOL_TARGETS_MAX], gap_ge[POOL_TARGETS_MAX];
+  __shared__ float red[POOL_THREADS / 32 + 1];
+  __shared__ float mx[POOL_MODELS_MAX], sum[POOL_MODELS_MAX];
+  __shared__ unsigned s_count, s_eligible;
+  const int tid = threadIdx.x, b = blockIdx.x, N = a.N, P = a.P;
+  const float* row = a.logits + (long long)b * N;
+  const int* trow = a.targets + (long long)b * P;
+
+  for (int i = tid; i < (1 << TARGET_HASH_LG); i += POOL_THREADS) { tgt_id[i] = 0; tgt_slot[i] = 0x7fffffff; }
+  for (int i = tid; i < POOL_TARGETS_MAX; i += POOL_THREADS) { slot_key[i] = 0ull; gap_rank[i] = 0; gap_greater[i] = 0; gap_ge[i] = 0; }
+  if (tid == 0) { s_count = 0; s_eligible = 0; }
+  pool_build_clicked(a, b, tid, clicked_tab);              // (its barriers also publish the initialisation above)
+  for (int p = tid; p < P; p += POOL_THREADS) {
+    const int id = trow[p];
+    if (id < 1 || id >= a.n_articles) continue;            // pad slot or an id no pool position can rank
+    for (unsigned h = pool_hash(id, TARGET_HASH_LG);; h = (h + 1) & ((1u << TARGET_HASH_LG) - 1)) {
+      const int old = atomicCAS(&tgt_id[h], 0, id);
+      if (old == 0 || old == id) { atomicMin(&tgt_slot[h], p); break; }
+    }
+  }
+  if (ENSEMBLE) pool_ensemble_stats(a, row, clicked_tab, mx, sum, red);
+  __syncthreads();
+
+  // locate: every target's key (a repeated pool id: the occurrence ranked first)
+#pragma unroll 1
+  for (int n0 = tid; n0 < N; n0 += POOL_BATCH * POOL_THREADS) {
+    unsigned long long key[POOL_BATCH];
+    int id[POOL_BATCH];
+    pool_raw_keys<ENSEMBLE>(a, row, mx, sum, n0, key, id);
+#pragma unroll
+    for (int j = 0; j < POOL_BATCH; ++j) {
+      if (key[j] == 0ull) continue;
+      const int slot = pool_target_slot(tgt_id, tgt_slot, id[j]);
+      if (slot >= 0 && pool_id_ok(a, clicked_tab, id[j])) atomicMax(&slot_key[slot], key[j]);
+    }
+  }
+  __syncthreads();
+  for (int p = tid; p < P; p += POOL_THREADS)
+    if (slot_key[p] != 0ull) tkey[atomicAdd(&s_count, 1u)] = slot_key[p];
+  __syncthreads();
+  const int T = (int)s_count;
+  pool_sort_desc(tkey, T, tid);
+
+  // count: the gap of every eligible position among the target keys, and among the target scores (the keys' upper 32 bits)
+  unsigned n_eligible = 0;
+#pragma unroll 1
+  for (int n0 = tid; n0 < N; n0 += POOL_BATCH * POOL_THREADS) {
+    unsigned long long key[POOL_BATCH];
+    int id[POOL_BATCH];
+    pool_raw_keys<ENSEMBLE>(a, row, mx, sum, n0, key, id);
+#pragma unroll
+    for (int j = 0; j < POOL_BATCH; ++j) {
+      if (key[j] == 0ull || !pool_id_ok(a, clicked_tab, id[j])) continue;
+      ++n_eligible;
+      const unsigned long long k = key[j];
+      const unsigned u = (unsigned)(k >> 32);
+      const int gt = pool_count_above(tkey, 0, T, [u](unsigned long long t) { return (unsigned)(t >> 32) > u; });
+      const int ge = pool_count_above(tkey, gt, T, [u](unsigned long long t) { return (unsigned)(t >> 32) >= u; });
+      const int kge = pool_count_above(tkey, gt, ge, [k](unsigned long long t) { return t >= k; });
+      if (kge < T) atomicAdd(&gap_rank[kge], 1);           // above targets kge.. (by key)
+      if (ge < T) atomicAdd(&gap_greater[ge], 1);          // a larger score than targets ge..
+      if (gt < T) atomicAdd(&gap_ge[gt], 1);               // a score at least that of targets gt..
+    }
+  }
+  atomicAdd(&s_eligible, n_eligible);
+  __syncthreads();
+  const int warp = tid >> 5;
+  if (warp == 0) pool_warp_scan(gap_rank, T);
+  else if (warp == 1) pool_warp_scan(gap_greater, T);
+  else if (warp == 2) pool_warp_scan(gap_ge, T);
+  __syncthreads();
+
+  for (int p = tid; p < P; p += POOL_THREADS) {
+    const long long o = (long long)b * P + p;
+    const unsigned long long k = slot_key[p];
+    if (k != 0ull) {
+      const int i = pool_count_above(tkey, 0, T, [k](unsigned long long t) { return t > k; });   // its place among the sorted keys
+      a.pos_out[o] = (int)~(unsigned)k;
+      a.rank_out[o] = gap_rank[i];
+      a.greater_out[o] = gap_greater[i];
+      a.equal_out[o] = gap_ge[i] - gap_greater[i] - 1;       // minus the target itself
+      a.score_out[o] = pool_key_score(k);
+    } else {
+      a.pos_out[o] = -1;
+      a.rank_out[o] = -1;
+      a.greater_out[o] = -1;
+      a.equal_out[o] = -1;
+      a.score_out[o] = CUDART_NAN_F;
+    }
+  }
+  if (tid == 0) a.n_eligible_out[b] = (int)s_eligible;
+}
+
+// the checks both entry points share; *lg: the exclusion table's log2 size (0: no exclusion)
+static int pool_check_models_and_history(const char* fn, int n_models, long long model_stride, int B, int N, const int* hist_article,
+                                         int H, int* lg) {
+  if (n_models < 1 || n_models > POOL_MODELS_MAX) { set_error("%s: need 1 <= n_models <= %d (got %d)", fn, POOL_MODELS_MAX, n_models); return NRM_EINVAL; }
+  if (n_models > 1 && model_stride < (long long)B * N) { set_error("%s: model_stride smaller than B * N", fn); return NRM_EINVAL; }
+  *lg = 0;
+  if (hist_article != nullptr) {
+    if (H <= 0) { set_error("%s: H must be positive with hist_article (got %d)", fn, H); return NRM_EINVAL; }
+    int l = 5;
+    while (l <= POOL_HASH_LG_MAX && (1LL << l) < 2LL * H) ++l;
+    if (l > POOL_HASH_LG_MAX) { set_error("%s: H = %d exceeds the %d history rows the exclusion table holds", fn, H, 1 << (POOL_HASH_LG_MAX - 1)); return NRM_EINVAL; }
+    *lg = l;
+  }
+  return NRM_OK;
+}
+
 int launch_pool_topk(const float* logits, int n_models, long long model_stride, int B, int N, int k, const int* pool_article, int n_articles,
                      const int* hist_article, int H, int* pos_out, float* val_out, cudaStream_t s) {
   if (k < 1 || k > N || k > POOL_TOPK_MAX) { set_error("nrm_pool_topk: need 1 <= k <= min(N, %d) (got k = %d, N = %d)", POOL_TOPK_MAX, k, N); return NRM_EINVAL; }
-  if (n_models < 1 || n_models > POOL_MODELS_MAX) { set_error("nrm_pool_topk: need 1 <= n_models <= %d (got %d)", POOL_MODELS_MAX, n_models); return NRM_EINVAL; }
-  if (n_models > 1 && model_stride < (long long)B * N) { set_error("nrm_pool_topk: model_stride smaller than B * N"); return NRM_EINVAL; }
-  int lg = 0;
-  if (hist_article != nullptr) {
-    if (H <= 0) { set_error("nrm_pool_topk: H must be positive with hist_article (got %d)", H); return NRM_EINVAL; }
-    lg = 5;
-    while (lg <= POOL_HASH_LG_MAX && (1LL << lg) < 2LL * H) ++lg;
-    if (lg > POOL_HASH_LG_MAX) { set_error("nrm_pool_topk: H = %d exceeds the %d history rows the exclusion table holds", H, 1 << (POOL_HASH_LG_MAX - 1)); return NRM_EINVAL; }
-  }
+  int lg;
+  if (const int rc = pool_check_models_and_history("nrm_pool_topk", n_models, model_stride, B, N, hist_article, H, &lg)) return rc;
   const PoolTopkArgs args{logits, n_models, model_stride, N, k, pool_article, n_articles, hist_article, H, lg, pos_out, val_out};
   const size_t smem = lg > 0 ? sizeof(int) << lg : 0;
   void (*kern)(const PoolTopkArgs) = n_models > 1 ? pool_topk_kernel<true> : pool_topk_kernel<false>;
@@ -315,6 +499,24 @@ int launch_pool_topk(const float* logits, int n_models, long long model_stride, 
     NRM_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(int) << POOL_HASH_LG_MAX)));
   kern<<<B, POOL_THREADS, smem, s>>>(args);
   NRM_LAUNCH_CHECK("pool_topk_kernel");
+  return NRM_OK;
+}
+
+int launch_pool_rank(const float* logits, int n_models, long long model_stride, int B, int N, const int* pool_article, int n_articles,
+                     const int* hist_article, int H, const int* targets, int P, int* pos_out, int* rank_out, int* greater_out,
+                     int* equal_out, float* score_out, int* n_eligible_out, cudaStream_t s) {
+  if (P < 1 || P > POOL_TARGETS_MAX) { set_error("nrm_pool_rank: need 1 <= P <= %d (got %d)", POOL_TARGETS_MAX, P); return NRM_EINVAL; }
+  int lg;
+  if (const int rc = pool_check_models_and_history("nrm_pool_rank", n_models, model_stride, B, N, hist_article, H, &lg)) return rc;
+  const PoolRankArgs args{logits, n_models, model_stride, N, pool_article, n_articles, hist_article, H, lg, targets, P,
+                          pos_out, rank_out, greater_out, equal_out, score_out, n_eligible_out};
+  const size_t smem = lg > 0 ? sizeof(int) << lg : 0;
+  void (*kern)(const PoolRankArgs) = n_models > 1 ? pool_rank_kernel<true> : pool_rank_kernel<false>;
+  static DeviceOnce configured[2];
+  if (configured[n_models > 1].first_time())
+    NRM_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(int) << POOL_HASH_LG_MAX)));
+  kern<<<B, POOL_THREADS, smem, s>>>(args);
+  NRM_LAUNCH_CHECK("pool_rank_kernel");
   return NRM_OK;
 }
 
@@ -328,4 +530,16 @@ extern "C" int nrm_pool_topk(const float* logits, int n_models, long long model_
   if (B <= 0 || N <= 0 || n_articles <= 0) { set_error("nrm_pool_topk: B, N, n_articles must be positive (got %d, %d, %d)", B, N, n_articles); return NRM_EINVAL; }
   return launch_pool_topk(logits, n_models, model_stride, B, N, k, pool_article, n_articles, hist_article, H, pos_out, val_out,
                           (cudaStream_t)stream);
+}
+
+extern "C" int nrm_pool_rank(const float* logits, int n_models, long long model_stride, int B, int N, const int* pool_article,
+                             int n_articles, const int* hist_article, int H, const int* targets, int P, int* pos_out, int* rank_out,
+                             int* greater_out, int* equal_out, float* score_out, int* n_eligible_out, void* stream) {
+  if (!logits || !pool_article || !targets || !pos_out || !rank_out || !greater_out || !equal_out || !score_out || !n_eligible_out) {
+    set_error("nrm_pool_rank: null pointer");
+    return NRM_EINVAL;
+  }
+  if (B <= 0 || N <= 0 || n_articles <= 0) { set_error("nrm_pool_rank: B, N, n_articles must be positive (got %d, %d, %d)", B, N, n_articles); return NRM_EINVAL; }
+  return launch_pool_rank(logits, n_models, model_stride, B, N, pool_article, n_articles, hist_article, H, targets, P, pos_out, rank_out,
+                          greater_out, equal_out, score_out, n_eligible_out, (cudaStream_t)stream);
 }

@@ -13,7 +13,14 @@ shared by all users, so the memory is that of a (B, H, chunk) forward, and the l
 GPU (`nrm_pool_topk`): the score is the logit for one model and, for an ensemble, the mean over the models of the softmax over the
 user's eligible articles (test.py:58-63); the order is Python's stable `sorted(..., reverse=True)` (test.py:124-127).  Eligible are
 the pool positions whose article id is in [1, n_articles), whose logits are not NaN and, with `exclude_clicked`, whose article
-is not among the user's non-pad history ids; duplicate ids in the pool are independent positions."""
+is not among the user's non-pad history ids; duplicate ids in the pool are independent positions.
+
+The same ranking measures itself (`nrm_pool_rank`): given each user's held-out clicked articles, `rank_targets` returns where every
+one lands in that user's ranking of the whole pool, `pool_metrics` turns those ranks into recall@k, nDCG@k, MRR and AUC, and
+`evaluate` runs the three steps from the models:
+
+    metrics, ranks = recommend.evaluate([m1, m2], table, hist_article, hist_time, hist_click, pool_time, targets, ks=(10, 100))
+    torch.nanmean(metrics['ndcg@10'])"""
 from __future__ import annotations
 
 import ctypes
@@ -24,6 +31,7 @@ import torch
 from . import _lib, engine, wire
 
 TOPK_MAX = 1024
+TARGETS_MAX = 1024
 MODELS_MAX = 16
 CHUNK_ALIGN = 8                       # the attention's candidate group: every multiple of it gives the same logits
 WORKSPACE_TARGET = 1 << 30            # chunk=None: the largest chunk whose workspace stays under 1 GiB
@@ -35,6 +43,16 @@ class Recommendations(NamedTuple):
     score: torch.Tensor       # [B,k] float32 ranking scores (NaN where the position is -1)
 
 
+class TargetRanks(NamedTuple):
+    """Per held-out target (b, p), counted over user b's eligible pool positions; -1 / NaN where the target is not rankable."""
+    position: torch.Tensor    # [B,P] int64 the target's pool position
+    rank: torch.Tensor        # [B,P] int64 positions ahead of it in top_articles' order: it is among top_articles(k) iff rank < k
+    greater: torch.Tensor     # [B,P] int64 positions with a strictly larger score
+    equal: torch.Tensor       # [B,P] int64 other positions with an equal score
+    score: torch.Tensor       # [B,P] float32 its ranking score
+    n_eligible: torch.Tensor  # [B] int64 the user's eligible positions
+
+
 def _stream(dev) -> ctypes.c_void_p:
     return ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
 
@@ -44,8 +62,9 @@ def _check_k(k, N: int) -> None:
         raise ValueError(f'k must be an integer in [1, min(N, {TOPK_MAX})] = [1, {min(N, TOPK_MAX)}], got {k!r}')
 
 
-def _check_users_and_pool(table, hist_article, hist_time, hist_click, pool_time, pool_article, k=None):
-    """-> (B, H, N, pool_article); ValueError for shapes / dtypes / layout / k, NrmError for tensors that are not on a CUDA device."""
+def _check_users_and_pool(table, hist_article, hist_time, hist_click, pool_time, pool_article, k=None, targets=None):
+    """-> (B, H, N, pool_article); ValueError for shapes / dtypes / layout / k / targets (with `targets`, also for a pool that
+    repeats an id), NrmError for tensors that are not on a CUDA device."""
     if not isinstance(table, wire.ArticleTable):
         raise ValueError('table must be a wire.ArticleTable')
     rows = table.rows
@@ -66,7 +85,12 @@ def _check_users_and_pool(table, hist_article, hist_time, hist_click, pool_time,
         raise ValueError(f'need B, H, N >= 1 (got {B}, {H}, {N})')
     if k is not None:
         _check_k(k, N)
-    tensors = (rows, hist_article, hist_time, hist_click, pool_article, pool_time)
+    if targets is not None:
+        _check_targets(targets, B)
+        if not targets.is_contiguous():
+            raise ValueError('targets must be contiguous')
+        _check_distinct_pool(pool_article, table.n)
+    tensors = (rows, hist_article, hist_time, hist_click, pool_article, pool_time) + ((targets,) if targets is not None else ())
     if not all(t.is_cuda for t in tensors):
         raise _lib.NrmError('recommend runs on CUDA tensors only (no CPU fallback)')
     if any(t.device != rows.device for t in tensors):
@@ -158,6 +182,136 @@ def select(logits: torch.Tensor, k: int, pool_article: torch.Tensor, n_articles:
     pos = pos.to(torch.int64)
     article = torch.where(pos >= 0, pa.to(torch.int64)[pos.clamp(min=0)], torch.full_like(pos, -1))
     return Recommendations(article, pos, val)
+
+
+def _check_targets(targets, B: int) -> int:
+    """-> P; ValueError unless targets is int32 [B,P] with 1 <= P <= 1024."""
+    if not isinstance(targets, torch.Tensor) or targets.dim() != 2 or targets.shape[0] != B or targets.dtype != torch.int32:
+        raise ValueError(f'targets must be int32 [B,P] with B = {B}, got {getattr(targets, "dtype", type(targets))} '
+                         f'{list(getattr(targets, "shape", []))}')
+    P = int(targets.shape[1])
+    if not 1 <= P <= TARGETS_MAX:
+        raise ValueError(f'targets must have 1 <= P <= {TARGETS_MAX} slots per user, got {P}')
+    return P
+
+
+def _check_distinct_pool(pool_article: torch.Tensor, n_articles: int) -> None:
+    """ValueError if an article id in [1, n_articles) occurs twice in the pool (one device sync for a CUDA pool)."""
+    ids = pool_article[(pool_article >= 1) & (pool_article < n_articles)]
+    if torch.unique(ids).numel() != ids.numel():
+        raise ValueError('pool_article holds a repeated article id: a target would have two ranks')
+
+
+def _rank(x, targets, pa, n_articles, ha) -> TargetRanks:
+    M, B, N = x.shape
+    P = int(targets.shape[1])
+    H = int(ha.shape[1]) if ha is not None else 0
+    dev = x.device
+    out = [torch.empty(B, P, dtype=torch.int32, device=dev) for _ in range(4)]
+    score = torch.empty(B, P, dtype=torch.float32, device=dev)
+    n_eligible = torch.empty(B, dtype=torch.int32, device=dev)
+    p = engine._ptr
+    _lib.check(_lib.load().nrm_pool_rank(p(x), M, B * N, B, N, p(pa), int(n_articles), p(ha), H, p(targets), P, *(p(t) for t in out),
+                                         p(score), p(n_eligible), _stream(dev)), 'nrm_pool_rank')
+    position, rank, greater, equal = (t.to(torch.int64) for t in out)
+    return TargetRanks(position, rank, greater, equal, score, n_eligible.to(torch.int64))
+
+
+def rank_targets(logits: torch.Tensor, targets: torch.Tensor, pool_article: torch.Tensor, n_articles: int, *,
+                 hist_article: Optional[torch.Tensor] = None) -> TargetRanks:
+    """Where each user's held-out targets land in the ranking `select` takes its first k entries of, on given logits ([B,N] or
+    [M,B,N] float32, M <= 16): the same eligibility, scores and stable order over the whole pool, with no limit on the rank.
+
+    `targets` int32 [B,P], 1 <= P <= 1024: article ids, 0 = pad slot.  A target is rankable if its id is in [1, n_articles), an
+    eligible pool position holds it, and no earlier slot of the user's row holds the same id; the others get position, rank,
+    greater and equal -1 and score NaN.  A rankable target is in `select(logits, k, ...)` iff its rank < k, at index rank.
+    `pool_article` must not repeat an id in [1, n_articles) (ValueError): a target would have two ranks.  That check costs one
+    device synchronisation per call."""
+    if logits.dim() == 2:
+        logits = logits.unsqueeze(0)
+    if logits.dim() != 3 or logits.dtype != torch.float32 or not 1 <= logits.shape[0] <= MODELS_MAX:
+        raise ValueError(f'logits must be float32 [B,N] or [M,B,N] with M <= {MODELS_MAX}, got {logits.dtype} {list(logits.shape)}')
+    M, B, N = logits.shape
+    _check_targets(targets, B)
+    if tuple(pool_article.shape) != (N,) or pool_article.dtype != torch.int32:
+        raise ValueError(f'pool_article must be int32 [{N}], got {pool_article.dtype} {list(pool_article.shape)}')
+    if hist_article is not None and (hist_article.dim() != 2 or hist_article.shape[0] != B or hist_article.dtype != torch.int32):
+        raise ValueError(f'hist_article must be int32 [B,H] with B = {B}, got {hist_article.dtype} {list(hist_article.shape)}')
+    _check_distinct_pool(pool_article, n_articles)
+    for t in (logits, targets, pool_article, hist_article):
+        if t is not None and not t.is_cuda:
+            raise _lib.NrmError('recommend runs on CUDA tensors only (no CPU fallback)')
+        if t is not None and t.device != logits.device:
+            raise ValueError('logits, targets, pool_article and hist_article must be on the same device')
+    return _rank(logits.contiguous(), targets.contiguous(), pool_article.contiguous(),
+                 n_articles, hist_article.contiguous() if hist_article is not None else None)
+
+
+def _check_ks(ks) -> tuple:
+    ks = tuple(ks)
+    if not ks or any(isinstance(k, bool) or not isinstance(k, int) or k < 1 for k in ks):
+        raise ValueError(f'ks must be a non-empty sequence of positive integers, got {ks!r}')
+    return ks
+
+
+def pool_metrics(ranks: TargetRanks, ks=(10,)) -> dict:
+    """Per-user metrics of pool recommendation from `rank_targets`' output, on its device.  T = the user's rankable targets.
+
+    For each k in `ks`, float32 [B]: `hit@k` 1 if some target has rank < k; `recall@k` #{rank < k} / T; `ndcg@k` the sum over
+    targets with rank < k of 1 / log2(rank + 2) over the ideal sum_{i < min(T, k)} 1 / log2(i + 2) (binary gains, as
+    `metrics.batch_metrics`).  Also `rr` 1 / (min rank + 1); `auc` the tie-averaged ROC AUC (sklearn's `roc_auc_score`) over the
+    user's eligible positions with the targets as positives, float32 [B]; `n_targets` T, int64 [B].  A user with T = 0, or (auc)
+    with no eligible position that is not a target, gets NaN: average with `torch.nanmean`.
+
+    The AUC needs no scores: a target with `greater` positions above it and `equal` tied has n_eligible - 1 - greater - equal below,
+    and summed over the targets the pairs of two targets contribute exactly T (T - 1) / 2, which leaves the target-negative pairs."""
+    ks = _check_ks(ks)
+    valid = ranks.rank >= 0
+    T = valid.sum(1)
+    Tf = T.to(torch.float64)
+    nan = torch.full_like(Tf, float('nan'))
+    rank = ranks.rank.to(torch.float64)
+    out = {}
+    for k in ks:
+        top = valid & (ranks.rank < k)
+        hits = top.sum(1).to(torch.float64)
+        dcg = torch.where(top, 1.0 / torch.log2(rank + 2.0), torch.zeros_like(rank)).sum(1)
+        ideal_terms = 1.0 / torch.log2(torch.arange(min(k, ranks.rank.shape[1]), dtype=torch.float64, device=rank.device) + 2.0)
+        ideal = torch.cumsum(ideal_terms, 0)[(T.clamp(max=k) - 1).clamp(min=0)]
+        out[f'hit@{k}'] = torch.where(T > 0, (hits > 0).to(torch.float64), nan).float()
+        out[f'recall@{k}'] = torch.where(T > 0, hits / Tf.clamp(min=1), nan).float()
+        out[f'ndcg@{k}'] = torch.where(T > 0, dcg / ideal, nan).float()
+    best = torch.where(valid, ranks.rank, torch.full_like(ranks.rank, torch.iinfo(torch.int64).max)).min(1).values
+    out['rr'] = torch.where(T > 0, 1.0 / (best.clamp(max=torch.iinfo(torch.int32).max).to(torch.float64) + 1.0), nan).float()
+    ne = ranks.n_eligible.to(torch.float64)
+    g, e = ranks.greater.to(torch.float64), ranks.equal.to(torch.float64)
+    below = torch.where(valid, ne[:, None] - 1.0 - g - e + 0.5 * e, torch.zeros_like(g)).sum(1)
+    n_neg = ne - Tf
+    out['auc'] = torch.where((T > 0) & (n_neg > 0), (below - Tf * (Tf - 1.0) / 2.0) / (Tf * n_neg).clamp(min=1), nan).float()
+    out['n_targets'] = T
+    return out
+
+
+def evaluate(models, table: wire.ArticleTable, hist_article, hist_time, hist_click, pool_time, targets, *, ks=(10,),
+             pool_article: Optional[torch.Tensor] = None, exclude_clicked: bool = True, chunk: Optional[int] = None):
+    """Offline evaluation of pool recommendation: `pool_logits` of every model in `models` (one `UserModel` or up to 16), then
+    `rank_targets` of each user's held-out clicked articles `targets` (int32 [B,P], 0 = pad) in the ranking `top_articles` uses,
+    then `pool_metrics`.  Arguments as for `top_articles`.  -> (metrics dict, TargetRanks)."""
+    if isinstance(models, torch.nn.Module):
+        models = [models]
+    models = list(models)
+    if not 1 <= len(models) <= MODELS_MAX:
+        raise ValueError(f'need 1 to {MODELS_MAX} models, got {len(models)}')
+    _check_chunk(chunk)
+    ks = _check_ks(ks)
+    B, H, N, pa = _check_users_and_pool(table, hist_article, hist_time, hist_click, pool_time, pool_article, targets=targets)
+    with torch.no_grad():
+        logits = torch.empty(len(models), B, N, dtype=torch.float32, device=hist_article.device)
+        c = chunk if chunk is not None else default_chunk(B, H, N)
+        for m, model in enumerate(models):
+            _forward_pool(model, table, hist_article, hist_time, hist_click, pool_time, pa, B, H, N, c, logits[m])
+        ranks = _rank(logits, targets, pa, table.n, hist_article if exclude_clicked else None)
+        return pool_metrics(ranks, ks), ranks
 
 
 def top_articles(models, table: wire.ArticleTable, hist_article, hist_time, hist_click, pool_time, k: int, *,
