@@ -7,7 +7,7 @@ Buffer names follow the training workspace (nrm_debug_ws_field): xh [B*H,64], e 
 dxt [R,64], dxin_h [B*H,66], dtp [2,R,64] (dL/dtp of the label and the text/img branch), plus logits [R]."""
 from __future__ import annotations
 
-from typing import Dict, Optional
+from typing import Dict, Optional, Tuple
 
 import torch
 
@@ -30,9 +30,11 @@ def grad_stage(key: str) -> str:
 
 
 def stage_references(p, x_history, x_target, x_global, G, gpu: Optional[Dict[str, torch.Tensor]] = None,
-                     dtype=torch.float64):
-    """p: parameters (dtype, on the inputs' device); x_*: packed rows; G [B,C]: the cotangent of the logits.
-    Returns (ref, grads): ref = dict of reference buffers (names as above), grads = parameter gradients by key."""
+                     dtype=torch.float64, training: bool = True, stats: Optional[Tuple[torch.Tensor, torch.Tensor]] = None):
+    """p: parameters (dtype, on the inputs' device); x_*: packed rows; G [B,C]: the cotangent of the logits, or None for the
+    forward stages alone (no backward buffers, no gradients).  training / stats: the head's BatchNorm, as M.head_forward takes
+    them (training=False: `stats` = (mean, var), the running statistics of `p` when None; the backward is then the frozen-
+    statistics one).  Returns (ref, grads): ref = dict of reference buffers (names as above), grads = parameter gradients by key."""
     B, H, _ = x_history.shape
     C = x_target.shape[1]
     R = B * C
@@ -57,9 +59,11 @@ def stage_references(p, x_history, x_target, x_global, G, gpu: Optional[Dict[str
     ti_P, ti_saved = M.attention_forward(p, TI, t_ti, pca_h)
     ref['e'] = torch.cat([lab_P.reshape(R, 64), ti_P.reshape(R, 64), eu_l, xt, pca_t], dim=1)
 
-    # head: BatchNorm statistics recomputed from the e it is fed
-    r, head_saved = M.head_forward(p, up('e', ref['e']), training=True)
+    # head: BatchNorm statistics recomputed from the e it is fed (training), or the given / running ones
+    r, head_saved = M.head_forward(p, up('e', ref['e']), training=training, stats=stats)
     ref['logits'] = r
+    if G is None:
+        return ref, grads
     ref['de'] = M.head_backward(p, head_saved, G.reshape(R).to(dtype), grads)
 
     # encoder backward

@@ -76,43 +76,18 @@ The FFMA backward of fp32 never writes dtp; each fp32 case says so with a DtpNot
 
 Set NRM_STAGEWISE_FLOORS=<path> to write the floors measured by a run as JSON.
 """
-import ctypes
-import json
-import os
 import warnings
 
-import numpy as np
 import pytest
 import torch
 
-import news_recommendation_model_b200 as nrm
-from news_recommendation_model_b200 import _lib
-from fixtures import load_weights
 from news_recommendation_model_b200.synthetic import make_batch
-from oracle import reference_port as O
+from stagewise_gpu import (CASE, CASE_IDS, DEV, PRECISIONS, USERS, DtpNotWritten, check_grad, check_rows, cotangent,
+                           params64, report_floors, ws_fields)
+from stagewise_gpu import batch as _batch, model as _model
 from stagewise_ref import grad_stage, stage_references
 
 pytestmark = pytest.mark.gpu
-
-DEV = 'cuda'
-USERS = 50
-PRECISIONS = ('fp32', 'bf16x3', 'bf16')
-
-# (id, B, H, C, make_batch options, regime)
-CASES = [
-    ('b2_h1_c1', 2, 1, 1, {}, 'smallest training batch'),
-    ('b1_h50_c5', 1, 50, 5, {}, 'B = 1: batch-stride branch of engine.forward_logits'),
-    ('b7_h65_c8', 7, 65, 8, {}, 'G = 1 with a full group of 8; history chunks of 64 + 1 rows'),
-    ('b150_h50_c9', 150, 50, 9, dict(variable_candidates=True),
-     'G = 2, 300 units over 148 CTAs: atomic dxh, groups of one impression on different CTAs, last group of 1'),
-    ('b160_h129_c17', 160, 129, 17, dict(variable_history=True),
-     'G = 3, B > 148: CTAs holding two impressions on the read-modify-write dxh path; chunks of 64 + 64 + 1 rows'),
-    ('b40_h64_c40', 40, 64, 40, {}, 'G = 5: 8 x 64 = 512 stacked rows, exactly 4 tiles per chunk'),
-    ('b300_h37_c5', 300, 37, 5, {}, 'G = 1 with several units per CTA; FFMA persistent backward with B > 148'),
-    ('b2000_h20_c5', 2000, 20, 5, {}, 'R = 10000 > 148 * 64: tensor-core head CTAs with several tiles, last-CTA BatchNorm sums'),
-]
-CASE_IDS = [c[0] for c in CASES]
-CASE = {c[0]: c for c in CASES}
 
 # rtol per buffer and precision (see the module docstring for the floors they come from): RTOL for every case with B >= 7, RTOL_SMALL
 # for the two ill-conditioned smallest batches (SMALL_CASES)
@@ -139,46 +114,7 @@ def rtol_for(precision, name, case_id):
     return (RTOL_SMALL if case_id in SMALL_CASES else RTOL)[precision][name]
 
 
-ATOL_FRACTION = 0.01   # atol = rtol / 100, for impressions whose own scale is near zero
 FLOORS = {}            # (precision, buffer, case id) -> worst err / impression scale seen by this run
-
-class DtpNotWritten(UserWarning):
-    """The precision under test does not write the dtp workspace buffer, so it is not compared."""
-
-
-WS_FIELDS = ('xh', 'e', 'de', 'dtp', 'dxh', 'dxt', 'dxin_h')
-MODE_TRAIN = 3         # MODE_BN_BATCH_STATS | MODE_KEEP_FOR_BWD
-
-
-def _batch(case):
-    _, B, H, C, kw, _ = case
-    return make_batch(B, H, C, seed=B * 1000 + H * 10 + C, user_num=USERS, fp32_exact=True, **kw)
-
-
-def _cotangent(B, C):
-    return torch.randn(B, C, generator=torch.Generator().manual_seed(B * 7 + C), dtype=torch.float32)
-
-
-def _model(precision):
-    model = nrm.UserModel(USERS)
-    model.load_state_dict(load_weights('train'), strict=False)
-    return model.to(DEV).train().set_precision(precision)
-
-
-def _ws_fields(model, B, H, C):
-    lib = _lib.load()
-    ws = model._runtime().train_ws
-    out = {}
-    for f in WS_FIELDS:
-        nb = ctypes.c_longlong()
-        off = lib.nrm_debug_ws_field(B, H, C, MODE_TRAIN, f.encode(), ctypes.byref(nb))
-        assert off >= 0, f
-        out[f] = ws[off:off + nb.value].view(torch.float32).clone()
-    R, NH = B * C, B * H
-    out['xh'] = out['xh'].view(NH, 64); out['dxh'] = out['dxh'].view(NH, 64); out['dxin_h'] = out['dxin_h'].view(NH, 66)
-    out['e'] = out['e'].view(R, 264); out['de'] = out['de'].view(R, 264); out['dxt'] = out['dxt'].view(R, 64)
-    out['dtp'] = out['dtp'].view(2, R, 64)
-    return out
 
 
 def gpu_step(model, x_history, x_target, x_global, G):
@@ -189,40 +125,16 @@ def gpu_step(model, x_history, x_target, x_global, G):
     torch.cuda.synchronize()
     B, H, C = x_history.shape[0], x_history.shape[1], x_target.shape[1]
     grads = {k: v.grad.detach().clone() for k, v in model.named_parameters() if v.grad is not None}
-    return out.detach().clone(), _ws_fields(model, B, H, C), grads
+    return out.detach().clone(), ws_fields(model, B, H, C), grads
 
 
 def run_case(case_id, precision):
     case = CASE[case_id]
     b = _batch(case)
     d = b.to(DEV)
-    G = _cotangent(case[1], case[3]).to(DEV)
+    G = cotangent(case[1], case[3]).to(DEV)
     logits, bufs, grads = gpu_step(_model(precision), d.x_history, d.x_target, d.x_global, G)
     return dict(logits=logits, bufs=bufs, grads=grads)
-
-
-def _params64():
-    p = O.load_params(load_weights('train'), dtype=torch.float64, user_num=USERS)
-    return {k: v.to(DEV) for k, v in p.items()}
-
-
-def _check_rows(name, got, ref, precision, case, failures):
-    """got / ref [B, n, k]; per impression scale."""
-    rtol = rtol_for(precision, name, case[0])
-    got, ref = got.double(), ref.double()
-    err = torch.nan_to_num((got - ref).abs(), nan=float('inf'))
-    imp = ref.abs().amax(dim=(1, 2))
-    buf = ref.abs().max()
-    ratio = err / imp.clamp_min(1e-30)[:, None, None]
-    key = (precision, name, case[0])
-    FLOORS[key] = max(FLOORS.get(key, 0.0), float(ratio.max()))
-    allowed = rtol * imp[:, None, None] + ATOL_FRACTION * rtol * buf
-    over = err / allowed.clamp_min(1e-30)
-    if float(over.max()) > 1.0:
-        b, n, k = np.unravel_index(int(over.argmax()), tuple(over.shape))
-        idx = 'h' if name in ('xh', 'dxh', 'dxin_h') else 'c'
-        failures.append(f'{name} [{precision}, {case[0]}: {case[5]}]: worst at b={b} {idx}={n} col={k}: gpu {float(got[b, n, k]):.6e} '
-                        f'ref {float(ref[b, n, k]):.6e}, err / impression scale {float(ratio[b, n, k]):.2e} > rtol {rtol:.1e}')
 
 
 def check_step(case, precision, res, failures):
@@ -231,13 +143,15 @@ def check_step(case, precision, res, failures):
     R = B * C
     b = _batch(case)
     bufs = {k: v.to(DEV) for k, v in res['bufs'].items()}
-    G = _cotangent(B, C).to(DEV)
+    G = cotangent(B, C).to(DEV)
     up = {k: bufs[k].double() for k in ('xh', 'e', 'de', 'dxh', 'dxt', 'dxin_h')}
     with torch.no_grad():
-        ref, grads = stage_references(_params64(), b.x_history.to(DEV), b.x_target.to(DEV), b.x_global.to(DEV), G.double(), gpu=up)
+        ref, grads = stage_references(params64(), b.x_history.to(DEV), b.x_target.to(DEV), b.x_global.to(DEV), G.double(), gpu=up)
     rows_h = lambda t: t.reshape(B, H, -1)
     rows_c = lambda t: t.reshape(B, C, -1)
-    chk = lambda name, g, r: _check_rows(name, g, r, precision, case, failures)
+    label = f'{precision}, {case[0]}: {case[5]}'
+    chk = lambda name, g, r: check_rows(name, g, r, rtol_for(precision, name, case[0]), label, FLOORS, (precision, name, case[0]),
+                                        failures)
     chk('xh', rows_h(bufs['xh']), rows_h(ref['xh']))
     chk('e_label', rows_c(bufs['e'][:, 0:64]), rows_c(ref['e'][:, 0:64]))
     chk('e_textimg', rows_c(bufs['e'][:, 64:128]), rows_c(ref['e'][:, 64:128]))
@@ -257,35 +171,15 @@ def check_step(case, precision, res, failures):
         if k == 'delta':
             continue
         name = 'grad_' + grad_stage(k)
-        g = res['grads'][k].to(DEV).double()
-        err = float(torch.nan_to_num((g - r).abs(), nan=float('inf')).max())
-        scale = max(float(r.abs().max()), 1e-30)
-        key = (precision, name, case[0])
-        FLOORS[key] = max(FLOORS.get(key, 0.0), err / scale)
-        rtol = rtol_for(precision, name, case[0])
-        if err > rtol * scale:
-            failures.append(f'{name} {k} [{precision}, {case[0]}: {case[5]}]: max err {err:.3e} = {err / scale:.2e} of max|ref| {scale:.3e} '
-                            f'> rtol {rtol:.1e}')
+        check_grad(name, k, res['grads'][k].to(DEV), r, rtol_for(precision, name, case[0]), label, FLOORS, (precision, name, case[0]),
+                   failures)
 
 
 @pytest.fixture(scope='module', autouse=True)
 def _report_floors():
     yield
-    if not FLOORS:
-        return
-    worst = {}
-    for (prec, name, cid), v in FLOORS.items():
-        key = (cid in SMALL_CASES, prec, name)
-        if v >= worst.get(key, (-1.0, ''))[0]:
-            worst[key] = (v, cid)
-    lines = ['measured floors (worst err / impression scale over the cases run):']
-    for (small, prec, name), (v, cid) in sorted(worst.items()):
-        lines.append(f'  {"small" if small else "B >= 7":6s} {prec:7s} {name:15s} {v:.3e} ({cid})   rtol {rtol_for(prec, name, cid):.1e}')
-    print('\n'.join(lines))
-    path = os.environ.get('NRM_STAGEWISE_FLOORS')
-    if path:
-        with open(path, 'w') as f:
-            json.dump({f'{p}/{n}/{c}': v for (p, n, c), v in sorted(FLOORS.items())}, f, indent=1)
+    report_floors(FLOORS, lambda k: (k[2] in SMALL_CASES, k[0], k[1]),
+                  lambda g: f'{"small" if g[0] else "B >= 7":6s} {g[1]:7s} {g[2]:15s}', lambda k: rtol_for(*k))
 
 
 @pytest.mark.parametrize('precision', PRECISIONS)
@@ -305,7 +199,7 @@ def test_trimmed_candidate_views_bit_identical(precision):
     b = make_batch(B, H, C, seed=404, user_num=USERS, variable_candidates=True).to(DEV)
     xt, xg = b.x_target[:, :keep], b.x_global[:, :keep]
     assert xt.stride(0) == C * xt.shape[2] and not xt.is_contiguous()
-    G = _cotangent(B, keep).to(DEV)
+    G = cotangent(B, keep).to(DEV)
     model = _model(precision)
     l_view, _, g_view = gpu_step(model, b.x_history, xt, xg, G)
     l_copy, _, g_copy = gpu_step(model, b.x_history, xt.contiguous(), xg.contiguous(), G)
@@ -324,7 +218,7 @@ def test_dxh_bit_identical_run_to_run(case_id, precision):
     soon as an element gets a third addend in run-dependent order (more groups, or chunks of one group added separately)."""
     case = CASE[case_id]
     b = _batch(case).to(DEV)
-    G = _cotangent(case[1], case[3]).to(DEV)
+    G = cotangent(case[1], case[3]).to(DEV)
     model = _model(precision)
     _, first, _ = gpu_step(model, b.x_history, b.x_target, b.x_global, G)
     _, second, _ = gpu_step(model, b.x_history, b.x_target, b.x_global, G)

@@ -43,19 +43,21 @@ def _capture(monkeypatch):
     return cap
 
 
-@pytest.mark.parametrize('B,H,C,kw', [(5, 13, 9, dict(variable_history=True, variable_candidates=True)), (2, 1, 1, {})])
-def test_chained_stages_equal_autograd_in_float64(B, H, C, kw, monkeypatch):
+PADDED = (5, 13, 9, dict(variable_history=True, variable_candidates=True))
+
+
+def _compare_with_autograd(B, H, C, kw, checkpoint, training, monkeypatch):
     b = make_batch(B, H, C, seed=11 + B, user_num=20, **kw)
-    p = O.load_params(load_weights('train'), dtype=torch.float64, user_num=20)
+    p = O.load_params(load_weights(checkpoint), dtype=torch.float64, user_num=20)
     G = torch.randn(B, C, generator=torch.Generator().manual_seed(3), dtype=torch.float64)
     leaves = {k: p[k].clone().requires_grad_(True) for k in O.TRAINABLE_KEYS}
     pa = dict(p, **leaves)
     cap = _capture(monkeypatch)
-    out = O.user_model_forward(pa, b.x_history, b.x_target, b.x_global, training=True, dtype=torch.float64,
+    out = O.user_model_forward(pa, b.x_history, b.x_target, b.x_global, training=training, dtype=torch.float64,
                                update_running_stats=False)
     out.backward(G)
     monkeypatch.undo()
-    ref, grads = stage_references(p, b.x_history, b.x_target, b.x_global, G)
+    ref, grads = stage_references(p, b.x_history, b.x_target, b.x_global, G, training=training)
 
     def same(name, got, want):
         assert got.shape == want.shape, name
@@ -71,6 +73,38 @@ def test_chained_stages_equal_autograd_in_float64(B, H, C, kw, monkeypatch):
     same('dxin_h', ref['dxin_h'][:, 0:64], torch.cat([emb_h.grad, time_h.grad], dim=2).reshape(B * H, 64))
     for i, prefix in enumerate((O.II + 'label_attention.mlp.', O.II + 'text_img_attention.mlp.')):
         same('dtp', ref['dtp'][i], cap['pre'][prefix].grad.reshape(B, C, H, 64).sum(2).reshape(R, 64))
+    assert leaves.keys() == {k for k in grads if k != 'delta'}
     for k, leaf in leaves.items():
         assert grad_stage(k) in ('head', 'attention', 'w1', 'embed')
         same(k, grads[k], leaf.grad)
+
+
+@pytest.mark.parametrize('B,H,C,kw', [PADDED, (2, 1, 1, {})])
+def test_chained_stages_equal_autograd_in_float64(B, H, C, kw, monkeypatch):
+    _compare_with_autograd(B, H, C, kw, 'train', True, monkeypatch)
+
+
+@pytest.mark.parametrize('checkpoint', ['train', 'validation'])
+@pytest.mark.parametrize('B,H,C,kw', [PADDED, (1, 1, 1, {})])
+def test_chained_eval_stages_equal_autograd_in_float64(B, H, C, kw, checkpoint, monkeypatch):
+    """Eval mode: BatchNorm with the checkpoint's running statistics, and the frozen-statistics backward (model.eval() with
+    gradients enabled).  The train checkpoint has running variances down to about 3.4e-4, the validation one near-dead
+    channels whose 1 / sqrt(var + eps) reaches about 316; bn.weight / bn.bias gradients are taken with the running-statistics
+    xhat."""
+    _compare_with_autograd(B, H, C, kw, checkpoint, False, monkeypatch)
+
+
+def test_forward_only_references_equal_the_chained_ones():
+    B, H, C, kw = PADDED
+    b = make_batch(B, H, C, seed=11 + B, user_num=20, **kw)
+    p = O.load_params(load_weights('validation'), dtype=torch.float64, user_num=20)
+    G = torch.randn(B, C, generator=torch.Generator().manual_seed(3), dtype=torch.float64)
+    stats = (p['bn.running_mean'] * 1.5, p['bn.running_var'] * 0.5)
+    full, _ = stage_references(p, b.x_history, b.x_target, b.x_global, G, training=False, stats=stats)
+    fwd, grads = stage_references(p, b.x_history, b.x_target, b.x_global, None, training=False, stats=stats)
+    assert fwd.keys() == {'xh', 'e', 'logits'}
+    for k, v in fwd.items():
+        assert torch.equal(v, full[k]), k
+    assert all(not bool(g.any()) for g in grads.values())
+    running, _ = stage_references(p, b.x_history, b.x_target, b.x_global, None, training=False)
+    assert not torch.equal(running['logits'], fwd['logits'])       # the given statistics are the ones used
