@@ -280,6 +280,27 @@ int nrm_pool_topk(const float* logits, int n_models, long long model_stride, int
 int nrm_pool_rank(const float* logits, int n_models, long long model_stride, int B, int N, const int* pool_article, int n_articles,
                   const int* hist_article, int H, const int* targets, int P, int* pos_out, int* rank_out, int* greater_out,
                   int* equal_out, float* score_out, int* n_eligible_out, void* stream);
+/*   nrm_pool_diversify: per user b, k of the user's candidates picked by greedy maximal marginal relevance (MMR), with an optional
+ *     cap per category.  cand_pos int32 / cand_score float32 [B,n_cand] are nrm_pool_topk's pos_out / val_out for k = n_cand (the
+ *     candidates, in that order: candidate index i is the slot); a slot at position -1 is not a candidate (nor is one whose position
+ *     is outside [0, N) or whose pool_article id is outside [1, n_articles), which nrm_pool_topk never writes).  article_rows: the
+ *     float32 [n_articles,80] article table (columns 0-63 the PCA vector, column 64 the category id).  In float32:
+ *       rel_i   min-max normalised score: (s_i - s_min) / (s_max - s_min) over the user's finite candidate scores, computed on
+ *               halved operands when s_max - s_min exceeds FLT_MAX; 1 if s_max == s_min; +inf -> 1, -inf -> 0;
+ *       u_i     v_i / sqrtf(sum_j v_ij^2) of the PCA columns v_i (correctly rounded sqrt and division; 0 for an all-zero v_i);
+ *       sim     u_i . u_j (fused multiply-adds in column order), 0 when either vector is zero;
+ *       m_i     max over the picked set S of sim(i, j), 0 while S is empty;
+ *       gain_i  lambda * rel_i - (1 - lambda) * m_i.
+ *     Each step picks the unpicked candidate with the largest gain, ties to the lower index; with max_per_category = q > 0 a
+ *     candidate whose category ((int) of column 64) already has q picks cannot be picked (q = 0: no cap).  The selection stops
+ *     after k picks or when nothing can be picked.  Per slot, int32 / float32 [B,k]: pos_out the pick's pool position, val_out its
+ *     candidate score, gain_out its gain when picked; slots left over get -1 / NaN / NaN.
+ *     1 <= k <= n_cand <= min(N, 512), 0 <= lambda <= 1, q >= 0.
+ *     Exactness: with lambda = 1 and q = 0 the gain is rel, which does not decrease along the candidates, and ties go to the lower
+ *     index, so pos_out / val_out are bit-identical to nrm_pool_topk's with the same k. */
+int nrm_pool_diversify(const int* cand_pos, const float* cand_score, int B, int n_cand, int k, float lambda, int max_per_category,
+                       const int* pool_article, int N, const float* article_rows, int n_articles, int* pos_out, float* val_out,
+                       float* gain_out, void* stream);
 
 /* ---- UserModel.loss (user_model.py:37-43) ---------------------------------------- */
 /* loss = (1-alpha) BCE(softmax(out), y) + alpha BCE(softmax(out + delta[id]), y), mean

@@ -83,6 +83,10 @@ int launch_pool_topk(const float* logits, int n_models, long long model_stride, 
 int launch_pool_rank(const float* logits, int n_models, long long model_stride, int B, int N, const int* pool_article, int n_articles,
                      const int* hist_article, int H, const int* targets, int P, int* pos_out, int* rank_out, int* greater_out,
                      int* equal_out, float* score_out, int* n_eligible_out, cudaStream_t s);
+// nrm_recommend.cu: per user, k of the nrm_pool_topk candidates picked by greedy maximal marginal relevance (nrm_pool_diversify)
+int launch_pool_diversify(const int* cand_pos, const float* cand_score, int B, int n_cand, int k, float lambda, int max_per_category,
+                          const int* pool_article, int N, const float* article_rows, int n_articles, int* pos_out, float* val_out,
+                          float* gain_out, cudaStream_t s);
 
 // nrm_head.cu
 int launch_bn_partial_sums(Workspace& w, cudaStream_t s);                 // -> w.bn_sums

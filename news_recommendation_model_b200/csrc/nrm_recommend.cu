@@ -520,6 +520,150 @@ int launch_pool_rank(const float* logits, int n_models, long long model_stride, 
   return NRM_OK;
 }
 
+// ---- nrm_pool_diversify: greedy maximal-marginal-relevance re-ranking of a user's nrm_pool_topk candidates ----------------------
+// One CTA per user, thread i owns candidate i (n_cand <= POOL_THREADS; the CTA is n_cand rounded up to a warp).  A thread keeps its
+// candidate's unit PCA vector (article row columns 0-63), relevance, category (column 64), running max similarity to the picks and
+// its state in registers.  Per step the winner of the last step publishes its vector and category to shared memory, every live
+// candidate updates its max similarity with one 64-term dot product and its category's pick count by comparing categories, and a
+// block arg-max over the keys pool_key(gain, i) picks the next candidate (unique keys: largest gain, ties to the lower index).
+// Every reduction reads the warp results in one fixed order, so the picks do not depend on timing.
+constexpr int PCA_COLS = 64, ARTICLE_COLS = 80, CATEGORY_COL = 64;
+
+struct PoolDiversifyArgs {
+  const int* cand_pos; const float* cand_score; int n_cand, k;
+  float lambda; int max_per_category;
+  const int* pool_article; int N;
+  const float* article_rows; int n_articles;
+  int* pos_out; float* val_out; float* gain_out;
+};
+
+// the largest v over the CTA, for every thread.  red[16] must not be read by another reduction before the barrier inside the next
+// call on the same buffer: alternate two buffers between consecutive calls.
+__device__ __forceinline__ unsigned long long diversify_block_max(unsigned long long v, unsigned long long* red) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const unsigned long long w = __shfl_xor_sync(0xffffffffu, v, o);
+    v = w > v ? w : v;
+  }
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
+  __syncthreads();
+  v = red[0];
+  for (int w = 1; w < (int)(blockDim.x >> 5); ++w) v = red[w] > v ? red[w] : v;
+  return v;
+}
+
+// a float's bits in an unsigned order that follows the float order (-0.0 == +0.0), as in pool_key
+__device__ __forceinline__ unsigned diversify_ordered(float x) {
+  const unsigned u = __float_as_uint(x + 0.0f);
+  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+
+__global__ void __launch_bounds__(POOL_THREADS, 1)
+pool_diversify_kernel(const PoolDiversifyArgs a) {
+  __shared__ unsigned long long red[2][POOL_THREADS / 32];
+  __shared__ float4 pick_vec[PCA_COLS / 4];
+  __shared__ int pick_cat;
+  const int i = threadIdx.x, b = blockIdx.x;
+  const long long o = (long long)b * a.n_cand + i;
+
+  // this thread's candidate: a slot past n_cand, at position -1 (or one select never writes) is none
+  int pos = i < a.n_cand ? a.cand_pos[o] : -1;
+  const int id = pos >= 0 && pos < a.N ? __ldg(a.pool_article + pos) : 0;
+  if (id < 1 || id >= a.n_articles) pos = -1;
+  const float score = pos >= 0 ? a.cand_score[o] : 0.f;
+  float u[PCA_COLS];
+  int cat = 0;
+  if (pos >= 0) {
+    const float* r = a.article_rows + (long long)id * ARTICLE_COLS;
+#pragma unroll
+    for (int j = 0; j < PCA_COLS; ++j) u[j] = __ldg(r + j);
+    cat = (int)__ldg(r + CATEGORY_COL);
+  } else {
+#pragma unroll
+    for (int j = 0; j < PCA_COLS; ++j) u[j] = 0.f;
+  }
+  float ss = 0.f;
+#pragma unroll
+  for (int j = 0; j < PCA_COLS; ++j) ss = fmaf(u[j], u[j], ss);
+  if (ss > 0.f) {                                          // an all-zero vector stays zero: similarity 0 to everything
+    const float nrm = __fsqrt_rn(ss);
+#pragma unroll
+    for (int j = 0; j < PCA_COLS; ++j) u[j] = __fdiv_rn(u[j], nrm);
+  }
+
+  // relevance: min-max over the finite candidate scores (0 in the ordered bits: none); +inf -> 1, -inf -> 0, all equal -> 1
+  const bool fin = pos >= 0 && isfinite(score);
+  const unsigned long long hi = diversify_block_max(fin ? diversify_ordered(score) : 0u, red[0]);
+  const unsigned long long lo = diversify_block_max(fin ? ~diversify_ordered(score) : 0u, red[1]);
+  const float s_max = pool_key_score(hi << 32), s_min = pool_key_score((~lo & 0xffffffffull) << 32);
+  float rel = 1.f;
+  if (score == -CUDART_INF_F) rel = 0.f;
+  else if (score != CUDART_INF_F && hi != 0ull && s_max > s_min) {
+    const float d = __fsub_rn(s_max, s_min);
+    rel = isfinite(d) ? __fdiv_rn(__fsub_rn(score, s_min), d)   // |s_max - s_min| beyond FLT_MAX: halve both operands first
+                      : __fdiv_rn(__fsub_rn(0.5f * score, 0.5f * s_min), __fsub_rn(0.5f * s_max, 0.5f * s_min));
+  }
+
+  const int q = a.max_per_category;
+  const float lam = a.lambda, mu = 1.f - a.lambda;
+  bool live = pos >= 0;                                    // a candidate, not picked, its category below the cap
+  float m = 0.f;
+  int same = 0, t = 0;                                     // t: picks so far
+  while (true) {
+    const float gain = __fsub_rn(__fmul_rn(lam, rel), __fmul_rn(mu, m));
+    const unsigned long long best = diversify_block_max(live ? pool_key(gain, i) : 0ull, red[t & 1]);
+    if (best == 0ull) break;                               // nothing left that may be picked
+    if (i == (int)~(unsigned)best) {
+      live = false;
+      const long long out = (long long)b * a.k + t;
+      a.pos_out[out] = pos;
+      a.val_out[out] = score;
+      a.gain_out[out] = gain;
+#pragma unroll
+      for (int j = 0; j < PCA_COLS / 4; ++j) pick_vec[j] = make_float4(u[4 * j], u[4 * j + 1], u[4 * j + 2], u[4 * j + 3]);
+      pick_cat = cat;
+    }
+    if (++t == a.k) break;
+    __syncthreads();                                       // the pick is published; red[(t - 1) & 1] has been read by every thread
+    if (live) {
+      float d = 0.f;
+#pragma unroll
+      for (int j = 0; j < PCA_COLS / 4; ++j) {
+        const float4 p = pick_vec[j];
+        d = fmaf(u[4 * j], p.x, d);
+        d = fmaf(u[4 * j + 1], p.y, d);
+        d = fmaf(u[4 * j + 2], p.z, d);
+        d = fmaf(u[4 * j + 3], p.w, d);
+      }
+      m = t == 1 ? d : fmaxf(m, d);                          // 0 only while nothing is picked: m may be negative
+      if (q > 0 && pick_cat == cat && ++same >= q) live = false;
+    }
+  }
+  for (int j = t + i; j < a.k; j += blockDim.x) {
+    const long long out = (long long)b * a.k + j;
+    a.pos_out[out] = -1;
+    a.val_out[out] = CUDART_NAN_F;
+    a.gain_out[out] = CUDART_NAN_F;
+  }
+}
+
+int launch_pool_diversify(const int* cand_pos, const float* cand_score, int B, int n_cand, int k, float lambda, int max_per_category,
+                          const int* pool_article, int N, const float* article_rows, int n_articles, int* pos_out, float* val_out,
+                          float* gain_out, cudaStream_t s) {
+  if (n_cand < 1 || n_cand > N || n_cand > POOL_THREADS) {
+    set_error("nrm_pool_diversify: need 1 <= n_cand <= min(N, %d) (got n_cand = %d, N = %d)", POOL_THREADS, n_cand, N);
+    return NRM_EINVAL;
+  }
+  if (k < 1 || k > n_cand) { set_error("nrm_pool_diversify: need 1 <= k <= n_cand (got k = %d, n_cand = %d)", k, n_cand); return NRM_EINVAL; }
+  if (!(lambda >= 0.f && lambda <= 1.f)) { set_error("nrm_pool_diversify: need 0 <= lambda <= 1 (got %g)", (double)lambda); return NRM_EINVAL; }
+  if (max_per_category < 0) { set_error("nrm_pool_diversify: max_per_category must be >= 0 (got %d)", max_per_category); return NRM_EINVAL; }
+  const PoolDiversifyArgs args{cand_pos, cand_score, n_cand, k, lambda, max_per_category, pool_article, N, article_rows, n_articles,
+                               pos_out, val_out, gain_out};
+  pool_diversify_kernel<<<B, (n_cand + 31) / 32 * 32, 0, s>>>(args);
+  NRM_LAUNCH_CHECK("pool_diversify_kernel");
+  return NRM_OK;
+}
+
 }  // namespace nrm
 
 using namespace nrm;
@@ -542,4 +686,16 @@ extern "C" int nrm_pool_rank(const float* logits, int n_models, long long model_
   if (B <= 0 || N <= 0 || n_articles <= 0) { set_error("nrm_pool_rank: B, N, n_articles must be positive (got %d, %d, %d)", B, N, n_articles); return NRM_EINVAL; }
   return launch_pool_rank(logits, n_models, model_stride, B, N, pool_article, n_articles, hist_article, H, targets, P, pos_out, rank_out,
                           greater_out, equal_out, score_out, n_eligible_out, (cudaStream_t)stream);
+}
+
+extern "C" int nrm_pool_diversify(const int* cand_pos, const float* cand_score, int B, int n_cand, int k, float lambda,
+                                  int max_per_category, const int* pool_article, int N, const float* article_rows, int n_articles,
+                                  int* pos_out, float* val_out, float* gain_out, void* stream) {
+  if (!cand_pos || !cand_score || !pool_article || !article_rows || !pos_out || !val_out || !gain_out) {
+    set_error("nrm_pool_diversify: null pointer");
+    return NRM_EINVAL;
+  }
+  if (B <= 0 || N <= 0 || n_articles <= 0) { set_error("nrm_pool_diversify: B, N, n_articles must be positive (got %d, %d, %d)", B, N, n_articles); return NRM_EINVAL; }
+  return launch_pool_diversify(cand_pos, cand_score, B, n_cand, k, lambda, max_per_category, pool_article, N, article_rows, n_articles,
+                               pos_out, val_out, gain_out, (cudaStream_t)stream);
 }

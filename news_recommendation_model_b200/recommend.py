@@ -20,10 +20,18 @@ one lands in that user's ranking of the whole pool, `pool_metrics` turns those r
 `evaluate` runs the three steps from the models:
 
     metrics, ranks = recommend.evaluate([m1, m2], table, hist_article, hist_time, hist_click, pool_time, targets, ks=(10, 100))
-    torch.nanmean(metrics['ndcg@10'])"""
+    torch.nanmean(metrics['ndcg@10'])
+
+A ranking by relevance alone tends to fill a user's list with near-copies.  `diversify` / `diverse_articles` re-rank each user's
+best candidates by greedy maximal marginal relevance over the articles' PCA vectors, optionally with a cap per category
+(`nrm_pool_diversify`), and `list_diversity` measures what that bought:
+
+    rec = recommend.diverse_articles(model, table, hist_article, hist_time, hist_click, pool_time, 10, lam=0.7, max_per_category=3)
+    ild, n_categories = recommend.list_diversity(table, rec.article)"""
 from __future__ import annotations
 
 import ctypes
+import numbers
 from typing import NamedTuple, Optional
 
 import torch
@@ -32,6 +40,7 @@ from . import _lib, engine, wire
 
 TOPK_MAX = 1024
 TARGETS_MAX = 1024
+CANDIDATES_MAX = 512                  # diversify: one thread per candidate in a 512-thread CTA
 MODELS_MAX = 16
 CHUNK_ALIGN = 8                       # the attention's candidate group: every multiple of it gives the same logits
 WORKSPACE_TARGET = 1 << 30            # chunk=None: the largest chunk whose workspace stays under 1 GiB
@@ -335,3 +344,130 @@ def top_articles(models, table: wire.ArticleTable, hist_article, hist_time, hist
         for m, model in enumerate(models):
             _forward_pool(model, table, hist_article, hist_time, hist_click, pool_time, pa, B, H, N, c, logits[m])
         return select(logits, k, pa, table.n, hist_article=hist_article if exclude_clicked else None)
+
+
+class DiverseRecommendations(NamedTuple):
+    article: torch.Tensor     # [B,k] int64 pool article ids in pick order (-1: fewer than k picks)
+    position: torch.Tensor    # [B,k] int64 positions in the pool (-1 likewise)
+    score: torch.Tensor       # [B,k] float32 the pick's ranking score, as `select` returns it (NaN where the position is -1)
+    gain: torch.Tensor        # [B,k] float32 its MMR objective when it was picked (NaN likewise)
+
+
+def _check_diversify(k, N: int, lam, candidates, max_per_category) -> tuple:
+    """-> (K', q); ValueError unless 1 <= k <= K' <= min(N, 512) (K' = candidates, default min(N, 512)), lam is a number in [0, 1]
+    and max_per_category is None or an integer >= 0 (q = 0: no cap)."""
+    kc = min(N, CANDIDATES_MAX) if candidates is None else candidates
+    if isinstance(kc, bool) or not isinstance(kc, int) or not 1 <= kc <= min(N, CANDIDATES_MAX):
+        raise ValueError(f'candidates must be an integer in [1, min(N, {CANDIDATES_MAX})] = [1, {min(N, CANDIDATES_MAX)}], got {kc!r}')
+    if isinstance(k, bool) or not isinstance(k, int) or not 1 <= k <= kc:
+        raise ValueError(f'k must be an integer in [1, candidates] = [1, {kc}], got {k!r}')
+    if isinstance(lam, bool) or not isinstance(lam, numbers.Real) or not 0.0 <= float(lam) <= 1.0:     # NaN fails the comparison
+        raise ValueError(f'lam must be a number in [0, 1], got {lam!r}')
+    q = 0 if max_per_category is None else max_per_category
+    if isinstance(q, bool) or not isinstance(q, int) or q < 0:
+        raise ValueError(f'max_per_category must be None or an integer >= 0, got {max_per_category!r}')
+    return kc, q
+
+
+def _check_table(table) -> None:
+    if not isinstance(table, wire.ArticleTable):
+        raise ValueError('table must be a wire.ArticleTable')
+    rows = table.rows
+    if rows.dtype != torch.float32 or rows.dim() != 2 or rows.shape[1] != wire.ARTICLE_COLS or not rows.is_contiguous():
+        raise ValueError(f'article table must be contiguous float32 [n, {wire.ARTICLE_COLS}]')
+
+
+def _diversify(cand: Recommendations, k: int, lam, q: int, pa, table) -> DiverseRecommendations:
+    B, kc = cand.position.shape
+    N = int(pa.shape[0])
+    dev = pa.device
+    cpos = cand.position.to(torch.int32)
+    pos = torch.empty(B, k, dtype=torch.int32, device=dev)
+    val = torch.empty(B, k, dtype=torch.float32, device=dev)
+    gain = torch.empty(B, k, dtype=torch.float32, device=dev)
+    p = engine._ptr
+    _lib.check(_lib.load().nrm_pool_diversify(p(cpos), p(cand.score), B, kc, k, float(lam), q, p(pa), N, p(table.rows), table.n,
+                                              p(pos), p(val), p(gain), _stream(dev)), 'nrm_pool_diversify')
+    pos = pos.to(torch.int64)
+    article = torch.where(pos >= 0, pa.to(torch.int64)[pos.clamp(min=0)], torch.full_like(pos, -1))
+    return DiverseRecommendations(article, pos, val, gain)
+
+
+def diversify(logits: torch.Tensor, k: int, pool_article: torch.Tensor, table: wire.ArticleTable, *, lam: float,
+              candidates: Optional[int] = None, max_per_category: Optional[int] = None,
+              hist_article: Optional[torch.Tensor] = None) -> DiverseRecommendations:
+    """Each user's `k` articles re-ranked for diversity by greedy maximal marginal relevance (MMR) over the article embeddings, on
+    given logits ([B,N] or [M,B,N] float32, M <= 16).
+
+    The candidates are `select(logits, candidates, pool_article, table.n, hist_article=hist_article)` (default candidates =
+    min(N, 512)): the user's best eligible positions with `select`'s scores.  Relevance is the score min-max normalised over the
+    user's candidates (finite scores; +inf -> 1, -inf -> 0, all equal -> 1), similarity the cosine of the articles' PCA vectors
+    (table columns 0-63; 0 for an all-zero vector).  Each step picks the candidate with the largest
+    gain = lam * relevance - (1 - lam) * (max similarity to the articles already picked), ties to the better `select` slot; with
+    `max_per_category` = q a category (table column 64) gets at most q picks.  It stops after k picks or when nothing can be picked;
+    the remaining slots hold article -1, position -1, score and gain NaN.  lam = 1 without a cap returns `select(logits, k, ...)`'s
+    positions and scores bit for bit; lam = 0 picks by dissimilarity alone.  1 <= k <= candidates <= min(N, 512), 0 <= lam <= 1."""
+    _check_table(table)
+    if logits.dim() not in (2, 3):
+        raise ValueError(f'logits must be float32 [B,N] or [M,B,N] with M <= {MODELS_MAX}, got {logits.dtype} {list(logits.shape)}')
+    kc, q = _check_diversify(k, int(logits.shape[-1]), lam, candidates, max_per_category)
+    if not logits.is_cuda or not table.rows.is_cuda:
+        raise _lib.NrmError('recommend runs on CUDA tensors only (no CPU fallback)')
+    if table.rows.device != logits.device:
+        raise ValueError('logits and the article table must be on the same device')
+    cand = select(logits, kc, pool_article, table.n, hist_article=hist_article)
+    return _diversify(cand, k, lam, q, pool_article.contiguous(), table)
+
+
+def diverse_articles(models, table: wire.ArticleTable, hist_article, hist_time, hist_click, pool_time, k: int, *, lam: float,
+                     candidates: Optional[int] = None, max_per_category: Optional[int] = None,
+                     pool_article: Optional[torch.Tensor] = None, exclude_clicked: bool = True,
+                     chunk: Optional[int] = None) -> DiverseRecommendations:
+    """`top_articles` re-ranked for diversity: `pool_logits` of every model in `models`, then `diversify`.  Arguments as for
+    `top_articles` and `diversify`."""
+    if isinstance(models, torch.nn.Module):
+        models = [models]
+    models = list(models)
+    if not 1 <= len(models) <= MODELS_MAX:
+        raise ValueError(f'need 1 to {MODELS_MAX} models, got {len(models)}')
+    _check_chunk(chunk)
+    _check_table(table)
+    N = int(pool_article.shape[0]) if pool_article is not None and pool_article.dim() == 1 else table.n - 1
+    kc, q = _check_diversify(k, N, lam, candidates, max_per_category)
+    B, H, N, pa = _check_users_and_pool(table, hist_article, hist_time, hist_click, pool_time, pool_article)
+    with torch.no_grad():
+        logits = torch.empty(len(models), B, N, dtype=torch.float32, device=hist_article.device)
+        c = chunk if chunk is not None else default_chunk(B, H, N)
+        for m, model in enumerate(models):
+            _forward_pool(model, table, hist_article, hist_time, hist_click, pool_time, pa, B, H, N, c, logits[m])
+        cand = select(logits, kc, pa, table.n, hist_article=hist_article if exclude_clicked else None)
+        return _diversify(cand, k, lam, q, pa, table)
+
+
+def list_diversity(table: wire.ArticleTable, article: torch.Tensor) -> tuple:
+    """What a recommendation list offers besides relevance, per user: -> (ild float32 [B], n_categories int64 [B]) for `article`
+    [B,k] (the `article` of `top_articles` / `diverse_articles`; ids outside [1, table.n), such as -1, are no article).
+    `ild`: intra-list diversity, the mean of 1 - cos(u_i, u_j) over the pairs of the list's articles, with the cosine of the PCA
+    vectors as `diversify` uses it (0 for an all-zero vector), in float64; NaN for fewer than two articles.  `n_categories`: the
+    number of distinct categories ((int) of table column 64) in the list.  Plain torch on the article's device (no kernel)."""
+    _check_table(table)
+    if not isinstance(article, torch.Tensor) or article.dim() != 2 or article.dtype.is_floating_point or article.dtype == torch.bool:
+        raise ValueError(f'article must be an integer [B,k] tensor, got {getattr(article, "dtype", type(article))}')
+    if article.device != table.rows.device:
+        raise ValueError('article and the article table must be on the same device')
+    valid = (article >= 1) & (article < table.n)
+    r = table.rows[torch.where(valid, article, torch.zeros_like(article)).long()]          # [B,k,80]
+    v = r[..., :64].double()
+    norm = v.norm(dim=-1, keepdim=True)
+    u = torch.where(norm > 0, v / norm.clamp(min=torch.finfo(torch.float64).tiny), torch.zeros_like(v))
+    sim = u @ u.transpose(1, 2)
+    k = article.shape[1]
+    upper = torch.ones(k, k, dtype=torch.bool, device=article.device).triu(1)
+    pair = valid[:, :, None] & valid[:, None, :] & upper
+    n_pairs = pair.sum((1, 2))
+    ild = torch.where(n_pairs > 0, torch.where(pair, 1.0 - sim, torch.zeros_like(sim)).sum((1, 2)) / n_pairs.clamp(min=1),
+                      torch.full_like(n_pairs, float('nan'), dtype=torch.float64))
+    cat = torch.where(valid, r[..., 64].double().trunc(), torch.full_like(valid, float('inf'), dtype=torch.float64)).sort(1).values
+    real = torch.isfinite(cat)
+    n_cat = real[:, :1].sum(1) + ((cat[:, 1:] != cat[:, :-1]) & real[:, 1:]).sum(1)
+    return ild.float(), n_cat.to(torch.int64)
