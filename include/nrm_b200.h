@@ -34,6 +34,7 @@
  *     (models/user_invariant_interest_model.py:14-22); x_target / x_global may be
  *     column-trimmed views as produced by test.py:53-54, hence the batch strides
  *     (in elements); rows inside one impression are contiguous;
+ *     every packed entry point returns NRM_EINVAL for a batch stride smaller than one impression;
  *   - parameters live in ONE flat float32 buffer whose layout is given by the
  *     nrm_layout_* functions (state_dict order of the reference, 16-byte aligned
  *     entries, `delta` last); gradients use the same layout;

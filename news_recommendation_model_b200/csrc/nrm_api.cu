@@ -404,10 +404,12 @@ extern "C" size_t nrm_workspace_e_offset(int B, int H, int C, int mode) {
   return (size_t)(reinterpret_cast<uintptr_t>(w.e) - 256);
 }
 
+// scores non-null: the attention kernels also export s_label / s_ti there (eval-mode forwards, nrm_forward_scores)
 static int forward_encoder_impl(const char* fn, const BatchPtrs& in, int B, int H, int C, const float* params, int mode, int precision,
-                                double* bn_sums, void* workspace, size_t workspace_bytes, void* stream) {
+                                double* bn_sums, float* scores, void* workspace, size_t workspace_bytes, void* stream) {
   Workspace w;
   NRM_TRY(get_workspace(fn, w, workspace, workspace_bytes, B, H, C, mode));
+  w.scores = scores;
   cudaStream_t s = (cudaStream_t)stream;
   NRM_TRY(encoder_forward(in, params, w, mode, precision, s));
   if (mode & NRM_MODE_BN_BATCH_STATS) {
@@ -419,42 +421,59 @@ static int forward_encoder_impl(const char* fn, const BatchPtrs& in, int B, int 
   return NRM_OK;
 }
 
-// compact wire format as the input of the row kernels (no expansion to the packed float64 tensors): needs the kernels that never
-// touch the packed rows again, i.e. the row-stacked tensor-core path
-static int compact_batch(const char* fn, const nrm_compact_batch* cb, int precision, CompactPtrs& cp) {
-  if (!cb || !cb->articles || cb->n_articles <= 0 || !cb->hist_article || !cb->hist_time || !cb->hist_click || !cb->cand_article || !cb->cand_time ||
-      (cb->label32 && !cb->label64)) {
+// packed float64 rows from the caller: one impression's rows are dense, the batch stride may be larger
+static int packed_batch(const char* fn, const double* x_history, const double* x_target, long long xt_bs, const double* x_global,
+                        long long xg_bs, int C, BatchPtrs& in) {
+  if (!x_history || !x_target || !x_global) { set_error("%s: null pointer", fn); return NRM_EINVAL; }
+  if (xt_bs < (long long)C * TC || xg_bs < (long long)C * GC) { set_error("%s: batch stride smaller than one impression", fn); return NRM_EINVAL; }
+  in = BatchPtrs{x_history, x_target, xt_bs, x_global, xg_bs};
+  return NRM_OK;
+}
+
+// the tables and ids every reader of a compact batch needs (labels aside)
+static int compact_struct(const char* fn, const nrm_compact_batch* cb) {
+  if (!cb || !cb->articles || cb->n_articles <= 0 || !cb->hist_article || !cb->hist_time || !cb->hist_click || !cb->cand_article || !cb->cand_time) {
     set_error("%s: bad compact batch", fn); return NRM_EINVAL;
   }
   if ((reinterpret_cast<uintptr_t>(cb->articles) & 15) != 0) { set_error("%s: the article table must be 16-byte aligned", fn); return NRM_EINVAL; }
+  return NRM_OK;
+}
+
+// compact wire format as the input of the row kernels (no expansion to the packed float64 tensors): needs the kernels that never
+// touch the packed rows again, i.e. the row-stacked tensor-core path.  `in` points into `cp`.
+static int compact_batch(const char* fn, const nrm_compact_batch* cb, int precision, CompactPtrs& cp, BatchPtrs& in) {
+  NRM_TRY(compact_struct(fn, cb));
+  if (cb->label32 && !cb->label64) { set_error("%s: bad compact batch", fn); return NRM_EINVAL; }
   if (precision == NRM_PRECISION_FP32) {
     set_error("%s: the compact wire format is read directly by the tensor-core precisions only (use nrm_expand_compact otherwise)", fn);
     return NRM_EUNSUPPORTED;
   }
   cp = CompactPtrs{cb->articles, cb->n_articles, cb->hist_article, cb->hist_time, cb->hist_click, cb->cand_article, cb->cand_time,
                    cb->label32, cb->label64};
+  in = BatchPtrs{nullptr, nullptr, 0, nullptr, 0};
+  in.compact = &cp;
   return NRM_OK;
 }
 
 extern "C" int nrm_forward_encoder(const double* x_history, const double* x_target, long long xt_bs, const double* x_global,
                                    long long xg_bs, int B, int H, int C, const float* params, int mode, int precision,
                                    double* bn_sums, void* workspace, size_t workspace_bytes, void* stream) {
-  NRM_TRY(check_shape("nrm_forward_encoder", B, H, C));
-  if (!x_history || !x_target || !x_global || !params) { set_error("nrm_forward_encoder: null pointer"); return NRM_EINVAL; }
-  if (xt_bs < (long long)C * TC || xg_bs < (long long)C * GC) { set_error("nrm_forward_encoder: batch stride smaller than one impression"); return NRM_EINVAL; }
-  const BatchPtrs in{x_history, x_target, xt_bs, x_global, xg_bs};
-  return forward_encoder_impl("nrm_forward_encoder", in, B, H, C, params, mode, precision, bn_sums, workspace, workspace_bytes, stream);
+  const char* fn = "nrm_forward_encoder";
+  NRM_TRY(check_shape(fn, B, H, C));
+  BatchPtrs in;
+  NRM_TRY(packed_batch(fn, x_history, x_target, xt_bs, x_global, xg_bs, C, in));
+  if (!params) { set_error("%s: null pointer", fn); return NRM_EINVAL; }
+  return forward_encoder_impl(fn, in, B, H, C, params, mode, precision, bn_sums, nullptr, workspace, workspace_bytes, stream);
 }
 
 extern "C" int nrm_forward_encoder_compact(const nrm_compact_batch* batch, int B, int H, int C, const float* params, int mode, int precision,
                                            double* bn_sums, void* workspace, size_t workspace_bytes, void* stream) {
-  NRM_TRY(check_shape("nrm_forward_encoder_compact", B, H, C));
-  if (!params) { set_error("nrm_forward_encoder_compact: null pointer"); return NRM_EINVAL; }
-  CompactPtrs cp;
-  NRM_TRY(compact_batch("nrm_forward_encoder_compact", batch, precision, cp));
-  BatchPtrs in{nullptr, nullptr, 0, nullptr, 0};
-  in.compact = &cp;
-  return forward_encoder_impl("nrm_forward_encoder_compact", in, B, H, C, params, mode, precision, bn_sums, workspace, workspace_bytes, stream);
+  const char* fn = "nrm_forward_encoder_compact";
+  NRM_TRY(check_shape(fn, B, H, C));
+  if (!params) { set_error("%s: null pointer", fn); return NRM_EINVAL; }
+  CompactPtrs cp; BatchPtrs in;
+  NRM_TRY(compact_batch(fn, batch, precision, cp, in));
+  return forward_encoder_impl(fn, in, B, H, C, params, mode, precision, bn_sums, nullptr, workspace, workspace_bytes, stream);
 }
 
 extern "C" int nrm_forward_head(int B, int H, int C, const float* params, float* bn_running_mean, float* bn_running_var,
@@ -473,9 +492,9 @@ extern "C" int nrm_forward_head(int B, int H, int C, const float* params, float*
   if (precision != NRM_PRECISION_FP32)
     return launch_head_forward_tc(params, w, precision, bn_running_mean, bn_running_var, bn_num_batches_tracked, training,
                                   (mode & NRM_MODE_KEEP_FOR_BWD) != 0, sums, rows, logits, (cudaStream_t)stream);
-  return launch_head_forward(params, w, bn_running_mean, bn_running_var, bn_num_batches_tracked, training,
-                             (mode & NRM_MODE_KEEP_FOR_BWD) != 0, sums, rows,
-                             logits, (cudaStream_t)stream);
+  // the BatchNorm finalisation (batch / running statistics, running-statistics update) is the prologue of the fused kernel
+  return launch_head_forward_fused(params, w, bn_running_mean, bn_running_var, bn_num_batches_tracked, training,
+                                   (mode & NRM_MODE_KEEP_FOR_BWD) != 0, sums, rows, logits, (cudaStream_t)stream);
 }
 
 extern "C" int nrm_forward(const double* x_history, const double* x_target, long long xt_bs, const double* x_global,
@@ -497,42 +516,39 @@ extern "C" int nrm_forward_compact(const nrm_compact_batch* batch, int B, int H,
 }
 
 // ---- attention scores (explanations): eval-mode forward that also exports s_label / s_ti -----------------------------------------
-static int forward_scores_impl(const char* fn, const BatchPtrs& in, int B, int H, int C, const float* params, float* bn_running_mean,
-                               float* bn_running_var, long long* bn_num_batches_tracked, int mode, int precision, float* logits,
-                               float* scores, void* workspace, size_t workspace_bytes, void* stream) {
+static int scores_args(const char* fn, int mode, const float* scores) {
   if (mode != NRM_MODE_EVAL) { set_error("%s: scores are exported by eval-mode forwards only (mode must be NRM_MODE_EVAL, got %d)", fn, mode); return NRM_EINVAL; }
   if (!scores) { set_error("%s: null scores", fn); return NRM_EINVAL; }
-  Workspace w;
-  NRM_TRY(get_workspace(fn, w, workspace, workspace_bytes, B, H, C, mode));
-  w.scores = scores;
-  NRM_TRY(encoder_forward(in, params, w, mode, precision, (cudaStream_t)stream));
-  return nrm_forward_head(B, H, C, params, bn_running_mean, bn_running_var, bn_num_batches_tracked, mode, precision, nullptr, 0,
-                          logits, workspace, workspace_bytes, stream);
+  return NRM_OK;
 }
 
 extern "C" int nrm_forward_scores(const double* x_history, const double* x_target, long long xt_bs, const double* x_global,
                                   long long xg_bs, int B, int H, int C, const float* params, float* bn_running_mean,
                                   float* bn_running_var, long long* bn_num_batches_tracked, int mode, int precision,
                                   float* logits, float* scores, void* workspace, size_t workspace_bytes, void* stream) {
-  NRM_TRY(check_shape("nrm_forward_scores", B, H, C));
-  if (!x_history || !x_target || !x_global || !params) { set_error("nrm_forward_scores: null pointer"); return NRM_EINVAL; }
-  if (xt_bs < (long long)C * TC || xg_bs < (long long)C * GC) { set_error("nrm_forward_scores: batch stride smaller than one impression"); return NRM_EINVAL; }
-  const BatchPtrs in{x_history, x_target, xt_bs, x_global, xg_bs};
-  return forward_scores_impl("nrm_forward_scores", in, B, H, C, params, bn_running_mean, bn_running_var, bn_num_batches_tracked, mode,
-                             precision, logits, scores, workspace, workspace_bytes, stream);
+  const char* fn = "nrm_forward_scores";
+  NRM_TRY(check_shape(fn, B, H, C));
+  BatchPtrs in;
+  NRM_TRY(packed_batch(fn, x_history, x_target, xt_bs, x_global, xg_bs, C, in));
+  if (!params) { set_error("%s: null pointer", fn); return NRM_EINVAL; }
+  NRM_TRY(scores_args(fn, mode, scores));
+  NRM_TRY(forward_encoder_impl(fn, in, B, H, C, params, mode, precision, nullptr, scores, workspace, workspace_bytes, stream));
+  return nrm_forward_head(B, H, C, params, bn_running_mean, bn_running_var, bn_num_batches_tracked, mode, precision, nullptr, 0,
+                          logits, workspace, workspace_bytes, stream);
 }
 
 extern "C" int nrm_forward_scores_compact(const nrm_compact_batch* batch, int B, int H, int C, const float* params, float* bn_running_mean,
                                           float* bn_running_var, long long* bn_num_batches_tracked, int mode, int precision,
                                           float* logits, float* scores, void* workspace, size_t workspace_bytes, void* stream) {
-  NRM_TRY(check_shape("nrm_forward_scores_compact", B, H, C));
-  if (!params) { set_error("nrm_forward_scores_compact: null pointer"); return NRM_EINVAL; }
-  CompactPtrs cp;
-  NRM_TRY(compact_batch("nrm_forward_scores_compact", batch, precision, cp));
-  BatchPtrs in{nullptr, nullptr, 0, nullptr, 0};
-  in.compact = &cp;
-  return forward_scores_impl("nrm_forward_scores_compact", in, B, H, C, params, bn_running_mean, bn_running_var, bn_num_batches_tracked,
-                             mode, precision, logits, scores, workspace, workspace_bytes, stream);
+  const char* fn = "nrm_forward_scores_compact";
+  NRM_TRY(check_shape(fn, B, H, C));
+  if (!params) { set_error("%s: null pointer", fn); return NRM_EINVAL; }
+  CompactPtrs cp; BatchPtrs in;
+  NRM_TRY(compact_batch(fn, batch, precision, cp, in));
+  NRM_TRY(scores_args(fn, mode, scores));
+  NRM_TRY(forward_encoder_impl(fn, in, B, H, C, params, mode, precision, nullptr, scores, workspace, workspace_bytes, stream));
+  return nrm_forward_head(B, H, C, params, bn_running_mean, bn_running_var, bn_num_batches_tracked, mode, precision, nullptr, 0,
+                          logits, workspace, workspace_bytes, stream);
 }
 
 // ---- recommendation from a shared pool: every user against the same N articles, in chunks of the pool ------------------------------
@@ -573,12 +589,8 @@ extern "C" int nrm_forward_pool(const nrm_compact_batch* users, int B, int H, in
   if (B <= 0 || H <= 0 || N <= 0) { set_error("%s: B, H, N must be positive (got %d, %d, %d)", fn, B, H, N); return NRM_EINVAL; }
   if (chunk <= 0 || chunk % 8 != 0) { set_error("%s: chunk must be a positive multiple of 8 (got %d)", fn, chunk); return NRM_EINVAL; }
   if (precision < NRM_PRECISION_FP32 || precision > NRM_PRECISION_BF16X3) { set_error("%s: unknown precision %d", fn, precision); return NRM_EINVAL; }
-  if (!users || !users->articles || users->n_articles <= 0 || !users->hist_article || !users->hist_time || !users->hist_click ||
-      !users->cand_article || !users->cand_time) {
-    set_error("%s: bad compact batch", fn); return NRM_EINVAL;
-  }
+  NRM_TRY(compact_struct(fn, users));
   if (users->label32 || users->label64) { set_error("%s: the pool has no labels (label32 / label64 must be null)", fn); return NRM_EINVAL; }
-  if ((reinterpret_cast<uintptr_t>(users->articles) & 15) != 0) { set_error("%s: the article table must be 16-byte aligned", fn); return NRM_EINVAL; }
   if (!params || !bn_running_mean || !bn_running_var || !logits) { set_error("%s: null pointer", fn); return NRM_EINVAL; }
   const int C = chunk < N ? chunk : N;
   NRM_TRY(check_shape(fn, B, H, C));
@@ -598,7 +610,7 @@ extern "C" int nrm_forward_pool(const nrm_compact_batch* users, int B, int H, in
     NRM_TRY(launch_expand_compact(u.articles, u.n_articles, nullptr, nullptr, nullptr, u.cand_article + c0, u.cand_time + c0, nullptr, 0, nc,
                                   nullptr, pc.xt, pc.xg, nullptr, s));
     const BatchPtrs in{pc.xh, pc.xt, 0, pc.xg, 0};
-    NRM_TRY(forward_encoder_impl(fn, in, B, H, nc, params, NRM_MODE_EVAL, precision, nullptr, pc.ws, pc.ws_bytes, stream));
+    NRM_TRY(forward_encoder_impl(fn, in, B, H, nc, params, NRM_MODE_EVAL, precision, nullptr, nullptr, pc.ws, pc.ws_bytes, stream));
     float* out = nc == N ? logits : pc.out;                 // a single chunk writes the [B,N] logits directly
     NRM_TRY(nrm_forward_head(B, H, nc, params, run_mean, run_var, nullptr, NRM_MODE_EVAL, precision, nullptr, 0, out, pc.ws, pc.ws_bytes, stream));
     if (out != logits)
@@ -607,6 +619,15 @@ extern "C" int nrm_forward_pool(const nrm_compact_batch* users, int B, int H, in
   return NRM_OK;
 }
 
+// head data gradients down to w.de and the BatchNorm backward sums: one tensor-core chain, or the FFMA dgrad + BatchNorm pass
+static int head_dgrad(const float* params, Workspace& w, int precision, const float* dlogits, float* grads, cudaStream_t s) {
+  if (precision != NRM_PRECISION_FP32) return launch_head_backward_dgrad_tc(params, w, precision, dlogits, grads, s);
+  NRM_TRY(launch_head_backward_dgrad(params, w, dlogits, s));
+  return launch_head_backward_bn(w, grads, s, 0);
+}
+
+// defer_wgrad: the head's weight gradients (only the optimizer needs them) are left to the next encoder backward on this stream, which
+// enqueues them on the side stream behind the w1 backward, beside its own tail, instead of in front of it
 static int backward_head(const char* fn, bool defer_wgrad, int B, int H, int C, const float* params, int precision, const float* dlogits, float* grads,
                          double* bn_bwd_sums, void* workspace, size_t workspace_bytes, void* stream) {
   NRM_TRY(check_shape(fn, B, H, C));
@@ -616,18 +637,13 @@ static int backward_head(const char* fn, bool defer_wgrad, int B, int H, int C, 
   cudaStream_t s = (cudaStream_t)stream;
   const bool tc = precision != NRM_PRECISION_FP32;
   const int tiles = tc ? head_tc_tiles(w.R) : 0;
-  if (!defer_wgrad) {
+  SideStream* ss = nullptr;
+  if (defer_wgrad && (ss = side_stream(s)) == nullptr) { set_error("%s: cannot create the side stream", fn); return NRM_ECUDA; }
+  {
     KernelTimer t("head_backward", s);
-    if (tc) NRM_TRY(launch_head_backward_dgrad_tc(params, w, precision, dlogits, grads, s));
-    else { NRM_TRY(launch_head_backward_dgrad(params, w, dlogits, s)); NRM_TRY(launch_head_backward_bn(w, grads, s, 0)); }
-    NRM_TRY(launch_head_backward_wgrad(params, w, grads, s, tiles, tc ? precision : 0));
-  } else {
-    SideStream* ss = side_stream(s);
-    if (ss == nullptr) { set_error("%s: cannot create the side stream", fn); return NRM_ECUDA; }
-    KernelTimer t("head_backward", s);
-    if (tc) NRM_TRY(launch_head_backward_dgrad_tc(params, w, precision, dlogits, grads, s)); else NRM_TRY(launch_head_backward_dgrad(params, w, dlogits, s));
-    ss->head_wgrad_pending = true; ss->wg_params = params; ss->wg_grads = grads; ss->wg_tiles = tiles; ss->wg_precision = tc ? precision : 0;
-    if (!tc) NRM_TRY(launch_head_backward_bn(w, grads, s, 0));
+    NRM_TRY(head_dgrad(params, w, precision, dlogits, grads, s));
+    if (defer_wgrad) { ss->head_wgrad_pending = true; ss->wg_params = params; ss->wg_grads = grads; ss->wg_tiles = tiles; ss->wg_precision = tc ? precision : 0; }
+    else NRM_TRY(launch_head_backward_wgrad(params, w, grads, s, tiles, tc ? precision : 0));
   }
   if (bn_bwd_sums != nullptr && bn_bwd_sums != w.bn_bwd_sums)
     NRM_CUDA(cudaMemcpyAsync(bn_bwd_sums, w.bn_bwd_sums, sizeof(double) * 2 * E, cudaMemcpyDeviceToDevice, s));
@@ -661,62 +677,42 @@ extern "C" int nrm_backward_encoder(const double* x_history, const double* x_tar
                                     const double* x_global, long long xg_bs, int B, int H, int C, const float* params,
                                     int mode, int precision, const double* bn_bwd_sums, long long bn_global_rows,
                                     float* grads, void* workspace, size_t workspace_bytes, void* stream) {
-  NRM_TRY(check_shape("nrm_backward_encoder", B, H, C));
-  if (!x_history || !x_target || !x_global || !params || !grads) { set_error("nrm_backward_encoder: null pointer"); return NRM_EINVAL; }
-  const BatchPtrs in{x_history, x_target, xt_bs, x_global, xg_bs};
-  return backward_encoder_impl("nrm_backward_encoder", in, B, H, C, params, mode, precision, bn_bwd_sums, bn_global_rows, grads, workspace,
-                               workspace_bytes, stream);
+  const char* fn = "nrm_backward_encoder";
+  NRM_TRY(check_shape(fn, B, H, C));
+  BatchPtrs in;
+  NRM_TRY(packed_batch(fn, x_history, x_target, xt_bs, x_global, xg_bs, C, in));
+  if (!params || !grads) { set_error("%s: null pointer", fn); return NRM_EINVAL; }
+  return backward_encoder_impl(fn, in, B, H, C, params, mode, precision, bn_bwd_sums, bn_global_rows, grads, workspace, workspace_bytes, stream);
 }
 
 extern "C" int nrm_backward_encoder_compact(const nrm_compact_batch* batch, int B, int H, int C, const float* params, int mode, int precision,
                                             const double* bn_bwd_sums, long long bn_global_rows, float* grads, void* workspace,
                                             size_t workspace_bytes, void* stream) {
-  NRM_TRY(check_shape("nrm_backward_encoder_compact", B, H, C));
-  if (!params || !grads) { set_error("nrm_backward_encoder_compact: null pointer"); return NRM_EINVAL; }
-  CompactPtrs cp;
-  NRM_TRY(compact_batch("nrm_backward_encoder_compact", batch, precision, cp));
-  BatchPtrs in{nullptr, nullptr, 0, nullptr, 0};
-  in.compact = &cp;
-  return backward_encoder_impl("nrm_backward_encoder_compact", in, B, H, C, params, mode, precision, bn_bwd_sums, bn_global_rows, grads, workspace,
-                               workspace_bytes, stream);
-}
-
-static int backward_impl(const char* fn, const BatchPtrs& in, int B, int H, int C, const float* params, int mode, int precision,
-                         const float* dlogits, float* grads, void* workspace, size_t workspace_bytes, void* stream) {
-  // Head and encoder backward in one call: the head's weight gradients (only the optimizer needs them) run on the side
-  // stream behind the w1 backward, beside the tail of the encoder backward, instead of in front of it.
-  const int training = mode & NRM_MODE_BN_BATCH_STATS;
-  Workspace w;
-  NRM_TRY(get_workspace(fn, w, workspace, workspace_bytes, B, H, C, NRM_MODE_KEEP_FOR_BWD));
-  cudaStream_t s = (cudaStream_t)stream;
-  SideStream* ss = side_stream(s);
-  if (ss == nullptr) { set_error("%s: cannot create the side stream", fn); return NRM_ECUDA; }
-  const bool htc = precision != NRM_PRECISION_FP32;
-  const int tiles = htc ? head_tc_tiles(w.R) : 0;
-  { KernelTimer t("head_backward", s);
-    if (htc) NRM_TRY(launch_head_backward_dgrad_tc(params, w, precision, dlogits, grads, s)); else NRM_TRY(launch_head_backward_dgrad(params, w, dlogits, s));
-    ss->head_wgrad_pending = true; ss->wg_params = params; ss->wg_grads = grads; ss->wg_tiles = tiles; ss->wg_precision = htc ? precision : 0;
-    if (!htc) NRM_TRY(launch_head_backward_bn(w, grads, s, 0)); }
-  NRM_TRY(launch_bn_backward_combine(params, w, training, w.bn_bwd_sums, w.R, htc, s));
-  return encoder_backward(in, params, w, precision, grads, s);     // enqueues the head weight gradients on the side stream and joins them
+  const char* fn = "nrm_backward_encoder_compact";
+  NRM_TRY(check_shape(fn, B, H, C));
+  if (!params || !grads) { set_error("%s: null pointer", fn); return NRM_EINVAL; }
+  CompactPtrs cp; BatchPtrs in;
+  NRM_TRY(compact_batch(fn, batch, precision, cp, in));
+  return backward_encoder_impl(fn, in, B, H, C, params, mode, precision, bn_bwd_sums, bn_global_rows, grads, workspace, workspace_bytes, stream);
 }
 
 extern "C" int nrm_backward(const double* x_history, const double* x_target, long long xt_bs, const double* x_global,
                             long long xg_bs, int B, int H, int C, const float* params, int mode, int precision,
                             const float* dlogits, float* grads, void* workspace, size_t workspace_bytes, void* stream) {
-  NRM_TRY(check_shape("nrm_backward", B, H, C));
-  if (!x_history || !x_target || !x_global || !params || !dlogits || !grads) { set_error("nrm_backward: null pointer"); return NRM_EINVAL; }
-  const BatchPtrs in{x_history, x_target, xt_bs, x_global, xg_bs};
-  return backward_impl("nrm_backward", in, B, H, C, params, mode, precision, dlogits, grads, workspace, workspace_bytes, stream);
+  const char* fn = "nrm_backward";
+  NRM_TRY(check_shape(fn, B, H, C));
+  BatchPtrs in;
+  NRM_TRY(packed_batch(fn, x_history, x_target, xt_bs, x_global, xg_bs, C, in));
+  NRM_TRY(backward_head(fn, true, B, H, C, params, precision, dlogits, grads, nullptr, workspace, workspace_bytes, stream));
+  return backward_encoder_impl(fn, in, B, H, C, params, mode, precision, nullptr, 0, grads, workspace, workspace_bytes, stream);
 }
 
 extern "C" int nrm_backward_compact(const nrm_compact_batch* batch, int B, int H, int C, const float* params, int mode, int precision,
                                     const float* dlogits, float* grads, void* workspace, size_t workspace_bytes, void* stream) {
-  NRM_TRY(check_shape("nrm_backward_compact", B, H, C));
-  if (!params || !dlogits || !grads) { set_error("nrm_backward_compact: null pointer"); return NRM_EINVAL; }
-  CompactPtrs cp;
-  NRM_TRY(compact_batch("nrm_backward_compact", batch, precision, cp));
-  BatchPtrs in{nullptr, nullptr, 0, nullptr, 0};
-  in.compact = &cp;
-  return backward_impl("nrm_backward_compact", in, B, H, C, params, mode, precision, dlogits, grads, workspace, workspace_bytes, stream);
+  const char* fn = "nrm_backward_compact";
+  NRM_TRY(check_shape(fn, B, H, C));
+  CompactPtrs cp; BatchPtrs in;
+  NRM_TRY(compact_batch(fn, batch, precision, cp, in));
+  NRM_TRY(backward_head(fn, true, B, H, C, params, precision, dlogits, grads, nullptr, workspace, workspace_bytes, stream));
+  return backward_encoder_impl(fn, in, B, H, C, params, mode, precision, nullptr, 0, grads, workspace, workspace_bytes, stream);
 }

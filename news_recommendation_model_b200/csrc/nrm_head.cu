@@ -95,16 +95,6 @@ int launch_bn_partial_sums(Workspace& w, cudaStream_t s) {
   return NRM_OK;
 }
 
-int launch_head_forward(const float* P, Workspace& w, float* run_mean, float* run_var, long long* nbt, int training, int keep,
-                        const double* bn_sums, long long global_rows, float* logits, cudaStream_t s) {
-  // the BatchNorm finalisation (batch / running statistics, running-statistics update) is the prologue of the fused kernel
-  return launch_head_forward_fused(P, w, run_mean, run_var, nbt, training, keep, bn_sums, global_rows, logits, s);
-}
-
-int launch_head_backward(const float* P, Workspace& w, const float* dlogits, float* G, cudaStream_t s) {
-  return launch_head_backward_fused(P, w, dlogits, G, s);
-}
-
 int launch_bn_backward_combine(const float* P, Workspace& w, int training, const double* bn_bwd_sums,
                                long long global_rows, bool de_holds_dx, cudaStream_t s) {
   const long long total4 = w.R * (E / 4);

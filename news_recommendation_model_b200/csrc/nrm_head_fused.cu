@@ -747,10 +747,4 @@ int launch_head_backward_wgrad(const float* P, Workspace& w, float* G, cudaStrea
   return NRM_OK;
 }
 
-int launch_head_backward_fused(const float* P, Workspace& w, const float* dlogits, float* G, cudaStream_t s) {
-  NRM_TRY(launch_head_backward_dgrad(P, w, dlogits, s));
-  NRM_TRY(launch_head_backward_bn(w, G, s, 0));
-  return launch_head_backward_wgrad(P, w, G, s, 0);
-}
-
 }  // namespace nrm

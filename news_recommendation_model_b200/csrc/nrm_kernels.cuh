@@ -58,7 +58,6 @@ int launch_head_forward_fused(const float* P, Workspace& w, float* run_mean, flo
 int launch_head_backward_dgrad(const float* P, Workspace& w, const float* dlogits, cudaStream_t s);
 int launch_head_backward_bn(Workspace& w, float* grads, cudaStream_t s, int dgrad_tiles);   // dgrad_tiles: row tiles of the dgrad kernel (0 = FFMA kernel's)                   // -> w.bn_bwd_sums, bn.weight / bn.bias gradients
 int launch_head_backward_wgrad(const float* P, Workspace& w, float* grads, cudaStream_t s, int dgrad_tiles, int tc_precision = 0);   // tc_precision != 0: products on tcgen05   // weight gradients of the five Linear layers + out_mlp.fc2
-int launch_head_backward_fused(const float* P, Workspace& w, const float* dlogits, float* grads, cudaStream_t s);   // -> w.bn_bwd_sums, w.dz, w.de
 
 // nrm_head_tc.cu  (tensor-core head; precision = bf16 / bf16x3)
 size_t head_tc_image_bytes();
@@ -90,9 +89,6 @@ int launch_pool_diversify(const int* cand_pos, const float* cand_score, int B, i
 
 // nrm_head.cu
 int launch_bn_partial_sums(Workspace& w, cudaStream_t s);                 // -> w.bn_sums
-int launch_head_forward(const float* P, Workspace& w, float* run_mean, float* run_var, long long* nbt,
-                        int training, int keep, const double* bn_sums, long long global_rows, float* logits, cudaStream_t s);
-int launch_head_backward(const float* P, Workspace& w, const float* dlogits, float* grads, cudaStream_t s);  // -> w.bn_bwd_sums
 int launch_bn_backward_combine(const float* P, Workspace& w, int training, const double* bn_bwd_sums,
                                long long global_rows, bool de_holds_dx, cudaStream_t s);  // w.de += BN path
 

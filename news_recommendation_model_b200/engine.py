@@ -11,7 +11,7 @@
 from __future__ import annotations
 
 import ctypes
-from typing import Dict, List, Optional, Tuple
+from typing import Dict, List, NamedTuple, Optional, Tuple
 
 import torch
 
@@ -153,9 +153,58 @@ class Runtime:
         return self.eval_ws
 
 
-def prepare_inputs(x_history, x_target, x_global):
+class Packed(NamedTuple):
+    """A batch of packed float64 rows as the packed entry points take it (`nrm_forward(xh, xt, xt_bs, xg, xg_bs, B, H, C, ...)`)."""
+    xh: torch.Tensor
+    xt: torch.Tensor
+    xt_bs: int              # batch strides in elements
+    xg: torch.Tensor
+    xg_bs: int
+    suffix = ''
+
+    @property
+    def args(self) -> tuple:
+        return _ptr(self.xh), _ptr(self.xt), self.xt_bs, _ptr(self.xg), self.xg_bs
+
+
+def packed(xh: torch.Tensor, xt: torch.Tensor, xg: torch.Tensor) -> Packed:
+    """The binding of packed tensors whose impressions are dense rows.  B = 1: a size-1 dimension may carry any stride, so the
+    library gets the dense one."""
+    B, C = xt.shape[0], xt.shape[1]
+    return Packed(xh, xt, xt.stride(0) if B > 1 else C * TGT_COLS, xg, xg.stride(0) if B > 1 else C * GLOBAL_COLS)
+
+
+class Compact(NamedTuple):
+    """A device `wire.CompactBatch` and its `ArticleTable` as the `_compact` entry points take them
+    (`nrm_forward_compact(&batch, B, H, C, ...)`): the row kernels read the article ids directly."""
+    struct: _lib.CompactBatchStruct
+    keep: tuple             # the tensors `struct` points into
+    suffix = '_compact'
+
+    @property
+    def args(self) -> tuple:
+        return (ctypes.byref(self.struct),)
+
+
+def compact(table, cb, label64: Optional[torch.Tensor] = None) -> Compact:
+    """`label64`: a float64 [B,C] buffer the first row kernel converts `cb.label` into (what the loss reads); None: no labels."""
+    label32 = cb.label if label64 is not None else None
+    struct = _lib.CompactBatchStruct(table.rows.data_ptr(), table.n, cb.hist_article.data_ptr(), cb.hist_time.data_ptr(),
+                                     cb.hist_click.data_ptr(), cb.cand_article.data_ptr(), cb.cand_time.data_ptr(),
+                                     label32.data_ptr() if label32 is not None else None,
+                                     label64.data_ptr() if label64 is not None else None)
+    return Compact(struct, (table, cb, label64))
+
+
+def call(inputs, entry: str, *rest) -> None:
+    """`entry` in the variant for `inputs`' wire format, with `inputs`' arguments first."""
+    name = entry + inputs.suffix
+    _lib.check(getattr(_lib.load(), name)(*inputs.args, *rest), name)
+
+
+def prepare_inputs(x_history, x_target, x_global) -> Packed:
     """Validate the packed float64 feature tensors (SURVEY.md 8b input conventions) and
-    return them with the batch strides the kernels need."""
+    return their binding."""
     if x_history.dim() != 3 or x_history.shape[2] != HIST_COLS:
         raise ValueError(f'x_history must be [B,H,{HIST_COLS}], got {tuple(x_history.shape)}')
     if x_target.dim() != 3 or x_target.shape[2] != TGT_COLS:
@@ -181,69 +230,81 @@ def prepare_inputs(x_history, x_target, x_global):
     xh, xt, xg = out
     if not xh.is_contiguous():
         xh = xh.contiguous()
-    return xh, xt, xg
+    return packed(xh, xt, xg)
+
+
+def forward(inputs, B, H, C, params, bn_mean, bn_var, bn_nbt, mode, precision, logits, ws, stream, bn_sums=None, exchange=None):
+    """Encoder and head forward of one batch.  `exchange` None: one call.  Otherwise the two halves of a synchronised-BatchNorm
+    forward: the encoder writes this rank's BatchNorm column sums into `bn_sums`, and `exchange(bn_sums)` returns the sums and the
+    row count the head normalises with."""
+    if exchange is None:
+        call(inputs, 'nrm_forward', B, H, C, _ptr(params), _ptr(bn_mean), _ptr(bn_var), _ptr(bn_nbt), mode, precision, _ptr(logits),
+             _ptr(ws), ws.numel(), stream)
+        return
+    call(inputs, 'nrm_forward_encoder', B, H, C, _ptr(params), mode, precision, _ptr(bn_sums), _ptr(ws), ws.numel(), stream)
+    sums, rows = exchange(bn_sums)
+    _lib.check(_lib.load().nrm_forward_head(B, H, C, _ptr(params), _ptr(bn_mean), _ptr(bn_var), _ptr(bn_nbt), mode, precision, _ptr(sums),
+                                            rows, _ptr(logits), _ptr(ws), ws.numel(), stream), 'nrm_forward_head')
+
+
+def backward(inputs, B, H, C, params, mode, precision, dlogits, grads, ws, stream, bn_sums=None, exchange=None, defer_wgrad=True):
+    """Head and encoder backward of one batch into `grads`.  `exchange` None: one call.  Otherwise the two halves, and
+    `exchange(bn_sums)` runs between them and returns the BatchNorm backward sums and row count the encoder combines with
+    (`bn_sums` None: this rank's own).  `defer_wgrad` False: the head's weight gradients are complete when `exchange` runs;
+    True: the encoder backward enqueues them beside its own tail."""
+    if exchange is None:
+        call(inputs, 'nrm_backward', B, H, C, _ptr(params), mode, precision, _ptr(dlogits), _ptr(grads), _ptr(ws), ws.numel(), stream)
+        return
+    head = 'nrm_backward_head_deferred' if defer_wgrad else 'nrm_backward_head'
+    _lib.check(getattr(_lib.load(), head)(B, H, C, _ptr(params), precision, _ptr(dlogits), _ptr(grads), _ptr(bn_sums), _ptr(ws), ws.numel(),
+                                          stream), head)
+    sums, rows = exchange(bn_sums)
+    call(inputs, 'nrm_backward_encoder', B, H, C, _ptr(params), mode, precision, _ptr(sums), rows, _ptr(grads), _ptr(ws), ws.numel(), stream)
 
 
 def forward_logits(rt: Runtime, flat: FlatParams, bn_mean, bn_var, bn_nbt, x_history, x_target, x_global,
                    mode: int, precision: int, dp=None):
-    """Run nrm_forward; returns (logits [B,C], token or None)."""
-    lib = _lib.load()
-    xh, xt, xg = prepare_inputs(x_history, x_target, x_global)
-    B, H, C = xh.shape[0], xh.shape[1], xt.shape[1]
-    dev = xh.device
+    """Run the forward (`forward`); returns (logits [B,C], token or None)."""
+    inputs = prepare_inputs(x_history, x_target, x_global)
+    B, H, C = inputs.xh.shape[0], inputs.xh.shape[1], inputs.xt.shape[1]
+    dev = inputs.xh.device
     if flat.device != dev:
         raise _lib.NrmError(f'model is on {flat.device} but inputs are on {dev}')
     ws = rt.workspace(B, H, C, mode, dev)
     logits = torch.empty(B, C, dtype=torch.float32, device=dev)
-    st = _stream(dev)
-    xt_bs = xt.stride(0) if B > 1 else C * TGT_COLS
-    xg_bs = xg.stride(0) if B > 1 else C * GLOBAL_COLS
+    sums = exchange = None
     if dp is not None and dp.sync_bn and (mode & MODE_BN_BATCH_STATS):
         sums = torch.empty(2 * E_DIM, dtype=torch.float64, device=dev)
-        _lib.check(lib.nrm_forward_encoder(_ptr(xh), _ptr(xt), xt_bs, _ptr(xg), xg_bs, B, H, C, _ptr(flat.buf), mode,
-                                           precision, _ptr(sums), _ptr(ws), ws.numel(), st), 'nrm_forward_encoder')
-        rows = dp.all_reduce_stats(sums, B * C)
-        _lib.check(lib.nrm_forward_head(B, H, C, _ptr(flat.buf), _ptr(bn_mean), _ptr(bn_var), _ptr(bn_nbt), mode, precision,
-                                        _ptr(sums), rows, _ptr(logits), _ptr(ws), ws.numel(), st), 'nrm_forward_head')
-    else:
-        _lib.check(lib.nrm_forward(_ptr(xh), _ptr(xt), xt_bs, _ptr(xg), xg_bs, B, H, C, _ptr(flat.buf), _ptr(bn_mean),
-                                   _ptr(bn_var), _ptr(bn_nbt), mode, precision, _ptr(logits), _ptr(ws), ws.numel(), st),
-                   'nrm_forward')
+        exchange = lambda s: (s, dp.all_reduce_stats(s, B * C))              # noqa: E731
+    forward(inputs, B, H, C, flat.buf, bn_mean, bn_var, bn_nbt, mode, precision, logits, ws, _stream(dev), sums, exchange)
     token = None
     if mode & MODE_KEEP_FOR_BWD:
-        token = StepToken(ws, B, H, C, mode, (xh, xt, xg, xt_bs, xg_bs), flat.total, dev)
+        token = StepToken(ws, B, H, C, mode, inputs, flat.total, dev)
         rt.train_ws_token = token
     return logits, token
 
 
 def backward_params(flat: FlatParams, token: StepToken, dlogits: torch.Tensor, precision: int, dp=None) -> torch.Tensor:
-    """Run nrm_backward for `token`; returns the flat gradient buffer."""
-    lib = _lib.load()
+    """Run the backward (`backward`) for `token`; returns the flat gradient buffer."""
     if token.done:
         raise _lib.NrmError('backward called twice for the same forward (activations already released)')
-    xh, xt, xg, xt_bs, xg_bs = token.inputs
     B, H, C, dev = token.B, token.H, token.C, token.device
-    ws = token.workspace
     g = token.grads()
     dl = dlogits.contiguous()
     if dl.dtype != torch.float32:
         dl = dl.float()
-    st = _stream(dev)
+    args = (token.inputs, B, H, C, flat.buf, token.mode, precision, dl, g, token.workspace, _stream(dev))
     if dp is None:
-        _lib.check(lib.nrm_backward(_ptr(xh), _ptr(xt), xt_bs, _ptr(xg), xg_bs, B, H, C, _ptr(flat.buf), token.mode, precision,
-                                    _ptr(dl), _ptr(g), _ptr(ws), ws.numel(), st), 'nrm_backward')
+        backward(*args)
     else:
         sync = dp.sync_bn and (token.mode & MODE_BN_BATCH_STATS)
+
+        def exchange(sums):
+            rows = dp.all_reduce_stats(sums, B * C) if sync else 0
+            dp.reduce_head_bucket(g, flat)          # overlaps with the encoder backward
+            return sums, rows
         sums = torch.empty(2 * E_DIM, dtype=torch.float64, device=dev) if sync else None
-        _lib.check(lib.nrm_backward_head(B, H, C, _ptr(flat.buf), precision, _ptr(dl), _ptr(g), _ptr(sums), _ptr(ws), ws.numel(), st),
-                   'nrm_backward_head')
-        rows = 0
-        if sync:
-            rows = dp.all_reduce_stats(sums, B * C)
-        dp.reduce_head_bucket(g, flat)          # overlaps with the encoder backward below
-        _lib.check(lib.nrm_backward_encoder(_ptr(xh), _ptr(xt), xt_bs, _ptr(xg), xg_bs, B, H, C, _ptr(flat.buf), token.mode,
-                                            precision, _ptr(sums), rows, _ptr(g), _ptr(ws), ws.numel(), st),
-                   'nrm_backward_encoder')
+        backward(*args, sums, exchange, defer_wgrad=False)
         dp.reduce_encoder_bucket(g, flat)
         dp.wait()
     token.done = True
@@ -348,23 +409,20 @@ def adam_step(param: torch.Tensor, grad: torch.Tensor, exp_avg: torch.Tensor, ex
 # ---------------------------------------------------------------------------------------
 def standalone_encoder(named: Dict[str, torch.Tensor], x_history, x_target, x_global) -> torch.Tensor:
     lib = _lib.load()
-    xh, xt, xg = prepare_inputs(x_history, x_target, x_global)
+    inputs = prepare_inputs(x_history, x_target, x_global)
     if any(p.requires_grad for p in named.values()) and torch.is_grad_enabled():
         raise _lib.NrmError('stand-alone encoder modules are inference-only (wrap the call in torch.no_grad()); '
                             'training runs through UserModel.forward')
-    dev = xh.device
+    dev = inputs.xh.device
     entries, fixed = layout()
     buf = torch.zeros(fixed, dtype=torch.float32, device=dev)
     for name, off, numel in entries:
         if name in named:
             buf[off:off + numel].copy_(named[name].detach().reshape(-1))
-    B, H, C = xh.shape[0], xh.shape[1], xt.shape[1]
+    B, H, C = inputs.xh.shape[0], inputs.xh.shape[1], inputs.xt.shape[1]
     need = int(lib.nrm_workspace_bytes(B, H, C, MODE_EVAL))
     ws = torch.empty(need, dtype=torch.uint8, device=dev)
-    xt_bs = xt.stride(0) if B > 1 else C * TGT_COLS
-    xg_bs = xg.stride(0) if B > 1 else C * GLOBAL_COLS
-    _lib.check(lib.nrm_forward_encoder(_ptr(xh), _ptr(xt), xt_bs, _ptr(xg), xg_bs, B, H, C, _ptr(buf), MODE_EVAL, 0, None,
-                                       _ptr(ws), need, _stream(dev)), 'nrm_forward_encoder')
+    call(inputs, 'nrm_forward_encoder', B, H, C, _ptr(buf), MODE_EVAL, 0, None, _ptr(ws), need, _stream(dev))
     off_e = int(lib.nrm_workspace_e_offset(B, H, C, MODE_EVAL))
     e = ws[off_e:off_e + 4 * B * C * E_DIM].view(torch.float32).view(B, C, E_DIM)
     return e.clone()

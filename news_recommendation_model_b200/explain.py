@@ -15,13 +15,13 @@ row embeds as the id-0 rows of the embedding tables, so its label features are n
 is told where they are."""
 from __future__ import annotations
 
-import ctypes
 from typing import NamedTuple, Optional, Union
 
 import torch
 
 from . import _lib, engine, wire
-from .config import GLOBAL_COLS, HIST_COLS, TGT_COLS
+from .config import HIST_COLS
+from .engine import _ptr, _stream
 
 TOPK_MAX = 64
 
@@ -39,15 +39,19 @@ class HistoryTopK(NamedTuple):
     text_img_score: torch.Tensor
 
 
-def _stream(dev) -> ctypes.c_void_p:
-    return ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-
-
-def _flat(model, dev):
-    flat = model.flat_parameters()
-    if flat.device != dev:
-        raise _lib.NrmError(f'model is on {flat.device} but inputs are on {dev}')
-    return flat
+def _scores(model, inputs, B, H, C, dev) -> AttentionScores:
+    """One eval-mode `nrm_forward_scores` of `inputs` (an engine binding)."""
+    with torch.no_grad():
+        flat = model.flat_parameters()
+        if flat.device != dev:
+            raise _lib.NrmError(f'model is on {flat.device} but inputs are on {dev}')
+        ws = model._runtime().workspace(B, H, C, engine.MODE_EVAL, dev)
+        logits = torch.empty(B, C, dtype=torch.float32, device=dev)
+        scores = torch.empty(2, B, C, H, dtype=torch.float32, device=dev)
+        engine.call(inputs, 'nrm_forward_scores', B, H, C, _ptr(flat.buf), _ptr(model.bn.running_mean), _ptr(model.bn.running_var),
+                    _ptr(model.bn.num_batches_tracked), engine.MODE_EVAL, model._precision_code(), _ptr(logits), _ptr(scores), _ptr(ws),
+                    ws.numel(), _stream(dev))
+    return AttentionScores(logits, scores[0], scores[1])
 
 
 def attention_scores(model, x_history, x_target, x_global) -> AttentionScores:
@@ -58,23 +62,9 @@ def attention_scores(model, x_history, x_target, x_global) -> AttentionScores:
     neither read as batch statistics nor updated, so explaining a batch in the middle of training does not move the model.
     Runs under `torch.no_grad()` in the model's precision; the logits equal `model.eval()(x_history, x_target, x_global)`
     bit for bit."""
-    lib = _lib.load()
     with torch.no_grad():
-        xh, xt, xg = engine.prepare_inputs(x_history, x_target, x_global)
-        B, H, C = xh.shape[0], xh.shape[1], xt.shape[1]
-        dev = xh.device
-        flat = _flat(model, dev)
-        ws = model._runtime().workspace(B, H, C, engine.MODE_EVAL, dev)
-        logits = torch.empty(B, C, dtype=torch.float32, device=dev)
-        scores = torch.empty(2, B, C, H, dtype=torch.float32, device=dev)
-        xt_bs = xt.stride(0) if B > 1 else C * TGT_COLS
-        xg_bs = xg.stride(0) if B > 1 else C * GLOBAL_COLS
-        p = engine._ptr
-        _lib.check(lib.nrm_forward_scores(p(xh), p(xt), xt_bs, p(xg), xg_bs, B, H, C, p(flat.buf), p(model.bn.running_mean),
-                                          p(model.bn.running_var), p(model.bn.num_batches_tracked), engine.MODE_EVAL,
-                                          model._precision_code(), p(logits), p(scores), p(ws), ws.numel(), _stream(dev)),
-                   'nrm_forward_scores')
-    return AttentionScores(logits, scores[0], scores[1])
+        inputs = engine.prepare_inputs(x_history, x_target, x_global)
+    return _scores(model, inputs, x_history.shape[0], x_history.shape[1], x_target.shape[1], inputs.xh.device)
 
 
 def attention_scores_compact(model, table: wire.ArticleTable, cb: wire.CompactBatch) -> AttentionScores:
@@ -95,21 +85,7 @@ def attention_scores_compact(model, table: wire.ArticleTable, cb: wire.CompactBa
                          (cb.cand_time, (B, C), torch.int32)):
         if tuple(t.shape) != shape or t.dtype != dt or not t.is_contiguous() or t.device != cb.hist_article.device:
             raise ValueError('CompactBatch tensors must be contiguous int32 / float32 [B,H] / [B,H,2] / [B,C] on one device')
-    lib = _lib.load()
-    dev = cb.hist_article.device
-    with torch.no_grad():
-        flat = _flat(model, dev)
-        ws = model._runtime().workspace(B, H, C, engine.MODE_EVAL, dev)
-        logits = torch.empty(B, C, dtype=torch.float32, device=dev)
-        scores = torch.empty(2, B, C, H, dtype=torch.float32, device=dev)
-        cs = _lib.CompactBatchStruct(table.rows.data_ptr(), table.n, cb.hist_article.data_ptr(), cb.hist_time.data_ptr(),
-                                     cb.hist_click.data_ptr(), cb.cand_article.data_ptr(), cb.cand_time.data_ptr(), None, None)
-        p = engine._ptr
-        _lib.check(lib.nrm_forward_scores_compact(ctypes.byref(cs), B, H, C, p(flat.buf), p(model.bn.running_mean),
-                                                  p(model.bn.running_var), p(model.bn.num_batches_tracked), engine.MODE_EVAL,
-                                                  model._precision_code(), p(logits), p(scores), p(ws), ws.numel(), _stream(dev)),
-                   'nrm_forward_scores_compact')
-    return AttentionScores(logits, scores[0], scores[1])
+    return _scores(model, engine.compact(table, cb), B, H, C, cb.hist_article.device)
 
 
 def top_history(scores: Union[AttentionScores, torch.Tensor], k: int, *, x_history: Optional[torch.Tensor] = None,

@@ -30,13 +30,13 @@ best candidates by greedy maximal marginal relevance over the articles' PCA vect
     ild, n_categories = recommend.list_diversity(table, rec.article)"""
 from __future__ import annotations
 
-import ctypes
 import numbers
 from typing import NamedTuple, Optional
 
 import torch
 
 from . import _lib, engine, wire
+from .engine import _stream
 
 TOPK_MAX = 1024
 TARGETS_MAX = 1024
@@ -60,10 +60,6 @@ class TargetRanks(NamedTuple):
     equal: torch.Tensor       # [B,P] int64 other positions with an equal score
     score: torch.Tensor       # [B,P] float32 its ranking score
     n_eligible: torch.Tensor  # [B] int64 the user's eligible positions
-
-
-def _stream(dev) -> ctypes.c_void_p:
-    return ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
 
 
 def _check_k(k, N: int) -> None:
@@ -134,10 +130,9 @@ def _forward_pool(model, table, hist_article, hist_time, hist_click, pool_time, 
     if flat.device != dev:
         raise _lib.NrmError(f'model is on {flat.device} but inputs are on {dev}')
     ws = torch.empty(int(lib.nrm_pool_workspace_bytes(B, H, N, chunk)), dtype=torch.uint8, device=dev)
-    cs = _lib.CompactBatchStruct(table.rows.data_ptr(), table.n, hist_article.data_ptr(), hist_time.data_ptr(), hist_click.data_ptr(),
-                                 pool_article.data_ptr(), pool_time.data_ptr(), None, None)
+    users = engine.compact(table, wire.CompactBatch(None, None, hist_article, hist_time, hist_click, pool_article, pool_time, None, None))
     p = engine._ptr
-    _lib.check(lib.nrm_forward_pool(ctypes.byref(cs), B, H, N, chunk, p(flat.buf), p(model.bn.running_mean), p(model.bn.running_var),
+    _lib.check(lib.nrm_forward_pool(*users.args, B, H, N, chunk, p(flat.buf), p(model.bn.running_mean), p(model.bn.running_var),
                                     model._precision_code(), p(out), p(ws), ws.numel(), _stream(dev)), 'nrm_forward_pool')
 
 

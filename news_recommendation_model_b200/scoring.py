@@ -12,7 +12,6 @@ Here the whole batch stays on the device until ONE copy back:
 `write_submission_file` mirrors `test.py:write_submission_file` without the worker processes."""
 from __future__ import annotations
 
-import ctypes
 import queue as _queue
 import zipfile
 from typing import List, Optional, Sequence, Tuple
@@ -21,14 +20,7 @@ import numpy as np
 import torch
 
 from . import _lib
-
-
-def _ptr(t: Optional[torch.Tensor]):
-    return ctypes.c_void_p(t.data_ptr()) if t is not None else None
-
-
-def _stream(dev):
-    return ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+from .engine import _ptr, _stream
 
 
 def score_epilogue(logits: torch.Tensor, empty_num: Optional[torch.Tensor] = None, want_ranks: bool = True

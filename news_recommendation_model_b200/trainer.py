@@ -17,7 +17,6 @@ Under data parallelism the graph is split around the gradient all-reduce.
 """
 from __future__ import annotations
 
-import ctypes
 import struct
 from typing import List, Optional
 
@@ -34,6 +33,7 @@ class _Slot:
         self.xh = torch.empty(B, H, HIST_COLS, dtype=torch.float64, device=dev)
         self.xt = torch.empty(B, C, TGT_COLS, dtype=torch.float64, device=dev)
         self.xg = torch.empty(B, C, GLOBAL_COLS, dtype=torch.float64, device=dev)
+        self.packed = engine.packed(self.xh, self.xt, self.xg)
         self.label = torch.empty(B, C, dtype=torch.float64, device=dev)
         self.uid = torch.empty(B, dtype=torch.int64, device=dev)
         self.ready = torch.cuda.Event()        # H2D of this slot finished
@@ -42,6 +42,7 @@ class _Slot:
         self.graph_adam: Optional[torch.cuda.CUDAGraph] = None
         self.used = False
         self.compact = None                    # device CompactBatch staging buffers (wire.py), allocated on first use
+        self.compact_inputs = None             # their engine.compact binding
         self.wire = 'packed'                   # what the last load() put into this slot
         self.rows = B                          # impressions the last load() put into this slot (< B: ragged last batch)
         self.graph_wire = None                 # wire format the captured graph was recorded for
@@ -149,31 +150,10 @@ class FusedTrainStep:
         loss_scratch = self.loss_scratch if loss_scratch is None else loss_scratch
         warming = getattr(self, '_warming', False)
         sync_bn = self.dp is not None and self.dp.sync_bn and not warming
-        direct = s.wire == 'compact' and self.compact_direct          # the slot's compact batch is the input itself
-        cb = ctypes.byref(s.cstruct) if direct else None
-        if not sync_bn:
-            if direct:
-                _lib.check(lib.nrm_forward_compact(cb, B, H, C, _p(f.buf), _p(m.bn.running_mean), _p(m.bn.running_var),
-                                                   _p(m.bn.num_batches_tracked), self.mode, self.precision, _p(self.logits), _p(self.ws),
-                                                   self.ws.numel(), st), 'nrm_forward_compact')
-            else:
-                _lib.check(lib.nrm_forward(_p(s.xh), _p(s.xt), C * TGT_COLS, _p(s.xg), C * GLOBAL_COLS, B, H, C, _p(f.buf),
-                                           _p(m.bn.running_mean), _p(m.bn.running_var), _p(m.bn.num_batches_tracked), self.mode,
-                                           self.precision, _p(self.logits), _p(self.ws), self.ws.numel(), st), 'nrm_forward')
-        else:
-            # synchronised BatchNorm: the two halves of the forward around the exchange of the column sums (2 x 264 doubles);
-            # N ranks x B impressions then reproduce one process on N * B
-            sums = self._bn_sums(0)
-            if direct:
-                _lib.check(lib.nrm_forward_encoder_compact(cb, B, H, C, _p(f.buf), self.mode, self.precision, _p(sums), _p(self.ws),
-                                                           self.ws.numel(), st), 'nrm_forward_encoder_compact')
-            else:
-                _lib.check(lib.nrm_forward_encoder(_p(s.xh), _p(s.xt), C * TGT_COLS, _p(s.xg), C * GLOBAL_COLS, B, H, C, _p(f.buf), self.mode,
-                                                   self.precision, _p(sums), _p(self.ws), self.ws.numel(), st), 'nrm_forward_encoder')
-            gsums = self._exchange_stats(0, sums, B * C)
-            _lib.check(lib.nrm_forward_head(B, H, C, _p(f.buf), _p(m.bn.running_mean), _p(m.bn.running_var), _p(m.bn.num_batches_tracked),
-                                            self.mode, self.precision, _p(gsums), B * C * self.world, _p(self.logits), _p(self.ws), self.ws.numel(), st),
-                       'nrm_forward_head')
+        # compact slot on the direct path: the compact batch is the input itself
+        inputs = s.compact_inputs if s.wire == 'compact' and self.compact_direct else s.packed
+        engine.forward(inputs, B, H, C, f.buf, m.bn.running_mean, m.bn.running_var, m.bn.num_batches_tracked, self.mode, self.precision,
+                       self.logits, self.ws, st, **(self._sync_bn(0, B * C) if sync_bn else {}))
         delta = f.buf[f.fixed:f.fixed + f.delta_numel]
         _lib.check(lib.nrm_loss_forward(_p(self.logits), _p(delta), f.delta_numel, _p(s.uid), _p(s.label), B, C, self.alpha, _p(loss_out),
                                         _p(loss_scratch), loss_scratch.numel(), st), 'nrm_loss_forward')
@@ -187,27 +167,15 @@ class FusedTrainStep:
             ddelta = self.grads[f.fixed:f.fixed + f.delta_numel]
             _lib.check(lib.nrm_loss_backward(_p(s.uid), B, C, _p(self.one), _p(self.dlogits), _p(ddelta), f.delta_numel,
                                              _p(loss_scratch), loss_scratch.numel(), st), 'nrm_loss_backward')
-        if not sync_bn:
-            if direct:
-                _lib.check(lib.nrm_backward_compact(cb, B, H, C, _p(f.buf), self.mode, self.precision, _p(self.dlogits), _p(self.grads),
-                                                    _p(self.ws), self.ws.numel(), st), 'nrm_backward_compact')
-            else:
-                _lib.check(lib.nrm_backward(_p(s.xh), _p(s.xt), C * TGT_COLS, _p(s.xg), C * GLOBAL_COLS, B, H, C, _p(f.buf), self.mode,
-                                            self.precision, _p(self.dlogits), _p(self.grads), _p(self.ws), self.ws.numel(), st),
-                           'nrm_backward')
-        else:
-            sums = self._bn_sums(1)
-            # head weight gradients stay on the library's side stream until the encoder backward has been enqueued
-            _lib.check(lib.nrm_backward_head_deferred(B, H, C, _p(f.buf), self.precision, _p(self.dlogits), _p(self.grads), _p(sums), _p(self.ws),
-                                                      self.ws.numel(), st), 'nrm_backward_head_deferred')
-            gsums = self._exchange_stats(1, sums, B * C)
-            if direct:
-                _lib.check(lib.nrm_backward_encoder_compact(cb, B, H, C, _p(f.buf), self.mode, self.precision, _p(gsums), B * C * self.world,
-                                                            _p(self.grads), _p(self.ws), self.ws.numel(), st), 'nrm_backward_encoder_compact')
-            else:
-                _lib.check(lib.nrm_backward_encoder(_p(s.xh), _p(s.xt), C * TGT_COLS, _p(s.xg), C * GLOBAL_COLS, B, H, C, _p(f.buf), self.mode,
-                                                    self.precision, _p(gsums), B * C * self.world, _p(self.grads), _p(self.ws), self.ws.numel(), st),
-                           'nrm_backward_encoder')
+        engine.backward(inputs, B, H, C, f.buf, self.mode, self.precision, self.dlogits, self.grads, self.ws, st,
+                        **(self._sync_bn(1, B * C) if sync_bn else {}))
+
+    def _sync_bn(self, which: int, local_rows: int) -> dict:
+        """Synchronised BatchNorm: the two halves of the forward (which = 0) or backward (1) around the exchange of the column sums
+        (2 x 264 doubles); N ranks x B impressions then reproduce one process on N * B.  In the backward the head weight gradients
+        stay on the library's side stream until the encoder backward has been enqueued."""
+        return {'bn_sums': self._bn_sums(which),
+                'exchange': lambda sums: (self._exchange_stats(which, sums, local_rows), local_rows * self.world)}
 
     def _bn_sums(self, which: int) -> torch.Tensor:
         if self.peer is not None:
@@ -284,10 +252,7 @@ class FusedTrainStep:
         if s.compact is None:
             s.compact = wire.CompactBatch(*[torch.zeros((self.B,) + tuple(getattr(batch, f).shape[1:]), dtype=getattr(batch, f).dtype, device=self.dev)
                                             for f in batch.__dataclass_fields__])
-            c = s.compact
-            s.cstruct = _lib.CompactBatchStruct(self.articles.rows.data_ptr(), int(self.articles.n), c.hist_article.data_ptr(),
-                                                c.hist_time.data_ptr(), c.hist_click.data_ptr(), c.cand_article.data_ptr(),
-                                                c.cand_time.data_ptr(), c.label.data_ptr(), s.label.data_ptr())
+            s.compact_inputs = engine.compact(self.articles, s.compact, s.label)
             self._expand(s)                                  # first launch of the kernel outside any graph capture
             # the zero fills / the expansion above run on the compute stream: the H2D copies below must not overtake them
             self.copy_stream.wait_stream(torch.cuda.current_stream(self.dev))

@@ -20,7 +20,6 @@ pinned `CompactBatch`es; `PrefetchLoader` does the same from a background thread
 no per-step collate of float64 `[B,200,80]`, no per-batch pinning)."""
 from __future__ import annotations
 
-import ctypes
 import queue
 import threading
 import time
@@ -32,6 +31,7 @@ import torch
 
 from . import _lib
 from .config import GLOBAL_COLS, HIST_COLS, TGT_COLS
+from .engine import _ptr, _stream
 from .synthetic import Batch
 
 ARTICLE_COLS = 80           # float32 per article row: pca 64 | cat | sub 5 | sent 3 | type | global 3 | pad 3
@@ -88,10 +88,6 @@ class CompactBatch:
         return int(self.hist_article.shape[0]), int(self.hist_article.shape[1]), int(self.cand_article.shape[1])
 
 
-def _ptr(t):
-    return ctypes.c_void_p(t.data_ptr()) if t is not None else None
-
-
 def expand_into(table: ArticleTable, cb: CompactBatch, xh: torch.Tensor, xt: torch.Tensor, xg: torch.Tensor,
                 label: Optional[torch.Tensor]) -> None:
     """Enqueue `nrm_expand_compact` on the current stream: device CompactBatch -> packed float64 tensors (preallocated)."""
@@ -111,7 +107,7 @@ def expand_into(table: ArticleTable, cb: CompactBatch, xh: torch.Tensor, xt: tor
     _lib.check(_lib.load().nrm_expand_compact(_ptr(table.rows), table.n, _ptr(cb.hist_article), _ptr(cb.hist_time), _ptr(cb.hist_click),
                                               _ptr(cb.cand_article), _ptr(cb.cand_time), _ptr(cb.label) if label is not None else None,
                                               B, H, C, _ptr(xh), _ptr(xt), _ptr(xg), _ptr(label),
-                                              ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)), 'nrm_expand_compact')
+                                              _stream(dev)), 'nrm_expand_compact')
 
 
 def expand(table: ArticleTable, cb: CompactBatch) -> Batch:

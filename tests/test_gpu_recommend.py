@@ -10,7 +10,7 @@ import torch
 import parity as P
 from fixtures import load_weights
 from recommend_ref import host_top_articles
-from news_recommendation_model_b200 import _lib, recommend, wire
+from news_recommendation_model_b200 import _lib, engine, recommend, wire
 
 pytestmark = pytest.mark.gpu
 
@@ -215,16 +215,15 @@ def test_bad_chunk_and_k_return_einval(precision):
     pa, pt = _pool(2000, seed=22)
     B, H, N = 2, 10, 2000
     table = _table()
-    cs = _lib.CompactBatchStruct(table.rows.data_ptr(), table.n, ha.data_ptr(), ht.data_ptr(), hc.data_ptr(), pa.data_ptr(), pt.data_ptr(),
-                                 None, None)
+    users = engine.compact(table, wire.CompactBatch(None, None, ha, ht, hc, pa, pt, None, None))
     flat = model.flat_parameters()
     ws = torch.empty(int(lib.nrm_pool_workspace_bytes(B, H, N, 16)), dtype=torch.uint8, device='cuda')
     logits = torch.zeros(B, N, device='cuda')
     p = lambda t: ctypes.c_void_p(t.data_ptr())
     code = model._precision_code()
-    assert lib.nrm_forward_pool(ctypes.byref(cs), B, H, N, 12, p(flat.buf), p(model.bn.running_mean), p(model.bn.running_var), code,
+    assert lib.nrm_forward_pool(*users.args, B, H, N, 12, p(flat.buf), p(model.bn.running_mean), p(model.bn.running_var), code,
                                 p(logits), p(ws), ws.numel(), None) == -1
-    assert lib.nrm_forward_pool(ctypes.byref(cs), B, H, N, 16, p(flat.buf), p(model.bn.running_mean), p(model.bn.running_var), code,
+    assert lib.nrm_forward_pool(*users.args, B, H, N, 16, p(flat.buf), p(model.bn.running_mean), p(model.bn.running_var), code,
                                 p(logits), p(ws), ws.numel(), None) == 0
     pos = torch.empty(B, 1025, dtype=torch.int32, device='cuda')
     val = torch.empty(B, 1025, device='cuda')

@@ -135,6 +135,13 @@ def test_argument_errors_are_reported_without_a_gpu():
     assert rc == -1 and b'nrm_adam_step' in lib.nrm_last_error()
     rc = lib.nrm_forward(None, None, 0, None, 0, 0, 1, 1, None, None, None, None, 0, 0, None, None, 0, None)
     assert rc == -1
+    # a batch stride below one impression (C * 78 / C * 3 doubles) is refused before the workspace is looked at, by every packed entry point
+    fake = ctypes.c_void_p(256)
+    B, H, C = 2, 3, 4
+    rc = lib.nrm_backward(fake, fake, C * 78 - 1, fake, C * 3, B, H, C, fake, 3, 2, fake, fake, None, 0, None)
+    assert rc == -1 and b'nrm_backward: batch stride' in lib.nrm_last_error()
+    rc = lib.nrm_backward_encoder(fake, fake, C * 78, fake, C * 3 - 1, B, H, C, fake, 3, 2, None, 0, fake, None, 0, None)
+    assert rc == -1 and b'nrm_backward_encoder: batch stride' in lib.nrm_last_error()
 
 
 def test_gelu_approximation_restated_in_numpy():

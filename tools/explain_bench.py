@@ -41,7 +41,8 @@ def card():
 def setup(model, b, k):
     lib = _lib.load()
     keep = b.x_target.shape[1] - int(b.empty_num.min())
-    xh, xt, xg = engine.prepare_inputs(b.x_history, b.x_target[:, :keep], b.x_global[:, :keep])
+    inputs = engine.prepare_inputs(b.x_history, b.x_target[:, :keep], b.x_global[:, :keep])
+    xh, xt = inputs.xh, inputs.xt
     B, H, C = xh.shape[0], xh.shape[1], xt.shape[1]
     dev = xh.device
     flat = model.flat_parameters()
@@ -53,7 +54,7 @@ def setup(model, b, k):
     p = engine._ptr
     prec = model._precision_code()
     st = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-    common = (p(xh), p(xt), xt.stride(0), p(xg), xg.stride(0), B, H, C, p(flat.buf), p(model.bn.running_mean), p(model.bn.running_var),
+    common = (*inputs.args, B, H, C, p(flat.buf), p(model.bn.running_mean), p(model.bn.running_var),
               p(model.bn.num_batches_tracked), engine.MODE_EVAL, prec, p(logits))
 
     def forward():

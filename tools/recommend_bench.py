@@ -81,16 +81,15 @@ def pool_call(model, table, cb, pa, pt, chunk):
     N = pa.shape[0]
     ws = torch.empty(int(lib.nrm_pool_workspace_bytes(B, H, N, chunk)), dtype=torch.uint8, device='cuda')
     logits = torch.empty(B, N, device='cuda')
-    cs = _lib.CompactBatchStruct(table.rows.data_ptr(), table.n, cb.hist_article.data_ptr(), cb.hist_time.data_ptr(), cb.hist_click.data_ptr(),
-                                 pa.data_ptr(), pt.data_ptr(), None, None)
+    users = engine.compact(table, wire.CompactBatch(None, None, cb.hist_article, cb.hist_time, cb.hist_click, pa, pt, None, None))
     p = engine._ptr
     flat = model.flat_parameters()
-    args = (ctypes.byref(cs), B, H, N, chunk, p(flat.buf), p(model.bn.running_mean), p(model.bn.running_var), model._precision_code(),
+    args = (*users.args, B, H, N, chunk, p(flat.buf), p(model.bn.running_mean), p(model.bn.running_var), model._precision_code(),
             p(logits), p(ws), ws.numel(), stream())
 
     def run():
         _lib.check(lib.nrm_forward_pool(*args), 'nrm_forward_pool')
-    run.logits, run.cs = logits, cs
+    run.logits, run.users = logits, users
     return run
 
 
