@@ -302,6 +302,24 @@ int nrm_pool_rank(const float* logits, int n_models, long long model_stride, int
 int nrm_pool_diversify(const int* cand_pos, const float* cand_score, int B, int n_cand, int k, float lambda, int max_per_category,
                        const int* pool_article, int N, const float* article_rows, int n_articles, int* pos_out, float* val_out,
                        float* gain_out, void* stream);
+/*   nrm_sample_negatives: k = C - C0 negatives per impression drawn from a pool, appended to the impression's own C0 candidates, in
+ *     place: cand_article int32 / cand_time uint32 / label32 float32 [B,C] are read in columns 0..C0-1 and written in columns
+ *     C0..C-1.  hist_article int32 [B,H] (0 = pad row).  pool_article int32 [N]; pool_cdf int64 [N] the inclusive prefix sum of the
+ *     positions' non-negative integer weights, where a position whose id is outside [1, n_articles) has weight 0; total = cdf[N-1]
+ *     (at most 2^62; 0 draws nothing).  step: int64 on the device, the number of completed optimizer steps t (FusedTrainStep passes
+ *     its Adam state, whose first field is the step).  Impression b (row index row_offset + b):
+ *       - attempt a = 0, 1, ... computes Philox4x32-10 of counter (a, row_offset + b, t & 0xffffffff, t >> 32) and key
+ *         (seed & 0xffffffff, seed >> 32), u = x0 | x1 << 32, r = (u * total) >> 64 (the high word of the 128-bit product), and
+ *         draws the first pool position n with cdf[n] > r, so position n is drawn with probability weight(n) / total;
+ *       - the drawn id is rejected if it is outside [1, n_articles), one of the impression's history ids, one of its C0 candidate
+ *         ids, or a negative already accepted for it; else the i-th accepted id fills column C0 + i with the cand_time of the
+ *         impression's first column c < C0 with label32 > 0 (time-matched to the positive) and label 0;
+ *       - sampling stops after k acceptances or 32 k attempts; the columns left, and all k columns of an impression without a
+ *         positive, become pads (article 0, time 0, label 0).
+ *     1 <= C - C0 <= 64, H + C <= 16384, 0 <= row_offset with row_offset + B < 2^31.  Results do not depend on timing. */
+int nrm_sample_negatives(const int* hist_article, int H, int* cand_article, unsigned* cand_time, float* label32, int B, int C, int C0,
+                         const int* pool_article, const long long* pool_cdf, int N, int n_articles, unsigned long long seed,
+                         const long long* step, int row_offset, void* stream);
 
 /* ---- UserModel.loss (user_model.py:37-43) ---------------------------------------- */
 /* loss = (1-alpha) BCE(softmax(out), y) + alpha BCE(softmax(out + delta[id]), y), mean

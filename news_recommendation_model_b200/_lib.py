@@ -75,6 +75,7 @@ SIGNATURES = {
     'nrm_pool_topk': (i32, [vp, i32, ll, i32, i32, i32, vp, i32, vp, i32, vp, vp, vp]),
     'nrm_pool_rank': (i32, [vp, i32, ll, i32, i32, vp, i32, vp, i32, vp, i32, vp, vp, vp, vp, vp, vp, vp]),
     'nrm_pool_diversify': (i32, [vp, vp, i32, i32, i32, f32, i32, vp, i32, vp, i32, vp, vp, vp, vp]),
+    'nrm_sample_negatives': (i32, [vp, i32, vp, vp, vp, i32, i32, i32, vp, vp, i32, i32, C.c_ulonglong, vp, i32, vp]),
 }
 
 

@@ -75,6 +75,10 @@ int launch_expand_compact(const float* articles, int n_articles, const int* hist
                           const int* cand_article, const unsigned* cand_time, const float* label32, long long NH, long long R,
                           double* x_history, double* x_target, double* x_global, double* label64, cudaStream_t s);
 
+// slot of article id `id` in an open-addressing table of 1 << lg ints (0 = empty), probed linearly: the exclusion sets of
+// nrm_recommend.cu and nrm_negatives.cu
+__device__ __forceinline__ unsigned pool_hash(int id, int lg) { return ((unsigned)id * 0x9E3779B1u) >> (32 - lg); }
+
 // nrm_recommend.cu: per user, the k best eligible positions of a shared article pool (nrm_pool_topk)
 int launch_pool_topk(const float* logits, int n_models, long long model_stride, int B, int N, int k, const int* pool_article, int n_articles,
                      const int* hist_article, int H, int* pos_out, float* val_out, cudaStream_t s);

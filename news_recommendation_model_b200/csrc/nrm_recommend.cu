@@ -43,8 +43,6 @@ __device__ __forceinline__ float pool_key_score(unsigned long long key) {
   return __uint_as_float((u & 0x80000000u) ? (u & 0x7fffffffu) : ~u);
 }
 
-__device__ __forceinline__ unsigned pool_hash(int id, int lg) { return ((unsigned)id * 0x9E3779B1u) >> (32 - lg); }
-
 __device__ __forceinline__ bool pool_clicked(const int* tab, int lg, int id) {
   if (lg == 0) return false;
   const unsigned m = (1u << lg) - 1;

@@ -65,11 +65,21 @@ class FusedTrainStep:
     SPARSE_DELTA_MIN = 65536
 
     def __init__(self, model, B: int, H: int, C: int, *, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=1e-5,
-                 alpha=0.95, use_graph=True, ring=8, nslots=2, articles=None):
+                 alpha=0.95, use_graph=True, ring=8, nslots=2, articles=None, negatives=None):
         """`articles`: a device `wire.ArticleTable`; with it `load()` also accepts `wire.CompactBatch`es (ids instead of
-        packed float64 rows) and the step starts with the expansion kernel."""
+        packed float64 rows) and the step starts with the expansion kernel.
+        `negatives`: a `negatives.NegativeSampler` (needs `articles`).  `C` is then the width after sampling: `load()` takes
+        CompactBatches of C - k candidate columns, and every step first appends k pool negatives per impression, drawn at step t =
+        the optimizer steps completed so far (read on the device, so every graph replay draws afresh) and row offset rank * B
+        under data parallelism.  Packed batches are refused."""
         self.model, self.B, self.H, self.C, self.alpha = model, B, H, C, float(alpha)
         self.articles = articles
+        self.negatives = negatives
+        if negatives is not None:
+            if articles is None:
+                raise ValueError('FusedTrainStep: negatives= needs articles=ArticleTable')
+            if C <= negatives.k:
+                raise ValueError(f'FusedTrainStep: C = {C} leaves no candidate column before the {negatives.k} negatives')
         self.flat = model.flat_parameters()
         dev = self.flat.device
         self.dev, self.lib = dev, _lib.load()
@@ -95,6 +105,7 @@ class FusedTrainStep:
         # AdamDeviceState: int64 step | lr, beta1, beta2, eps, wd, grad_scale, step_size, bc2_sqrt
         raw = struct.pack('<q8f', 0, lr, betas[0], betas[1], eps, weight_decay, 1.0, 0.0, 0.0)
         self.adam_state = torch.frombuffer(bytearray(raw), dtype=torch.uint8).to(dev)
+        self.adam_step = self.adam_state[:8].view(torch.int64)     # the step field: the sampler's t
         ws_bytes = int(self.lib.nrm_workspace_bytes(B, H, C, self.mode))
         self.ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
         ls_bytes = int(self.lib.nrm_loss_scratch_bytes(B, C))
@@ -112,6 +123,7 @@ class FusedTrainStep:
         self.use_graph = use_graph and not (self.dp is not None and self.dp.sync_bn and self.peer is None)
         self.one_graph = self.dp is None or self.peer is not None
         self.world = world
+        self.row_offset = self.dp.rank * B if self.dp is not None and negatives is not None else 0    # of the sampler's Philox counter
         self._tail_scratch = {}
         self._warmup()
 
@@ -247,20 +259,29 @@ class FusedTrainStep:
         if self.articles is None:
             raise _lib.NrmError('FusedTrainStep: pass articles=ArticleTable to feed CompactBatches')
         b, bh, bc = batch.shape
-        if b > self.B or (bh, bc) != (self.H, self.C):
-            raise ValueError(f'CompactBatch of shape {batch.shape} does not fit this step (B <= {self.B}, H = {self.H}, C = {self.C})')
+        C0 = self.C - (self.negatives.k if self.negatives is not None else 0)
+        if b > self.B or (bh, bc) != (self.H, C0):
+            raise ValueError(f'CompactBatch of shape {batch.shape} does not fit this step (B <= {self.B}, H = {self.H}, C = {C0}'
+                             + (f' before the {self.negatives.k} negatives)' if self.negatives is not None else ')'))
         if s.compact is None:
-            s.compact = wire.CompactBatch(*[torch.zeros((self.B,) + tuple(getattr(batch, f).shape[1:]), dtype=getattr(batch, f).dtype, device=self.dev)
+            cand = ('cand_article', 'cand_time', 'label')       # [B, C]: the loaded columns, then the negatives
+            s.compact = wire.CompactBatch(*[torch.zeros((self.B,) + ((self.C,) if f in cand else tuple(getattr(batch, f).shape[1:])),
+                                                        dtype=getattr(batch, f).dtype, device=self.dev)
                                             for f in batch.__dataclass_fields__])
             s.compact_inputs = engine.compact(self.articles, s.compact, s.label)
-            self._expand(s)                                  # first launch of the kernel outside any graph capture
+            self._expand(s)                                  # first launch of the kernels outside any graph capture
             # the zero fills / the expansion above run on the compute stream: the H2D copies below must not overtake them
             self.copy_stream.wait_stream(torch.cuda.current_stream(self.dev))
         with torch.cuda.stream(self.copy_stream):
             if s.used:
                 self.copy_stream.wait_event(s.consumed)
             fields = ('hist_article', 'hist_time', 'hist_click', 'cand_article', 'cand_time', 'label')
-            if b == self.B:                                  # full batch: one multi-tensor copy call (host time, not bytes, is what counts here)
+            if self.negatives is not None:                   # into the first C0 columns
+                dst = [getattr(s.compact, f)[:b] for f in fields[:3]] + [getattr(s.compact, f)[:b, :C0] for f in fields[3:]]
+                for d, f in zip(dst, fields):
+                    d.copy_(getattr(batch, f), non_blocking=True)
+                s.uid[:b].copy_(batch.user_id, non_blocking=True)
+            elif b == self.B:                                # full batch: one multi-tensor copy call (host time, not bytes, is what counts here)
                 torch._foreach_copy_([getattr(s.compact, f) for f in fields] + [s.uid], [getattr(batch, f) for f in fields] + [batch.user_id],
                                      non_blocking=True)
             else:
@@ -277,10 +298,13 @@ class FusedTrainStep:
         s.rows = b                                           # b < B: ragged last batch (expanded whole, trained on its first b rows)
         return s
 
-    def _expand(self, s: _Slot):
-        """Compact slot -> what the forward reads: nothing to do on the direct path (the row kernels read the compact batch; the
-        labels are converted by the first of them), the packed float64 tensors otherwise."""
+    def _expand(self, s: _Slot, rows: Optional[int] = None):
+        """Compact slot -> what the forward reads: the pool negatives appended to its first `rows` impressions (with a sampler),
+        then nothing more on the direct path (the row kernels read the compact batch; the labels are converted by the first of
+        them), the packed float64 tensors otherwise."""
         from . import wire
+        if self.negatives is not None:
+            self.negatives.sample_into(s.compact, self.C - self.negatives.k, self.adam_step, self.row_offset, rows)
         if self.compact_direct:
             return
         wire.expand_into(self.articles, s.compact, s.xh, s.xt, s.xg, s.label)
@@ -288,6 +312,8 @@ class FusedTrainStep:
     def load(self, batch) -> _Slot:
         """Enqueue the H2D copy of a (pinned) host batch into the next slot (round robin).  `batch` is a packed
         `synthetic.Batch`-like object (x_history, x_target, x_global, label, user_id) or a `wire.CompactBatch`."""
+        if self.negatives is not None and not hasattr(batch, 'hist_article'):
+            raise ValueError('FusedTrainStep: with negatives= the step takes CompactBatches only (the sampler appends article ids)')
         s = self.slots[self.loaded % len(self.slots)]
         self.loaded += 1
         if hasattr(batch, 'hist_article'):
@@ -328,7 +354,7 @@ class FusedTrainStep:
                 scratch = self._tail_scratch[s.rows] = torch.zeros(int(self.lib.nrm_loss_scratch_bytes(s.rows, self.C)),
                                                                    dtype=torch.uint8, device=self.dev)
             if s.wire == 'compact':
-                self._expand(s)
+                self._expand(s, s.rows)
             self._forward_backward(s, loss_out, B=s.rows, loss_scratch=scratch)
             self._adam()
         elif self.use_graph:
