@@ -200,9 +200,9 @@ int nrm_backward_encoder(const double* x_history, const double* x_target, long l
 /* ---- the compact wire format as a direct input (no expansion to the packed float64 tensors) ----------------------------
  * nrm_expand_compact (below) rebuilds the reference's packed tensors for the entry points above.  These variants hand the
  * article table + per-impression ids / time buckets / click features straight to the row kernels instead: the 36 MB of
- * float64 rows are neither written nor read.  Same results, bit for bit.  Tensor-core precisions only (the FFMA attention
- * kernels of precision fp32 read the packed rows): NRM_EUNSUPPORTED otherwise.  label32 / label64 are optional (both null):
- * when given, the float32 labels are converted to the float64 labels nrm_loss_forward reads. */
+ * float64 rows are neither written nor read.  Same results, bit for bit, in every precision: only the row kernels read the batch,
+ * every later kernel reads the workspace.  label32 / label64 are optional (both null): when given, the float32 labels are
+ * converted to the float64 labels nrm_loss_forward reads. */
 typedef struct {
   const float* articles; int n_articles;      /* [n,80] float32, row 0 = the all-zero pad article                 */
   const int* hist_article; const unsigned* hist_time; const float* hist_click;   /* [B,H], [B,H] packed buckets, [B,H,2] */
@@ -227,8 +227,7 @@ int nrm_backward_encoder_compact(const nrm_compact_batch* batch, int B, int H, i
  * rows get scores too (the reference does not mask them; they contribute to the pooled sum).
  *   nrm_forward_scores[_compact]: nrm_forward[_compact] in mode NRM_MODE_EVAL (any other mode: NRM_EINVAL; BatchNorm reads its
  *     running statistics and nothing is written to them) that also writes `scores`; the logits are bit-identical to nrm_forward's
- *     for the same precision, the workspace is nrm_workspace_bytes(B, H, C, NRM_MODE_EVAL).  The compact variant has
- *     nrm_forward_compact's precision limits.
+ *     for the same precision, the workspace is nrm_workspace_bytes(B, H, C, NRM_MODE_EVAL).
  *   nrm_history_topk: per (branch, b, c) row the k largest scores and their history positions, descending, ties to the lower
  *     position (Python's stable sorted(..., reverse=True)); idx_out int32 / val_out float32 [2,B,C,k], 1 <= k <= min(H, 64).  Pad rows
  *     are left out: all-zero rows of x_history [B,H,80] or hist_article [B,H] == 0 (at most one of the two; both null: none); slots
@@ -251,8 +250,9 @@ int nrm_history_topk(const float* scores, int B, int C, int H, int k, const doub
  *     every b), in the same precision (all three).  BatchNorm reads its running statistics only.
  *     users->hist_* are the users' [B,H] / [B,H,2] compact histories; users->cand_article / cand_time are the pool's [N] ids and
  *     packed time buckets (one time for all users); label32 / label64 must be null.  The pool is processed in chunks of `chunk`
- *     articles (a positive multiple of 8, the attention's candidate group: any such chunk gives the same bits); the workspace
- *     is nrm_pool_workspace_bytes(B, H, N, chunk) bytes, 256-byte aligned, and grows with B * chunk.
+ *     articles (a positive multiple of 8, the attention's candidate group: any such chunk gives the same bits).  The row kernels
+ *     read the users and the chunk's ids as they are, nothing is expanded to packed rows: the workspace, nrm_pool_workspace_bytes(B,
+ *     H, N, chunk) bytes, 256-byte aligned, is that of one eval forward of B users x `chunk` candidates plus its [B, chunk] logits.
  *   nrm_pool_topk: per user b the k pool positions with the largest score, descending, ties to the lower position (Python's
  *     stable sorted(..., reverse=True), test.py:124-127); pos_out int32 / val_out float32 [B,k], 1 <= k <= min(N, 1024).
  *     logits: n_models >= 1 (at most 16) stacked [B,N] slices, model m at logits + m * model_stride.  Position n is eligible

@@ -266,12 +266,12 @@ static int encoder_forward(const BatchPtrs& in, const float* P, Workspace& w, in
   { KernelTimer t("w1_forward", s); NRM_TRY(launch_w1_forward(P, w, s)); }
   NRM_CUDA(cudaStreamWaitEvent(s, ss->join_tp, 0));          // join: operand images, transposed head matrices, tp
   if (!tc) {
-    { KernelTimer t("attention_forward_label", s); NRM_TRY(launch_attention_forward(in, P, w, 0, precision, s)); }
-    { KernelTimer t("attention_forward_textimg", s); NRM_TRY(launch_attention_forward(in, P, w, 1, precision, s)); }
+    { KernelTimer t("attention_forward_label", s); NRM_TRY(launch_attention_forward(P, w, 0, s)); }
+    { KernelTimer t("attention_forward_textimg", s); NRM_TRY(launch_attention_forward(P, w, 1, s)); }
   } else {
     // tensor-core path: one launch covers both branches
     KernelTimer t("attention_forward", s);
-    NRM_TRY(launch_attention_forward_rs(in, w, precision, s));
+    NRM_TRY(launch_attention_forward_rs(w, precision, s));
   }
   // join: the id sort (long finished: it ran under the w1 / attention kernels) comes back to the caller's stream HERE, so a
   // training-mode forward that is never followed by a backward (validation with gradients enabled, a graph capture of the
@@ -287,7 +287,7 @@ static int encoder_backward(const BatchPtrs& in, const float* P, Workspace& w, i
   // tensor-core precisions: the row-stacked backward sums over rows (weight gradients, dtp); its label branch exports dhid for the
   // input-gradient kernel
   { KernelTimer t("attention_backward_label", s);
-    if (tc) NRM_TRY(launch_attention_backward_rs(w, 0, precision, true, s)); else NRM_TRY(launch_attention_backward(in, P, w, 0, precision, s)); }
+    if (tc) NRM_TRY(launch_attention_backward_rs(w, 0, precision, true, s)); else NRM_TRY(launch_attention_backward(P, w, 0, s)); }
   if (tc) {
     // the label branch's input gradients (dxh, dxt) come from the dhid tiles the kernel above exported
     KernelTimer t("attention_input_grad_label", s);
@@ -299,7 +299,7 @@ static int encoder_backward(const BatchPtrs& in, const float* P, Workspace& w, i
   NRM_CUDA(cudaEventRecord(ss->fork2, s));
   NRM_CUDA(cudaStreamWaitEvent(ss->stream, ss->fork2, 0));
   { KernelTimer t("attention_backward_textimg", s);
-    if (tc) NRM_TRY(launch_attention_backward_rs(w, 1, precision, false, s)); else NRM_TRY(launch_attention_backward(in, P, w, 1, precision, s)); }
+    if (tc) NRM_TRY(launch_attention_backward_rs(w, 1, precision, false, s)); else NRM_TRY(launch_attention_backward(P, w, 1, s)); }
   // w1: dxin_h = dxh W1, dW1 = dxh^T xin_h, db1 = colsum(dxh)
   { KernelTimer t("w1_backward", ss->stream);
     if (tc) NRM_TRY(launch_w1_backward_tc(P, w, G, precision, ss->stream)); else NRM_TRY(launch_w1_backward(P, w, G, ss->stream)); }
@@ -311,7 +311,7 @@ static int encoder_backward(const BatchPtrs& in, const float* P, Workspace& w, i
   }
   { KernelTimer t("attention_finish", s);
     if (tc) NRM_TRY(launch_attention_finish_tc(P, w, G, s));   // one pass for both branches
-    else { NRM_TRY(launch_attention_finish(P, w, 0, precision, G, s)); NRM_TRY(launch_attention_finish(P, w, 1, precision, G, s)); } }
+    else { NRM_TRY(launch_attention_finish(P, w, 0, G, s)); NRM_TRY(launch_attention_finish(P, w, 1, G, s)); } }
   NRM_CUDA(cudaStreamWaitEvent(s, ss->join2, 0));          // join: dxin_h ready
   // fork: the sentiment / instant Linear gradients (side stream) next to the table gradients (two latency-bound kernel
   // pairs that write disjoint gradient ranges)
@@ -430,28 +430,17 @@ static int packed_batch(const char* fn, const double* x_history, const double* x
   return NRM_OK;
 }
 
-// the tables and ids every reader of a compact batch needs (labels aside)
-static int compact_struct(const char* fn, const nrm_compact_batch* cb) {
+// compact wire format as the input of the row kernels (no expansion to the packed float64 tensors); cand_bs: the batch stride of the
+// candidate ids, C, or 0 when every impression has the same candidates
+static int compact_batch(const char* fn, const nrm_compact_batch* cb, int cand_bs, BatchPtrs& in) {
   if (!cb || !cb->articles || cb->n_articles <= 0 || !cb->hist_article || !cb->hist_time || !cb->hist_click || !cb->cand_article || !cb->cand_time) {
     set_error("%s: bad compact batch", fn); return NRM_EINVAL;
   }
   if ((reinterpret_cast<uintptr_t>(cb->articles) & 15) != 0) { set_error("%s: the article table must be 16-byte aligned", fn); return NRM_EINVAL; }
-  return NRM_OK;
-}
-
-// compact wire format as the input of the row kernels (no expansion to the packed float64 tensors): needs the kernels that never
-// touch the packed rows again, i.e. the row-stacked tensor-core path.  `in` points into `cp`.
-static int compact_batch(const char* fn, const nrm_compact_batch* cb, int precision, CompactPtrs& cp, BatchPtrs& in) {
-  NRM_TRY(compact_struct(fn, cb));
   if (cb->label32 && !cb->label64) { set_error("%s: bad compact batch", fn); return NRM_EINVAL; }
-  if (precision == NRM_PRECISION_FP32) {
-    set_error("%s: the compact wire format is read directly by the tensor-core precisions only (use nrm_expand_compact otherwise)", fn);
-    return NRM_EUNSUPPORTED;
-  }
-  cp = CompactPtrs{cb->articles, cb->n_articles, cb->hist_article, cb->hist_time, cb->hist_click, cb->cand_article, cb->cand_time,
-                   cb->label32, cb->label64};
-  in = BatchPtrs{nullptr, nullptr, 0, nullptr, 0};
-  in.compact = &cp;
+  in = BatchPtrs{};
+  in.compact = CompactPtrs{cb->articles, cb->n_articles, cand_bs, cb->hist_article, cb->hist_time, cb->hist_click, cb->cand_article,
+                           cb->cand_time, cb->label32, cb->label64};
   return NRM_OK;
 }
 
@@ -471,8 +460,8 @@ extern "C" int nrm_forward_encoder_compact(const nrm_compact_batch* batch, int B
   const char* fn = "nrm_forward_encoder_compact";
   NRM_TRY(check_shape(fn, B, H, C));
   if (!params) { set_error("%s: null pointer", fn); return NRM_EINVAL; }
-  CompactPtrs cp; BatchPtrs in;
-  NRM_TRY(compact_batch(fn, batch, precision, cp, in));
+  BatchPtrs in;
+  NRM_TRY(compact_batch(fn, batch, C, in));
   return forward_encoder_impl(fn, in, B, H, C, params, mode, precision, bn_sums, nullptr, workspace, workspace_bytes, stream);
 }
 
@@ -543,8 +532,8 @@ extern "C" int nrm_forward_scores_compact(const nrm_compact_batch* batch, int B,
   const char* fn = "nrm_forward_scores_compact";
   NRM_TRY(check_shape(fn, B, H, C));
   if (!params) { set_error("%s: null pointer", fn); return NRM_EINVAL; }
-  CompactPtrs cp; BatchPtrs in;
-  NRM_TRY(compact_batch(fn, batch, precision, cp, in));
+  BatchPtrs in;
+  NRM_TRY(compact_batch(fn, batch, C, in));
   NRM_TRY(scores_args(fn, mode, scores));
   NRM_TRY(forward_encoder_impl(fn, in, B, H, C, params, mode, precision, nullptr, scores, workspace, workspace_bytes, stream));
   return nrm_forward_head(B, H, C, params, bn_running_mean, bn_running_var, bn_num_batches_tracked, mode, precision, nullptr, 0,
@@ -552,11 +541,11 @@ extern "C" int nrm_forward_scores_compact(const nrm_compact_batch* batch, int B,
 }
 
 // ---- recommendation from a shared pool: every user against the same N articles, in chunks of the pool ------------------------------
-// Workspace: the users' history as packed float64 rows (expanded once), one pool chunk as packed x_target / x_global rows, the chunk's
-// [B,C] logits and the eval workspace of a (B, H, C) forward.  The encoder reads the chunk's candidate rows with batch stride 0, so
-// all B users see the same rows without a copy per user.  C is a multiple of 8, the row-stacked attention's candidate group (rs::CG),
-// so every chunk groups candidates exactly as one forward over all N columns would: the logits are that forward's, bit for bit.
-struct PoolCarve { double* xh; double* xt; double* xg; float* out; void* ws; size_t ws_bytes, bytes; };
+// Workspace: the chunk's [B,C] logits and the eval workspace of a (B, H, C) forward.  The row kernels read the users' compact histories
+// as they are and the chunk's candidate ids with batch stride 0, so all B users see the same candidates without a copy per user.  C is
+// a multiple of 8, the row-stacked attention's candidate group (rs::CG), so every chunk groups candidates exactly as one forward over
+// all N columns would: the logits are that forward's, bit for bit.
+struct PoolCarve { float* out; void* ws; size_t ws_bytes, bytes; };
 static void carve_pool(PoolCarve& pc, void* base, int B, int H, int N, int chunk) {
   const int C = chunk < N ? chunk : N;
   size_t off = 0;
@@ -565,9 +554,6 @@ static void carve_pool(PoolCarve& pc, void* base, int B, int H, int N, int chunk
     off += (bytes + 255) & ~(size_t)255;
     return p;
   };
-  pc.xh = (double*)take(sizeof(double) * B * H * HC);
-  pc.xt = (double*)take(sizeof(double) * C * TC);
-  pc.xg = (double*)take(sizeof(double) * C * GC);
   pc.out = (float*)take(sizeof(float) * B * C);
   Workspace w;
   pc.ws_bytes = carve_workspace(w, nullptr, B, H, C, NRM_MODE_EVAL);
@@ -589,7 +575,8 @@ extern "C" int nrm_forward_pool(const nrm_compact_batch* users, int B, int H, in
   if (B <= 0 || H <= 0 || N <= 0) { set_error("%s: B, H, N must be positive (got %d, %d, %d)", fn, B, H, N); return NRM_EINVAL; }
   if (chunk <= 0 || chunk % 8 != 0) { set_error("%s: chunk must be a positive multiple of 8 (got %d)", fn, chunk); return NRM_EINVAL; }
   if (precision < NRM_PRECISION_FP32 || precision > NRM_PRECISION_BF16X3) { set_error("%s: unknown precision %d", fn, precision); return NRM_EINVAL; }
-  NRM_TRY(compact_struct(fn, users));
+  BatchPtrs in;
+  NRM_TRY(compact_batch(fn, users, 0, in));
   if (users->label32 || users->label64) { set_error("%s: the pool has no labels (label32 / label64 must be null)", fn); return NRM_EINVAL; }
   if (!params || !bn_running_mean || !bn_running_var || !logits) { set_error("%s: null pointer", fn); return NRM_EINVAL; }
   const int C = chunk < N ? chunk : N;
@@ -599,18 +586,14 @@ extern "C" int nrm_forward_pool(const nrm_compact_batch* users, int B, int H, in
   carve_pool(pc, workspace, B, H, N, chunk);
   if (pc.bytes > workspace_bytes) { set_error("%s: workspace too small (%zu < %zu bytes)", fn, workspace_bytes, pc.bytes); return NRM_EWORKSPACE; }
   cudaStream_t s = (cudaStream_t)stream;
-  const nrm_compact_batch& u = *users;
-  NRM_TRY(launch_expand_compact(u.articles, u.n_articles, u.hist_article, u.hist_time, u.hist_click, nullptr, nullptr, nullptr, (long long)B * H, 0,
-                                pc.xh, nullptr, nullptr, nullptr, s));
   // the BatchNorm buffers are only read in eval mode: the head's training-only writes never happen
   float* run_mean = const_cast<float*>(bn_running_mean);
   float* run_var = const_cast<float*>(bn_running_var);
   for (int c0 = 0; c0 < N; c0 += C) {
     const int nc = N - c0 < C ? N - c0 : C;
-    NRM_TRY(launch_expand_compact(u.articles, u.n_articles, nullptr, nullptr, nullptr, u.cand_article + c0, u.cand_time + c0, nullptr, 0, nc,
-                                  nullptr, pc.xt, pc.xg, nullptr, s));
-    const BatchPtrs in{pc.xh, pc.xt, 0, pc.xg, 0};
-    NRM_TRY(forward_encoder_impl(fn, in, B, H, nc, params, NRM_MODE_EVAL, precision, nullptr, nullptr, pc.ws, pc.ws_bytes, stream));
+    BatchPtrs chunk_in = in;
+    chunk_in.compact.cand_article += c0; chunk_in.compact.cand_time += c0;
+    NRM_TRY(forward_encoder_impl(fn, chunk_in, B, H, nc, params, NRM_MODE_EVAL, precision, nullptr, nullptr, pc.ws, pc.ws_bytes, stream));
     float* out = nc == N ? logits : pc.out;                 // a single chunk writes the [B,N] logits directly
     NRM_TRY(nrm_forward_head(B, H, nc, params, run_mean, run_var, nullptr, NRM_MODE_EVAL, precision, nullptr, 0, out, pc.ws, pc.ws_bytes, stream));
     if (out != logits)
@@ -691,8 +674,8 @@ extern "C" int nrm_backward_encoder_compact(const nrm_compact_batch* batch, int 
   const char* fn = "nrm_backward_encoder_compact";
   NRM_TRY(check_shape(fn, B, H, C));
   if (!params || !grads) { set_error("%s: null pointer", fn); return NRM_EINVAL; }
-  CompactPtrs cp; BatchPtrs in;
-  NRM_TRY(compact_batch(fn, batch, precision, cp, in));
+  BatchPtrs in;
+  NRM_TRY(compact_batch(fn, batch, C, in));
   return backward_encoder_impl(fn, in, B, H, C, params, mode, precision, bn_bwd_sums, bn_global_rows, grads, workspace, workspace_bytes, stream);
 }
 
@@ -711,8 +694,8 @@ extern "C" int nrm_backward_compact(const nrm_compact_batch* batch, int B, int H
                                     const float* dlogits, float* grads, void* workspace, size_t workspace_bytes, void* stream) {
   const char* fn = "nrm_backward_compact";
   NRM_TRY(check_shape(fn, B, H, C));
-  CompactPtrs cp; BatchPtrs in;
-  NRM_TRY(compact_batch(fn, batch, precision, cp, in));
+  BatchPtrs in;
+  NRM_TRY(compact_batch(fn, batch, C, in));
   NRM_TRY(backward_head(fn, true, B, H, C, params, precision, dlogits, grads, nullptr, workspace, workspace_bytes, stream));
   return backward_encoder_impl(fn, in, B, H, C, params, mode, precision, nullptr, 0, grads, workspace, workspace_bytes, stream);
 }

@@ -66,30 +66,15 @@ __device__ __forceinline__ void load_att_weights(const float* __restrict__ P, At
   }
 }
 
-// Stage history rows [r0, r0+64) of impression b: h[row][k] and hT[k][row]; rows >= H are zero.
-template <int BRANCH>
-__device__ __forceinline__ void load_history_tile(const double* __restrict__ xh, const float* __restrict__ xhp,
-                                                  long long b, int H, int r0, float* h, float* hT) {
-  if (BRANCH == 0) {
-    // w1-projected label features, fp32 [NH,64]
-    for (int f = threadIdx.x; f < HT * 16; f += ATT_THREADS) {
-      const int row = f >> 4, k4 = f & 15;
-      float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (r0 + row < H) v = __ldg(reinterpret_cast<const float4*>(xhp + (b * H + r0 + row) * 64) + k4);
-      *reinterpret_cast<float4*>(h + row * 64 + 4 * k4) = v;
-      hT[(4 * k4 + 0) * TS + row] = v.x; hT[(4 * k4 + 1) * TS + row] = v.y;
-      hT[(4 * k4 + 2) * TS + row] = v.z; hT[(4 * k4 + 3) * TS + row] = v.w;
-    }
-  } else {
-    // PCA columns 4..67 of the packed float64 rows, converted in registers
-    for (int f = threadIdx.x; f < HT * 32; f += ATT_THREADS) {
-      const int row = f >> 5, k2 = f & 31;
-      double2 v = make_double2(0.0, 0.0);
-      if (r0 + row < H) v = __ldg(reinterpret_cast<const double2*>(xh + (b * H + r0 + row) * HC + 4) + k2);
-      const float a = (float)v.x, c = (float)v.y;
-      *reinterpret_cast<float2*>(h + row * 64 + 2 * k2) = make_float2(a, c);
-      hT[(2 * k2 + 0) * TS + row] = a; hT[(2 * k2 + 1) * TS + row] = c;
-    }
+// Stage history rows [r0, r0+64) of impression b from fp32 [NH,64] rows: h[row][k] and hT[k][row]; rows >= H are zero.
+__device__ __forceinline__ void load_history_tile(const float* __restrict__ hist, long long b, int H, int r0, float* h, float* hT) {
+  for (int f = threadIdx.x; f < HT * 16; f += ATT_THREADS) {
+    const int row = f >> 4, k4 = f & 15;
+    float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (r0 + row < H) v = __ldg(reinterpret_cast<const float4*>(hist + (b * H + r0 + row) * 64) + k4);
+    *reinterpret_cast<float4*>(h + row * 64 + 4 * k4) = v;
+    hT[(4 * k4 + 0) * TS + row] = v.x; hT[(4 * k4 + 1) * TS + row] = v.y;
+    hT[(4 * k4 + 2) * TS + row] = v.z; hT[(4 * k4 + 3) * TS + row] = v.w;
   }
 }
 
@@ -136,11 +121,12 @@ __device__ __forceinline__ float reduce16(float v) {   // sum over the 16 lanes 
 // ---------------------------------------------------------------------------------
 // forward: grid = B (one impression per CTA), 256 threads, ~108 KB shared
 // ---------------------------------------------------------------------------------
+// hist: the branch's history rows, fp32 [NH,64] (branch 0: w1-projected label features w.xh, branch 1: the PCA slice w.pca_h).
 // kScores: also store every valid row's score s[c][h] to scores [2][B][C][H] (nrm_forward_scores); with kScores = false the kernel
 // is the one nrm_forward has always launched.
 template <int BRANCH, bool kScores>
 __global__ void __launch_bounds__(ATT_THREADS, 2)
-attention_forward_kernel(const double* __restrict__ xh, const float* __restrict__ xhp, int B, int H, int C,
+attention_forward_kernel(const float* __restrict__ hist, int B, int H, int C,
                          const float* __restrict__ P, float* __restrict__ e, float* __restrict__ scores) {
   pdl_wait();                                          // programmatic dependent launch: see nrm_common.cuh
   pdl_trigger();
@@ -156,7 +142,7 @@ attention_forward_kernel(const double* __restrict__ xh, const float* __restrict_
   for (long long b = blockIdx.x; b < B; b += gridDim.x) {
     for (int r0 = 0; r0 < H; r0 += HT) {
       __syncthreads();
-      load_history_tile<BRANCH>(xh, xhp, b, H, r0, sm.h, sm.hT);
+      load_history_tile(hist, b, H, r0, sm.h, sm.hT);
       for (int c0 = 0; c0 < C; c0 += CCH) {
         const int nc = min(CCH, C - c0);
         __syncthreads();
@@ -215,7 +201,7 @@ attention_forward_kernel(const double* __restrict__ xh, const float* __restrict_
 // ---------------------------------------------------------------------------------
 template <int BRANCH>
 __global__ void __launch_bounds__(ATT_THREADS, 1)
-attention_backward_kernel(const double* __restrict__ xh, const float* __restrict__ xhp, int B, int H, int C,
+attention_backward_kernel(const float* __restrict__ hist, int B, int H, int C,
                           const float* __restrict__ P, const float* __restrict__ e, const float* __restrict__ de,
                           float* __restrict__ dxh, float* __restrict__ dxt, float* __restrict__ part) {
   pdl_wait();                                          // programmatic dependent launch: see nrm_common.cuh
@@ -237,7 +223,7 @@ attention_backward_kernel(const double* __restrict__ xh, const float* __restrict
   for (long long b = blockIdx.x; b < B; b += gridDim.x) {
     for (int r0 = 0; r0 < H; r0 += HT) {
       __syncthreads();
-      load_history_tile<BRANCH>(xh, xhp, b, H, r0, sm.h, sm.hT);
+      load_history_tile(hist, b, H, r0, sm.h, sm.hT);
       float dhacc[4][4];
 #pragma unroll
       for (int r = 0; r < 4; ++r)
@@ -499,37 +485,34 @@ attention_compose_kernel(const float* __restrict__ part, int nparts, AttOffsets 
 // ---------------------------------------------------------------------------------
 static int att_bwd_grid(int B) { return min(B, min(sm_count(), ATT_BWD_CTAS_MAX)); }
 
-int launch_attention_forward(const BatchPtrs& in, const float* P, Workspace& w, int branch, int precision, cudaStream_t s) {
-  if (precision != NRM_PRECISION_FP32) { set_error("attention: the FFMA kernels run precision fp32 only (got %d)", precision); return NRM_EUNSUPPORTED; }
+int launch_attention_forward(const float* P, Workspace& w, int branch, cudaStream_t s) {
   const size_t smem = sizeof(AttSmemFwd);
   // w.scores non-null: the score-exporting instantiations
-  void (*k)(const double*, const float*, int, int, int, const float*, float*, float*) =
+  void (*k)(const float*, int, int, int, const float*, float*, float*) =
       w.scores != nullptr ? (branch == 0 ? attention_forward_kernel<0, true> : attention_forward_kernel<1, true>)
                           : (branch == 0 ? attention_forward_kernel<0, false> : attention_forward_kernel<1, false>);
   NRM_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  launch_pdl(k, dim3(w.B), dim3(ATT_THREADS), smem, s, in.xh, (const float*)w.xh, w.B, w.H, w.C, P, w.e, w.scores);
+  launch_pdl(k, dim3(w.B), dim3(ATT_THREADS), smem, s, branch == 0 ? w.xh : w.pca_h, w.B, w.H, w.C, P, w.e, w.scores);
   NRM_LAUNCH_CHECK("attention_forward_kernel");
   return NRM_OK;
 }
 
-int launch_attention_backward(const BatchPtrs& in, const float* P, Workspace& w, int branch, int precision, cudaStream_t s) {
-  if (precision != NRM_PRECISION_FP32) { set_error("attention: the FFMA kernels run precision fp32 only (got %d)", precision); return NRM_EUNSUPPORTED; }
+int launch_attention_backward(const float* P, Workspace& w, int branch, cudaStream_t s) {
   const size_t smem = sizeof(AttSmemBwd);
   const int grid = att_bwd_grid(w.B);
   float* part = w.att_part + (long long)branch * ATT_BWD_CTAS_MAX * ATT_PARTIAL;
   if (branch == 0) {
     NRM_CUDA(cudaFuncSetAttribute(attention_backward_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    launch_pdl(attention_backward_kernel<0>, dim3(grid), dim3(ATT_THREADS), smem, s, in.xh, w.xh, w.B, w.H, w.C, P, w.e, w.de, w.dxh, w.dxt, part);
+    launch_pdl(attention_backward_kernel<0>, dim3(grid), dim3(ATT_THREADS), smem, s, w.xh, w.B, w.H, w.C, P, w.e, w.de, w.dxh, w.dxt, part);
   } else {
     NRM_CUDA(cudaFuncSetAttribute(attention_backward_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    launch_pdl(attention_backward_kernel<1>, dim3(grid), dim3(ATT_THREADS), smem, s, in.xh, w.xh, w.B, w.H, w.C, P, w.e, w.de, w.dxh, w.dxt, part);
+    launch_pdl(attention_backward_kernel<1>, dim3(grid), dim3(ATT_THREADS), smem, s, w.pca_h, w.B, w.H, w.C, P, w.e, w.de, w.dxh, w.dxt, part);
   }
   NRM_LAUNCH_CHECK("attention_backward_kernel");
   return NRM_OK;
 }
 
-int launch_attention_finish(const float* P, Workspace& w, int branch, int precision, float* grads, cudaStream_t s) {
-  if (precision != NRM_PRECISION_FP32) { set_error("attention: the FFMA kernels run precision fp32 only (got %d)", precision); return NRM_EUNSUPPORTED; }
+int launch_attention_finish(const float* P, Workspace& w, int branch, float* grads, cudaStream_t s) {
   const float* part = w.att_part + (long long)branch * ATT_BWD_CTAS_MAX * ATT_PARTIAL;
   launch_pdl(attention_compose_kernel, dim3(64), dim3(256), 0, s, part, att_bwd_grid(w.B), branch == 0 ? ATT_LABEL : ATT_TI, grads);
   NRM_LAUNCH_CHECK("attention_compose_kernel");

@@ -469,7 +469,7 @@ int launch_attention_prep_rs(const float* P, Workspace& w, cudaStream_t s) {
 }
 
 template <int SPLIT>
-static int launch_fwd_rs(const BatchPtrs& in, Workspace& w, cudaStream_t s) {
+static int launch_fwd_rs(Workspace& w, cudaStream_t s) {
   constexpr int NP = SPLIT == 3 ? 2 : 1;
   const size_t smem = sizeof(rs::Smem<NP>);
   const long long G = (w.C + rs::CG - 1) / rs::CG, U = 2LL * w.B * G;
@@ -482,9 +482,9 @@ static int launch_fwd_rs(const BatchPtrs& in, Workspace& w, cudaStream_t s) {
 }
 
 // both branches in one launch; w.scores non-null: the score-exporting kernels (nrm_attention_rs_scores.cu)
-int launch_attention_forward_rs(const BatchPtrs& in, Workspace& w, int precision, cudaStream_t s) {
+int launch_attention_forward_rs(Workspace& w, int precision, cudaStream_t s) {
   if (w.scores != nullptr) return launch_attention_forward_rs_scores(w, precision, s);
-  return precision == NRM_PRECISION_BF16 ? launch_fwd_rs<1>(in, w, s) : launch_fwd_rs<3>(in, w, s);
+  return precision == NRM_PRECISION_BF16 ? launch_fwd_rs<1>(w, s) : launch_fwd_rs<3>(w, s);
 }
 
 size_t attention_rs_image_bytes() { return (size_t)rs::img_bytes(); }

@@ -20,13 +20,11 @@ struct RowFields {
   int tix[4], cat, sub[5], typ;
   float s0, s1, s2;
 };
-struct CompactArgs {
-  const float* articles; int n_articles;
-  const int* hist_article; const unsigned* hist_time; const float* hist_click;
-  const int* cand_article; const unsigned* cand_time;
-  const float* label32; double* label64;
-};
-__device__ __forceinline__ const float* compact_article(const CompactArgs& ca, bool is_hist, long long r) {
+// position of history row r, or of candidate row r (impression r / C, column r % C), in the compact id arrays
+__device__ __forceinline__ long long compact_index(const CompactPtrs& ca, bool is_hist, long long r, int C) {
+  return is_hist ? r : (long long)((int)r / C) * ca.cand_bs + (int)r % C;
+}
+__device__ __forceinline__ const float* compact_article(const CompactPtrs& ca, bool is_hist, long long r) {
   int art = is_hist ? ca.hist_article[r] : ca.cand_article[r];
   art = (art < 0 || art >= ca.n_articles) ? 0 : art;         // out-of-range ids read the pad article (as nrm_expand_compact does)
   return ca.articles + (long long)art * 80;
@@ -35,7 +33,7 @@ __device__ __forceinline__ const float* compact_article(const CompactArgs& ca, b
 template <bool COMPACT>
 __global__ void __launch_bounds__(256)
 embed_rows_kernel(const double* __restrict__ xh, const double* __restrict__ xt, long long xt_bs,
-                  const double* __restrict__ xg, long long xg_bs, const CompactArgs ca, int H, int C, long long NH, long long N,
+                  const double* __restrict__ xg, long long xg_bs, const CompactPtrs ca, int H, int C, long long NH, long long N,
                   const float* __restrict__ P, float* __restrict__ xin_h, float* __restrict__ e, float* __restrict__ pca_h,
                   int* __restrict__ keys32, int* __restrict__ keys8) {
   pdl_wait();                                          // programmatic dependent launch: see nrm_common.cuh
@@ -53,7 +51,7 @@ embed_rows_kernel(const double* __restrict__ xh, const double* __restrict__ xt, 
   const float* art = nullptr;
   RowFields f;
   if (COMPACT) {
-    const long long r = is_hist ? row : row - NH;
+    const long long r = compact_index(ca, is_hist, is_hist ? row : row - NH, C);
     art = compact_article(ca, is_hist, r);
     const unsigned t = is_hist ? ca.hist_time[r] : ca.cand_time[r];
     f.tix[0] = (int)(t & 0xfffu); f.tix[1] = (int)((t >> 12) & 0xfu); f.tix[2] = (int)((t >> 16) & 0x1fu); f.tix[3] = (int)((t >> 21) & 0x1fu);
@@ -497,7 +495,7 @@ table_grad_l2_kernel(const SortPair sp, const float* __restrict__ gpart32, const
 template <bool COMPACT>
 __global__ void __launch_bounds__(256)
 small_linear_grad_kernel(const double* __restrict__ xh, const double* __restrict__ xt, long long xt_bs,
-                         const double* __restrict__ xg, long long xg_bs, const CompactArgs ca, int C, long long NH, long long N,
+                         const double* __restrict__ xg, long long xg_bs, const CompactPtrs ca, int C, long long NH, long long N,
                          const float* __restrict__ xin_h, const float* __restrict__ e,
                          const float* __restrict__ dxin_h, const float* __restrict__ dxt, const float* __restrict__ de,
                          float* __restrict__ part) {
@@ -522,7 +520,7 @@ small_linear_grad_kernel(const double* __restrict__ xh, const double* __restrict
     const float* dvp = is_hist ? (dxin_h + row * XIN + 32) : (dxt + r * D + 32);
     float in[3], gl[3] = {0.f, 0.f, 0.f};
     if (COMPACT) {
-      const float* art = compact_article(ca, is_hist, is_hist ? row : r);
+      const float* art = compact_article(ca, is_hist, compact_index(ca, is_hist, is_hist ? row : r, C));
       const float2 a = __ldg(reinterpret_cast<const float2*>(art + 70));      // sentiment 70-72
       in[0] = a.x; in[1] = a.y; in[2] = __ldg(art + 72);
       if (!is_hist) { gl[0] = __ldg(art + 74); gl[1] = __ldg(art + 75); gl[2] = __ldg(art + 76); }
@@ -631,20 +629,11 @@ small_linear_grad_finish_kernel(const float* __restrict__ part, int nparts, floa
 // ---------------------------------------------------------------------------------
 // host-side launchers
 // ---------------------------------------------------------------------------------
-static CompactArgs compact_args(const BatchPtrs& in) {
-  CompactArgs ca{};
-  if (in.compact != nullptr) {
-    const CompactPtrs& c = *in.compact;
-    ca = CompactArgs{c.articles, c.n_articles, c.hist_article, c.hist_time, c.hist_click, c.cand_article, c.cand_time, c.label32, c.label64};
-  }
-  return ca;
-}
-
 int launch_embed_rows(const BatchPtrs& in, const float* P, Workspace& w, bool with_keys, cudaStream_t s) {
   const int grid = (int)((w.N + 31) / 32);
-  const CompactArgs ca = compact_args(in);
-  if (in.compact != nullptr) {
-    const int tail = ca.label32 != nullptr ? (int)((w.R + 255) / 256) : 0;       // label conversion blocks
+  const CompactPtrs& ca = in.compact;
+  if (ca.articles != nullptr) {
+    const int tail = ca.label32 != nullptr ? (int)((w.R + 255) / 256) : 0;       // label conversion blocks ([B,C] dense labels: cand_bs == C)
     launch_pdl(embed_rows_kernel<true>, dim3(grid + tail), dim3(256), 0, s, in.xh, in.xt, in.xt_bs, in.xg, in.xg_bs, ca, w.H, w.C, w.NH, w.N, P, w.xin_h, w.e, w.pca_h, with_keys ? w.keys32 : nullptr, with_keys ? w.keys8 : nullptr);
   } else {
     launch_pdl(embed_rows_kernel<false>, dim3(grid), dim3(256), 0, s, in.xh, in.xt, in.xt_bs, in.xg, in.xg_bs, ca, w.H, w.C, w.NH, w.N, P, w.xin_h, w.e, w.pca_h, with_keys ? w.keys32 : nullptr, with_keys ? w.keys8 : nullptr);
@@ -696,8 +685,8 @@ int launch_small_linear_grads(const BatchPtrs& in, Workspace& w, float* grads, c
   // one row per lane and pass: enough CTAs to cover the rows once, at most one wave of 2 CTAs per SM
   int nparts = (int)((w.N + 255) / 256);
   nparts = max(1, min(nparts, min(1024, 2 * sm_count())));
-  const CompactArgs ca = compact_args(in);
-  if (in.compact != nullptr)
+  const CompactPtrs& ca = in.compact;
+  if (ca.articles != nullptr)
     launch_pdl(small_linear_grad_kernel<true>, dim3(nparts), dim3(256), 0, s, in.xh, in.xt, in.xt_bs, in.xg, in.xg_bs, ca, w.C, w.NH, w.N, w.xin_h, w.e, w.dxin_h, w.dxt, w.de, w.small_part);
   else
     launch_pdl(small_linear_grad_kernel<false>, dim3(nparts), dim3(256), 0, s, in.xh, in.xt, in.xt_bs, in.xg, in.xg_bs, ca, w.C, w.NH, w.N, w.xin_h, w.e, w.dxin_h, w.dxt, w.de, w.small_part);

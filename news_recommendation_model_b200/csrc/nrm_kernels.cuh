@@ -7,15 +7,17 @@ namespace nrm {
 // compact wire format (nrm_wire.cu): the article table resident in HBM + per-impression ids / time buckets / click features
 struct CompactPtrs {
   const float* articles; int n_articles;     // [n,80] float32: pca 64 | category | sub-category 5 | sentiment 3 | type | 3 global statistics | pad
+  int cand_bs;                               // batch stride of cand_article / cand_time: C, or 0 when every impression has the same candidates
   const int* hist_article; const unsigned* hist_time; const float* hist_click;   // [B,H], [B,H], [B,H,2]
   const int* cand_article; const unsigned* cand_time;                            // [B,C], [B,C]
-  const float* label32; double* label64;     // optional: float32 labels -> the float64 labels the loss kernels read
+  const float* label32; double* label64;     // optional ([B,C] dense, so cand_bs == C): float32 labels -> the float64 labels the loss kernels read
 };
+// The caller's batch.  Only the row kernels (launch_embed_rows, launch_small_linear_grads) read it; every later kernel reads the workspace.
 struct BatchPtrs {
   const double* xh;               // [B,H,80]
   const double* xt; long long xt_bs;   // [B,C,78], batch stride in doubles
   const double* xg; long long xg_bs;   // [B,C,3]
-  const CompactPtrs* compact = nullptr;   // non-null: the packed pointers above are unused, the row kernels read the compact format
+  CompactPtrs compact;            // compact.articles non-null: the packed pointers above are unused, the row kernels read the compact format
 };
 
 // nrm_embed.cu
@@ -32,9 +34,9 @@ int launch_w1_backward(const float* P, Workspace& w, float* grads, cudaStream_t 
 int launch_w1_backward_tc(const float* P, Workspace& w, float* grads, int precision, cudaStream_t s);
 
 // nrm_attention.cu  (precision fp32: FFMA kernels; branch 0 = label attention on w1-projected features, 1 = text/img PCA)
-int launch_attention_forward(const BatchPtrs& in, const float* P, Workspace& w, int branch, int precision, cudaStream_t s);
-int launch_attention_backward(const BatchPtrs& in, const float* P, Workspace& w, int branch, int precision, cudaStream_t s);
-int launch_attention_finish(const float* P, Workspace& w, int branch, int precision, float* grads, cudaStream_t s);
+int launch_attention_forward(const float* P, Workspace& w, int branch, cudaStream_t s);
+int launch_attention_backward(const float* P, Workspace& w, int branch, cudaStream_t s);
+int launch_attention_finish(const float* P, Workspace& w, int branch, float* grads, cudaStream_t s);
 
 // nrm_attention_tc.cu  (precision = bf16 / bf16x3: tcgen05 tensor-core tiles)
 int launch_candidate_tp(const float* P, Workspace& w, cudaStream_t s);            // per-candidate tp -> w.tp (needs w.e target rows)
@@ -44,7 +46,7 @@ int launch_attention_finish_tc(const float* P, Workspace& w, float* grads, cudaS
 size_t attention_rs_image_bytes();
 int rsprof_read(long long* host_out64);                                         // -DNRM_RS_PROFILE builds only
 int launch_attention_prep_rs(const float* P, Workspace& w, cudaStream_t s);       // weight image -> w.att_rs_img (weights only)
-int launch_attention_forward_rs(const BatchPtrs& in, Workspace& w, int precision, cudaStream_t s);   // both branches, one launch
+int launch_attention_forward_rs(Workspace& w, int precision, cudaStream_t s);   // both branches, one launch
 int launch_attention_forward_rs_scores(Workspace& w, int precision, cudaStream_t s);   // the same + scores to w.scores (nrm_attention_rs_scores.cu)
 // nrm_attention_rs_bwd.cu: sums over rows (weight gradients, dtp) of one branch; export_dhid also writes the dhid tiles / scores
 int launch_attention_backward_rs(Workspace& w, int branch, int precision, bool export_dhid, cudaStream_t s);

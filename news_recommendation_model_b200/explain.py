@@ -69,13 +69,9 @@ def attention_scores(model, x_history, x_target, x_global) -> AttentionScores:
 
 def attention_scores_compact(model, table: wire.ArticleTable, cb: wire.CompactBatch) -> AttentionScores:
     """`attention_scores` for a device `wire.CompactBatch` and its `ArticleTable`: the row kernels read the compact format
-    directly (`nrm_forward_scores_compact`); precision 'fp32', whose kernels read packed rows, expands it first
-    (`wire.expand`).  Same results, bit for bit, as `attention_scores` on `wire.expand(table, cb)`."""
+    directly (`nrm_forward_scores_compact`).  Same results, bit for bit, as `attention_scores` on `wire.expand(table, cb)`."""
     if not (table.rows.is_cuda and cb.hist_article.is_cuda):
         raise _lib.NrmError('attention_scores_compact runs on CUDA tensors only (no CPU fallback)')
-    if model.precision == 'fp32':
-        b = wire.expand(table, cb)
-        return attention_scores(model, b.x_history, b.x_target, b.x_global)
     if table.rows.dtype != torch.float32 or table.rows.dim() != 2 or table.rows.shape[1] != wire.ARTICLE_COLS \
             or not table.rows.is_contiguous():
         raise ValueError(f'article table must be contiguous float32 [n, {wire.ARTICLE_COLS}]')

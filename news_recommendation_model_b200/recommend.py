@@ -7,8 +7,8 @@ device), score all of them for every active user and return each user's k best, 
     logits = recommend.pool_logits(model, table, hist_article, hist_time, hist_click, pool_time)      # [B, n-1]: every real article
     rec = recommend.top_articles([m1, m2], table, hist_article, hist_time, hist_click, pool_time, 10)  # rec.article [B,10], best first
 
-`pool_logits` runs the eval forward over the pool in chunks (`nrm_forward_pool`): the pool rows are expanded once per chunk and
-shared by all users, so the memory is that of a (B, H, chunk) forward, and the logits are, bit for bit, those of
+`pool_logits` runs the eval forward over the pool in chunks (`nrm_forward_pool`): the row kernels read the users' ids and each chunk's
+article ids as they are, the chunk shared by all users, so the memory is that of a (B, H, chunk) forward, and the logits are, bit for bit, those of
 `model.eval()(x_history, x_target, x_global)` with the pool broadcast as every user's candidates.  `top_articles` selects on the
 GPU (`nrm_pool_topk`): the score is the logit for one model and, for an ensemble, the mean over the models of the softmax over the
 user's eligible articles (test.py:58-63); the order is Python's stable `sorted(..., reverse=True)` (test.py:124-127).  Eligible are

@@ -67,7 +67,7 @@ class FusedTrainStep:
     def __init__(self, model, B: int, H: int, C: int, *, lr=1e-3, betas=(0.9, 0.999), eps=1e-8, weight_decay=1e-5,
                  alpha=0.95, use_graph=True, ring=8, nslots=2, articles=None, negatives=None):
         """`articles`: a device `wire.ArticleTable`; with it `load()` also accepts `wire.CompactBatch`es (ids instead of
-        packed float64 rows) and the step starts with the expansion kernel.
+        packed float64 rows), which the row kernels of the step read directly.
         `negatives`: a `negatives.NegativeSampler` (needs `articles`).  `C` is then the width after sampling: `load()` takes
         CompactBatches of C - k candidate columns, and every step first appends k pool negatives per impression, drawn at step t =
         the optimizer steps completed so far (read on the device, so every graph replay draws afresh) and row offset rank * B
@@ -87,9 +87,6 @@ class FusedTrainStep:
         world = self.dp.world if self.dp is not None else 1
         self.precision = model._precision_code()
         self.mode = engine.MODE_BN_BATCH_STATS | engine.MODE_KEEP_FOR_BWD
-        # compact batches go straight into the row kernels (no expansion to the packed float64 tensors) in the tensor-core precisions;
-        # the FFMA attention of precision fp32 reads the packed rows, so it gets nrm_expand_compact in front
-        self.compact_direct = self.precision != 0
         n = self.flat.total
         # data parallel: the flat gradient buffer in symmetric (peer-mapped) memory, so that the Adam kernel of every rank can read
         # all of them (dp.PeerContext); None -> NCCL all-reduce between two graphs
@@ -162,8 +159,7 @@ class FusedTrainStep:
         loss_scratch = self.loss_scratch if loss_scratch is None else loss_scratch
         warming = getattr(self, '_warming', False)
         sync_bn = self.dp is not None and self.dp.sync_bn and not warming
-        # compact slot on the direct path: the compact batch is the input itself
-        inputs = s.compact_inputs if s.wire == 'compact' and self.compact_direct else s.packed
+        inputs = s.compact_inputs if s.wire == 'compact' else s.packed
         engine.forward(inputs, B, H, C, f.buf, m.bn.running_mean, m.bn.running_var, m.bn.num_batches_tracked, self.mode, self.precision,
                        self.logits, self.ws, st, **(self._sync_bn(0, B * C) if sync_bn else {}))
         delta = f.buf[f.fixed:f.fixed + f.delta_numel]
@@ -269,8 +265,8 @@ class FusedTrainStep:
                                                         dtype=getattr(batch, f).dtype, device=self.dev)
                                             for f in batch.__dataclass_fields__])
             s.compact_inputs = engine.compact(self.articles, s.compact, s.label)
-            self._expand(s)                                  # first launch of the kernels outside any graph capture
-            # the zero fills / the expansion above run on the compute stream: the H2D copies below must not overtake them
+            self._sample_negatives(s)                        # first launch of the sampler outside any graph capture
+            # the zero fills / the sampler above run on the compute stream: the H2D copies below must not overtake them
             self.copy_stream.wait_stream(torch.cuda.current_stream(self.dev))
         with torch.cuda.stream(self.copy_stream):
             if s.used:
@@ -295,19 +291,14 @@ class FusedTrainStep:
             ev.record(self.copy_stream)
             loader.release(batch, ev)
         s.wire = 'compact'
-        s.rows = b                                           # b < B: ragged last batch (expanded whole, trained on its first b rows)
+        s.rows = b                                           # b < B: ragged last batch (trained on its first b rows)
         return s
 
-    def _expand(self, s: _Slot, rows: Optional[int] = None):
-        """Compact slot -> what the forward reads: the pool negatives appended to its first `rows` impressions (with a sampler),
-        then nothing more on the direct path (the row kernels read the compact batch; the labels are converted by the first of
-        them), the packed float64 tensors otherwise."""
-        from . import wire
+    def _sample_negatives(self, s: _Slot, rows: Optional[int] = None):
+        """With a sampler: append the pool negatives to the first `rows` impressions of a compact slot (the only kind a step with
+        a sampler loads).  The row kernels then read the compact batch as it is; the first of them converts the labels."""
         if self.negatives is not None:
             self.negatives.sample_into(s.compact, self.C - self.negatives.k, self.adam_step, self.row_offset, rows)
-        if self.compact_direct:
-            return
-        wire.expand_into(self.articles, s.compact, s.xh, s.xt, s.xg, s.label)
 
     def load(self, batch) -> _Slot:
         """Enqueue the H2D copy of a (pinned) host batch into the next slot (round robin).  `batch` is a packed
@@ -353,8 +344,7 @@ class FusedTrainStep:
             if scratch is None:
                 scratch = self._tail_scratch[s.rows] = torch.zeros(int(self.lib.nrm_loss_scratch_bytes(s.rows, self.C)),
                                                                    dtype=torch.uint8, device=self.dev)
-            if s.wire == 'compact':
-                self._expand(s, s.rows)
+            self._sample_negatives(s, s.rows)
             self._forward_backward(s, loss_out, B=s.rows, loss_scratch=scratch)
             self._adam()
         elif self.use_graph:
@@ -363,8 +353,7 @@ class FusedTrainStep:
                 s.graph_fb = torch.cuda.CUDAGraph()
                 s.loss_slot = self.loss_dev.new_zeros(())
                 with torch.cuda.graph(s.graph_fb, capture_error_mode='thread_local'):       # other threads (a loader) may call CUDA meanwhile
-                    if s.wire == 'compact':
-                        self._expand(s)
+                    self._sample_negatives(s)
                     self._forward_backward(s, s.loss_slot)
                     if self.one_graph:
                         self._adam()                     # single process or peer-memory data parallel: the whole step is ONE graph
@@ -380,8 +369,7 @@ class FusedTrainStep:
                 s.graph_adam.replay()
             loss_out = s.loss_slot.view(1)
         else:
-            if s.wire == 'compact':
-                self._expand(s)
+            self._sample_negatives(s)
             self._forward_backward(s, loss_out)
             if self.dp is not None and self.peer is None:
                 self.dp.buckets.reduce(self.grads, 0, self.grads.numel())

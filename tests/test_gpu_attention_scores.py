@@ -123,7 +123,7 @@ def test_top_history_is_a_stable_descending_sort_without_pad_rows(precision, k):
         assert torch.isnan(val.cpu()[i < 0]).all()
 
 
-@pytest.mark.parametrize('precision', ['bf16', 'bf16x3'])
+@pytest.mark.parametrize('precision', PRECISIONS)
 def test_top_history_reads_pad_rows_from_the_compact_batch(precision):
     model, _ = _model(precision, user_num=40)
     table = wire.make_article_table(3000, seed=5).to('cuda')

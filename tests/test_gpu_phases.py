@@ -17,8 +17,7 @@ pytestmark = pytest.mark.gpu
 
 H, C = 50, 5
 MODE_TRAIN = 3                 # NRM_MODE_BN_BATCH_STATS | NRM_MODE_KEEP_FOR_BWD
-CASES = [(fmt, precision, B) for fmt in ('packed', 'compact') for precision in ('fp32', 'bf16', 'bf16x3') for B in (1, 33)
-         if not (fmt == 'compact' and precision == 'fp32')]      # the compact format is read directly by the tensor-core precisions only
+CASES = [(fmt, precision, B) for fmt in ('packed', 'compact') for precision in ('fp32', 'bf16', 'bf16x3') for B in (1, 33)]
 
 
 def _p(t):

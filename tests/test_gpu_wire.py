@@ -5,7 +5,7 @@ import pytest
 import torch
 
 import news_recommendation_model_b200 as nrm
-from news_recommendation_model_b200 import wire
+from news_recommendation_model_b200 import _lib, wire
 from fixtures import load_weights
 from oracle.wire_port import expand_reference
 
@@ -55,33 +55,38 @@ def test_scoring_forward_is_identical_for_both_wire_formats():
 
 
 @pytest.mark.parametrize('precision', ['bf16x3', 'fp32'])
-def test_fused_train_step_is_identical_for_both_wire_formats(precision):
-    """bf16x3: the compact batch is the direct input of the row kernels (nrm_forward_compact / nrm_backward_compact, no packed tensors);
-    fp32: it is expanded on the GPU first (the FFMA attention kernels read the packed rows).  Either way three training steps end
-    with the same bits as feeding the reference's packed float64 tensors."""
+def test_compact_train_step_launches_what_the_packed_one_does_and_ends_with_its_bits(precision):
+    """The compact batch is the direct input of the row kernels (nrm_forward_compact / nrm_backward_compact, no packed tensors) in
+    every precision: an eager step launches as many kernels as one fed the packed tensors (no expansion kernel runs), and three
+    training steps end with the same bits as feeding the reference's packed float64 tensors."""
     B, H, C = 64, 50, 5
+    lib = _lib.load()
     table = wire.make_article_table(2000, seed=5)
     batches = [wire.make_compact_batch(table, B, H, C, seed=20 + i, user_num=100) for i in range(3)]
-    results = []
+    results, launches = [], []
     for fmt in ('packed', 'compact'):
         m = nrm.UserModel(100)
         m.load_state_dict(load_weights('train'), strict=False)
         m.to('cuda').train().set_precision(precision)
         tr = nrm.FusedTrainStep(m, B, H, C, lr=1e-3, weight_decay=1e-5, articles=table.to('cuda'))
-        assert tr.compact_direct == (precision != 'fp32')
-        losses = []
+        feeds = []
         for cb in batches:
             if fmt == 'packed':
                 xh, xt, xg = _host_packed(table, cb)
-                feed = nrm.synthetic.Batch(cb.impression_id, cb.user_id, xh, xt, xg, cb.label.double(), cb.label.double(), cb.empty_num).pin()
+                feeds.append(nrm.synthetic.Batch(cb.impression_id, cb.user_id, xh, xt, xg, cb.label.double(), cb.label.double(), cb.empty_num).pin())
             else:
-                feed = cb.pin()
-            losses.append(tr.step(feed).item())
+                feeds.append(cb.pin())
+        losses = [tr.step(feed).item() for feed in feeds]
         torch.cuda.synchronize()
-        results.append((losses, m.flat_parameters().buf.clone(), m.bn.running_mean.clone()))
-    (l0, p0, r0), (l1, p1, r1) = results
+        results.append((losses, m.flat_parameters().buf.clone(), m.bn.running_mean.clone(), m.bn.running_var.clone()))
+        tr.use_graph = False                     # one step more, eager: count the library's kernel launches
+        n0 = lib.nrm_launch_count()
+        tr.step(feeds[0]).item()
+        launches.append(lib.nrm_launch_count() - n0)
+    (l0, p0, r0, v0), (l1, p1, r1, v1) = results
     assert l0 == l1
-    assert torch.equal(p0, p1) and torch.equal(r0, r1)
+    assert torch.equal(p0, p1) and torch.equal(r0, r1) and torch.equal(v0, v1)
+    assert launches[0] == launches[1] > 0, launches
 
 
 def test_slot_recaptures_its_graph_when_the_wire_format_changes():
